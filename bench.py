@@ -17,6 +17,8 @@ roofline : algorithmic HBM bytes (2 B per genotype + row metadata + sums traffic
 cpu_baseline : the CPU oracle (a C port of the reference algorithm; the Nim reference cannot be
            built in this image) on a bounded sample of the same cohort.
 --impl reference : that oracle with all host threads, as the reference arm.
+--dump-outputs DIR : after the timed steps, what the headline's last step computed, as DIR/<name>.npy (see dump_outputs);
+           the inputs are a pure function of the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -30,11 +32,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark leaves the tree as it found it (it may be read-only)
 
 SEED = 0x6E696D70
 N_SAMPLES = 500_000
 V_PER_GPU = 125_000
 MISS_RATE = 0.005
+DUMP_BYTES = 60_000_000                 # --dump-outputs: data bytes in all, under 64 MB with the .npy headers
 
 
 def parse_args():
@@ -54,7 +58,33 @@ def parse_args():
     ap.add_argument("--config", type=int, default=3, choices=[2, 3, 4, 5],
                     help="BASELINE.json config to time as the headline (default 3: the genome-wide shard)")
     ap.add_argument("--no-extra", action="store_true", help="skip the short timings of configs 2, 4 and 5 (N = 1 only)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm sizes its sample from a calibration timing, so its outputs differ from run to run")
+    return args
+
+
+def locus_fields(loci):
+    """The per-locus records (nb.LOCUS_DTYPE, any shape) as one array per field."""
+    return {"loci_" + f: loci[f] for f in ("klass", "used", "eaidx", "ngt", "nmiss", "neff", "imputed")}
+
+
+def dump_outputs(path, arrays):
+    """Write every array as <path>/<name>.npy in float64 (the integer fields are exact there).  When they hold more
+    than DUMP_BYTES in all, each array larger than an equal share keeps a sample of that many positions, drawn from a
+    generator seeded by SEED and the array's size and kept in order: the same positions in every run."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    share = DUMP_BYTES // 8 // len(arrays)
+    sample = sum(a.size for a in arrays.values()) * 8 > DUMP_BYTES
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        if sample and a.size > share:
+            a = a.ravel()[np.sort(np.random.default_rng([SEED, a.size]).choice(a.size, share, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ---- synthetic score rows / cohort parameters (SURVEY.md 8d) -------------------------------------
@@ -244,14 +274,19 @@ def time_resident(nb, torch, dev, n, V, miss_lo, miss_hi, steps=20, warmup=5, po
     return t, out, shape, 2.0 * n * V + 32.0 * V + 16.0 * n
 
 
-def extra_configs(nb, torch, dev, peak):
-    """configs[1], [3] and [4] of BASELINE.json, a few launches each, so that the driver's line carries them."""
-    ex = {}
-    t, out, shape, alg = time_resident(nb, torch, dev, 100_000, 697, 0.005, 0.005)
+def extra_configs(nb, torch, dev, peak, steps=None, warmup=None):
+    """configs[1], [3] and [4] of BASELINE.json, a few launches each -> (timings, outputs of each config's last call).
+    steps / warmup: timed and untimed calls of each config (None: 20 / 5 launches of configs 2 and 5, 5 / 1 calls of
+    config 4, the short timings beside the genome-wide headline)."""
+    ex, outs = {}, {}
+    reps = {} if steps is None else dict(steps=steps, warmup=warmup)
+    t, out, shape, alg = time_resident(nb, torch, dev, 100_000, 697, 0.005, 0.005, **reps)
+    outs["config2"] = {"scores": out["scores"], "nloci": out["nloci"], **locus_fields(out["loci"])}
     ex["config2"] = {"workload": "697 loci (the wood height score's size) x 100,000 samples, 0.5% missing, one launch",
                      "value": 100_000 * 697 / t, "unit": "genotypes/s", "launch_us": t * 1e6, "roofline_frac": alg / t / 1e9 / peak,
                      "grid": shape["grid"], "row_groups": shape.get("row_groups"), "l2": "flushed before every timed launch"}
-    t, out, shape, alg = time_resident(nb, torch, dev, 50_000, 10_000, 0.0, 0.10)
+    t, out, shape, alg = time_resident(nb, torch, dev, 50_000, 10_000, 0.0, 0.10, **reps)
+    outs["config5"] = {"scores": out["scores"], "nloci": out["nloci"], **locus_fields(out["loci"])}
     ex["config5"] = {"workload": "10,000 loci x 50,000 samples, per-locus missing rate U(0, 0.10), --maxmis 0.05 (default policies), one launch",
                      "value": 50_000 * 10_000 / t, "unit": "genotypes/s", "launch_us": t * 1e6, "roofline_frac": alg / t / 1e9 / peak,
                      "loci_over_maxmis": int((out["loci"]["klass"] == 4).sum()), "grid": shape["grid"], "row_groups": shape.get("row_groups"),
@@ -278,11 +313,13 @@ def extra_configs(nb, torch, dev, peak):
     sc_out = [pin_s[k].numpy() for k in range(S)]
     lo_out = [pin_l[k].numpy().view(nb.LOCUS_DTYPE) for k in range(S)]
     ts = []
-    for rep in range(6):
+    steps4, warmup4 = (5, 1) if steps is None else (steps, warmup)
+    for rep in range(warmup4 + steps4):
         t0 = time.perf_counter()
-        eng.score_resident_multi(lists, [0.0] * S, sc_out, lo_out)
+        nloci4 = [nl for _, nl, _ in eng.score_resident_multi(lists, [0.0] * S, sc_out, lo_out)]
         ts.append(time.perf_counter() - t0)
-    t = float(np.median(ts[1:]))
+    t = float(np.median(ts[warmup4:]))
+    outs["config4"] = {"scores": np.stack(sc_out), "nloci": nloci4, **locus_fields(np.stack(lo_out))}
     ex["config4"] = {"workload": f"{S} score definitions x {V} loci x {n} samples over one resident 8 GB slab, one npc_score_resident_multi call "
                                  "(wall clock: row tables H2D, tally + contraction kernels, 18 x n scores and records D2H)",
                      "value": float(V) * n * S / t, "unit": "genotype-score cells/s", "call_ms": t * 1e3,
@@ -290,7 +327,7 @@ def extra_configs(nb, torch, dev, peak):
                      "substitution": "BASELINE names 18 bundled score files; 4 of the bundled files are score definitions, so 18 synthetic "
                                      "definitions over one site set stand in (DESIGN.md section 7)"}
     eng.close()
-    return ex
+    return ex, outs
 
 
 # ---- B200 arm -------------------------------------------------------------------------------------
@@ -319,9 +356,12 @@ def b200_arm(args):
         torch.cuda.set_stream(stream)
         peaks_path = os.path.join(ROOT, "MEASURED_PEAKS.json")
         peak = float(json.load(open(peaks_path))["hbm_gbs"]) if os.path.exists(peaks_path) else 6650.0
-        ex = extra_configs(nb, torch, dev, peak)[f"config{args.config}"]
+        ex, outs = extra_configs(nb, torch, dev, peak, args.steps, args.warmup)
+        ex, outs = ex[f"config{args.config}"], outs[f"config{args.config}"]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outs)
         line = {"metric": "genotypes scored/sec (variants x samples)", "value": ex["value"], "unit": ex["unit"], "n_gpus": 1,
-                "steps": 20, "warmup": 5, "ms_per_step": ex.get("launch_us", ex.get("call_ms", 0.0) * 1e3) / 1e3, "higher_is_better": True,
+                "steps": args.steps, "warmup": args.warmup, "ms_per_step": ex.get("launch_us", ex.get("call_ms", 0.0) * 1e3) / 1e3, "higher_is_better": True,
                 "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
                 "config": {"workload": ex["workload"], "l2": ex.get("l2", "8 GB slab: larger than L2")},
                 "roofline": {"bound": "hbm", "frac": ex.get("roofline_frac"), "peak": peak, "unit": "GB/s"}, "detail": ex}
@@ -422,6 +462,11 @@ def b200_arm(args):
     genotypes_step = float(n) * V * world
     value = genotypes_step / (ms_step * 1e-3)
     assert int(nl.item()) == V * world, (int(nl.item()), V * world)
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path holds after the last step: the per-sample sums (combined over the ranks when
+        # N > 1), nloci, and the per-locus records of this rank's shard
+        dump_outputs(args.dump_outputs, {"sums": total.cpu().numpy(), "nloci": nl.cpu().numpy(),
+                                         **locus_fields(eng.partial(want_loci=True)["loci"])})
 
     # N > 1: the combine is checked, not assumed.  Every rank scores the first Vp rows of its shard into a
     # fresh context and the ranks combine them through the same npc_comm_combine; rank 0 then scores every
@@ -563,7 +608,7 @@ def b200_arm(args):
         eng.close()
         del gt, d_rows
         torch.cuda.empty_cache()
-        extra = extra_configs(nb, torch, dev, peak)
+        extra, _ = extra_configs(nb, torch, dev, peak)
 
     if rank == 0:
         line = {
