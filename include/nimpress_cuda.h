@@ -31,6 +31,9 @@
  * `gt_width` bytes (1, 2 or 4), value = (allele+1)<<1 | phased, 0|phase = missing allele,
  * width-specific sentinels missing = MIN, vector_end = MIN+1 (both ignored, and a vector_end
  * ends the sample), rows `row_stride` bytes apart (row_stride % 16 == 0).
+ *
+ * Or, for a context created with gt_width = NPC_GT_BED (ploidy 2), rows of a PLINK 1 `.bed` fileset as stored:
+ * 2 bits per sample, low bits first, ceil(n/4) bytes per row (DESIGN.md 4.7, npc_bed.cuh).
  */
 /*
  * Environment (diagnostics and tests; none is needed in normal use):
@@ -76,6 +79,16 @@ enum { NPC_KIND_GT = 0,      /* record found, FILTER passes: decode its genotype
        NPC_KIND_ABSENT = 2,  /* findVariant returned nil               (:536-551)           */
        NPC_KIND_FILTER = 3,  /* FILTER not in {".","PASS"}, !ignorefilt (:553-558)          */
        NPC_CLASS_MAXMIS = 4  /* nmissing/n > maxmis                     (:565-571)          */ };
+
+/* gt_width of a context whose rows are PLINK 1 `.bed` rows (SNP-major): ploidy must be 2.  Per sample a 2-bit code,
+ * sample s in bits 2*(s%4) of byte s/4: 00 = homozygous A1, 01 = missing, 10 = heterozygous, 11 = homozygous A2, with
+ * A2 = REF (eaidx 0) and A1 = the one ALT (eaidx 1); the padding codes of a row's last byte are ignored.  Every
+ * npc_score_block* / npc_score_resident call takes such rows (npc_score_resident_multi scores one definition at a time);
+ * a GT-kind row names eaidx 0 or 1.  The split count / accumulate calls return NPC_EUNSUPPORTED. */
+#define NPC_GT_BED 0
+
+/* Bytes of one genotype row of n samples in a layout (gt_width 1, 2, 4 or NPC_GT_BED). */
+int64_t npc_gt_row_bytes(int64_t n_samples, int32_t ploidy, int32_t gt_width);
 
 typedef struct npc_ctx npc_ctx;
 
@@ -295,7 +308,9 @@ int npc_set_dosage_rows(npc_ctx *ctx, int32_t on);
 /* Which kernels npc_score_block* uses for this context: shape[0] = 2 for the fused tile kernel in
  * its default mode, 1 in exact-order mode (int8 / int16 diploid cohorts that fit one resident pass),
  * 3 for cohorts too wide for that (> ~1.2 M samples per GPU: tally + decide over all samples, then the
- * tile kernel in "decided" mode once per slab of the sample axis),
+ * tile kernel in "decided" mode once per slab of the sample axis), 4 for NPC_GT_BED rows (k_count_bed,
+ * k_decide, k_accum_bed; then shape[1] = CTAs of the accumulate pass, shape[2] = warps per CTA,
+ * shape[3] = samples per thread, shape[4] = rows per tile: 4 in the default mode, 1 in exact order),
  * 0 for the count/decide/accumulate sequence; then grid (tile kernel: sample slabs * 1000 + row
  * groups), consumer warps, chunks per thread, rows
  * per tile, raw stages * 1000 + index-ring tiles, lag * 100 + tiles per decider pass * 10 + decider warps, dynamic

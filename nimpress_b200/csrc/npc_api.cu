@@ -16,6 +16,7 @@
 #include "npc_multi.cuh"
 #include "npc_reduce.cuh"
 #include "npc_dosage.cuh"
+#include "npc_bed.cuh"
 
 using namespace npc;
 
@@ -78,6 +79,10 @@ struct npc_ctx {
     // FORMAT/DS rows (npc_dosage.cuh): fp32 dosages, one per sample
     bool ds = false;
     double *d_ds_part = nullptr;            // [max_rows][n_blocks] block sums of the tally pass
+    // PLINK 1 .bed rows (npc_bed.cuh, gt_width = NPC_GT_BED): 2 bits per sample
+    bool bed = false;
+    double *d_bed_tab = nullptr;            // per batch of BED_RB rows: the accumulate pass's value tables
+    int32_t *d_bed_off = nullptr;           // ... and the slab row of every row it loads
     // cross-GPU combine (npc_reduce.cuh)
     cudaEvent_t ev_multi = nullptr;         // npc_score_resident_multi: orders its copy-stream work against the compute stream
     cudaEvent_t ev_reduce = nullptr;        // "this context's partial sums are final"
@@ -107,6 +112,10 @@ static int fail(npc_ctx *ctx, int code, const char *msg) {
 
 extern "C" int npc_version(void) { return 200; }
 
+extern "C" int64_t npc_gt_row_bytes(int64_t n_samples, int32_t ploidy, int32_t gt_width) {
+    return gt_width == NPC_GT_BED ? (n_samples + 3) / 4 : n_samples * ploidy * gt_width;
+}
+
 extern "C" int npc_warmup(int device) {
     if (cudaSetDevice(device) != cudaSuccess || cudaFree(nullptr) != cudaSuccess) { cudaGetLastError(); return NPC_ECUDA; }
     return NPC_OK;
@@ -129,7 +138,7 @@ extern "C" void npc_destroy(npc_ctx *ctx) {
     if (ctx->ev_slab) cudaEventDestroy(ctx->ev_slab);
     if (ctx->ev_reduce) cudaEventDestroy(ctx->ev_reduce);
     if (ctx->ev_multi) cudaEventDestroy(ctx->ev_multi);
-    cudaFree(ctx->d_nloci_total); cudaFree(ctx->d_bridge); cudaFree(ctx->d_gather); cudaFree(ctx->d_ds_part);
+    cudaFree(ctx->d_nloci_total); cudaFree(ctx->d_bridge); cudaFree(ctx->d_gather); cudaFree(ctx->d_ds_part); cudaFree(ctx->d_bed_tab); cudaFree(ctx->d_bed_off);
     if (ctx->comm && g_nccl.lib) g_nccl.CommDestroy(ctx->comm);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -314,7 +323,7 @@ static int create_impl(npc_ctx *c) {
     NPC_CUDA(c, cudaMalloc(&c->d_rowp, r1 * sizeof(RowP)));
     c->log_cap = std::max<int64_t>(r1, 1024);
     NPC_CUDA(c, cudaMalloc(&c->d_log, c->log_cap * sizeof(npc_locus)));
-    c->row_stride = ((c->n * c->ploidy * c->width + 127) / 128) * 128;
+    c->row_stride = ((npc_gt_row_bytes(c->n, c->ploidy, c->width) + 127) / 128) * 128;
     if (c->row_stride == 0) c->row_stride = 128;
     c->h_gt.assign(c->n_slots, nullptr); c->d_gt.assign(c->n_slots, nullptr);
     c->ev_h2d.assign(c->n_slots, nullptr); c->ev_done.assign(c->n_slots, nullptr);
@@ -343,13 +352,14 @@ extern "C" int npc_create2(npc_ctx **out, int device, int64_t n_samples, int32_t
                            int64_t max_rows_per_block, int32_t n_slots, int64_t staging_rows) {
     if (!out) return NPC_EINVAL;
     *out = nullptr;
-    if (n_samples < 0 || ploidy < 1 || ploidy > 64 || (gt_width != 1 && gt_width != 2 && gt_width != 4) ||
+    if (n_samples < 0 || ploidy < 1 || ploidy > 64 || (gt_width != 1 && gt_width != 2 && gt_width != 4 && gt_width != NPC_GT_BED) ||
+        (gt_width == NPC_GT_BED && ploidy != 2) ||
         max_rows_per_block < 1 || n_slots < 0 || n_slots == 1 || staging_rows < 1 || staging_rows > max_rows_per_block) {
         g_create_error = "npc_create: invalid argument";
         return NPC_EINVAL;
     }
     npc_ctx *c = new npc_ctx();
-    c->device = device; c->n = n_samples; c->ploidy = ploidy; c->width = gt_width;
+    c->device = device; c->n = n_samples; c->ploidy = ploidy; c->width = gt_width; c->bed = gt_width == NPC_GT_BED;
     c->max_rows = max_rows_per_block; c->n_slots = n_slots; c->staging_rows = staging_rows;
     c->pol.imp_locus = NPC_LOCUS_PS; c->pol.imp_missing = NPC_MISSING_HOMREF; c->pol.imp_sample = NPC_SAMPLE_INT_PS;
     c->pol.mincs = 100; c->pol.maxmis = 0.05; c->pol.n_total = n_samples;      // defaults of main (:670-687)
@@ -422,6 +432,11 @@ extern "C" int npc_kernel_shape2(const npc_ctx *ctx, int64_t n_rows, int32_t sha
     const bool wide = !(ctx->exact ? ctx->exact_cfg.ok : ctx->fast.ok) && ctx->wide.ok;
     const npc_ctx::TileCfg &t = wide ? (ctx->exact ? ctx->wide_exact : ctx->wide) : ctx->exact ? ctx->exact_cfg : fast_config(ctx, n_rows);
     memset(shape, 0, 8 * sizeof(int32_t));
+    if (ctx->bed) {
+        shape[0] = 4; shape[1] = (int32_t)((ctx->n + 8 * BED_THREADS - 1) / (8 * BED_THREADS)); shape[2] = BED_THREADS / 32;
+        shape[3] = 8; shape[4] = ctx->exact ? 1 : 4;
+        return NPC_OK;
+    }
     if (!t.ok) return NPC_OK;
     shape[0] = wide ? 3 : ctx->exact ? 1 : 2; shape[1] = t.Gs * 1000 + (ctx->exact ? 1 : t.Gr); shape[2] = t.nc; shape[3] = t.K;
     shape[4] = F4_R; shape[5] = t.Sr * 1000 + t.Sc; shape[6] = t.L * 100 + t.GD * 10 + t.A; shape[7] = (int32_t)t.smem;
@@ -434,7 +449,7 @@ extern "C" int npc_plan_shape(int64_t n_samples, int32_t gt_width, int32_t num_s
     if (!plan || n_samples < 0 || num_sms < 1 || max_smem < 1 || n_rows < 0) return NPC_EINVAL;
     npc_ctx *c = new npc_ctx;
     c->n = n_samples; c->ploidy = 2; c->width = gt_width;
-    c->row_stride = ((c->n * c->ploidy * c->width + 127) / 128) * 128;
+    c->row_stride = ((npc_gt_row_bytes(c->n, c->ploidy, c->width) + 127) / 128) * 128;
     plan_shapes(c, num_sms, max_smem);
     const bool wide = !(exact ? c->exact_cfg.ok : c->fast.ok) && c->wide.ok;
     const npc_ctx::TileCfg &t = wide ? (exact ? c->wide_exact : c->wide) : exact ? c->exact_cfg : fast_config(c, n_rows);
@@ -452,7 +467,7 @@ extern "C" int npc_plan_shape(int64_t n_samples, int32_t gt_width, int32_t num_s
 
 extern "C" int npc_set_dosage_rows(npc_ctx *ctx, int32_t on) {
     if (!ctx) return NPC_EINVAL;
-    if (on && (ctx->width != 4 || ctx->ploidy != 1))
+    if (on && (ctx->width != 4 || ctx->ploidy != 1 || ctx->bed))
         return fail(ctx, NPC_EINVAL, "npc_set_dosage_rows: create the context with ploidy 1 and gt_width 4 (one fp32 DS value per sample)");
     ctx->ds = on != 0;
     return NPC_OK;
@@ -484,8 +499,17 @@ static int check_block(npc_ctx *c, const void *gt, int64_t row_stride, int64_t n
     if (n_rows < 0 || n_gt_rows < 0 || n_rows > c->max_rows || n_gt_rows > c->max_rows)
         return fail(c, NPC_EINVAL, "block larger than max_rows_per_block");
     if (n_rows && !rows) return fail(c, NPC_EINVAL, "rows is NULL");
-    if (n_gt_rows && (!gt || ((uintptr_t)gt & 15) || (row_stride & 15) || row_stride < c->n * c->ploidy * c->width))
-        return fail(c, NPC_EINVAL, "genotype slab must be 16-byte aligned with row_stride % 16 == 0 and >= n*ploidy*width");
+    if (n_gt_rows && (!gt || ((uintptr_t)gt & 15) || (row_stride & 15) || row_stride < npc_gt_row_bytes(c->n, c->ploidy, c->width)))
+        return fail(c, NPC_EINVAL, "genotype slab must be 16-byte aligned with row_stride % 16 == 0 and >= the bytes of a row");
+    return NPC_OK;
+}
+
+// .bed rows carry one ALT: a decoded row names REF (0) or that ALT (1).  Checked where the rows are on the host.
+static int check_bed_rows(npc_ctx *c, const npc_row *rows, int64_t n_rows, int on_device) {
+    if (!c->bed || on_device) return NPC_OK;
+    for (int64_t i = 0; i < n_rows; i++)
+        if (rows[i].kind == NPC_KIND_GT && rows[i].gt_row >= 0 && rows[i].eaidx != 0 && rows[i].eaidx != 1)
+            return fail(c, NPC_EINVAL, "PLINK .bed rows: the effect allele of a genotype row is REF (eaidx 0) or the one ALT (eaidx 1)");
     return NPC_OK;
 }
 
@@ -655,8 +679,49 @@ static int launch_dosage(npc_ctx *c, const uint8_t *gt, int64_t row_stride, cons
     return NPC_OK;
 }
 
+// PLINK .bed rows: popc tally, the common decision, table-indexed accumulate (npc_bed.cuh)
+static int launch_bed(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows) {
+    if (n_rows == 0) return NPC_OK;
+    int rc = ensure_log(c, n_rows);
+    if (rc) return rc;
+    NPC_CUDA(c, cudaMemsetAsync(c->d_counts, 0, n_rows * 2 * sizeof(ull), c->stream));
+    if (c->n) {
+        // as k_count_i8x2: ~4096 blocks, up to 64 chunks (of 64 samples) per thread
+        const int64_t nchunks = (c->n + 63) / 64;
+        const int64_t s_min = (nchunks + 16383) / 16384, s_max = (nchunks + 1023) / 1024, want = (4096 + n_rows - 1) / n_rows;
+        const unsigned slabs = (unsigned)std::min<int64_t>(std::max<int64_t>(std::min(std::max(want, s_min), s_max), 1), 65535);
+        k_count_bed<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->d_counts);
+        c->launches++;
+    }
+    k_decide<<<(unsigned)((n_rows + 127) / 128), 128, 0, c->stream>>>(d_rows, n_rows, c->d_counts, c->pol, c->n, c->d_rowp,
+                                                                      c->d_log + c->log_len, c->d_nloci);
+    c->launches++;
+    c->log_len += n_rows;
+    if (c->n) {
+        const int64_t n_batches = (n_rows + BED_RB - 1) / BED_RB, E = c->exact ? BED_RB * 4 : BED_RB * 8;
+        if (!c->d_bed_tab) {
+            const int64_t max_batches = (std::max<int64_t>(c->max_rows, 1) + BED_RB - 1) / BED_RB;
+            NPC_CUDA(c, cudaMalloc(&c->d_bed_tab, (size_t)max_batches * BED_RB * 8 * sizeof(double)));
+            NPC_CUDA(c, cudaMalloc(&c->d_bed_off, (size_t)max_batches * BED_RB * sizeof(int32_t)));
+        }
+        const unsigned pgrid = (unsigned)((n_batches * E + 255) / 256);
+        const unsigned grid = (unsigned)((c->n + 8 * BED_THREADS - 1) / (8 * BED_THREADS));
+        if (c->exact) {
+            k_bed_prep<true><<<pgrid, 256, 0, c->stream>>>(c->d_rowp, n_rows, n_batches, c->d_bed_tab, c->d_bed_off);
+            k_accum_bed<true><<<grid, BED_THREADS, 0, c->stream>>>(gt, row_stride, c->d_bed_tab, c->d_bed_off, n_rows, c->n, c->d_sums);
+        } else {
+            k_bed_prep<false><<<pgrid, 256, 0, c->stream>>>(c->d_rowp, n_rows, n_batches, c->d_bed_tab, c->d_bed_off);
+            k_accum_bed<false><<<grid, BED_THREADS, 0, c->stream>>>(gt, row_stride, c->d_bed_tab, c->d_bed_off, n_rows, c->n, c->d_sums);
+        }
+        c->launches += 2;
+    }
+    NPC_CUDA(c, cudaGetLastError());
+    return NPC_OK;
+}
+
 static int launch_block(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows) {
     if (c->ds) return launch_dosage(c, gt, row_stride, d_rows, n_rows);
+    if (c->bed) return launch_bed(c, gt, row_stride, d_rows, n_rows);
     if (c->exact ? c->exact_cfg.ok : c->fast.ok) return launch_fused(c, c->exact ? c->exact_cfg : fast_config(c, n_rows), c->exact, gt, row_stride, d_rows, n_rows);
     if (c->wide.ok && env_int("NPC_WIDE", 1)) return launch_wide(c, c->exact, gt, row_stride, d_rows, n_rows);
     int rc = launch_count(c, gt, row_stride, d_rows, n_rows, c->d_counts);
@@ -690,6 +755,7 @@ extern "C" int npc_score_block(npc_ctx *ctx, int32_t slot, int64_t n_gt_rows, co
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     if (!ctx->d_gt[slot]) NPC_CUDA(ctx, cudaMalloc(&ctx->d_gt[slot], (size_t)ctx->row_stride * (size_t)std::max<int64_t>(ctx->staging_rows, 1)));
     int rc = check_block(ctx, ctx->d_gt[slot], ctx->row_stride, n_gt_rows, rows, n_rows);
+    if (!rc) rc = check_bed_rows(ctx, rows, n_rows, 0);
     if (rc) return rc;
     if (n_gt_rows)
         NPC_CUDA(ctx, cudaMemcpyAsync(ctx->d_gt[slot], ctx->h_gt[slot], (size_t)n_gt_rows * ctx->row_stride,
@@ -711,6 +777,7 @@ extern "C" int npc_score_block(npc_ctx *ctx, int32_t slot, int64_t n_gt_rows, co
 extern "C" int npc_score_block_device(npc_ctx *ctx, const void *gt_dev, int64_t row_stride, int64_t n_gt_rows,
                                       const npc_row *rows, int64_t n_rows, int32_t rows_on_device) {
     int rc = check_block(ctx, gt_dev, row_stride, n_gt_rows, rows, n_rows);
+    if (!rc) rc = check_bed_rows(ctx, rows, n_rows, rows_on_device);
     if (rc) return rc;
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     const npc_row *d_rows;
@@ -725,6 +792,7 @@ extern "C" int npc_count_block_device(npc_ctx *ctx, const void *gt_dev, int64_t 
     if (rc) return rc;
     if (!counts_dev) return fail(ctx, NPC_EINVAL, "counts_dev is NULL");
     if (ctx->ds) return fail(ctx, NPC_EUNSUPPORTED, "the split count / accumulate calls take hard-call (GT) rows only");
+    if (ctx->bed) return fail(ctx, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not PLINK .bed rows");
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     const npc_row *d_rows;
     if ((rc = upload_rows(ctx, rows, n_rows, rows_on_device, &d_rows))) return rc;
@@ -738,6 +806,7 @@ extern "C" int npc_accumulate_block_device(npc_ctx *ctx, const void *gt_dev, int
     if (rc) return rc;
     if (!counts_dev) return fail(ctx, NPC_EINVAL, "counts_dev is NULL");
     if (ctx->ds) return fail(ctx, NPC_EUNSUPPORTED, "the split count / accumulate calls take hard-call (GT) rows only");
+    if (ctx->bed) return fail(ctx, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not PLINK .bed rows");
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     const npc_row *d_rows;
     if ((rc = upload_rows(ctx, rows, n_rows, rows_on_device, &d_rows))) return rc;
@@ -766,7 +835,7 @@ extern "C" int npc_resident_reserve(npc_ctx *ctx, int64_t capacity_rows, int64_t
 
 extern "C" int npc_resident_adopt(npc_ctx *ctx, const void *gt_dev, int64_t row_stride, int64_t n_gt_rows) {
     if (!ctx || n_gt_rows < 0 || (n_gt_rows && !gt_dev)) return NPC_EINVAL;
-    if (((uintptr_t)gt_dev & 15) || (row_stride & 15) || row_stride < ctx->n * ctx->ploidy * ctx->width)
+    if (((uintptr_t)gt_dev & 15) || (row_stride & 15) || row_stride < npc_gt_row_bytes(ctx->n, ctx->ploidy, ctx->width))
         return fail(ctx, NPC_EINVAL, "npc_resident_adopt: slab must be 16-byte aligned, row_stride a multiple of 16 holding a whole row");
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     NPC_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -800,6 +869,7 @@ extern "C" int npc_score_resident(npc_ctx *ctx, const npc_row *rows, int64_t n_r
     for (int64_t i = 0; i < n_rows; i++)
         if (rows[i].kind == NPC_KIND_GT && rows[i].gt_row >= ctx->slab_rows)
             return fail(ctx, NPC_EINVAL, "npc_score_resident: gt_row outside the resident slab");
+    if (int rc = check_bed_rows(ctx, rows, n_rows, 0)) return rc;
     // every upload issued so far must have landed
     for (int s = 0; s < ctx->n_slots; s++) NPC_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_h2d[s], 0));
     for (int64_t r0 = 0; r0 < n_rows; r0 += ctx->max_rows) {

@@ -13,6 +13,12 @@ LOCUS = {"ps": 0, "homref": 1, "fail": 2, "ignore": 3}          # ImputeMethodLo
 MISSING = {"homref": 0, "ignore": 1}                             # ImputeMethodMissing (:413)
 SAMPLE = {"ps": 0, "homref": 1, "fail": 2, "int_ps": 3, "int_fail": 4}   # ImputeMethodSample (:414)
 KIND_GT, KIND_NOTCOV, KIND_ABSENT, KIND_FILTER, CLASS_MAXMIS = range(5)
+GT_BED = 0        # gt_width of a context over PLINK 1 .bed rows (2 bits per sample, ploidy 2): NPC_GT_BED
+
+
+def gt_row_bytes(n_samples, ploidy, gt_width):
+    """npc_gt_row_bytes: bytes of one genotype row in a layout."""
+    return int(load_library().npc_gt_row_bytes(int(n_samples), int(ploidy), int(gt_width)))
 
 ROW_DTYPE = np.dtype([("gt_row", "<i4"), ("eaidx", "<i4"), ("beta", "<f8"), ("eaf", "<f8"),
                       ("ref_is_ea", "<i4"), ("kind", "<i4")], align=True)
@@ -87,6 +93,7 @@ def load_library():
         "npc_set_exact_order": (C.c_int, [vp, i32]),
         "npc_set_dosage_rows": (C.c_int, [vp, i32]),
         "npc_synth_fill_device": (C.c_int, [vp, vp, i64, i64, i64, C.c_uint64, vp, vp, vp]),
+        "npc_gt_row_bytes": (i64, [i64, i32, i32]),
         "npc_version": (C.c_int, []),
         "npc_warmup": (C.c_int, [C.c_int]),
     }

@@ -232,7 +232,7 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
 
     // staging slots of ~8 MB: big enough for efficient H2D copies, small enough that pinning three of them per
     // device does not dominate a short run (pinning costs ~1 ms per MB); scoring launches are sized separately
-    const int64_t row_bytes = std::max<int64_t>(16, n * ploidy * gt_width);
+    const int64_t row_bytes = std::max<int64_t>(16, npc_gt_row_bytes(n, ploidy, gt_width));
     struct Dev {
         Ctx ctx;
         int32_t slot = -1; uint8_t *stage = nullptr; int64_t stride = 0, staged = 0, slab_base = 0, slab_cap = 0, block_rows = 1;
@@ -346,7 +346,7 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
                 v.stage = (uint8_t *)ptr; v.staged = 0;
             }
             uint8_t *dst = v.stage + v.staged * v.stride;
-            if (first) memcpy(dst, first, (size_t)n * ploidy * gt_width);   // a record named by two ranges: same bytes
+            if (first) memcpy(dst, first, (size_t)npc_gt_row_bytes(n, ploidy, gt_width));   // a record named by two ranges: same bytes
             else {
                 // BCF with the context's layout: the GT payload goes from the inflated blocks straight into the pinned row
                 const bool direct = vcf.load_gt_into(rec, dst, gt_width, ploidy);
@@ -473,6 +473,10 @@ bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores
     for (int attempt = 0; attempt < 6; attempt++) {
         std::unique_ptr<VariantSource> vcf = open_variant_source(genotype_path, seekable);
         if (!vcf) return false;
+        if (vcf->plink_rows()) {                    // PLINK fileset: its 2-bit rows as stored, read by offset (no index pass)
+            if (p.use_ds) throw InputError("--dosage: a PLINK fileset holds hard calls only, no FORMAT/DS");
+            width = NPC_GT_BED; ploidy = 2; seekable = false;
+        }
         vcf->set_dosage_mode(p.use_ds);
         try {
             run_pass(scores, *vcf, genotype_path, seekable, cov, p, width, ploidy, outs);

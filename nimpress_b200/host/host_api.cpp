@@ -194,7 +194,7 @@ int nph_read_gt(const char *genotype_path, uint8_t *out, int64_t row_bytes, int6
             if (k >= max_records) return NPH_ECAPACITY;
             if (rec.has_gt) {
                 vcf->load_gt(rec);
-                const int64_t bytes = vcf->n_samples() * rec.ploidy * rec.gt_width;
+                const int64_t bytes = npc_gt_row_bytes(vcf->n_samples(), rec.ploidy, rec.gt_width);
                 if (bytes > row_bytes) return NPH_ECAPACITY;
                 memcpy(out + k * row_bytes, rec.gt, (size_t)bytes);
                 *width = rec.gt_width; *ploidy = rec.ploidy;
@@ -231,10 +231,10 @@ int nph_format_float(double v, char *buf, int32_t buflen) {
 // ------------------------------------------------------------------------------------------
 
 static const char *USAGE =
-    "Compute polygenic scores from a VCF/BCF.\n\n"
+    "Compute polygenic scores from a VCF/BCF or a PLINK 1 binary fileset.\n\n"
     "Usage:\n"
-    "  nimpress [options] <scoredef> <genotypes.vcf>\n"
-    "  nimpress [options] <scoredef1>,<scoredef2>,... <genotypes.vcf>   (one pass, a \"#score\" line per file; not in the reference)\n"
+    "  nimpress [options] <scoredef> <genotypes.vcf|.bcf|.bed>\n"
+    "  nimpress [options] <scoredef1>,<scoredef2>,... <genotypes.vcf|.bcf|.bed>   (one pass, a \"#score\" line per file; not in the reference)\n"
     "  nimpress (-h | --help)\n"
     "  nimpress --version\n\n"
     "Options:\n"
@@ -267,6 +267,9 @@ static const char *USAGE =
     "                     in range order (not a reference option).\n"
     "  --dosage           Score FORMAT/DS (expected ALT-allele dosage, one float per sample) instead of\n"
     "                     FORMAT/GT (not a reference option: the reference lists it under Future).\n"
+    "                     Not with a PLINK fileset.\n"
+    "PLINK 1 fileset (not a reference input): X.bed with X.bim and X.fam, recognised by its magic bytes.\n"
+    "  REF = A2 (.bim column 6), ALT = A1 (column 5), sample names = .fam IID; FILTER is always \".\".\n"
     "  --exact-order      Add every locus to the running sums in score-file order, bit for bit\n"
     "                     like the reference (default: sum tiles of four loci first; same\n"
     "                     products, scores equal to ~1e-15 relative) (not a reference option).\n";
@@ -344,9 +347,9 @@ int nph_main(int argc, char **argv) {
             else if (npos < 2) pos[npos++] = a;
             else throw InputError("too many arguments");
         }
-        if (npos != 2) throw InputError("expected <scoredef> <genotypes.vcf>");
+        if (npos != 2) throw InputError("expected <scoredef> <genotypes.vcf|.bcf|.bed>");
     } catch (const InputError &e) {
-        std::cerr << e.what() << "\n" << "Usage:\n  nimpress [options] <scoredef> <genotypes.vcf>\n";
+        std::cerr << e.what() << "\n" << "Usage:\n  nimpress [options] <scoredef> <genotypes.vcf|.bcf|.bed>\n";
         return 1;
     }
     // several score files, one pass (not a reference feature) -- unless the whole argument names a file, as it would for the reference

@@ -1,6 +1,11 @@
 #include "variant_source.hpp"
 #include "region_index.hpp"
 #include "fast_inflate.hpp"
+#include "../../include/nimpress_cuda.h"
+
+#include <fcntl.h>
+#include <sys/stat.h>
+#include <unistd.h>
 
 #include <algorithm>
 #include <atomic>
@@ -821,6 +826,133 @@ private:
 };
 
 // ------------------------------------------------------------------------------------------
+// PLINK 1 binary fileset (.bed + .bim + .fam), DESIGN.md 4.7 -- not a reference input
+// ------------------------------------------------------------------------------------------
+
+// The .bim is read whole at open (it sizes and checks the .bed); next() walks its lines in file order, and a row of the
+// .bed is read by offset only when the driver asks for it (load_gt / load_gt_into): a few hundred scored loci on a
+// genome-wide fileset read a few hundred rows, no index needed.  Per line: CHROM = column 1 (compared literally),
+// POS = column 4, ALT = A1 (column 5; "0" = no ALT), REF = A2 (column 6), rlen = len(REF), FILTER ".".
+class PlinkSource : public VariantSource {
+public:
+    ~PlinkSource() override { if (fd_ >= 0) ::close(fd_); }
+    // false: a sibling file cannot be opened.  Throws InputError on a malformed fileset.
+    bool open(const std::string &bed_path, uint8_t mode) {
+        if (mode == 0x00) throw InputError("PLINK .bed " + bed_path + ": individual-major mode (mode byte 00) is not supported");
+        if (mode != 0x01) throw InputError("PLINK .bed " + bed_path + ": unknown mode byte");
+        const std::string prefix = bed_path.size() > 4 && bed_path.compare(bed_path.size() - 4, 4, ".bed") == 0
+                                       ? bed_path.substr(0, bed_path.size() - 4) : bed_path;
+        FILE *fam = fopen((prefix + ".fam").c_str(), "rb");
+        if (!fam) return false;
+        FILE *bim = fopen((prefix + ".bim").c_str(), "rb");
+        if (!bim) { fclose(fam); return false; }
+        std::string line;
+        auto getline = [&line](FILE *f) {
+            line.clear();
+            int ch;
+            while ((ch = fgetc(f)) != EOF && ch != '\n') line += (char)ch;
+            if (!line.empty() && line.back() == '\r') line.pop_back();
+            return ch != EOF || !line.empty();
+        };
+        auto fields = [&line]() {
+            std::vector<std::string> f;
+            size_t i = 0;
+            while (i < line.size()) {
+                while (i < line.size() && (line[i] == ' ' || line[i] == '\t')) i++;
+                size_t j = i;
+                while (j < line.size() && line[j] != ' ' && line[j] != '\t') j++;
+                if (j > i) f.emplace_back(line, i, j - i);
+                i = j;
+            }
+            return f;
+        };
+        int64_t ln = 0;
+        while (getline(fam)) {
+            ln++;
+            std::vector<std::string> f = fields();
+            if (f.empty()) continue;
+            if (f.size() < 2) { fclose(fam); fclose(bim); throw InputError("PLINK .fam line " + std::to_string(ln) + ": fewer than 2 columns"); }
+            samples_.push_back(f[1]);                                   // IID
+        }
+        fclose(fam);
+        std::unordered_map<std::string, int32_t> ids;
+        ln = 0;
+        try {
+            while (getline(bim)) {
+                ln++;
+                std::vector<std::string> f = fields();
+                if (f.empty()) continue;
+                const std::string where = "PLINK .bim line " + std::to_string(ln);
+                if (f.size() < 6) throw InputError(where + ": fewer than 6 columns");
+                Line L;
+                auto it = ids.find(f[0]);
+                if (it == ids.end()) { it = ids.emplace(f[0], (int32_t)contigs_.size()).first; contigs_.push_back(f[0]); }
+                L.contig = it->second;
+                L.pos = parse_int_nim(f[3], (where + " POS").c_str());
+                if (L.pos < 1) throw InputError(where + ": bad POS " + f[3]);
+                L.alt = f[4]; L.ref = f[5];
+                lines_.push_back(std::move(L));
+            }
+        } catch (...) { fclose(bim); throw; }
+        fclose(bim);
+        fd_ = ::open(bed_path.c_str(), O_RDONLY);
+        if (fd_ < 0) return false;
+        struct stat st;
+        if (fstat(fd_, &st) != 0) return false;
+        row_bytes_ = npc_gt_row_bytes((int64_t)samples_.size(), 2, NPC_GT_BED);
+        const int64_t want = 3 + (int64_t)lines_.size() * row_bytes_;
+        if ((int64_t)st.st_size != want)
+            throw InputError("PLINK .bed " + bed_path + " holds " + std::to_string((long long)st.st_size) + " bytes; " +
+                             std::to_string(lines_.size()) + " variants x " + std::to_string(samples_.size()) + " samples need " + std::to_string(want));
+        return true;
+    }
+    bool plink_rows() const override { return true; }
+    void load_gt(VariantRecord &rec) override {
+        buf_.resize((size_t)std::max<int64_t>(row_bytes_, 1));
+        read_row(buf_.data());
+        fill(rec, buf_.data());
+    }
+    bool load_gt_into(VariantRecord &rec, uint8_t *dst, int want_width, int want_ploidy) override {
+        if (want_width != NPC_GT_BED || want_ploidy != 2) { load_gt(rec); return false; }
+        read_row(dst);
+        fill(rec, dst);
+        return true;
+    }
+protected:
+    bool next_raw(VariantRecord &rec) override {
+        if (cur_ + 1 >= (int64_t)lines_.size()) { cur_ = (int64_t)lines_.size(); return false; }
+        const Line &L = lines_[(size_t)++cur_];
+        rec.contig_id = L.contig; rec.contig = &contigs_[(size_t)L.contig];
+        rec.pos = L.pos; rec.ref = L.ref; rec.rlen = (int64_t)L.ref.size();
+        rec.alts.clear();
+        if (L.alt != "0") rec.alts.push_back(L.alt);
+        rec.filter = ".";
+        rec.has_gt = true; rec.gt = nullptr; rec.gt_width = NPC_GT_BED; rec.ploidy = 2;
+        return true;
+    }
+    InflateStream *stream() override { return nullptr; }               // no index-driven mode: use_regions returns false
+    int contig_rank(const VariantRecord &rec) const override { return rec.contig_id; }
+    int contig_rank(const std::string &) const override { return -1; }
+private:
+    struct Line { int32_t contig; int64_t pos; std::string ref, alt; };
+    void read_row(uint8_t *dst) {
+        const int64_t off = 3 + cur_ * row_bytes_;
+        int64_t got = 0;
+        while (got < row_bytes_) {
+            const ssize_t r = pread(fd_, dst + got, (size_t)(row_bytes_ - got), (off_t)(off + got));
+            if (r <= 0) throw InputError("PLINK .bed: read failed at byte " + std::to_string((long long)(off + got)));
+            got += r;
+        }
+    }
+    void fill(VariantRecord &rec, const uint8_t *row) const { rec.has_gt = true; rec.gt = row; rec.gt_width = NPC_GT_BED; rec.ploidy = 2; }
+    std::vector<std::string> contigs_;
+    std::vector<Line> lines_;
+    std::vector<uint8_t> buf_;
+    int64_t cur_ = -1, row_bytes_ = 0;
+    int fd_ = -1;
+};
+
+// ------------------------------------------------------------------------------------------
 // index-driven region mode
 // ------------------------------------------------------------------------------------------
 
@@ -914,6 +1046,18 @@ bool VariantSource::next(VariantRecord &rec) {
 }
 
 std::unique_ptr<VariantSource> open_variant_source(const std::string &path, bool seekable) {
+    {   // a PLINK 1 .bed is recognised by its magic bytes 6c 1b, then the mode byte (not by the file name)
+        uint8_t m[3] = { 0, 0, 0 };
+        FILE *f = fopen(path.c_str(), "rb");
+        if (!f) return nullptr;
+        const size_t got = fread(m, 1, 3, f);
+        fclose(f);
+        if (got == 3 && m[0] == 0x6c && m[1] == 0x1b) {
+            auto src = std::make_unique<PlinkSource>();
+            if (!src->open(path, m[2])) return nullptr;
+            return src;
+        }
+    }
     auto s = std::make_unique<InflateStream>();
     if (!s->open(path, seekable)) return nullptr;
     uint8_t magic[5] = { 0 };

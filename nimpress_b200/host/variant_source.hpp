@@ -101,6 +101,8 @@ public:
     // FORMAT/DS instead of FORMAT/GT (not a reference feature: README.md:162-165 lists dosage input under "Future"):
     // load_gt / load_gt_into then deliver one BCF float per value, gt_width = 4, ploidy = values per sample.
     virtual void set_dosage_mode(bool on) { dosage_ = on; }
+    // true for a PLINK 1 fileset: load_gt delivers .bed rows (gt_width NPC_GT_BED = 0, ploidy 2, ceil(n/4) bytes)
+    virtual bool plink_rows() const { return false; }
     bool dosage_mode() const { return dosage_; }
     const std::vector<std::string> &samples() const { return samples_; }
     int64_t n_samples() const { return (int64_t)samples_.size(); }
@@ -122,7 +124,8 @@ private:
     int64_t seeks_ = 0;
 };
 
-// nullptr: the file cannot be opened or is neither VCF nor BCF (the reference: open() == false).
+// nullptr: the file cannot be opened or is neither VCF, BCF nor a PLINK 1 .bed (the reference: open() == false); for a .bed
+// also when its .bim or .fam sibling cannot be opened.  A malformed fileset throws InputError (see PlinkSource).
 // seekable: read BGZF block by block with one zlib stream so that VariantSource::use_regions can jump (no inflate pool).
 std::unique_ptr<VariantSource> open_variant_source(const std::string &path, bool seekable = false);
 
