@@ -41,15 +41,12 @@
  *   NPC_EXACT=1              exact-order mode for every context (as npc_set_exact_order)
  *   NPC_TILE_K / _SR / _SC / _L / _A / _GR / _GD / _NC1   launch shape of the fused tile kernel (chunks per thread, raw
  *                            stages, index tiles, lag, decider warps, row groups, tiles per decider pass, most warps at K = 1)
- *   NPC_TILE_LONG=0          no separate grid split for long launches; NPC_TILE_LONG_MB=<MB>: what counts as long (default 1536, or 192 when short launches split the rows too)
- *   NPC_TILE_V=4             the round-1 tile kernel (npc_fused4.cuh) instead of the pair-lookup kernel (npc_fused5.cuh)
+ *   NPC_TILE_LONG_MB=<MB>    what counts as a long launch, which may split the grid differently (default 1536, or 192 when short launches split the rows too)
  *   NPC_TILE_SLEEP=<ns>      auxiliary warps of the tile kernel poll + nanosleep instead of a suspended try_wait
  *   NPC_MULTI=0 | 1          npc_score_resident_multi: never / always the tensor-core contraction (default: >= 3 definitions)
  *   NPC_MULTI_PARTS=<n>      split of a tile's entry range over work units in the contraction (default: chosen from the tile count)
  *   NPC_TIMING=1             phase wall times of npc_score_resident_multi on stderr
  *   NPC_TRACE=1              keep %globaltimer stamps of the tile kernel's CTA 0 (npc_trace)
- *   NPC_STAGE_WC=1           write-combined pinned staging slots (measured on B200 / PCIe Gen5: no difference, 55 GB/s either way)
- *   NPC_WIDE=0               cohorts wider than one resident pass: the round-1 two-kernel sequence instead of decided-mode slabs
  */
 #ifndef NIMPRESS_CUDA_H
 #define NIMPRESS_CUDA_H

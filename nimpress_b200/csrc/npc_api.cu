@@ -11,7 +11,6 @@
 #include <unordered_map>
 #include <vector>
 
-#include "npc_fused4.cuh"
 #include "npc_fused5.cuh"
 #include "npc_multi.cuh"
 #include "npc_reduce.cuh"
@@ -48,7 +47,6 @@ struct npc_ctx {
     struct TileCfg {
         bool ok = false;
         int Gs = 1, Gr = 1, K = 1, nc = 1, slab = 0, Sr = 3, Sc = 16, L = 15, A = 2, GD = 8;
-        int ver = 5;                        // 5: pair-lookup kernel (npc_fused5.cuh); 4: the round-1 kernel (npc_fused4.cuh, NPC_TILE_V=4)
         uint32_t smem = 0;
     };
     TileCfg fast;                           // default: sample slabs x row groups, tile-wise summation
@@ -150,26 +148,29 @@ static int env_int(const char *name, int dflt) {
     return v && *v ? atoi(v) : dflt;
 }
 
-static const void *tile_kernel(int ver, int K, bool exact, int width, int nc) {
-    if (ver == 5 && width == 2) {
+// NCMAX of the k_fused_pair instance that runs nc warps of K chunks per thread: 24 or 28 for int8 GT at K = 1, else 16.
+static int instance_warps(int width, int K, int nc) {
+    if (width != 1 || K != 1) return 16;
+    return nc > F5_NC_WIDE ? F5_NC_MAX : nc > 16 ? F5_NC_WIDE : 16;
+}
+
+static const void *tile_kernel(int K, bool exact, int width, int nc) {
+    if (width == 2) {
         if (K == 1) return exact ? (const void *)k_fused_pair<1, true, 2> : (const void *)k_fused_pair<1, false, 2>;
         return exact ? (const void *)k_fused_pair<2, true, 2> : (const void *)k_fused_pair<2, false, 2>;
     }
-    if (ver == 5) {
-        if (K == 1 && nc > F5_NC_WIDE) return exact ? (const void *)k_fused_pair<1, true, 1, F5_NC_MAX> : (const void *)k_fused_pair<1, false, 1, F5_NC_MAX>;
-        if (K == 1 && nc > 16) return exact ? (const void *)k_fused_pair<1, true, 1, F5_NC_WIDE> : (const void *)k_fused_pair<1, false, 1, F5_NC_WIDE>;
-        if (K == 1) return exact ? (const void *)k_fused_pair<1, true> : (const void *)k_fused_pair<1, false>;
-        return exact ? (const void *)k_fused_pair<2, true> : (const void *)k_fused_pair<2, false>;
-    }
-    if (K == 1) return exact ? (const void *)k_fused_tile4<1, true> : (const void *)k_fused_tile4<1, false>;
-    return exact ? (const void *)k_fused_tile4<2, true> : (const void *)k_fused_tile4<2, false>;
+    const int inst = instance_warps(width, K, nc);
+    if (inst == F5_NC_MAX) return exact ? (const void *)k_fused_pair<1, true, 1, F5_NC_MAX> : (const void *)k_fused_pair<1, false, 1, F5_NC_MAX>;
+    if (inst == F5_NC_WIDE) return exact ? (const void *)k_fused_pair<1, true, 1, F5_NC_WIDE> : (const void *)k_fused_pair<1, false, 1, F5_NC_WIDE>;
+    if (K == 1) return exact ? (const void *)k_fused_pair<1, true> : (const void *)k_fused_pair<1, false>;
+    return exact ? (const void *)k_fused_pair<2, true> : (const void *)k_fused_pair<2, false>;
 }
 
 // Consumer shape for a CTA that owns nch chunks (of 8 samples) of every row: K chunks per thread, nc warps.  One chunk
 // per thread as long as the warps fit the SM's registers (int8 GT: up to 24 warps on the 72-register instance, cohorts
 // up to ~909,000 samples per GPU), two (up to 16 warps) above that.
-static bool tile_shape(int ver, int width, int64_t nch, int &K, int64_t &nc) {
-    const int max1 = ver == 5 && width == 1 ? std::max(1, std::min(F5_NC_MAX, env_int("NPC_TILE_NC1", F5_NC_MAX))) : 16;
+static bool tile_shape(int width, int64_t nch, int &K, int64_t &nc) {
+    const int max1 = width == 1 ? std::max(1, std::min(F5_NC_MAX, env_int("NPC_TILE_NC1", F5_NC_MAX))) : 16;
     K = env_int("NPC_TILE_K", 0);
     if (K != 1 && K != 2) K = nch <= 32 * max1 ? 1 : 2;
     nc = (nch + 32 * K - 1) / (32 * K);
@@ -184,31 +185,26 @@ static bool tile_config(const npc_ctx *c, int gr, int max_smem, npc_ctx::TileCfg
     const int gs = (int)std::min<int64_t>(c->num_sms / gr, std::max<int64_t>(1, C / 32));
     if (gs < 1) return false;
     const int64_t nch = (C + gs - 1) / gs;
-    const int ver = env_int("NPC_TILE_V", 5) == 4 ? 4 : 5;
     int K; int64_t nc;
-    if (!tile_shape(ver, c->width, nch, K, nc)) return false;
-    const int W = c->width;                            // 1 or 2 (int16 GT: pair kernel only)
+    if (!tile_shape(c->width, nch, K, nc)) return false;
+    const int W = c->width;                            // 1 or 2 (int16 GT)
     const int slab = (int)(nc * 32 * K * 16 * W);
     int Sr = env_int("NPC_TILE_SR", 0), Sc = env_int("NPC_TILE_SC", 0), L = env_int("NPC_TILE_L", 0), A = env_int("NPC_TILE_A", 2);
     int GD = env_int("NPC_TILE_GD", 0);
-    if (W != 1 && ver != 5) return false;
-    const int stage = F4_R * (ver == 5 ? slab / K : slab);           // bytes of a raw stage
-    auto smem_of = [&](int sr, int sc) {
-        return ver == 5 ? (int)Fused5Smem::make(sr, sc, slab, (int)nc, K, W).total : (int)Fused4Smem::make(sr, sc, slab).total;
-    };
+    const int stage = F5_R * slab / K;                 // bytes of a raw stage
+    auto smem_of = [&](int sr, int sc) { return (int)Fused5Smem::make(sr, sc, slab, (int)nc, K, W).total; };
     // K = 2: one raw stage per chunk set, ~110 KB of them, at least 3
     // (a quarter stage of slack: 19-20 warps, 38-40 KB stages, measured 0.93 / 0.965 on three stages against 0.91 / 0.94 on two)
-    if (Sr <= 0) Sr = std::max(ver == 5 && K == 2 ? 3 : 2, std::min(8, (112 * 1024 + (ver == 5 ? stage / 4 : 0)) / stage));
+    if (Sr <= 0) Sr = std::max(K == 2 ? 3 : 2, std::min(8, (112 * 1024 + stage / 4) / stage));
     if (Sc <= 0) {
         Sc = 32;
         while (Sc > 2 && smem_of(Sr, Sc) > max_smem) Sc--;
     }
-    while (Sr > (ver == 5 && K == 2 ? 3 : 2) && smem_of(Sr, Sc) > max_smem) Sr--;
+    while (Sr > (K == 2 ? 3 : 2) && smem_of(Sr, Sc) > max_smem) Sr--;
     // Deciders work on groups of GD tiles and the first tile of a group waits for the last: the lag must cover a
     // whole group plus the grid-wide round trip of the tally word (~6 us under load; a tile streams in
     // 4 * slab bytes / 42 GB/s per SM).  8 tiles per pass where the rings leave that much lag, else 4.
-    if (ver != 5) GD = 8;
-    else if (GD != 4 && GD != 8) {
+    if (GD != 4 && GD != 8) {
         const double tile_us = 4.0 * slab / 41.9e3;
         GD = Sc - 1 >= 8 + 1 + (int)std::ceil(6.0 / tile_us) ? 8 : 4;
     }
@@ -217,7 +213,6 @@ static bool tile_config(const npc_ctx *c, int gr, int max_smem, npc_ctx::TileCfg
     t.Gs = gs; t.Gr = gr; t.K = K; t.nc = (int)nc; t.slab = slab; t.Sr = Sr; t.Sc = Sc; t.L = L; t.GD = GD;
     t.A = std::max(1, std::min(2, A));
     t.smem = (uint32_t)smem_of(Sr, Sc);
-    t.ver = ver;
     t.ok = true;
     return true;
 }
@@ -244,7 +239,7 @@ static void plan_shapes(npc_ctx *c, int num_sms, int max_smem) {
         if (gs < 1) break;
         const int64_t nch = (C + gs - 1) / gs;
         int k; int64_t nc;
-        if (!tile_shape(env_int("NPC_TILE_V", 5) == 4 ? 4 : 5, c->width, nch, k, nc)) continue;
+        if (!tile_shape(c->width, nch, k, nc)) continue;
         if (force_gr && gr != force_gr) continue;
         const double score = (double)gs * gr * std::min<int64_t>(nc * k, 14) * ((double)nch / (double)(nc * 32 * k));
         cand.emplace_back(score, gr);
@@ -261,19 +256,24 @@ static void plan_shapes(npc_ctx *c, int num_sms, int max_smem) {
     // 2 row groups on 27 warps fill 97.8 % of the lanes, 148 x 1 on 14 warps 94.3 %: 0.938 against 0.920 of the
     // roofline); short ones keep round 1's rule -- more row groups leave a CTA fewer tiles to hide ramp-up and
     // drain behind, and k_add_partials grows with them.
-    if (c->fast.ok && !force_gr && env_int("NPC_TILE_LONG", 1)) {
+    if (c->fast.ok && !force_gr) {
         double have = 0.0, best = 0.0; int best_gr = 0;
         for (const auto &sc : cand) { if (sc.second == c->fast.Gr) have = sc.first; if (sc.first > best) { best = sc.first; best_gr = sc.second; } }
         if (best_gr && best_gr != c->fast.Gr && best > have * 1.02) tile_config(c, best_gr, max_smem, c->fast_long);
     }
     tile_config(c, 1, max_smem, c->exact_cfg);
-    if (!c->fast.ok && c->width == 1 && env_int("NPC_TILE_V", 5) != 4) {
+    if (!c->fast.ok && c->width == 1) {
         // no shape holds a whole row's share in one CTA: the fewest equal slabs (multiples of 1024 samples) the tile kernel can hold
         for (int S = 2; S <= 64 && !c->wide.ok; S++) {
             const int64_t ns = ((c->n + S - 1) / S + 1023) / 1024 * 1024;
             if (tile_config(c, 1, max_smem, c->wide, ns) && tile_config(c, 1, max_smem, c->wide_exact, ns)) { c->wide_n = ns; c->wide_slabs = (int)((c->n + ns - 1) / ns); }
             else c->wide.ok = c->wide_exact.ok = false;
         }
+        // ONE decider warp: in decided mode the local "tile counted" barrier is the deciders' only gate, and a warp that
+        // takes every A-th group of 8 tiles would wait on a ring slot's barrier 8*A tiles apart -- with 8*A > Sc it
+        // skips a phase of that slot and the parity test passes a whole ring turn early (in the normal mode the poll
+        // of the grid-wide tally word is the real gate, so the early pass is harmless there)
+        c->wide.A = c->wide_exact.A = 1;
     }
 }
 
@@ -281,20 +281,19 @@ static int fused_configure(npc_ctx *c, const cudaDeviceProp &prop) {
     const int max_smem = (int)prop.sharedMemPerBlockOptin;
     plan_shapes(c, prop.multiProcessorCount, max_smem);
     if (!c->fast.ok && !c->exact_cfg.ok && !c->wide.ok) return NPC_OK;
-    for (int ex = 0; ex < 5; ex++) {
-        const npc_ctx::TileCfg &t = ex == 0 ? c->fast : ex == 1 ? c->exact_cfg : ex == 2 ? c->wide : ex == 3 ? c->wide_exact : c->fast_long;
-        if (!t.ok) continue;
+    const std::pair<const npc_ctx::TileCfg *, bool> cfgs[] = {
+        { &c->fast, false }, { &c->fast_long, false }, { &c->exact_cfg, true }, { &c->wide, false }, { &c->wide_exact, true } };
+    for (const auto &[t, exact] : cfgs) {
+        if (!t->ok) continue;
         // the device's maximum, not this shape's need: the attribute belongs to the kernel function, which other contexts
         // of the process (and this context's other shapes) launch with other sizes
-        cudaError_t e = cudaFuncSetAttribute(tile_kernel(t.ver, t.K, (ex & 1) != 0, c->width, t.nc), cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
+        cudaError_t e = cudaFuncSetAttribute(tile_kernel(t->K, exact, c->width, t->nc), cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem);
         if (e != cudaSuccess) { c->err = std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(e); return NPC_ECUDA; }
     }
-    if (c->fast.ok || c->exact_cfg.ok || c->wide.ok) {
-        const size_t words = 2 * (size_t)std::max<int64_t>(c->max_rows, 1);
-        NPC_CUDA(c, cudaMalloc(&c->d_fcounts, words * sizeof(ull)));
-        NPC_CUDA(c, cudaMemset(c->d_fcounts, 0, words * sizeof(ull)));
-        if (env_int("NPC_TRACE", 0)) { NPC_CUDA(c, cudaMalloc(&c->d_trace, 8 * sizeof(ull))); NPC_CUDA(c, cudaMemset(c->d_trace, 0, 8 * sizeof(ull))); }
-    }
+    const size_t words = 2 * (size_t)std::max<int64_t>(c->max_rows, 1);
+    NPC_CUDA(c, cudaMalloc(&c->d_fcounts, words * sizeof(ull)));
+    NPC_CUDA(c, cudaMemset(c->d_fcounts, 0, words * sizeof(ull)));
+    if (env_int("NPC_TRACE", 0)) { NPC_CUDA(c, cudaMalloc(&c->d_trace, 8 * sizeof(ull))); NPC_CUDA(c, cudaMemset(c->d_trace, 0, 8 * sizeof(ull))); }
     const int max_gr = std::max(c->fast.ok ? c->fast.Gr : 1, c->fast_long.ok ? c->fast_long.Gr : 1);
     if (max_gr > 1) NPC_CUDA(c, cudaMalloc(&c->d_partials, (size_t)(max_gr - 1) * (size_t)c->n * sizeof(double)));
     c->exact = env_int("NPC_EXACT", 0) != 0;
@@ -332,8 +331,8 @@ static int create_impl(npc_ctx *c) {
         // pinned host slots only: the device copy of a slot is allocated when npc_score_block first needs it
         // (the resident path uploads straight into the slab)
         const size_t bytes = (size_t)c->row_stride * (size_t)std::max<int64_t>(c->staging_rows, 1);
-        // NPC_STAGE_WC=1: write-combined pinned memory (measured: no difference, the H2D copy runs at the PCIe rate either way)
-        NPC_CUDA(c, cudaHostAlloc((void **)&c->h_gt[s], bytes, env_int("NPC_STAGE_WC", 0) ? cudaHostAllocWriteCombined : cudaHostAllocDefault));
+        // (write-combined memory was measured no faster: the H2D copy runs at the PCIe rate either way)
+        NPC_CUDA(c, cudaHostAlloc((void **)&c->h_gt[s], bytes, cudaHostAllocDefault));
         NPC_CUDA(c, cudaEventCreateWithFlags(&c->ev_h2d[s], cudaEventDisableTiming));
         NPC_CUDA(c, cudaEventCreateWithFlags(&c->ev_done[s], cudaEventDisableTiming));
     }
@@ -427,19 +426,29 @@ static const npc_ctx::TileCfg &fast_config(const npc_ctx *c, int64_t n_rows) {
     return n_rows * c->row_stride >= long_bytes ? c->fast_long : c->fast;
 }
 
+// What a launch of n_rows GT rows runs (launch_block), and what npc_kernel_shape2 and npc_plan_shape report: 0 the generic
+// two-kernel sequence, 1 the tile kernel in exact order, 2 in default order, 3 tally + decide, then the tile kernel in
+// decided mode over the wide slabs (only where no resident shape fits).  t: the tile kernel's shape in modes 1-3.
+static int launch_mode(const npc_ctx *c, bool exact, int64_t n_rows, const npc_ctx::TileCfg *&t) {
+    t = exact ? &c->exact_cfg : &fast_config(c, n_rows);
+    if (t->ok) return exact ? 1 : 2;
+    t = exact ? &c->wide_exact : &c->wide;
+    return t->ok ? 3 : 0;
+}
+
 extern "C" int npc_kernel_shape2(const npc_ctx *ctx, int64_t n_rows, int32_t shape[8]) {
     if (!ctx || !shape || n_rows < 0) return NPC_EINVAL;
-    const bool wide = !(ctx->exact ? ctx->exact_cfg.ok : ctx->fast.ok) && ctx->wide.ok;
-    const npc_ctx::TileCfg &t = wide ? (ctx->exact ? ctx->wide_exact : ctx->wide) : ctx->exact ? ctx->exact_cfg : fast_config(ctx, n_rows);
     memset(shape, 0, 8 * sizeof(int32_t));
     if (ctx->bed) {
         shape[0] = 4; shape[1] = (int32_t)((ctx->n + 8 * BED_THREADS - 1) / (8 * BED_THREADS)); shape[2] = BED_THREADS / 32;
         shape[3] = 8; shape[4] = ctx->exact ? 1 : 4;
         return NPC_OK;
     }
-    if (!t.ok) return NPC_OK;
-    shape[0] = wide ? 3 : ctx->exact ? 1 : 2; shape[1] = t.Gs * 1000 + (ctx->exact ? 1 : t.Gr); shape[2] = t.nc; shape[3] = t.K;
-    shape[4] = F4_R; shape[5] = t.Sr * 1000 + t.Sc; shape[6] = t.L * 100 + t.GD * 10 + t.A; shape[7] = (int32_t)t.smem;
+    const npc_ctx::TileCfg *t;
+    const int mode = launch_mode(ctx, ctx->exact, n_rows, t);
+    if (!mode) return NPC_OK;
+    shape[0] = mode; shape[1] = t->Gs * 1000 + t->Gr; shape[2] = t->nc; shape[3] = t->K;
+    shape[4] = F5_R; shape[5] = t->Sr * 1000 + t->Sc; shape[6] = t->L * 100 + t->GD * 10 + t->A; shape[7] = (int32_t)t->smem;
     return NPC_OK;
 }
 extern "C" int npc_kernel_shape(const npc_ctx *ctx, int32_t shape[8]) { return npc_kernel_shape2(ctx, 0, shape); }
@@ -451,14 +460,13 @@ extern "C" int npc_plan_shape(int64_t n_samples, int32_t gt_width, int32_t num_s
     c->n = n_samples; c->ploidy = 2; c->width = gt_width;
     c->row_stride = ((npc_gt_row_bytes(c->n, c->ploidy, c->width) + 127) / 128) * 128;
     plan_shapes(c, num_sms, max_smem);
-    const bool wide = !(exact ? c->exact_cfg.ok : c->fast.ok) && c->wide.ok;
-    const npc_ctx::TileCfg &t = wide ? (exact ? c->wide_exact : c->wide) : exact ? c->exact_cfg : fast_config(c, n_rows);
+    const npc_ctx::TileCfg *t;
+    const int mode = launch_mode(c, exact != 0, n_rows, t);
     memset(plan, 0, 16 * sizeof(int32_t));
-    if (t.ok) {
-        const int A = wide ? 1 : t.A;
-        const int32_t v[16] = { wide ? 3 : exact ? 1 : 2, t.Gs, exact || wide ? 1 : t.Gr, t.K, t.nc, t.slab, t.Sr, t.Sc, t.L, A, t.GD, (int32_t)t.smem,
-                                (t.nc + 2 + A) * 32, t.K == 1 && c->width == 1 ? (t.nc > F5_NC_WIDE ? F5_NC_MAX : t.nc > 16 ? F5_NC_WIDE : 16) : 16,
-                                wide ? c->wide_slabs : 1, wide ? (int32_t)c->wide_n : (int32_t)std::min<int64_t>(c->n, INT32_MAX) };
+    if (mode) {
+        const int32_t v[16] = { mode, t->Gs, t->Gr, t->K, t->nc, t->slab, t->Sr, t->Sc, t->L, t->A, t->GD, (int32_t)t->smem,
+                                (t->nc + 2 + t->A) * 32, instance_warps(c->width, t->K, t->nc),
+                                mode == 3 ? c->wide_slabs : 1, mode == 3 ? (int32_t)c->wide_n : (int32_t)std::min<int64_t>(c->n, INT32_MAX) };
         memcpy(plan, v, sizeof(v));
     }
     delete c;
@@ -522,21 +530,22 @@ static int upload_rows(npc_ctx *c, const npc_row *rows, int64_t n_rows, int on_d
     return NPC_OK;
 }
 
+// Blocks per row of the tally kernels (256 threads, rows of `units`): cheap to run but not free to schedule, so up to 64 units
+// per thread (5.8 TB/s on an 8 GB slab against 4.6 TB/s at 4), fewer only to keep ~4096 blocks, at least min_units a block.
+static unsigned tally_grid_y(int64_t units, int64_t n_rows, int64_t min_units) {
+    const int64_t s_min = (units + 16383) / 16384, s_max = (units + min_units - 1) / min_units, want = (4096 + n_rows - 1) / n_rows;
+    return (unsigned)std::min<int64_t>(std::max<int64_t>(std::min(std::max(want, s_min), s_max), 1), 65535);
+}
+
 static int launch_count(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows,
                         ull *counts) {
     NPC_CUDA(c, cudaMemsetAsync(counts, 0, n_rows * 2 * sizeof(ull), c->stream));
     if (n_rows == 0 || c->n == 0) return NPC_OK;
     if (c->width == 1 && c->ploidy == 2) {
-        const int64_t nchunks = (c->n + 7) / 8;
-        // blocks are cheap to run but not free to schedule: up to 64 chunks per thread (5.8 TB/s on an 8 GB
-        // slab against 4.6 TB/s at 4 per thread), fewer only to keep ~4096 blocks in the grid
-        const int64_t s_min = (nchunks + 16383) / 16384, s_max = (nchunks + 1023) / 1024, want = (4096 + n_rows - 1) / n_rows;
-        const unsigned slabs = (unsigned)std::min<int64_t>(std::max<int64_t>(std::min(std::max(want, s_min), s_max), 1), 65535);
+        const unsigned slabs = tally_grid_y((c->n + 7) / 8, n_rows, 1024);                   // units: chunks of 8 samples
         k_count_i8x2<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
     } else {
-        const int64_t s_min = (c->n + 16383) / 16384, s_max = (c->n + 2047) / 2048, want = (4096 + n_rows - 1) / n_rows;   // as above
-        const unsigned slabs = (unsigned)std::min<int64_t>(std::max<int64_t>(std::min(std::max(want, s_min), s_max), 1), 65535);
-        dim3 grid((unsigned)n_rows, slabs);
+        dim3 grid((unsigned)n_rows, tally_grid_y(c->n, n_rows, 2048));                        // units: samples
         if (c->width == 1) k_count_generic<int8_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->ploidy, counts);
         else if (c->width == 2) k_count_generic<int16_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->ploidy, counts);
         else k_count_generic<int32_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->ploidy, counts);
@@ -572,35 +581,29 @@ static int launch_decide_accum(npc_ctx *c, const uint8_t *gt, int64_t row_stride
     return NPC_OK;
 }
 
-// count -> decide -> accumulate in one persistent cooperative launch (npc_fused4.cuh)
+// count -> decide -> accumulate in one persistent cooperative launch (npc_fused5.cuh)
 static int launch_fused(npc_ctx *c, const npc_ctx::TileCfg &t, bool exact, const uint8_t *gt, int64_t row_stride,
                         const npc_row *d_rows, int64_t n_rows) {
     if (n_rows == 0) return NPC_OK;
     int rc = ensure_log(c, n_rows);
     if (rc) return rc;
-    const int64_t half_words = std::max<int64_t>(c->max_rows, 1);
-    ull *counts = c->d_fcounts, *counts_next = nullptr;
-    int64_t n_zero = 0;
-    if (t.ver == 5) {                                  // double buffer: this launch clears the words the next one uses
-        counts = c->d_fcounts + (size_t)c->fcounts_half * half_words;
-        counts_next = c->d_fcounts + (size_t)(c->fcounts_half ^ 1) * half_words;
-        n_zero = c->fcounts_dirty[c->fcounts_half ^ 1];
-        c->fcounts_dirty[c->fcounts_half ^ 1] = 0;
-        c->fcounts_dirty[c->fcounts_half] = n_rows;
-        c->fcounts_half ^= 1;
-    } else NPC_CUDA(c, cudaMemsetAsync(c->d_fcounts, 0, n_rows * sizeof(ull), c->stream));
-    const int64_t tiles = (n_rows + F4_R - 1) / F4_R;
+    const int64_t tiles = (n_rows + F5_R - 1) / F5_R;
     const int gr = exact ? 1 : (int)std::max<int64_t>(1, std::min<int64_t>(t.Gr, tiles / 16));   // >= 16 tiles per row group
+    // the tally words are a double buffer: this launch counts into half h and clears the words of half h ^ 1 the next one uses
+    const int64_t half_words = std::max<int64_t>(c->max_rows, 1), h = c->fcounts_half;
     FusedParams P;
     P.gt = gt; P.row_stride = row_stride; P.n = c->n; P.rows = d_rows; P.n_rows = n_rows; P.pol = c->pol;
-    P.sums = c->d_sums; P.counts = counts; P.log = c->d_log + c->log_len; P.nloci = c->d_nloci;
-    P.counts_next = counts_next; P.n_zero = n_zero; P.trace = c->d_trace;
+    P.sums = c->d_sums; P.counts = c->d_fcounts + h * half_words; P.log = c->d_log + c->log_len; P.nloci = c->d_nloci;
+    P.counts_next = c->d_fcounts + (h ^ 1) * half_words; P.n_zero = c->fcounts_dirty[h ^ 1]; P.trace = c->d_trace;
+    c->fcounts_dirty[h ^ 1] = 0;
+    c->fcounts_dirty[h] = n_rows;
+    c->fcounts_half ^= 1;
     P.Sr = t.Sr; P.Sc = t.Sc; P.L = t.L; P.A = t.A; P.nc = t.nc; P.slab_stride = t.slab; P.GD = t.GD;
     P.Gs = t.Gs; P.Gr = gr; P.partials = c->d_partials;
     P.aux_sleep_ns = (uint32_t)env_int("NPC_TILE_SLEEP", 0);
     P.decided = nullptr;
     void *args[] = { &P };
-    NPC_CUDA(c, cudaLaunchCooperativeKernel(tile_kernel(t.ver, t.K, exact, c->width, t.nc), dim3(t.Gs * gr), dim3((t.nc + 2 + t.A) * 32), args, t.smem, c->stream));
+    NPC_CUDA(c, cudaLaunchCooperativeKernel(tile_kernel(t.K, exact, c->width, t.nc), dim3(t.Gs * gr), dim3((t.nc + 2 + t.A) * 32), args, t.smem, c->stream));
     c->launches++;
     // Row groups > 1: a second, wide kernel adds the groups' partial sums in group order.  (Folding this into the tile
     // kernel -- the last group of a slab to finish adds them -- was measured in round 2: one CTA per slab doing
@@ -618,7 +621,8 @@ static int launch_fused(npc_ctx *c, const npc_ctx::TileCfg &t, bool exact, const
 // then the tile kernel in "decided" mode once per slab of the sample axis -- it decodes and accumulates, the deciders
 // read the rows' contributions from d_rowp.  The slab is read twice (4 B/genotype), the second time at the tile
 // kernel's rate instead of k_accum's.
-static int launch_wide(npc_ctx *c, bool exact, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows) {
+static int launch_wide(npc_ctx *c, const npc_ctx::TileCfg &t, bool exact, const uint8_t *gt, int64_t row_stride,
+                       const npc_row *d_rows, int64_t n_rows) {
     if (n_rows == 0) return NPC_OK;
     int rc = launch_count(c, gt, row_stride, d_rows, n_rows, c->d_counts);
     if (rc) return rc;
@@ -628,7 +632,6 @@ static int launch_wide(npc_ctx *c, bool exact, const uint8_t *gt, int64_t row_st
     c->launches++;
     NPC_CUDA(c, cudaGetLastError());
     c->log_len += n_rows;
-    const npc_ctx::TileCfg &t = exact ? c->wide_exact : c->wide;
     for (int s = 0; s < c->wide_slabs; s++) {
         const int64_t s0 = (int64_t)s * c->wide_n, ns = std::min<int64_t>(c->wide_n, c->n - s0);
         if (ns <= 0) break;
@@ -636,16 +639,12 @@ static int launch_wide(npc_ctx *c, bool exact, const uint8_t *gt, int64_t row_st
         memset(&P, 0, sizeof(P));
         P.gt = gt + s0 * 2; P.row_stride = row_stride; P.n = ns; P.rows = d_rows; P.n_rows = n_rows; P.pol = c->pol;
         P.sums = c->d_sums + s0; P.counts = c->d_fcounts; P.log = nullptr; P.nloci = c->d_nloci;
-        // ONE decider warp: in this mode the local "tile counted" barrier is the deciders' only gate, and a warp that
-        // takes every A-th group of 8 tiles would wait on a ring slot's barrier 8*A tiles apart -- with 8*A > Sc it
-        // skips a phase of that slot and the parity test passes a whole ring turn early (in the normal mode the poll
-        // of the grid-wide tally word is the real gate, so the early pass is harmless there)
-        P.Sr = t.Sr; P.Sc = t.Sc; P.L = t.L; P.A = 1; P.nc = t.nc; P.slab_stride = t.slab; P.GD = t.GD;
+        P.Sr = t.Sr; P.Sc = t.Sc; P.L = t.L; P.A = t.A; P.nc = t.nc; P.slab_stride = t.slab; P.GD = t.GD;
         P.Gs = t.Gs; P.Gr = 1; P.partials = nullptr;
         P.aux_sleep_ns = (uint32_t)env_int("NPC_TILE_SLEEP", 0);
         P.decided = c->d_rowp;
         void *args[] = { &P };
-        NPC_CUDA(c, cudaLaunchCooperativeKernel(tile_kernel(t.ver, t.K, exact, c->width, t.nc), dim3(t.Gs), dim3((t.nc + 2 + 1) * 32), args, t.smem, c->stream));
+        NPC_CUDA(c, cudaLaunchCooperativeKernel(tile_kernel(t.K, exact, c->width, t.nc), dim3(t.Gs), dim3((t.nc + 2 + t.A) * 32), args, t.smem, c->stream));
         c->launches++;
     }
     return NPC_OK;
@@ -686,10 +685,7 @@ static int launch_bed(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const n
     if (rc) return rc;
     NPC_CUDA(c, cudaMemsetAsync(c->d_counts, 0, n_rows * 2 * sizeof(ull), c->stream));
     if (c->n) {
-        // as k_count_i8x2: ~4096 blocks, up to 64 chunks (of 64 samples) per thread
-        const int64_t nchunks = (c->n + 63) / 64;
-        const int64_t s_min = (nchunks + 16383) / 16384, s_max = (nchunks + 1023) / 1024, want = (4096 + n_rows - 1) / n_rows;
-        const unsigned slabs = (unsigned)std::min<int64_t>(std::max<int64_t>(std::min(std::max(want, s_min), s_max), 1), 65535);
+        const unsigned slabs = tally_grid_y((c->n + 63) / 64, n_rows, 1024);                 // units: chunks of 64 samples
         k_count_bed<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->d_counts);
         c->launches++;
     }
@@ -722,8 +718,10 @@ static int launch_bed(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const n
 static int launch_block(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows) {
     if (c->ds) return launch_dosage(c, gt, row_stride, d_rows, n_rows);
     if (c->bed) return launch_bed(c, gt, row_stride, d_rows, n_rows);
-    if (c->exact ? c->exact_cfg.ok : c->fast.ok) return launch_fused(c, c->exact ? c->exact_cfg : fast_config(c, n_rows), c->exact, gt, row_stride, d_rows, n_rows);
-    if (c->wide.ok && env_int("NPC_WIDE", 1)) return launch_wide(c, c->exact, gt, row_stride, d_rows, n_rows);
+    const npc_ctx::TileCfg *t;
+    const int mode = launch_mode(c, c->exact, n_rows, t);
+    if (mode == 1 || mode == 2) return launch_fused(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
+    if (mode == 3) return launch_wide(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
     int rc = launch_count(c, gt, row_stride, d_rows, n_rows, c->d_counts);
     if (rc) return rc;
     return launch_decide_accum(c, gt, row_stride, d_rows, n_rows, c->d_counts);

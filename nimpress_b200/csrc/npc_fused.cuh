@@ -1,6 +1,6 @@
-// npc_fused.cuh -- shared pieces of the fused persistent kernels (npc_fused4.cuh): launch
-// parameters, the packed tally word, and the PTX wrappers for mbarrier / TMA bulk copies / relaxed
-// global loads and REDs / shared-memory loads with raw 32-bit addresses.
+// npc_fused.cuh -- shared pieces of the fused persistent tile kernel (npc_fused5.cuh): launch
+// parameters, the packed tally word, the PTX wrappers for mbarrier / TMA bulk copies / relaxed
+// global loads and REDs / shared-memory loads with raw 32-bit addresses, and k_add_partials.
 #pragma once
 #include "npc_kernels.cuh"
 
@@ -110,6 +110,11 @@ __device__ __forceinline__ uint32_t lds_u8(uint32_t addr) {
     asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(addr));
     return v;
 }
+__device__ __forceinline__ uint32_t lds_u32(uint32_t addr) {
+    uint32_t v;
+    asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(addr));
+    return v;
+}
 __device__ __forceinline__ double lds_f64(uint32_t addr) {
     double v;
     asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(addr));
@@ -133,6 +138,15 @@ __device__ __forceinline__ void sts_v1(uint32_t addr, uint32_t a) {
 }
 __device__ __forceinline__ void red_shared_add_u32(uint32_t addr, uint32_t v) {
     asm volatile("red.shared.add.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
+}
+
+// sums[s] = ((sums[s] + p0[s]) + p1[s]) + ...: the row groups' partial sums, in group (= row) order
+__global__ void k_add_partials(double *__restrict__ sums, const double *__restrict__ partials, int64_t n, int n_partials) {
+    const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= n) return;
+    double a = sums[s];
+    for (int g = 0; g < n_partials; g++) a = __dadd_rn(a, partials[(int64_t)g * n + s]);
+    sums[s] = a;
 }
 
 }  // namespace npc

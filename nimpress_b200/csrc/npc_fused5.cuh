@@ -1,16 +1,16 @@
-// npc_fused5.cuh -- the default roofline kernel, second generation ("pair lookup").
-//
-// Same pipeline as npc_fused4.cuh (TMA raw ring -> COUNT -> grid-wide tally dependency -> DECIDE ->
-// ACCUMULATE over tiles of four score rows, every genotype byte read from HBM exactly once); what
-// changed is what the round-1 ncu source page showed to be the bound: the consumer warps were never
-// waiting, they were issuing 336 instructions per (tile, warp), 75 of them for the tallies alone.
+// npc_fused5.cuh -- the default roofline kernel ("pair lookup"): count -> decide -> accumulate in one
+// persistent cooperative launch.  A TMA raw ring feeds COUNT, a grid-wide tally dependency gates
+// DECIDE, and ACCUMULATE runs over tiles of four score rows; every genotype byte is read from HBM
+// exactly once.  The consumer warps are bound by the instructions they issue, not by waiting (the
+// round-1 tile kernel issued 336 per (tile, warp), 75 of them for the tallies alone), so every step
+// below is built to issue few:
 //
 //  * COUNT looks up TWO samples at a time.  A 32-bit word of the raw row holds two diploid int8
 //    samples (4 allele bytes).  On the fast path (every byte < 8: alleles REF, ALT1, ALT2 or missing,
 //    no sentinel) each byte carries its allele code (allele+1, 0 = missing) in bits 1-2, and ONE
 //    byte-wise dot product, dp4a(w & 0x06060606, {132, 2, 8, 32}, table), is the address of the pair's
-//    4-byte entry: a mask, an IDP.4A and an LDS.32 per two genotypes (v1: two folds, two PRMT and two
-//    LDS.U16).  The entry index is 66*c0 + c1 + 4*c2 + 16*c3: injective over all 256 code
+//    4-byte entry: a mask, an IDP.4A and an LDS.32 per two genotypes.  The entry index is
+//    66*c0 + c1 + 4*c2 + 16*c3: injective over all 256 code
 //    combinations, and -- unlike the plain base-4 index, whose top digit never reaches the bank
 //    bits -- the 16 combinations of REF / ALT1 alleles fall into 16 different banks, so the lookups of a
 //    warp are conflict-free on ordinary data (measured with base-4: 1.85 wavefronts per lookup).
@@ -21,8 +21,12 @@
 //  * Tallies leave the warp with two RED.shared.add.u32 per chunk into per-lane counters (three
 //    warps share a counter: 6-bit fields hold 3 x 16), no warp reduction, no lane-0 epilogue; the
 //    publisher warp, which has time to spare, does the cross-lane sum once per tile.
-//  * DECIDE and ACCUMULATE are those of v1 (two conflict-free 16-entry fp64 tables per tile, two
-//    LDS.64 and two DADD per sample per four genotypes); the index-ring byte of a sample pair is
+//  * DECIDE builds, per tile, two 16-entry fp64 tables T01[b0|b1<<2] = v0[b0]+v1[b1] and
+//    T23[b2|b3<<2] = v2[b2]+v3[b3] of the rows' contributions (constant rows and dropped rows fold
+//    in as constants).  16 doubles span exactly the 32 banks: every lookup is conflict-free (one
+//    256-entry table was measured at 3-way conflicts: its hot entries share 9 of 16 bank pairs).
+//  * ACCUMULATE: sums[s] = (sums[s] + T01[..]) + T23[..] -- two LDS.64 and two DADD per sample per
+//    four genotypes, no per-row branches.  The index-ring byte of a sample pair is
 //    [sample 0: rows a,b | sample 1: rows a,b], one byte for rows (0,1) and one for rows (2,3).
 //
 //  * Wide cohorts.  One chunk (8 samples) per consumer thread up to 28 warps (~1.06 M samples on 148 CTAs); above that
@@ -31,11 +35,20 @@
 //    of ring and 1.4 us of streaming) the deciders take 4 tiles per pass instead of 8: the first tile of a pass waits
 //    for its last to be counted by the whole grid, and that wait must fit the lag.
 //
-// Rounding and the EXACT mode are as in npc_fused4.cuh: every addend is the reference's rounded
-// product fl(dosage*beta) (src/nimpress.nim:640); the default mode adds rows (0,1) and (2,3) of a
-// tile to each other first, EXACT adds row by row in score-file order, bit for bit the reference.
+// Rounding: the contributions of rows (0,1) and of rows (2,3) of a tile are added to each other
+// first and then, in that order, to the running sum.  Every addend is still the reference's rounded
+// product fl(dosage*beta); only the association differs from the reference's left-to-right chain
+// (src/nimpress.nim:639-640), so scores agree to a few ulp of the running sum (tests assert <= 1e-12
+// relative; the contract is 1e-9).  The result is deterministic; the association depends on how the
+// rows are cut into launches and row groups (DESIGN 4.1), not on the sample slabs.
+//
+// EXACT = true (npc_set_exact_order) keeps everything above except the pre-summing: the tile's
+// block holds the four rows' 4-entry tables and ACCUMULATE does one lookup and one DADD per
+// genotype, rows in order -- the same rounded products and the same rounded adds as
+// `scores[i] += dosages[i]*beta` (src/nimpress.nim:640), bit for bit.  It runs on a 1-D grid (every
+// CTA sees every row) so that the per-sample chain is the reference's.
 #pragma once
-#include "npc_fused4.cuh"   // lds_u32 and the shared PTX helpers
+#include "npc_fused.cuh"
 
 namespace npc {
 

@@ -160,7 +160,7 @@ def nb():
 
 
 def slab_starts(n, p):
-    """First sample of every CTA's share of the sample axis (npc_fused5.cuh:139-142); in decided mode, of every wide
+    """First sample of every CTA's share of the sample axis (npc_fused5.cuh:152-155); in decided mode, of every wide
     slab and of the CTA shares inside the first one."""
     n_slab = p["wide_samples"] if p["mode"] == 3 else n
     C, gs = -(-n_slab // 8), max(p["sample_slabs"], 1)
@@ -261,6 +261,9 @@ def test_instance_parity(nb, name, mode):
     eng.set_policy(); eng.set_exact_order(exact); eng.reset()
     shape = eng.kernel_shape_for(R)
     assert shape["fused"] == want_plan["mode"], shape
+    p = case_plan(name, exact)                             # the context reports the launch the planner chose
+    for k in ("decider_warps", "decider_tiles", "lag", "raw_stages", "index_tiles", "smem_bytes"):
+        assert shape[k] == p[k], (k, shape, p)
     if want_plan["mode"]:
         for k in ("chunks_per_thread", "consumer_warps"):
             assert shape[k] == want_plan[k], (k, shape)
