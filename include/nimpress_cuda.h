@@ -39,10 +39,9 @@
  * Environment (diagnostics and tests; none is needed in normal use):
  *   NPC_FUSED=0              two-kernel sequence instead of the fused tile kernel
  *   NPC_EXACT=1              exact-order mode for every context (as npc_set_exact_order)
- *   NPC_TILE_K / _SR / _SC / _L / _A / _GR / _GD / _NC1   launch shape of the fused tile kernel (chunks per thread, raw
- *                            stages, index tiles, lag, decider warps, row groups, tiles per decider pass, most warps at K = 1)
+ *   NPC_TILE_K / _SR / _SC / _L / _A / _GR / _GD   launch shape of the fused tile kernel (chunks per thread, raw
+ *                            stages, index tiles, lag, decider warps, row groups, tiles per decider pass)
  *   NPC_TILE_LONG_MB=<MB>    what counts as a long launch, which may split the grid differently (default 1536, or 192 when short launches split the rows too)
- *   NPC_TILE_SLEEP=<ns>      auxiliary warps of the tile kernel poll + nanosleep instead of a suspended try_wait
  *   NPC_MULTI=0 | 1          npc_score_resident_multi: never / always the tensor-core contraction (default: >= 3 definitions)
  *   NPC_MULTI_PARTS=<n>      split of a tile's entry range over work units in the contraction (default: chosen from the tile count)
  *   NPC_TIMING=1             phase wall times of npc_score_resident_multi on stderr

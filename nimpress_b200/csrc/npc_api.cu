@@ -170,23 +170,28 @@ static const void *tile_kernel(int K, bool exact, int width, int nc) {
 // per thread as long as the warps fit the SM's registers (int8 GT: up to 24 warps on the 72-register instance, cohorts
 // up to ~909,000 samples per GPU), two (up to 16 warps) above that.
 static bool tile_shape(int width, int64_t nch, int &K, int64_t &nc) {
-    const int max1 = width == 1 ? std::max(1, std::min(F5_NC_MAX, env_int("NPC_TILE_NC1", F5_NC_MAX))) : 16;
+    const int max1 = width == 1 ? F5_NC_MAX : 16;
     K = env_int("NPC_TILE_K", 0);
     if (K != 1 && K != 2) K = nch <= 32 * max1 ? 1 : 2;
     nc = (nch + 32 * K - 1) / (32 * K);
     return nc <= (K == 1 ? max1 : 16);                // else: cohort too wide for one resident pass
 }
 
+// The sample axis of C chunks under `gr` row groups: gs slabs (one CTA each, gs * gr CTAs at most one per SM) of nch chunks,
+// and the consumer shape that holds a slab.  False when no such split exists.
+static bool slab_split(const npc_ctx *c, int64_t C, int gr, int &gs, int64_t &nch, int &K, int64_t &nc) {
+    gs = (int)std::min<int64_t>(c->num_sms / gr, std::max<int64_t>(1, C / 32));
+    if (gs < 1) return false;
+    nch = (C + gs - 1) / gs;
+    return tile_shape(c->width, nch, K, nc);
+}
+
 // Launch shape of the tile kernel for `gr` row groups: Gs sample slabs (one CTA each), a raw ring of Sr
 // stages (one chunk set of 4 rows each; ~110 KB of loads in flight per SM), the rest of shared memory as
 // index-ring slots, lag L = Sc - 1 tiles, A decider warps deciding GD tiles per pass.
 static bool tile_config(const npc_ctx *c, int gr, int max_smem, npc_ctx::TileCfg &t, int64_t n_samples = -1) {
-    const int64_t C = ((n_samples < 0 ? c->n : n_samples) + 7) / 8;
-    const int gs = (int)std::min<int64_t>(c->num_sms / gr, std::max<int64_t>(1, C / 32));
-    if (gs < 1) return false;
-    const int64_t nch = (C + gs - 1) / gs;
-    int K; int64_t nc;
-    if (!tile_shape(c->width, nch, K, nc)) return false;
+    int gs, K; int64_t nch, nc;
+    if (!slab_split(c, ((n_samples < 0 ? c->n : n_samples) + 7) / 8, gr, gs, nch, K, nc)) return false;
     const int W = c->width;                            // 1 or 2 (int16 GT)
     const int slab = (int)(nc * 32 * K * 16 * W);
     int Sr = env_int("NPC_TILE_SR", 0), Sc = env_int("NPC_TILE_SC", 0), L = env_int("NPC_TILE_L", 0), A = env_int("NPC_TILE_A", 2);
@@ -235,12 +240,8 @@ static void plan_shapes(npc_ctx *c, int num_sms, int max_smem) {
     // found cohorts whose best-scoring split did not fit and silently lost the fused path)
     std::vector<std::pair<double, int>> cand;
     for (int gr = 1; gr <= 16; gr++) {
-        const int gs = (int)std::min<int64_t>(c->num_sms / gr, std::max<int64_t>(1, C / 32));
-        if (gs < 1) break;
-        const int64_t nch = (C + gs - 1) / gs;
-        int k; int64_t nc;
-        if (!tile_shape(c->width, nch, k, nc)) continue;
-        if (force_gr && gr != force_gr) continue;
+        int gs, k; int64_t nch, nc;
+        if (!slab_split(c, C, gr, gs, nch, k, nc) || (force_gr && gr != force_gr)) continue;
         const double score = (double)gs * gr * std::min<int64_t>(nc * k, 14) * ((double)nch / (double)(nc * 32 * k));
         cand.emplace_back(score, gr);
     }
@@ -426,10 +427,13 @@ static const npc_ctx::TileCfg &fast_config(const npc_ctx *c, int64_t n_rows) {
     return n_rows * c->row_stride >= long_bytes ? c->fast_long : c->fast;
 }
 
-// What a launch of n_rows GT rows runs (launch_block), and what npc_kernel_shape2 and npc_plan_shape report: 0 the generic
-// two-kernel sequence, 1 the tile kernel in exact order, 2 in default order, 3 tally + decide, then the tile kernel in
-// decided mode over the wide slabs (only where no resident shape fits).  t: the tile kernel's shape in modes 1-3.
+// What a launch of n_rows rows runs (launch_block), and what npc_kernel_shape2 and npc_plan_shape report: 0 the generic
+// tally, decide, accumulate sequence, 1 the tile kernel in exact order, 2 in default order, 3 tally + decide, then the tile
+// kernel in decided mode over the wide slabs (only where no resident shape fits), 4 the sequence on PLINK .bed rows.
+// t: the tile kernel's shape in modes 1-3.
 static int launch_mode(const npc_ctx *c, bool exact, int64_t n_rows, const npc_ctx::TileCfg *&t) {
+    t = nullptr;
+    if (c->bed) return 4;
     t = exact ? &c->exact_cfg : &fast_config(c, n_rows);
     if (t->ok) return exact ? 1 : 2;
     t = exact ? &c->wide_exact : &c->wide;
@@ -439,16 +443,15 @@ static int launch_mode(const npc_ctx *c, bool exact, int64_t n_rows, const npc_c
 extern "C" int npc_kernel_shape2(const npc_ctx *ctx, int64_t n_rows, int32_t shape[8]) {
     if (!ctx || !shape || n_rows < 0) return NPC_EINVAL;
     memset(shape, 0, 8 * sizeof(int32_t));
-    if (ctx->bed) {
-        shape[0] = 4; shape[1] = (int32_t)((ctx->n + 8 * BED_THREADS - 1) / (8 * BED_THREADS)); shape[2] = BED_THREADS / 32;
-        shape[3] = 8; shape[4] = ctx->exact ? 1 : 4;
-        return NPC_OK;
-    }
     const npc_ctx::TileCfg *t;
-    const int mode = launch_mode(ctx, ctx->exact, n_rows, t);
-    if (!mode) return NPC_OK;
-    shape[0] = mode; shape[1] = t->Gs * 1000 + t->Gr; shape[2] = t->nc; shape[3] = t->K;
-    shape[4] = F5_R; shape[5] = t->Sr * 1000 + t->Sc; shape[6] = t->L * 100 + t->GD * 10 + t->A; shape[7] = (int32_t)t->smem;
+    shape[0] = launch_mode(ctx, ctx->exact, n_rows, t);
+    if (shape[0] == 4) {
+        shape[1] = (int32_t)((ctx->n + 8 * BED_THREADS - 1) / (8 * BED_THREADS)); shape[2] = BED_THREADS / 32;
+        shape[3] = 8; shape[4] = ctx->exact ? 1 : 4;
+    } else if (shape[0]) {
+        shape[1] = t->Gs * 1000 + t->Gr; shape[2] = t->nc; shape[3] = t->K;
+        shape[4] = F5_R; shape[5] = t->Sr * 1000 + t->Sc; shape[6] = t->L * 100 + t->GD * 10 + t->A; shape[7] = (int32_t)t->smem;
+    }
     return NPC_OK;
 }
 extern "C" int npc_kernel_shape(const npc_ctx *ctx, int32_t shape[8]) { return npc_kernel_shape2(ctx, 0, shape); }
@@ -537,163 +540,63 @@ static unsigned tally_grid_y(int64_t units, int64_t n_rows, int64_t min_units) {
     return (unsigned)std::min<int64_t>(std::max<int64_t>(std::min(std::max(want, s_min), s_max), 1), 65535);
 }
 
-static int launch_count(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows,
+// Tallies of n_rows rows into counts: two words a row; for dosage rows the missing count alone, the block sums of the
+// called dosages go to d_ds_part.
+static int launch_tally(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows,
                         ull *counts) {
-    NPC_CUDA(c, cudaMemsetAsync(counts, 0, n_rows * 2 * sizeof(ull), c->stream));
+    NPC_CUDA(c, cudaMemsetAsync(counts, 0, n_rows * (c->ds ? 1 : 2) * sizeof(ull), c->stream));
     if (n_rows == 0 || c->n == 0) return NPC_OK;
-    if (c->width == 1 && c->ploidy == 2) {
-        const unsigned slabs = tally_grid_y((c->n + 7) / 8, n_rows, 1024);                   // units: chunks of 8 samples
-        k_count_i8x2<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
-    } else {
-        dim3 grid((unsigned)n_rows, tally_grid_y(c->n, n_rows, 2048));                        // units: samples
-        if (c->width == 1) k_count_generic<int8_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->ploidy, counts);
-        else if (c->width == 2) k_count_generic<int16_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->ploidy, counts);
-        else k_count_generic<int32_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->ploidy, counts);
-    }
-    c->launches++;
-    NPC_CUDA(c, cudaGetLastError());
-    return NPC_OK;
-}
-
-static int launch_decide_accum(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows,
-                               int64_t n_rows, const ull *counts) {
-    if (n_rows == 0) return NPC_OK;
-    int rc = ensure_log(c, n_rows);
-    if (rc) return rc;
-    k_decide<<<(unsigned)((n_rows + 127) / 128), 128, 0, c->stream>>>(d_rows, n_rows, counts, c->pol, c->n, c->d_rowp,
-                                                                      c->d_log + c->log_len, c->d_nloci);
-    c->launches++;
-    NPC_CUDA(c, cudaGetLastError());
-    c->log_len += n_rows;
-    if (c->n == 0) return NPC_OK;
-    if (c->width == 1 && c->ploidy == 2) {
-        const int64_t nchunks = (c->n + 7) / 8;
-        k_accum_i8x2<64, 8><<<(unsigned)((nchunks + 255) / 256), 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows,
-                                                                                     c->n, c->d_sums);
-    } else {
-        const unsigned grid = (unsigned)((c->n + 255) / 256);
-        if (c->width == 1) k_accum_generic<int8_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
-        else if (c->width == 2) k_accum_generic<int16_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
-        else k_accum_generic<int32_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
-    }
-    c->launches++;
-    NPC_CUDA(c, cudaGetLastError());
-    return NPC_OK;
-}
-
-// count -> decide -> accumulate in one persistent cooperative launch (npc_fused5.cuh)
-static int launch_fused(npc_ctx *c, const npc_ctx::TileCfg &t, bool exact, const uint8_t *gt, int64_t row_stride,
-                        const npc_row *d_rows, int64_t n_rows) {
-    if (n_rows == 0) return NPC_OK;
-    int rc = ensure_log(c, n_rows);
-    if (rc) return rc;
-    const int64_t tiles = (n_rows + F5_R - 1) / F5_R;
-    const int gr = exact ? 1 : (int)std::max<int64_t>(1, std::min<int64_t>(t.Gr, tiles / 16));   // >= 16 tiles per row group
-    // the tally words are a double buffer: this launch counts into half h and clears the words of half h ^ 1 the next one uses
-    const int64_t half_words = std::max<int64_t>(c->max_rows, 1), h = c->fcounts_half;
-    FusedParams P;
-    P.gt = gt; P.row_stride = row_stride; P.n = c->n; P.rows = d_rows; P.n_rows = n_rows; P.pol = c->pol;
-    P.sums = c->d_sums; P.counts = c->d_fcounts + h * half_words; P.log = c->d_log + c->log_len; P.nloci = c->d_nloci;
-    P.counts_next = c->d_fcounts + (h ^ 1) * half_words; P.n_zero = c->fcounts_dirty[h ^ 1]; P.trace = c->d_trace;
-    c->fcounts_dirty[h ^ 1] = 0;
-    c->fcounts_dirty[h] = n_rows;
-    c->fcounts_half ^= 1;
-    P.Sr = t.Sr; P.Sc = t.Sc; P.L = t.L; P.A = t.A; P.nc = t.nc; P.slab_stride = t.slab; P.GD = t.GD;
-    P.Gs = t.Gs; P.Gr = gr; P.partials = c->d_partials;
-    P.aux_sleep_ns = (uint32_t)env_int("NPC_TILE_SLEEP", 0);
-    P.decided = nullptr;
-    void *args[] = { &P };
-    NPC_CUDA(c, cudaLaunchCooperativeKernel(tile_kernel(t.K, exact, c->width, t.nc), dim3(t.Gs * gr), dim3((t.nc + 2 + t.A) * 32), args, t.smem, c->stream));
-    c->launches++;
-    // Row groups > 1: a second, wide kernel adds the groups' partial sums in group order.  (Folding this into the tile
-    // kernel -- the last group of a slab to finish adds them -- was measured in round 2: one CTA per slab doing
-    // Gr - 1 dependent L2 reads per sample took 12 us where this kernel takes ~4, launch included.)
-    if (gr > 1) {
-        k_add_partials<<<(unsigned)((c->n + 255) / 256), 256, 0, c->stream>>>(c->d_sums, c->d_partials, c->n, gr - 1);
-        c->launches++;
-        NPC_CUDA(c, cudaGetLastError());
-    }
-    c->log_len += n_rows;
-    return NPC_OK;
-}
-
-// Cohorts too wide for one resident pass: tally + decide over all samples (the two kernels of the generic sequence),
-// then the tile kernel in "decided" mode once per slab of the sample axis -- it decodes and accumulates, the deciders
-// read the rows' contributions from d_rowp.  The slab is read twice (4 B/genotype), the second time at the tile
-// kernel's rate instead of k_accum's.
-static int launch_wide(npc_ctx *c, const npc_ctx::TileCfg &t, bool exact, const uint8_t *gt, int64_t row_stride,
-                       const npc_row *d_rows, int64_t n_rows) {
-    if (n_rows == 0) return NPC_OK;
-    int rc = launch_count(c, gt, row_stride, d_rows, n_rows, c->d_counts);
-    if (rc) return rc;
-    if ((rc = ensure_log(c, n_rows))) return rc;
-    k_decide<<<(unsigned)((n_rows + 127) / 128), 128, 0, c->stream>>>(d_rows, n_rows, c->d_counts, c->pol, c->n, c->d_rowp,
-                                                                      c->d_log + c->log_len, c->d_nloci);
-    c->launches++;
-    NPC_CUDA(c, cudaGetLastError());
-    c->log_len += n_rows;
-    for (int s = 0; s < c->wide_slabs; s++) {
-        const int64_t s0 = (int64_t)s * c->wide_n, ns = std::min<int64_t>(c->wide_n, c->n - s0);
-        if (ns <= 0) break;
-        FusedParams P;
-        memset(&P, 0, sizeof(P));
-        P.gt = gt + s0 * 2; P.row_stride = row_stride; P.n = ns; P.rows = d_rows; P.n_rows = n_rows; P.pol = c->pol;
-        P.sums = c->d_sums + s0; P.counts = c->d_fcounts; P.log = nullptr; P.nloci = c->d_nloci;
-        P.Sr = t.Sr; P.Sc = t.Sc; P.L = t.L; P.A = t.A; P.nc = t.nc; P.slab_stride = t.slab; P.GD = t.GD;
-        P.Gs = t.Gs; P.Gr = 1; P.partials = nullptr;
-        P.aux_sleep_ns = (uint32_t)env_int("NPC_TILE_SLEEP", 0);
-        P.decided = c->d_rowp;
-        void *args[] = { &P };
-        NPC_CUDA(c, cudaLaunchCooperativeKernel(tile_kernel(t.K, exact, c->width, t.nc), dim3(t.Gs), dim3((t.nc + 2 + t.A) * 32), args, t.smem, c->stream));
-        c->launches++;
-    }
-    return NPC_OK;
-}
-
-// FORMAT/DS rows: tally pass (block sums + missing counts), decide, accumulate in row order
-static int launch_dosage(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows) {
-    if (n_rows == 0) return NPC_OK;
-    int rc = ensure_log(c, n_rows);
-    if (rc) return rc;
-    const int64_t n_blocks = std::max<int64_t>((c->n + DS_BLOCK - 1) / DS_BLOCK, 1);
-    if (!c->d_ds_part) NPC_CUDA(c, cudaMalloc(&c->d_ds_part, (size_t)std::max<int64_t>(c->max_rows, 1) * (size_t)n_blocks * sizeof(double)));
-    NPC_CUDA(c, cudaMemsetAsync(c->d_counts, 0, n_rows * sizeof(ull), c->stream));
-    if (c->n) {
-        for (int64_t r0 = 0; r0 < n_rows; r0 += 65535) {
+    if (c->ds) {
+        const int64_t n_blocks = (c->n + DS_BLOCK - 1) / DS_BLOCK;
+        if (!c->d_ds_part) NPC_CUDA(c, cudaMalloc(&c->d_ds_part, (size_t)std::max<int64_t>(c->max_rows, 1) * (size_t)n_blocks * sizeof(double)));
+        for (int64_t r0 = 0; r0 < n_rows; r0 += 65535) {                                        // grid y: at most 65,535 rows
             const int64_t nr = std::min<int64_t>(65535, n_rows - r0);
             k_count_ds<<<dim3((unsigned)((n_blocks + 7) / 8), (unsigned)nr), 256, 0, c->stream>>>(gt, row_stride, d_rows + r0, c->n, n_blocks,
-                                                                                               c->d_ds_part + r0 * n_blocks, c->d_counts + r0);
+                                                                                               c->d_ds_part + r0 * n_blocks, counts + r0);
             c->launches++;
         }
-    }
-    k_decide_ds<<<(unsigned)((n_rows + 127) / 128), 128, 0, c->stream>>>(d_rows, n_rows, c->d_ds_part, c->n ? n_blocks : 0, c->d_counts, c->pol, c->n,
-                                                                        c->d_rowp, c->d_log + c->log_len, c->d_nloci);
-    c->launches++;
-    c->log_len += n_rows;
-    if (c->n) {
-        k_accum_ds<<<(unsigned)((c->n + 255) / 256), 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->d_sums);
+    } else {
+        if (c->bed) {
+            const unsigned slabs = tally_grid_y((c->n + 63) / 64, n_rows, 1024);             // units: chunks of 64 samples
+            k_count_bed<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
+        } else if (c->width == 1 && c->ploidy == 2) {
+            const unsigned slabs = tally_grid_y((c->n + 7) / 8, n_rows, 1024);               // units: chunks of 8 samples
+            k_count_i8x2<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
+        } else {
+            dim3 grid((unsigned)n_rows, tally_grid_y(c->n, n_rows, 2048));                    // units: samples
+            if (c->width == 1) k_count_generic<int8_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->ploidy, counts);
+            else if (c->width == 2) k_count_generic<int16_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->ploidy, counts);
+            else k_count_generic<int32_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->ploidy, counts);
+        }
         c->launches++;
     }
     NPC_CUDA(c, cudaGetLastError());
     return NPC_OK;
 }
 
-// PLINK .bed rows: popc tally, the common decision, table-indexed accumulate (npc_bed.cuh)
-static int launch_bed(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows) {
+// The decision for each of n_rows tallied rows: its contributions to d_rowp, its record appended to the locus log
+static int launch_decide(npc_ctx *c, const npc_row *d_rows, int64_t n_rows, const ull *counts) {
     if (n_rows == 0) return NPC_OK;
     int rc = ensure_log(c, n_rows);
     if (rc) return rc;
-    NPC_CUDA(c, cudaMemsetAsync(c->d_counts, 0, n_rows * 2 * sizeof(ull), c->stream));
-    if (c->n) {
-        const unsigned slabs = tally_grid_y((c->n + 63) / 64, n_rows, 1024);                 // units: chunks of 64 samples
-        k_count_bed<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->d_counts);
-        c->launches++;
-    }
-    k_decide<<<(unsigned)((n_rows + 127) / 128), 128, 0, c->stream>>>(d_rows, n_rows, c->d_counts, c->pol, c->n, c->d_rowp,
-                                                                      c->d_log + c->log_len, c->d_nloci);
+    const unsigned grid = (unsigned)((n_rows + 127) / 128);
+    if (c->ds)
+        k_decide_ds<<<grid, 128, 0, c->stream>>>(d_rows, n_rows, c->d_ds_part, (c->n + DS_BLOCK - 1) / DS_BLOCK, counts, c->pol, c->n,
+                                                c->d_rowp, c->d_log + c->log_len, c->d_nloci);
+    else
+        k_decide<<<grid, 128, 0, c->stream>>>(d_rows, n_rows, counts, c->pol, c->n, c->d_rowp, c->d_log + c->log_len, c->d_nloci);
     c->launches++;
+    NPC_CUDA(c, cudaGetLastError());
     c->log_len += n_rows;
-    if (c->n) {
+    return NPC_OK;
+}
+
+// The decided rows' contributions (d_rowp) added to the sums
+static int launch_accum(npc_ctx *c, const uint8_t *gt, int64_t row_stride, int64_t n_rows) {
+    if (n_rows == 0 || c->n == 0) return NPC_OK;
+    if (c->ds) {
+        k_accum_ds<<<(unsigned)((c->n + 255) / 256), 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->d_sums);
+    } else if (c->bed) {
         const int64_t n_batches = (n_rows + BED_RB - 1) / BED_RB, E = c->exact ? BED_RB * 4 : BED_RB * 8;
         if (!c->d_bed_tab) {
             const int64_t max_batches = (std::max<int64_t>(c->max_rows, 1) + BED_RB - 1) / BED_RB;
@@ -709,22 +612,104 @@ static int launch_bed(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const n
             k_bed_prep<false><<<pgrid, 256, 0, c->stream>>>(c->d_rowp, n_rows, n_batches, c->d_bed_tab, c->d_bed_off);
             k_accum_bed<false><<<grid, BED_THREADS, 0, c->stream>>>(gt, row_stride, c->d_bed_tab, c->d_bed_off, n_rows, c->n, c->d_sums);
         }
-        c->launches += 2;
+        c->launches++;                                                                          // k_bed_prep
+    } else if (c->width == 1 && c->ploidy == 2) {
+        const int64_t nchunks = (c->n + 7) / 8;
+        k_accum_i8x2<64, 8><<<(unsigned)((nchunks + 255) / 256), 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows,
+                                                                                     c->n, c->d_sums);
+    } else {
+        const unsigned grid = (unsigned)((c->n + 255) / 256);
+        if (c->width == 1) k_accum_generic<int8_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
+        else if (c->width == 2) k_accum_generic<int16_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
+        else k_accum_generic<int32_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
     }
+    c->launches++;
     NPC_CUDA(c, cudaGetLastError());
     return NPC_OK;
 }
 
-static int launch_block(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows) {
-    if (c->ds) return launch_dosage(c, gt, row_stride, d_rows, n_rows);
-    if (c->bed) return launch_bed(c, gt, row_stride, d_rows, n_rows);
-    const npc_ctx::TileCfg *t;
-    const int mode = launch_mode(c, c->exact, n_rows, t);
-    if (mode == 1 || mode == 2) return launch_fused(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
-    if (mode == 3) return launch_wide(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
-    int rc = launch_count(c, gt, row_stride, d_rows, n_rows, c->d_counts);
+// The tile kernel's parameters for shape t over every sample and one row group; each mode then sets its own fields
+static FusedParams fused_params(const npc_ctx *c, const npc_ctx::TileCfg &t, const uint8_t *gt, int64_t row_stride,
+                                const npc_row *d_rows, int64_t n_rows) {
+    FusedParams P;
+    memset(&P, 0, sizeof(P));
+    P.gt = gt; P.row_stride = row_stride; P.n = c->n; P.rows = d_rows; P.n_rows = n_rows; P.pol = c->pol;
+    P.sums = c->d_sums; P.nloci = c->d_nloci;
+    P.Sr = t.Sr; P.Sc = t.Sc; P.L = t.L; P.A = t.A; P.nc = t.nc; P.slab_stride = t.slab; P.GD = t.GD;
+    P.Gs = t.Gs; P.Gr = 1;
+    return P;
+}
+
+// One cooperative launch of the tile kernel: P.Gs sample slabs x P.Gr row groups
+static int launch_tile(npc_ctx *c, const npc_ctx::TileCfg &t, bool exact, FusedParams &P) {
+    void *args[] = { &P };
+    NPC_CUDA(c, cudaLaunchCooperativeKernel(tile_kernel(t.K, exact, c->width, t.nc), dim3(P.Gs * P.Gr), dim3((t.nc + 2 + t.A) * 32), args, t.smem, c->stream));
+    c->launches++;
+    return NPC_OK;
+}
+
+// count -> decide -> accumulate in one persistent cooperative launch (npc_fused5.cuh)
+static int launch_fused(npc_ctx *c, const npc_ctx::TileCfg &t, bool exact, const uint8_t *gt, int64_t row_stride,
+                        const npc_row *d_rows, int64_t n_rows) {
+    if (n_rows == 0) return NPC_OK;
+    int rc = ensure_log(c, n_rows);
     if (rc) return rc;
-    return launch_decide_accum(c, gt, row_stride, d_rows, n_rows, c->d_counts);
+    const int64_t tiles = (n_rows + F5_R - 1) / F5_R;
+    FusedParams P = fused_params(c, t, gt, row_stride, d_rows, n_rows);
+    P.Gr = exact ? 1 : (int)std::max<int64_t>(1, std::min<int64_t>(t.Gr, tiles / 16));   // >= 16 tiles per row group
+    P.partials = c->d_partials;
+    // the tally words are a double buffer: this launch counts into half h and clears the words of half h ^ 1 the next one uses
+    const int64_t half_words = std::max<int64_t>(c->max_rows, 1), h = c->fcounts_half;
+    P.counts = c->d_fcounts + h * half_words; P.log = c->d_log + c->log_len; P.trace = c->d_trace;
+    P.counts_next = c->d_fcounts + (h ^ 1) * half_words; P.n_zero = c->fcounts_dirty[h ^ 1];
+    c->fcounts_dirty[h ^ 1] = 0;
+    c->fcounts_dirty[h] = n_rows;
+    c->fcounts_half ^= 1;
+    if ((rc = launch_tile(c, t, exact, P))) return rc;
+    // Row groups > 1: a second, wide kernel adds the groups' partial sums in group order.  (Folding this into the tile
+    // kernel -- the last group of a slab to finish adds them -- was measured in round 2: one CTA per slab doing
+    // Gr - 1 dependent L2 reads per sample took 12 us where this kernel takes ~4, launch included.)
+    if (P.Gr > 1) {
+        k_add_partials<<<(unsigned)((c->n + 255) / 256), 256, 0, c->stream>>>(c->d_sums, c->d_partials, c->n, P.Gr - 1);
+        c->launches++;
+        NPC_CUDA(c, cudaGetLastError());
+    }
+    c->log_len += n_rows;
+    return NPC_OK;
+}
+
+// Cohorts too wide for one resident pass: tally + decide over all samples (the two kernels of the generic sequence),
+// then the tile kernel in "decided" mode once per slab of the sample axis -- it decodes and accumulates, the deciders
+// read the rows' contributions from d_rowp.  The slab is read twice (4 B/genotype), the second time at the tile
+// kernel's rate instead of k_accum's.
+static int launch_wide(npc_ctx *c, const npc_ctx::TileCfg &t, bool exact, const uint8_t *gt, int64_t row_stride,
+                       const npc_row *d_rows, int64_t n_rows) {
+    if (n_rows == 0) return NPC_OK;
+    int rc = launch_tally(c, gt, row_stride, d_rows, n_rows, c->d_counts);
+    if (!rc) rc = launch_decide(c, d_rows, n_rows, c->d_counts);
+    if (rc) return rc;
+    FusedParams P = fused_params(c, t, gt, row_stride, d_rows, n_rows);
+    P.decided = c->d_rowp;
+    for (int s = 0; s < c->wide_slabs; s++) {
+        const int64_t s0 = (int64_t)s * c->wide_n, ns = std::min<int64_t>(c->wide_n, c->n - s0);
+        if (ns <= 0) break;
+        P.gt = gt + s0 * 2; P.n = ns; P.sums = c->d_sums + s0;
+        if ((rc = launch_tile(c, t, exact, P))) return rc;
+    }
+    return NPC_OK;
+}
+
+static int launch_block(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows) {
+    const npc_ctx::TileCfg *t;
+    switch (launch_mode(c, c->exact, n_rows, t)) {
+    case 1: case 2: return launch_fused(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
+    case 3: return launch_wide(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
+    default: {                                                                                  // 0, 4
+        int rc = launch_tally(c, gt, row_stride, d_rows, n_rows, c->d_counts);
+        if (!rc) rc = launch_decide(c, d_rows, n_rows, c->d_counts);
+        return rc ? rc : launch_accum(c, gt, row_stride, n_rows);
+    }
+    }
 }
 
 // ---- staged blocks -----------------------------------------------------------------------
@@ -783,32 +768,33 @@ extern "C" int npc_score_block_device(npc_ctx *ctx, const void *gt_dev, int64_t 
     return launch_block(ctx, (const uint8_t *)gt_dev, row_stride, d_rows, n_rows);
 }
 
+// The split calls' checks and row upload: hard-call rows of the BCF layouts only
+static int split_prologue(npc_ctx *c, const void *gt_dev, int64_t row_stride, int64_t n_gt_rows, const npc_row *rows,
+                          int64_t n_rows, int32_t rows_on_device, const int64_t *counts_dev, const npc_row **d_rows) {
+    int rc = check_block(c, gt_dev, row_stride, n_gt_rows, rows, n_rows);
+    if (rc) return rc;
+    if (!counts_dev) return fail(c, NPC_EINVAL, "counts_dev is NULL");
+    if (c->ds) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take hard-call (GT) rows only");
+    if (c->bed) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not PLINK .bed rows");
+    NPC_CUDA(c, cudaSetDevice(c->device));
+    return upload_rows(c, rows, n_rows, rows_on_device, d_rows);
+}
+
 extern "C" int npc_count_block_device(npc_ctx *ctx, const void *gt_dev, int64_t row_stride, int64_t n_gt_rows,
                                       const npc_row *rows, int64_t n_rows, int32_t rows_on_device,
                                       int64_t *counts_dev) {
-    int rc = check_block(ctx, gt_dev, row_stride, n_gt_rows, rows, n_rows);
-    if (rc) return rc;
-    if (!counts_dev) return fail(ctx, NPC_EINVAL, "counts_dev is NULL");
-    if (ctx->ds) return fail(ctx, NPC_EUNSUPPORTED, "the split count / accumulate calls take hard-call (GT) rows only");
-    if (ctx->bed) return fail(ctx, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not PLINK .bed rows");
-    NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     const npc_row *d_rows;
-    if ((rc = upload_rows(ctx, rows, n_rows, rows_on_device, &d_rows))) return rc;
-    return launch_count(ctx, (const uint8_t *)gt_dev, row_stride, d_rows, n_rows, (ull *)counts_dev);
+    int rc = split_prologue(ctx, gt_dev, row_stride, n_gt_rows, rows, n_rows, rows_on_device, counts_dev, &d_rows);
+    return rc ? rc : launch_tally(ctx, (const uint8_t *)gt_dev, row_stride, d_rows, n_rows, (ull *)counts_dev);
 }
 
 extern "C" int npc_accumulate_block_device(npc_ctx *ctx, const void *gt_dev, int64_t row_stride, int64_t n_gt_rows,
                                            const npc_row *rows, int64_t n_rows, int32_t rows_on_device,
                                            const int64_t *counts_dev) {
-    int rc = check_block(ctx, gt_dev, row_stride, n_gt_rows, rows, n_rows);
-    if (rc) return rc;
-    if (!counts_dev) return fail(ctx, NPC_EINVAL, "counts_dev is NULL");
-    if (ctx->ds) return fail(ctx, NPC_EUNSUPPORTED, "the split count / accumulate calls take hard-call (GT) rows only");
-    if (ctx->bed) return fail(ctx, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not PLINK .bed rows");
-    NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     const npc_row *d_rows;
-    if ((rc = upload_rows(ctx, rows, n_rows, rows_on_device, &d_rows))) return rc;
-    return launch_decide_accum(ctx, (const uint8_t *)gt_dev, row_stride, d_rows, n_rows, (const ull *)counts_dev);
+    int rc = split_prologue(ctx, gt_dev, row_stride, n_gt_rows, rows, n_rows, rows_on_device, counts_dev, &d_rows);
+    if (!rc) rc = launch_decide(ctx, d_rows, n_rows, (const ull *)counts_dev);
+    return rc ? rc : launch_accum(ctx, (const uint8_t *)gt_dev, row_stride, n_rows);
 }
 
 // ---- resident slab ---------------------------------------------------------------------------
@@ -883,12 +869,19 @@ extern "C" int npc_score_resident(npc_ctx *ctx, const npc_row *rows, int64_t n_r
 
 // ---- results -------------------------------------------------------------------------------
 
-static int fetch_log(npc_ctx *c, npc_locus *loci_out, int64_t loci_cap, int64_t *n_loci_out) {
+// sums (n doubles from the device array `sums`), nloci and the locus log to the host; returns when they have landed
+static int copy_out(npc_ctx *c, const double *sums, double *sums_out, int64_t *nloci_out, npc_locus *loci_out, int64_t loci_cap,
+                    int64_t *n_loci_out) {
+    if (c->n) NPC_CUDA(c, cudaMemcpyAsync(sums_out, sums, c->n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    ull nl = 0;
+    NPC_CUDA(c, cudaMemcpyAsync(&nl, c->d_nloci, sizeof(ull), cudaMemcpyDeviceToHost, c->stream));
     if (n_loci_out) *n_loci_out = c->log_len;
     if (loci_out) {
         if (loci_cap < c->log_len) return fail(c, NPC_EINVAL, "loci_out too small");
         NPC_CUDA(c, cudaMemcpyAsync(loci_out, c->d_log, c->log_len * sizeof(npc_locus), cudaMemcpyDeviceToHost, c->stream));
     }
+    NPC_CUDA(c, cudaStreamSynchronize(c->stream));
+    if (nloci_out) *nloci_out = (int64_t)nl;
     return NPC_OK;
 }
 
@@ -900,15 +893,8 @@ extern "C" int npc_finish(npc_ctx *ctx, double offset, double *scores_out, int64
         k_finalize<<<(unsigned)((ctx->n + 255) / 256), 256, 0, ctx->stream>>>(ctx->d_sums, ctx->n, ctx->d_nloci, offset, ctx->d_out);
         ctx->launches++;
         NPC_CUDA(ctx, cudaGetLastError());
-        NPC_CUDA(ctx, cudaMemcpyAsync(scores_out, ctx->d_out, ctx->n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
     }
-    ull nl = 0;
-    NPC_CUDA(ctx, cudaMemcpyAsync(&nl, ctx->d_nloci, sizeof(ull), cudaMemcpyDeviceToHost, ctx->stream));
-    int rc = fetch_log(ctx, loci_out, loci_cap, n_loci_out);
-    if (rc) return rc;
-    NPC_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    if (nloci_out) *nloci_out = (int64_t)nl;
-    return NPC_OK;
+    return copy_out(ctx, ctx->d_out, scores_out, nloci_out, loci_out, loci_cap, n_loci_out);
 }
 
 // ---- several score definitions over the resident slab ------------------------------------------
@@ -1043,7 +1029,7 @@ static int multi_contract(npc_ctx *c, int32_t S, const npc_row *const *rows, con
 
     // ---- tallies once per entry: launched first, so that the pass over the slab (the long pole) runs while the host
     // pushes the row tables of every definition through the copy stream
-    int rc = launch_count(c, c->d_slab, c->slab_stride, d_erows, E, d_ecounts);
+    int rc = launch_tally(c, c->d_slab, c->slab_stride, d_erows, E, d_ecounts);
     if (rc) return rc;
     cudaStream_t cs = c->copy_stream;
     if (!c->ev_multi) NPC_CUDA(c, cudaEventCreateWithFlags(&c->ev_multi, cudaEventDisableTiming));
@@ -1166,15 +1152,7 @@ extern "C" int npc_partial(npc_ctx *ctx, double *sums_out, int64_t *nloci_out, n
                            int64_t *n_loci_out) {
     if (!ctx || !sums_out) return NPC_EINVAL;
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
-    if (ctx->n)
-        NPC_CUDA(ctx, cudaMemcpyAsync(sums_out, ctx->d_sums, ctx->n * sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
-    ull nl = 0;
-    NPC_CUDA(ctx, cudaMemcpyAsync(&nl, ctx->d_nloci, sizeof(ull), cudaMemcpyDeviceToHost, ctx->stream));
-    int rc = fetch_log(ctx, loci_out, loci_cap, n_loci_out);
-    if (rc) return rc;
-    NPC_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-    if (nloci_out) *nloci_out = (int64_t)nl;
-    return NPC_OK;
+    return copy_out(ctx, ctx->d_sums, sums_out, nloci_out, loci_out, loci_cap, n_loci_out);
 }
 
 extern "C" int npc_partial_device_ptr(npc_ctx *ctx, double **sums_dev, int64_t **nloci_dev) {

@@ -25,10 +25,6 @@ struct FusedParams {
     // Group g > 0 accumulates into partials[(g-1)*n ..]; k_add_partials folds them in group order.
     int32_t Gs, Gr;
     double *partials;
-    // wait policy of the auxiliary warps (producer, publisher, deciders): 0 = hardware-suspended try_wait;
-    // > 0 = test, then sleep this many ns.  A suspended try_wait wakes every few dozen cycles and costs
-    // ~4 issue slots per wake-up; four such warps take a quarter of an SM's issue bandwidth.
-    uint32_t aux_sleep_ns;
     // pair kernel: the tally words of the NEXT launch (the other half of a double buffer), cleared by this one so
     // that no memset sits between launches; n_zero words.  nullptr: the caller cleared `counts` itself.
     ull *counts_next;
@@ -70,20 +66,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
         "bra WAIT_%=;\n"
         "DONE_%=:\n"
         "}\n" ::"r"(bar), "r"(parity), "r"(0x989680u) : "memory");   // suspend-time hint: sleep in hardware, do not spin
-}
-// for warps that run far ahead of the work they wait on: poll, sleep `ns`, poll again
-__device__ __forceinline__ void mbar_wait_sleep(uint32_t bar, uint32_t parity, uint32_t ns) {
-    if (ns == 0) { mbar_wait(bar, parity); return; }
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAITS_%=:\n"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONES_%=;\n"
-        "nanosleep.u32 %2;\n"
-        "bra WAITS_%=;\n"
-        "DONES_%=:\n"
-        "}\n" ::"r"(bar), "r"(parity), "r"(ns) : "memory");
 }
 // TMA bulk copy global -> shared, completion counted in bytes on an mbarrier; the slab is read
 // once, so it is marked evict-first in L2.

@@ -216,7 +216,7 @@ k_fused_pair(const FusedParams P) {
                 for (int k = 0; k < K; k++) {                        // one raw stage per chunk set of the tile
                     const uint32_t lo = (uint32_t)k * hslab;
                     const uint32_t bytes = slab_bytes > lo ? min(slab_bytes - lo, hslab) : 0u;
-                    mbar_wait_sleep(bar_rempty + 8u * s, ph ^ 1u, P.aux_sleep_ns);
+                    mbar_wait(bar_rempty + 8u * s, ph ^ 1u);
                     if (mine) { s_reaidx[s * R + (lane % R)] = is_gt ? cur.eaidx : 0; s_rtb[s * R + (lane % R)] = my_tb; }
                     if (lane == 0) s_rflags[s] = gt_mask | (((odd_all >> (R * j)) & ((1u << R) - 1u)) << 4);
                     __syncwarp();
@@ -235,7 +235,7 @@ k_fused_pair(const FusedParams P) {
         // 64-bit RED per row: tallies and arrival count in the same word, so the data is the flag
         int s = 0; uint32_t ph = 0;
         for (int64_t t = 0; t < (P.decided ? 0 : n_tiles); t++) {
-            mbar_wait_sleep(bar_cnt + 8u * s, ph, P.aux_sleep_ns);
+            mbar_wait(bar_cnt + 8u * s, ph);
             const uint32_t base = sb + M.cnt + (uint32_t)s * cnt_slot + (uint32_t)lane * 4u;
             uint32_t d01 = 0, m01 = 0, d23 = 0, m23 = 0;             // 16-bit halves: row a | row b
             for (int g = 0; g < NG; g++) {
@@ -276,7 +276,7 @@ k_fused_pair(const FusedParams P) {
             if (have) row = P.rows[my_row];                          // in flight while we wait
             {   // the grid cannot have arrived before this CTA has: sleep on the local barrier of the group's last tile first
                 const int64_t tl = t0 + ng - 1;
-                mbar_wait_sleep(bar_cnt + 8u * (uint32_t)(tl % Sc), (uint32_t)((tl / Sc) & 1), P.aux_sleep_ns);
+                mbar_wait(bar_cnt + 8u * (uint32_t)(tl % Sc), (uint32_t)((tl / Sc) & 1));
             }
             double v0 = 0.0, v1 = 0.0, v2 = 0.0, v3 = 0.0;           // a dropped row adds +0.0: the identity
             int used = 0;
