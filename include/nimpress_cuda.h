@@ -34,6 +34,16 @@
  *
  * Or, for a context created with gt_width = NPC_GT_BED (ploidy 2), rows of a PLINK 1 `.bed` fileset as stored:
  * 2 bits per sample, low bits first, ceil(n/4) bytes per row (DESIGN.md 4.7, npc_bed.cuh).
+ *
+ * Or, for a context created with gt_width = NPC_GT_DOSE255 (ploidy 2), fixed-point dosage rows as the host makes them
+ * from a BGEN v1.2 file (layout 2, 8-bit probabilities, diploid, biallelic; DESIGN.md 4.8, npc_dose255.cuh): n
+ * little-endian uint16 per row, k = 255 x the expected ALT dosage (unphased: 510 - 2*P(hom allele 1) - P(het);
+ * phased: (255 - h0) + (255 - h1), all in units of 1/255), 0..510; any value above 510 (the host writes 0xFFFF) is a
+ * missing sample.  A row whose effect allele is REF (eaidx 0) uses k' = 510 - k.  Tally: nmiss, and
+ * neff_num = sum of k' over called samples as an exact integer; the reference's real tally is neff = fl(neff_num / 255)
+ * and npc_locus.neff reports neff_num (units of 1/255).  Accumulate: scores[s] += fl(fl(k'/255) * beta) (cm for a
+ * missing sample) in score-row order, the reference's chain, in every mode.  Hard calls (k = 0, 255, 510) therefore
+ * score bit for bit as the same genotypes in int8 GT rows in exact order.
  */
 /*
  * Environment (diagnostics and tests; none is needed in normal use):
@@ -83,7 +93,13 @@ enum { NPC_KIND_GT = 0,      /* record found, FILTER passes: decode its genotype
  * a GT-kind row names eaidx 0 or 1.  The split count / accumulate calls return NPC_EUNSUPPORTED. */
 #define NPC_GT_BED 0
 
-/* Bytes of one genotype row of n samples in a layout (gt_width 1, 2, 4 or NPC_GT_BED). */
+/* gt_width of a context whose rows are fixed-point dosage rows (2 bytes per sample, see above): ploidy must be 2.  Every
+ * npc_score_block* / npc_score_resident call takes such rows (npc_score_resident_multi scores one definition at a time);
+ * a GT-kind row names eaidx 0 (REF) or 1 (the ALT).  npc_set_exact_order changes nothing: the sums always follow the
+ * reference's chain.  The split count / accumulate calls return NPC_EUNSUPPORTED. */
+#define NPC_GT_DOSE255 255
+
+/* Bytes of one genotype row of n samples in a layout (gt_width 1, 2, 4, NPC_GT_BED or NPC_GT_DOSE255). */
 int64_t npc_gt_row_bytes(int64_t n_samples, int32_t ploidy, int32_t gt_width);
 
 typedef struct npc_ctx npc_ctx;
@@ -307,7 +323,8 @@ int npc_set_dosage_rows(npc_ctx *ctx, int32_t on);
  * tile kernel in "decided" mode once per slab of the sample axis), 4 for NPC_GT_BED rows (k_count_bed,
  * k_decide, k_accum_bed; then shape[1] = CTAs of the accumulate pass, shape[2] = warps per CTA,
  * shape[3] = samples per thread, shape[4] = rows per tile: 4 in the default mode, 1 in exact order),
- * 0 for the count/decide/accumulate sequence; then grid (tile kernel: sample slabs * 1000 + row
+ * 5 for NPC_GT_DOSE255 rows (k_count_dose255, k_decide_dose255, k_accum_dose255; then shape[1] = CTAs of the
+ * accumulate pass, shape[2] = warps per CTA, shape[3] = 8 samples per thread), 0 for the count/decide/accumulate sequence; then grid (tile kernel: sample slabs * 1000 + row
  * groups), consumer warps, chunks per thread, rows
  * per tile, raw stages * 1000 + index-ring tiles, lag * 100 + tiles per decider pass * 10 + decider warps, dynamic
  * shared-memory bytes. */

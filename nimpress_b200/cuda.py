@@ -14,6 +14,7 @@ MISSING = {"homref": 0, "ignore": 1}                             # ImputeMethodM
 SAMPLE = {"ps": 0, "homref": 1, "fail": 2, "int_ps": 3, "int_fail": 4}   # ImputeMethodSample (:414)
 KIND_GT, KIND_NOTCOV, KIND_ABSENT, KIND_FILTER, CLASS_MAXMIS = range(5)
 GT_BED = 0        # gt_width of a context over PLINK 1 .bed rows (2 bits per sample, ploidy 2): NPC_GT_BED
+GT_DOSE255 = 255  # gt_width of a context over fixed-point dosage rows of BGEN files (uint16 255 x dosage, ploidy 2): NPC_GT_DOSE255
 
 
 def gt_row_bytes(n_samples, ploidy, gt_width):

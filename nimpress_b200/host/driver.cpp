@@ -138,7 +138,9 @@ struct SlabOverflow {};                            // several score files, and t
 struct NoIndex {};                                 // the index-driven pass is not possible / not worthwhile: stream the file
 
 // WARN lines of one score file, in the reference's order (:326, :527-530, :538-541, :554-557, :567-570, :575-579)
-std::string make_warnings(const ScoreFile &score, const Matcher &M, const std::vector<npc_locus> &loci, int64_t n, const ScoreParams &p) {
+// real_tally: dosage rows (FORMAT/DS, BGEN), whose effect-allele tally is not an integer allele count
+std::string make_warnings(const ScoreFile &score, const Matcher &M, const std::vector<npc_locus> &loci, int64_t n, const ScoreParams &p,
+                          bool real_tally) {
     std::string w;
     const std::vector<ScoreEntry> &E = score.entries;
     for (int64_t i = 0; i < (int64_t)E.size(); i++) {
@@ -159,7 +161,7 @@ std::string make_warnings(const ScoreFile &score, const Matcher &M, const std::v
             const double missingrate = (double)L.nmiss / (double)n;
             w += "WARN Locus " + span + " has " + format_float_nim(missingrate * 100) +
                  "% of samples missing a genotype. This exceeds the missingness threshold; imputing all dosages at this locus.\n";
-        } else if (p.use_ds) {
+        } else if (real_tally) {
             // dosage rows: the tally is a real number, the reference's exact binomial test is not defined on it
         } else if (!std::isnan(e.eaf) && binom_test(L.neff, (n - L.nmiss) * 2, e.eaf) < p.afmisp) {
             w += "WARN Variant " + id + " cohort EAF is " + format_float_nim((double)L.neff / (double)((n - L.nmiss) * 2)) + " in " +
@@ -240,6 +242,12 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
         std::string err;
     };
     std::vector<Dev> devs(D);
+    // rows still being converted by the source's workers land in the devices' pinned slots: let them finish before the
+    // slots go, whichever way this pass ends
+    struct RowsGuard {
+        VariantSource &v;
+        ~RowsGuard() { try { v.wait_rows(); } catch (...) {} }
+    } rows_guard{ vcf };
     npc_policy pol = { p.imp_locus, p.imp_missing, p.imp_sample, 0, p.mincs, p.maxmis };
     auto open_dev = [&](int d) {
         Dev &v = devs[d];
@@ -276,6 +284,7 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
 
     auto flush_stage = [&](Dev &v) {
         if (v.slot < 0) return;
+        vcf.wait_rows();
         v.ctx.ck(npc_stage_upload(v.ctx.h, v.slot, v.staged, v.slab_base), "npc_stage_upload");
         v.slab_base += v.staged; v.staged = 0; v.slot = -1;
     };
@@ -346,7 +355,10 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
                 v.stage = (uint8_t *)ptr; v.staged = 0;
             }
             uint8_t *dst = v.stage + v.staged * v.stride;
-            if (first) memcpy(dst, first, (size_t)npc_gt_row_bytes(n, ploidy, gt_width));   // a record named by two ranges: same bytes
+            if (first) {                                            // a record named by two ranges: same bytes
+                vcf.wait_rows();
+                memcpy(dst, first, (size_t)npc_gt_row_bytes(n, ploidy, gt_width));
+            }
             else {
                 // BCF with the context's layout: the GT payload goes from the inflated blocks straight into the pinned row
                 const bool direct = vcf.load_gt_into(rec, dst, gt_width, ploidy);
@@ -457,7 +469,7 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
     for (int k = 0; k < S; k++) {
         outs[k].loci.assign(scores[k]->entries.size(), npc_locus());
         for (size_t j = 0; j < order[k].size(); j++) outs[k].loci[order[k][j]] = logs[k][j];
-        outs[k].warnings = make_warnings(*scores[k], *ps[k].M, outs[k].loci, n, p);
+        outs[k].warnings = make_warnings(*scores[k], *ps[k].M, outs[k].loci, n, p, p.use_ds || gt_width == NPC_GT_DOSE255);
     }
     timer.mark("WARN lines (binomial tests)");
 }
@@ -473,13 +485,17 @@ bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores
     for (int attempt = 0; attempt < 6; attempt++) {
         std::unique_ptr<VariantSource> vcf = open_variant_source(genotype_path, seekable);
         if (!vcf) return false;
-        if (vcf->plink_rows()) {                    // PLINK fileset: its 2-bit rows as stored, read by offset (no index pass)
-            if (p.use_ds) throw InputError("--dosage: a PLINK fileset holds hard calls only, no FORMAT/DS");
-            width = NPC_GT_BED; ploidy = 2; seekable = false;
+        // PLINK fileset, BGEN file: rows in a layout of their own, read by offset (no index pass)
+        const int fixed = vcf->fixed_layout();
+        ScoreParams q = p;
+        if (fixed == NPC_GT_BED && p.use_ds) throw InputError("--dosage: a PLINK fileset holds hard calls only, no FORMAT/DS");
+        if (fixed != VariantSource::NO_FIXED_LAYOUT) {
+            width = fixed; ploidy = 2; seekable = false;
+            q.use_ds = false;                       // BGEN rows are dosages already: --dosage changes nothing
         }
-        vcf->set_dosage_mode(p.use_ds);
+        vcf->set_dosage_mode(q.use_ds);
         try {
-            run_pass(scores, *vcf, genotype_path, seekable, cov, p, width, ploidy, outs);
+            run_pass(scores, *vcf, genotype_path, seekable, cov, q, width, ploidy, outs);
             return true;
         } catch (const NoIndex &) {
             seekable = false;

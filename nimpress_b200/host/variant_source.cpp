@@ -12,6 +12,7 @@
 #include <climits>
 #include <condition_variable>
 #include <cstring>
+#include <deque>
 #include <map>
 #include <mutex>
 #include <thread>
@@ -906,7 +907,7 @@ public:
                              std::to_string(lines_.size()) + " variants x " + std::to_string(samples_.size()) + " samples need " + std::to_string(want));
         return true;
     }
-    bool plink_rows() const override { return true; }
+    int fixed_layout() const override { return NPC_GT_BED; }
     void load_gt(VariantRecord &rec) override {
         buf_.resize((size_t)std::max<int64_t>(row_bytes_, 1));
         read_row(buf_.data());
@@ -950,6 +951,288 @@ private:
     std::vector<uint8_t> buf_;
     int64_t cur_ = -1, row_bytes_ = 0;
     int fd_ = -1;
+};
+
+// ------------------------------------------------------------------------------------------
+// BGEN v1.2, layout 2, 8-bit probabilities (DESIGN.md 4.8) -- not a reference input
+// ------------------------------------------------------------------------------------------
+
+// One genotype block -> one row of fixed-point dosages (NPC_GT_DOSE255): per sample k = 255 x the expected ALT dosage as
+// a little-endian uint16, 0xFFFF for a missing sample.  Each thread that converts blocks has one of these: its own file
+// descriptor, inflate tables and buffers.
+class BgenBlockReader {
+public:
+    BgenBlockReader(const std::string &path, int64_t n, bool compressed) : n_(n), compressed_(compressed) {
+        fd_ = ::open(path.c_str(), O_RDONLY);
+        if (fd_ < 0) throw InputError("BGEN " + path + ": cannot reopen the file");
+    }
+    ~BgenBlockReader() { if (fd_ >= 0) ::close(fd_); }
+    BgenBlockReader(const BgenBlockReader &) = delete;
+    BgenBlockReader &operator=(const BgenBlockReader &) = delete;
+    // off / C: file offset and length of the genotype block after its C field; what: the variant, for messages
+    void convert(int64_t off, uint32_t C, uint8_t *dst, const std::string &what) {
+        in_.resize((size_t)C + 16);
+        int64_t got = 0;
+        while (got < (int64_t)C) {
+            const ssize_t r = pread(fd_, in_.data() + got, (size_t)(C - got), (off_t)(off + got));
+            if (r <= 0) throw InputError("BGEN: read failed in the genotype block of " + what);
+            got += r;
+        }
+        const uint8_t *p = in_.data();
+        size_t len = C;
+        if (compressed_) {
+            if (C < 4) throw InputError("BGEN: genotype block of " + what + " is too short");
+            uint32_t D;
+            memcpy(&D, in_.data(), 4);
+            out_.resize((size_t)D + 16);
+            // a zlib stream: 2-byte header, raw deflate, Adler-32.  This engine's decoder first, zlib where it does not finish.
+            const uint8_t *z = in_.data() + 4;
+            const size_t zl = C - 4;
+            bool ok = zl >= 6 && (z[0] & 0x0F) == 8 && !(z[1] & 0x20) && fast_inflate(z + 2, zl - 6, out_.data(), D, tabs_);
+            if (ok) {
+                const uint32_t want = (uint32_t)z[zl - 4] << 24 | (uint32_t)z[zl - 3] << 16 | (uint32_t)z[zl - 2] << 8 | z[zl - 1];
+                ok = (uint32_t)adler32(1L, out_.data(), D) == want;
+            }
+            if (!ok) {
+                uLongf dl = D;
+                if (uncompress(out_.data(), &dl, z, (uLong)zl) != Z_OK || dl != D)
+                    throw InputError("BGEN: corrupt compressed genotype block of " + what);
+            }
+            p = out_.data(); len = D;
+        }
+        decode(p, len, dst, what);
+    }
+private:
+    void decode(const uint8_t *p, size_t len, uint8_t *dst, const std::string &what) const {
+        auto bad = [&](const std::string &m) { return InputError("BGEN: variant " + what + ": " + m); };
+        if (len < 8) throw bad("genotype block too short");
+        uint32_t N; uint16_t K;
+        memcpy(&N, p, 4); memcpy(&K, p + 4, 2);
+        const int pmin = p[6], pmax = p[7];
+        if ((int64_t)N != n_) throw bad("genotype block holds " + std::to_string(N) + " samples, the header " + std::to_string(n_));
+        if (K != 2) throw bad(std::to_string(K) + " alleles (only biallelic variants are supported)");
+        if (pmin != 2 || pmax != 2) throw bad("ploidy " + std::to_string(pmin) + ".." + std::to_string(pmax) + " (only diploid samples are supported)");
+        if (len < 8 + (size_t)n_ + 2) throw bad("genotype block too short");
+        const uint8_t *ploidy = p + 8, *q = p + 8 + n_;
+        const bool phased = q[0] != 0;
+        const int B = q[1];
+        if (B != 8) throw bad(std::to_string(B) + " bits per probability (only 8 are supported)");
+        if (len < 8 + (size_t)n_ + 2 + 2 * (size_t)n_) throw bad("genotype block too short");
+        const uint8_t *pr = q + 2;
+        for (int64_t i = 0; i < n_; i++) {
+            const uint32_t a = pr[2 * i], b = pr[2 * i + 1];
+            uint32_t k;
+            if (ploidy[i] & 0x80) k = 0xFFFF;
+            else if (phased) k = 510 - a - b;                             // (255 - h0) + (255 - h1)
+            else {
+                if (a + b > 255) throw bad("sample " + std::to_string(i) + ": P(hom allele 1) + P(het) > 1");
+                k = 510 - 2 * a - b;                                      // P(het) + 2 P(hom allele 2), in 1/255
+            }
+            const uint16_t v = (uint16_t)k;
+            memcpy(dst + 2 * i, &v, 2);
+        }
+    }
+    int fd_ = -1;
+    int64_t n_;
+    bool compressed_;
+    std::vector<uint8_t> in_, out_;
+    FastInflateTables tabs_;
+};
+
+// The header and sample identifiers are read at open; next() walks the variant headers and skips each genotype block by
+// its length (there is no index: a .bgi is an SQLite file).  A block is read and converted only when a score row matched
+// its variant (load_gt / load_gt_into).  load_gt_into hands the block to a pool of NIMPRESS_THREADS workers and returns;
+// wait_rows() waits for every block posted so far.  Per variant: CHROM = chromosome (compared literally), POS, REF =
+// allele 1, ALT = allele 2 (and any further alleles), rlen = len(REF), FILTER ".".
+class BgenSource : public VariantSource {
+public:
+    ~BgenSource() override {
+        {
+            std::lock_guard<std::mutex> g(mu_);
+            stop_ = true;
+        }
+        cv_.notify_all();
+        for (auto &t : workers_) t.join();
+        if (fp_) fclose(fp_);
+    }
+    // false: the file cannot be read, or the .sample it needs cannot be opened.  Throws InputError on a malformed file.
+    bool open(const std::string &path) {
+        path_ = path;
+        fp_ = fopen(path.c_str(), "rb");
+        if (!fp_) return false;
+        fseeko(fp_, 0, SEEK_END);
+        size_ = (int64_t)ftello(fp_);
+        fseeko(fp_, 0, SEEK_SET);
+        const std::string where = "BGEN " + path;
+        uint32_t offset, LH, M, N, flags;
+        if (!rd(&offset, 4) || !rd(&LH, 4) || !rd(&M, 4) || !rd(&N, 4)) throw InputError(where + ": truncated header");
+        if (LH < 20) throw InputError(where + ": header length " + std::to_string(LH) + " < 20");
+        if (offset < LH) throw InputError(where + ": variant data offset " + std::to_string(offset) + " lies inside the header block");
+        if ((int64_t)LH + 4 > size_ || fseeko(fp_, (off_t)LH, SEEK_SET) != 0 || !rd(&flags, 4)) throw InputError(where + ": truncated header");
+        const int comp = flags & 3, layout = (flags >> 2) & 15;
+        if (comp == 2) throw InputError(where + ": zstd-compressed genotype blocks are not supported");
+        if (comp == 3) throw InputError(where + ": unknown compression " + std::to_string(comp));
+        if (layout != 2) throw InputError(where + ": layout " + std::to_string(layout) + " is not supported (layout 2 only)");
+        compressed_ = comp == 1;
+        n_ = N; m_ = M;
+        if (flags & 0x80000000u) {                                        // sample identifier block
+            uint32_t LSI, NS;
+            if (!rd(&LSI, 4) || !rd(&NS, 4)) throw InputError(where + ": truncated sample identifier block");
+            if (NS != N) throw InputError(where + ": " + std::to_string(NS) + " sample identifiers for " + std::to_string(N) + " samples");
+            for (uint32_t i = 0; i < N; i++) samples_.push_back(str16(where + ": truncated sample identifier block"));
+        } else {
+            const std::string stem = path.size() > 5 && path.compare(path.size() - 5, 5, ".bgen") == 0 ? path.substr(0, path.size() - 5) : path;
+            FILE *sf = fopen((stem + ".sample").c_str(), "rb");
+            if (!sf) return false;
+            std::string line;
+            int64_t ln = 0;
+            for (;;) {
+                line.clear();
+                int ch;
+                while ((ch = fgetc(sf)) != EOF && ch != '\n') line += (char)ch;
+                if (ch == EOF && line.empty()) break;
+                if (++ln <= 2) continue;                                 // header line, type line
+                size_t i = 0;
+                std::string cols[2];
+                for (int c = 0; c < 2; c++) {
+                    while (i < line.size() && isspace((unsigned char)line[i])) i++;
+                    const size_t j0 = i;
+                    while (i < line.size() && !isspace((unsigned char)line[i])) i++;
+                    cols[c] = line.substr(j0, i - j0);
+                }
+                if (cols[0].empty() && cols[1].empty()) continue;
+                if (cols[1].empty()) { fclose(sf); throw InputError(where + ": .sample line " + std::to_string(ln) + " has fewer than 2 columns"); }
+                samples_.push_back(cols[1]);                             // ID_2
+            }
+            fclose(sf);
+            if ((int64_t)samples_.size() != (int64_t)N)
+                throw InputError(where + ": the .sample file names " + std::to_string(samples_.size()) + " samples, the header " + std::to_string(N));
+        }
+        pos_ = 4 + (int64_t)offset;
+        if (pos_ > size_ || fseeko(fp_, (off_t)pos_, SEEK_SET) != 0) throw InputError(where + ": truncated before the first variant");
+        const unsigned hc = std::max(1u, std::thread::hardware_concurrency());
+        threads_ = (int)std::min<unsigned>(hc > 2 ? hc - 1 : hc, 32u);
+        if (const char *e = getenv("NIMPRESS_THREADS")) if (*e) threads_ = std::max(1, atoi(e));
+        return true;
+    }
+    int fixed_layout() const override { return NPC_GT_DOSE255; }
+    void load_gt(VariantRecord &rec) override {
+        buf_.resize((size_t)std::max<int64_t>(2 * n_, 1));
+        inline_reader().convert(blk_off_, blk_len_, buf_.data(), what_);
+        fill(rec, buf_.data());
+    }
+    bool load_gt_into(VariantRecord &rec, uint8_t *dst, int want_width, int want_ploidy) override {
+        if (want_width != NPC_GT_DOSE255 || want_ploidy != 2) { load_gt(rec); return false; }
+        if (threads_ <= 1) inline_reader().convert(blk_off_, blk_len_, dst, what_);
+        else {
+            std::lock_guard<std::mutex> g(mu_);
+            if (workers_.empty())
+                for (int t = 0; t < threads_; t++) workers_.emplace_back([this] { work(); });
+            jobs_.push_back(Job{ blk_off_, blk_len_, dst, what_ });
+            pending_++;
+            cv_.notify_one();
+        }
+        fill(rec, dst);
+        return true;
+    }
+    void wait_rows() override {
+        std::unique_lock<std::mutex> lk(mu_);
+        done_.wait(lk, [this] { return pending_ == 0; });
+        if (!err_.empty()) { std::string e; e.swap(err_); throw InputError(e); }
+    }
+protected:
+    bool next_raw(VariantRecord &rec) override {
+        if (read_ >= m_) return false;
+        const std::string where = "BGEN " + path_ + ": variant block " + std::to_string(read_ + 1) + " of " + std::to_string(m_);
+        const std::string trunc = where + " is truncated";
+        id_ = str16(trunc);
+        str16(trunc);                                                     // rsid
+        std::string chrom = str16(trunc);
+        uint32_t pos; uint16_t K;
+        if (!rd(&pos, 4) || !rd(&K, 2)) throw InputError(trunc);
+        rec.alts.clear();
+        rec.ref.clear();
+        for (uint16_t a = 0; a < K; a++) {
+            uint32_t L;
+            if (!rd(&L, 4) || pos_ + (int64_t)L > size_) throw InputError(trunc);
+            std::string s(L, '\0');
+            if (L && !rd(&s[0], L)) throw InputError(trunc);
+            if (a == 0) rec.ref = std::move(s); else rec.alts.push_back(std::move(s));
+        }
+        uint32_t C;
+        if (!rd(&C, 4)) throw InputError(trunc);
+        blk_off_ = pos_; blk_len_ = C;
+        if (pos_ + (int64_t)C > size_ || fseeko(fp_, (off_t)(pos_ + C), SEEK_SET) != 0) throw InputError(trunc);
+        pos_ += C;
+        read_++;
+        auto it = ids_.find(chrom);
+        if (it == ids_.end()) { it = ids_.emplace(chrom, (int32_t)contigs_.size()).first; contigs_.push_back(chrom); }
+        rec.contig_id = it->second; rec.contig = &contigs_[(size_t)it->second];
+        rec.pos = pos; rec.rlen = (int64_t)rec.ref.size(); rec.filter = ".";
+        rec.has_gt = true; rec.gt = nullptr; rec.gt_width = NPC_GT_DOSE255; rec.ploidy = 2;
+        what_ = chrom + ":" + std::to_string(pos) + " (" + id_ + ")";
+        return true;
+    }
+    InflateStream *stream() override { return nullptr; }               // no index-driven mode: use_regions returns false
+    int contig_rank(const VariantRecord &rec) const override { return rec.contig_id; }
+    int contig_rank(const std::string &) const override { return -1; }
+private:
+    struct Job { int64_t off; uint32_t len; uint8_t *dst; std::string what; };
+    bool rd(void *dst, size_t n) {
+        if (fread(dst, 1, n, fp_) != n) return false;
+        pos_ += (int64_t)n;
+        return true;
+    }
+    std::string str16(const std::string &err) {
+        uint16_t L;
+        if (!rd(&L, 2)) throw InputError(err);
+        std::string s(L, '\0');
+        if (L && !rd(&s[0], L)) throw InputError(err);
+        return s;
+    }
+    BgenBlockReader &inline_reader() {
+        if (!inline_) inline_ = std::make_unique<BgenBlockReader>(path_, n_, compressed_);
+        return *inline_;
+    }
+    void fill(VariantRecord &rec, const uint8_t *row) const { rec.has_gt = true; rec.gt = row; rec.gt_width = NPC_GT_DOSE255; rec.ploidy = 2; }
+    void work() {
+        std::unique_ptr<BgenBlockReader> r;
+        for (;;) {
+            Job j;
+            {
+                std::unique_lock<std::mutex> lk(mu_);
+                cv_.wait(lk, [this] { return stop_ || !jobs_.empty(); });
+                if (jobs_.empty()) return;
+                j = std::move(jobs_.front());
+                jobs_.pop_front();
+            }
+            std::string e;
+            try {
+                if (!r) r = std::make_unique<BgenBlockReader>(path_, n_, compressed_);
+                r->convert(j.off, j.len, j.dst, j.what);
+            } catch (const InputError &x) { e = x.what(); }
+            std::lock_guard<std::mutex> g(mu_);
+            if (!e.empty() && err_.empty()) err_ = e;
+            if (--pending_ == 0) done_.notify_all();
+        }
+    }
+    std::string path_, id_, what_;
+    FILE *fp_ = nullptr;
+    int64_t size_ = 0, pos_ = 0, n_ = 0, m_ = 0, read_ = 0, blk_off_ = 0;
+    uint32_t blk_len_ = 0;
+    bool compressed_ = false;
+    std::vector<std::string> contigs_;
+    std::unordered_map<std::string, int32_t> ids_;
+    std::vector<uint8_t> buf_;
+    std::unique_ptr<BgenBlockReader> inline_;
+    int threads_ = 1;
+    std::mutex mu_;
+    std::condition_variable cv_, done_;
+    std::deque<Job> jobs_;
+    int64_t pending_ = 0;
+    bool stop_ = false;
+    std::string err_;
+    std::vector<std::thread> workers_;
 };
 
 // ------------------------------------------------------------------------------------------
@@ -1046,15 +1329,21 @@ bool VariantSource::next(VariantRecord &rec) {
 }
 
 std::unique_ptr<VariantSource> open_variant_source(const std::string &path, bool seekable) {
-    {   // a PLINK 1 .bed is recognised by its magic bytes 6c 1b, then the mode byte (not by the file name)
-        uint8_t m[3] = { 0, 0, 0 };
+    {   // a PLINK 1 .bed is recognised by its magic bytes 6c 1b, then the mode byte, a BGEN file by "bgen" at bytes 16-19
+        // (not by the file name)
+        uint8_t m[20] = { 0 };
         FILE *f = fopen(path.c_str(), "rb");
         if (!f) return nullptr;
-        const size_t got = fread(m, 1, 3, f);
+        const size_t got = fread(m, 1, 20, f);
         fclose(f);
-        if (got == 3 && m[0] == 0x6c && m[1] == 0x1b) {
+        if (got >= 3 && m[0] == 0x6c && m[1] == 0x1b) {
             auto src = std::make_unique<PlinkSource>();
             if (!src->open(path, m[2])) return nullptr;
+            return src;
+        }
+        if (got == 20 && !memcmp(m + 16, "bgen", 4)) {
+            auto src = std::make_unique<BgenSource>();
+            if (!src->open(path)) return nullptr;
             return src;
         }
     }

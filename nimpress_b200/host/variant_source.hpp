@@ -101,8 +101,14 @@ public:
     // FORMAT/DS instead of FORMAT/GT (not a reference feature: README.md:162-165 lists dosage input under "Future"):
     // load_gt / load_gt_into then deliver one BCF float per value, gt_width = 4, ploidy = values per sample.
     virtual void set_dosage_mode(bool on) { dosage_ = on; }
-    // true for a PLINK 1 fileset: load_gt delivers .bed rows (gt_width NPC_GT_BED = 0, ploidy 2, ceil(n/4) bytes)
-    virtual bool plink_rows() const { return false; }
+    // The one device layout this source's rows come in, or NO_FIXED_LAYOUT for VCF / BCF (whose layout follows the records):
+    // NPC_GT_BED for a PLINK 1 fileset (.bed rows as stored, ploidy 2, ceil(n/4) bytes), NPC_GT_DOSE255 for a BGEN file
+    // (one uint16 dosage numerator per sample, ploidy 2).
+    static constexpr int NO_FIXED_LAYOUT = -1;
+    virtual int fixed_layout() const { return NO_FIXED_LAYOUT; }
+    // Rows that load_gt_into handed to worker threads are complete once this returns; a worker's InputError is rethrown
+    // here.  Call before the rows' bytes are read.
+    virtual void wait_rows() {}
     bool dosage_mode() const { return dosage_; }
     const std::vector<std::string> &samples() const { return samples_; }
     int64_t n_samples() const { return (int64_t)samples_.size(); }
@@ -124,8 +130,9 @@ private:
     int64_t seeks_ = 0;
 };
 
-// nullptr: the file cannot be opened or is neither VCF, BCF nor a PLINK 1 .bed (the reference: open() == false); for a .bed
-// also when its .bim or .fam sibling cannot be opened.  A malformed fileset throws InputError (see PlinkSource).
+// nullptr: the file cannot be opened or is neither VCF, BCF, a PLINK 1 .bed nor a BGEN file (the reference: open() == false);
+// for a .bed also when its .bim or .fam sibling cannot be opened, for a BGEN file without sample identifiers when its
+// .sample cannot be opened.  A malformed fileset or BGEN header throws InputError (see PlinkSource, BgenSource).
 // seekable: read BGZF block by block with one zlib stream so that VariantSource::use_regions can jump (no inflate pool).
 std::unique_ptr<VariantSource> open_variant_source(const std::string &path, bool seekable = false);
 
