@@ -44,6 +44,18 @@
  * and npc_locus.neff reports neff_num (units of 1/255).  Accumulate: scores[s] += fl(fl(k'/255) * beta) (cm for a
  * missing sample) in score-row order, the reference's chain, in every mode.  Hard calls (k = 0, 255, 510) therefore
  * score bit for bit as the same genotypes in int8 GT rows in exact order.
+ *
+ * Or, for a context created with gt_width = NPC_GT_DOSE32 (ploidy 2), 32-bit fixed-point dosage rows as the host makes
+ * them from a BGEN v1.2 file at any bit depth B from 1 to 16, haploid and diploid samples (DESIGN.md 4.9,
+ * npc_dose32.cuh): a 16-byte row header, uint32 D = 2^B - 1 then 12 zero bytes, then n little-endian uint32 words, one
+ * per sample: bits 0-23 k = D x the expected ALT dosage, bits 24-25 the ploidy p (1 or 2), bit 31 missing (the host
+ * writes 0xFFFFFFFF).  A sample is called when bit 31 is clear, p is 1 or 2 and k <= p*D; every other word is a missing
+ * sample.  The host writes unphased diploid: 2D - 2*b0 - b1; phased diploid: (D - h0) + (D - h1); haploid: D - b0.  A
+ * row whose effect allele is REF (eaidx 0) uses k' = p*D - k.  Tally: nmiss, and neff_num = sum of k' over called
+ * samples as an exact integer; neff = fl(neff_num / D) and npc_locus.neff reports neff_num (units of 1/D of that row).
+ * Accumulate: scores[s] += fl(fl(k'/D) * beta) (cm for a missing sample) in score-row order, the reference's chain, in
+ * every mode.  With D = 255 and diploid samples a row scores bit for bit as the same NPC_GT_DOSE255 row; hard calls
+ * (k' = 0, D, 2D) score bit for bit as the same genotypes in int8 GT rows in exact order, haploid samples included.
  */
 /*
  * Environment (diagnostics and tests; none is needed in normal use):
@@ -99,7 +111,11 @@ enum { NPC_KIND_GT = 0,      /* record found, FILTER passes: decode its genotype
  * reference's chain.  The split count / accumulate calls return NPC_EUNSUPPORTED. */
 #define NPC_GT_DOSE255 255
 
-/* Bytes of one genotype row of n samples in a layout (gt_width 1, 2, 4, NPC_GT_BED or NPC_GT_DOSE255). */
+/* gt_width of a context whose rows are 32-bit fixed-point dosage rows (a 16-byte header, then 4 bytes per sample, see
+ * above): ploidy must be 2.  Calls, effect alleles, exact order and the split calls as for NPC_GT_DOSE255. */
+#define NPC_GT_DOSE32 32
+
+/* Bytes of one genotype row of n samples in a layout (gt_width 1, 2, 4, NPC_GT_BED, NPC_GT_DOSE255 or NPC_GT_DOSE32). */
 int64_t npc_gt_row_bytes(int64_t n_samples, int32_t ploidy, int32_t gt_width);
 
 typedef struct npc_ctx npc_ctx;
@@ -324,7 +340,8 @@ int npc_set_dosage_rows(npc_ctx *ctx, int32_t on);
  * k_decide, k_accum_bed; then shape[1] = CTAs of the accumulate pass, shape[2] = warps per CTA,
  * shape[3] = samples per thread, shape[4] = rows per tile: 4 in the default mode, 1 in exact order),
  * 5 for NPC_GT_DOSE255 rows (k_count_dose255, k_decide_dose255, k_accum_dose255; then shape[1] = CTAs of the
- * accumulate pass, shape[2] = warps per CTA, shape[3] = 8 samples per thread), 0 for the count/decide/accumulate sequence; then grid (tile kernel: sample slabs * 1000 + row
+ * accumulate pass, shape[2] = warps per CTA, shape[3] = 8 samples per thread), 6 for NPC_GT_DOSE32 rows (k_count_dose32,
+ * k_decide_dose32, k_accum_dose32; shape[1..3] as for 5, with 4 samples per thread), 0 for the count/decide/accumulate sequence; then grid (tile kernel: sample slabs * 1000 + row
  * groups), consumer warps, chunks per thread, rows
  * per tile, raw stages * 1000 + index-ring tiles, lag * 100 + tiles per decider pass * 10 + decider warps, dynamic
  * shared-memory bytes. */

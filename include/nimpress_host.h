@@ -24,6 +24,8 @@
  *   NIMPRESS_TIMING=1        phase wall times on stderr
  *   NIMPRESS_SLAB_ROWS=<n>   cap the device-resident genotype rows (tests: forces scoring in rounds)
  *   NIMPRESS_SPLIT=<k>       with one device: k contexts on it, combined by npc_reduce (tests of the multi-GPU path on one GPU)
+ *   NIMPRESS_READ_DOSE32=1   nph_read_gt on a BGEN file: every block as a 32-bit dosage row (NPC_GT_DOSE32) instead of a
+ *                            2-byte one (NPC_GT_DOSE255, which refuses other bit depths and haploid samples)
  */
 #ifndef NIMPRESS_HOST_H
 #define NIMPRESS_HOST_H

@@ -17,6 +17,7 @@
 #include "npc_dosage.cuh"
 #include "npc_bed.cuh"
 #include "npc_dose255.cuh"
+#include "npc_dose32.cuh"
 
 using namespace npc;
 
@@ -84,6 +85,9 @@ struct npc_ctx {
     int32_t *d_bed_off = nullptr;           // ... and the slab row of every row it loads
     // fixed-point dosage rows from BGEN files (npc_dose255.cuh, gt_width = NPC_GT_DOSE255): uint16 per sample
     bool dose255 = false;
+    // 32-bit fixed-point dosage rows from BGEN files at any bit depth (npc_dose32.cuh, gt_width = NPC_GT_DOSE32): a 16-byte
+    // header holding the row's denominator, then uint32 per sample
+    bool dose32 = false;
     // cross-GPU combine (npc_reduce.cuh)
     cudaEvent_t ev_multi = nullptr;         // npc_score_resident_multi: orders its copy-stream work against the compute stream
     cudaEvent_t ev_reduce = nullptr;        // "this context's partial sums are final"
@@ -116,6 +120,7 @@ extern "C" int npc_version(void) { return 200; }
 extern "C" int64_t npc_gt_row_bytes(int64_t n_samples, int32_t ploidy, int32_t gt_width) {
     if (gt_width == NPC_GT_BED) return (n_samples + 3) / 4;
     if (gt_width == NPC_GT_DOSE255) return n_samples * 2;
+    if (gt_width == NPC_GT_DOSE32) return D32_HEADER + n_samples * 4;
     return n_samples * ploidy * gt_width;
 }
 
@@ -358,15 +363,16 @@ extern "C" int npc_create2(npc_ctx **out, int device, int64_t n_samples, int32_t
     if (!out) return NPC_EINVAL;
     *out = nullptr;
     if (n_samples < 0 || ploidy < 1 || ploidy > 64 ||
-        (gt_width != 1 && gt_width != 2 && gt_width != 4 && gt_width != NPC_GT_BED && gt_width != NPC_GT_DOSE255) ||
-        ((gt_width == NPC_GT_BED || gt_width == NPC_GT_DOSE255) && ploidy != 2) ||
+        (gt_width != 1 && gt_width != 2 && gt_width != 4 && gt_width != NPC_GT_BED && gt_width != NPC_GT_DOSE255 &&
+         gt_width != NPC_GT_DOSE32) ||
+        ((gt_width == NPC_GT_BED || gt_width == NPC_GT_DOSE255 || gt_width == NPC_GT_DOSE32) && ploidy != 2) ||
         max_rows_per_block < 1 || n_slots < 0 || n_slots == 1 || staging_rows < 1 || staging_rows > max_rows_per_block) {
         g_create_error = "npc_create: invalid argument";
         return NPC_EINVAL;
     }
     npc_ctx *c = new npc_ctx();
     c->device = device; c->n = n_samples; c->ploidy = ploidy; c->width = gt_width; c->bed = gt_width == NPC_GT_BED;
-    c->dose255 = gt_width == NPC_GT_DOSE255;
+    c->dose255 = gt_width == NPC_GT_DOSE255; c->dose32 = gt_width == NPC_GT_DOSE32;
     c->max_rows = max_rows_per_block; c->n_slots = n_slots; c->staging_rows = staging_rows;
     c->pol.imp_locus = NPC_LOCUS_PS; c->pol.imp_missing = NPC_MISSING_HOMREF; c->pol.imp_sample = NPC_SAMPLE_INT_PS;
     c->pol.mincs = 100; c->pol.maxmis = 0.05; c->pol.n_total = n_samples;      // defaults of main (:670-687)
@@ -437,12 +443,13 @@ static const npc_ctx::TileCfg &fast_config(const npc_ctx *c, int64_t n_rows) {
 // What a launch of n_rows rows runs (launch_block), and what npc_kernel_shape2 and npc_plan_shape report: 0 the generic
 // tally, decide, accumulate sequence, 1 the tile kernel in exact order, 2 in default order, 3 tally + decide, then the tile
 // kernel in decided mode over the wide slabs (only where no resident shape fits), 4 the sequence on PLINK .bed rows, 5 the
-// sequence on fixed-point dosage rows (BGEN).
+// sequence on fixed-point dosage rows (BGEN), 6 the sequence on 32-bit fixed-point dosage rows (BGEN at any bit depth).
 // t: the tile kernel's shape in modes 1-3.
 static int launch_mode(const npc_ctx *c, bool exact, int64_t n_rows, const npc_ctx::TileCfg *&t) {
     t = nullptr;
     if (c->bed) return 4;
     if (c->dose255) return 5;
+    if (c->dose32) return 6;
     t = exact ? &c->exact_cfg : &fast_config(c, n_rows);
     if (t->ok) return exact ? 1 : 2;
     t = exact ? &c->wide_exact : &c->wide;
@@ -459,6 +466,8 @@ extern "C" int npc_kernel_shape2(const npc_ctx *ctx, int64_t n_rows, int32_t sha
         shape[3] = 8; shape[4] = ctx->exact ? 1 : 4;
     } else if (shape[0] == 5) {
         shape[1] = (int32_t)((ctx->n + 8 * D255_THREADS - 1) / (8 * D255_THREADS)); shape[2] = D255_THREADS / 32; shape[3] = 8;
+    } else if (shape[0] == 6) {
+        shape[1] = (int32_t)((ctx->n + 4 * D32_THREADS - 1) / (4 * D32_THREADS)); shape[2] = D32_THREADS / 32; shape[3] = 4;
     } else if (shape[0]) {
         shape[1] = t->Gs * 1000 + t->Gr; shape[2] = t->nc; shape[3] = t->K;
         shape[4] = F5_R; shape[5] = t->Sr * 1000 + t->Sc; shape[6] = t->L * 100 + t->GD * 10 + t->A; shape[7] = (int32_t)t->smem;
@@ -528,7 +537,7 @@ static int check_block(npc_ctx *c, const void *gt, int64_t row_stride, int64_t n
 
 // .bed and dosage rows carry one ALT: a decoded row names REF (0) or that ALT (1).  Checked where the rows are on the host.
 static int check_bed_rows(npc_ctx *c, const npc_row *rows, int64_t n_rows, int on_device) {
-    if (!(c->bed || c->dose255) || on_device) return NPC_OK;
+    if (!(c->bed || c->dose255 || c->dose32) || on_device) return NPC_OK;
     for (int64_t i = 0; i < n_rows; i++)
         if (rows[i].kind == NPC_KIND_GT && rows[i].gt_row >= 0 && rows[i].eaidx != 0 && rows[i].eaidx != 1)
             return fail(c, NPC_EINVAL, c->bed ? "PLINK .bed rows: the effect allele of a genotype row is REF (eaidx 0) or the one ALT (eaidx 1)"
@@ -574,6 +583,9 @@ static int launch_tally(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const
         } else if (c->dose255) {
             const unsigned slabs = tally_grid_y((c->n + 7) / 8, n_rows, 1024);               // units: chunks of 8 samples
             k_count_dose255<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
+        } else if (c->dose32) {
+            const unsigned slabs = tally_grid_y((c->n + 3) / 4, n_rows, 1024);               // units: chunks of 4 samples
+            k_count_dose32<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
         } else if (c->width == 1 && c->ploidy == 2) {
             const unsigned slabs = tally_grid_y((c->n + 7) / 8, n_rows, 1024);               // units: chunks of 8 samples
             k_count_i8x2<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
@@ -589,8 +601,9 @@ static int launch_tally(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const
     return NPC_OK;
 }
 
-// The decision for each of n_rows tallied rows: its contributions to d_rowp, its record appended to the locus log
-static int launch_decide(npc_ctx *c, const npc_row *d_rows, int64_t n_rows, const ull *counts) {
+// The decision for each of n_rows tallied rows: its contributions to d_rowp, its record appended to the locus log.  gt: the
+// rows' slab, whose row headers hold the denominators of 32-bit dosage rows
+static int launch_decide(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows, const ull *counts) {
     if (n_rows == 0) return NPC_OK;
     int rc = ensure_log(c, n_rows);
     if (rc) return rc;
@@ -600,6 +613,9 @@ static int launch_decide(npc_ctx *c, const npc_row *d_rows, int64_t n_rows, cons
                                                 c->d_rowp, c->d_log + c->log_len, c->d_nloci);
     else if (c->dose255)
         k_decide_dose255<<<grid, 128, 0, c->stream>>>(d_rows, n_rows, counts, c->pol, c->n, c->d_rowp, c->d_log + c->log_len, c->d_nloci);
+    else if (c->dose32)
+        k_decide_dose32<<<grid, 128, 0, c->stream>>>(gt, row_stride, d_rows, n_rows, counts, c->pol, c->n, c->d_rowp,
+                                                     c->d_log + c->log_len, c->d_nloci);
     else
         k_decide<<<grid, 128, 0, c->stream>>>(d_rows, n_rows, counts, c->pol, c->n, c->d_rowp, c->d_log + c->log_len, c->d_nloci);
     c->launches++;
@@ -633,6 +649,9 @@ static int launch_accum(npc_ctx *c, const uint8_t *gt, int64_t row_stride, int64
     } else if (c->dose255) {
         const unsigned grid = (unsigned)((c->n + 8 * D255_THREADS - 1) / (8 * D255_THREADS));
         k_accum_dose255<<<grid, D255_THREADS, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->d_sums);
+    } else if (c->dose32) {
+        const unsigned grid = (unsigned)((c->n + 4 * D32_THREADS - 1) / (4 * D32_THREADS));
+        k_accum_dose32<<<grid, D32_THREADS, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->d_sums);
     } else if (c->width == 1 && c->ploidy == 2) {
         const int64_t nchunks = (c->n + 7) / 8;
         k_accum_i8x2<64, 8><<<(unsigned)((nchunks + 255) / 256), 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows,
@@ -706,7 +725,7 @@ static int launch_wide(npc_ctx *c, const npc_ctx::TileCfg &t, bool exact, const 
                        const npc_row *d_rows, int64_t n_rows) {
     if (n_rows == 0) return NPC_OK;
     int rc = launch_tally(c, gt, row_stride, d_rows, n_rows, c->d_counts);
-    if (!rc) rc = launch_decide(c, d_rows, n_rows, c->d_counts);
+    if (!rc) rc = launch_decide(c, gt, row_stride, d_rows, n_rows, c->d_counts);
     if (rc) return rc;
     FusedParams P = fused_params(c, t, gt, row_stride, d_rows, n_rows);
     P.decided = c->d_rowp;
@@ -724,9 +743,9 @@ static int launch_block(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const
     switch (launch_mode(c, c->exact, n_rows, t)) {
     case 1: case 2: return launch_fused(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
     case 3: return launch_wide(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
-    default: {                                                                                  // 0, 4, 5
+    default: {                                                                                  // 0, 4, 5, 6
         int rc = launch_tally(c, gt, row_stride, d_rows, n_rows, c->d_counts);
-        if (!rc) rc = launch_decide(c, d_rows, n_rows, c->d_counts);
+        if (!rc) rc = launch_decide(c, gt, row_stride, d_rows, n_rows, c->d_counts);
         return rc ? rc : launch_accum(c, gt, row_stride, n_rows);
     }
     }
@@ -796,7 +815,7 @@ static int split_prologue(npc_ctx *c, const void *gt_dev, int64_t row_stride, in
     if (!counts_dev) return fail(c, NPC_EINVAL, "counts_dev is NULL");
     if (c->ds) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take hard-call (GT) rows only");
     if (c->bed) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not PLINK .bed rows");
-    if (c->dose255) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not BGEN dosage rows");
+    if (c->dose255 || c->dose32) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not BGEN dosage rows");
     NPC_CUDA(c, cudaSetDevice(c->device));
     return upload_rows(c, rows, n_rows, rows_on_device, d_rows);
 }
@@ -814,7 +833,7 @@ extern "C" int npc_accumulate_block_device(npc_ctx *ctx, const void *gt_dev, int
                                            const int64_t *counts_dev) {
     const npc_row *d_rows;
     int rc = split_prologue(ctx, gt_dev, row_stride, n_gt_rows, rows, n_rows, rows_on_device, counts_dev, &d_rows);
-    if (!rc) rc = launch_decide(ctx, d_rows, n_rows, (const ull *)counts_dev);
+    if (!rc) rc = launch_decide(ctx, (const uint8_t *)gt_dev, row_stride, d_rows, n_rows, (const ull *)counts_dev);
     return rc ? rc : launch_accum(ctx, (const uint8_t *)gt_dev, row_stride, n_rows);
 }
 

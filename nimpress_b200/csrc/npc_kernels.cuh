@@ -28,7 +28,7 @@ struct RowP {
     int32_t mode;
     int32_t eaidx;
     int32_t gt_row;
-    int32_t pad;
+    int32_t pad;             // 32-bit dosage rows: the row's denominator D (npc_dose32.cuh); 0 elsewhere
 };
 
 struct Policy {

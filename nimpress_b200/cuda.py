@@ -15,6 +15,7 @@ SAMPLE = {"ps": 0, "homref": 1, "fail": 2, "int_ps": 3, "int_fail": 4}   # Imput
 KIND_GT, KIND_NOTCOV, KIND_ABSENT, KIND_FILTER, CLASS_MAXMIS = range(5)
 GT_BED = 0        # gt_width of a context over PLINK 1 .bed rows (2 bits per sample, ploidy 2): NPC_GT_BED
 GT_DOSE255 = 255  # gt_width of a context over fixed-point dosage rows of BGEN files (uint16 255 x dosage, ploidy 2): NPC_GT_DOSE255
+GT_DOSE32 = 32    # gt_width of a context over 32-bit fixed-point dosage rows of BGEN files at any bit depth (ploidy 2): NPC_GT_DOSE32
 
 
 def gt_row_bytes(n_samples, ploidy, gt_width):

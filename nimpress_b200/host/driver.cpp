@@ -469,7 +469,8 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
     for (int k = 0; k < S; k++) {
         outs[k].loci.assign(scores[k]->entries.size(), npc_locus());
         for (size_t j = 0; j < order[k].size(); j++) outs[k].loci[order[k][j]] = logs[k][j];
-        outs[k].warnings = make_warnings(*scores[k], *ps[k].M, outs[k].loci, n, p, p.use_ds || gt_width == NPC_GT_DOSE255);
+        outs[k].warnings = make_warnings(*scores[k], *ps[k].M, outs[k].loci, n, p,
+                                         p.use_ds || gt_width == NPC_GT_DOSE255 || gt_width == NPC_GT_DOSE32);
     }
     timer.mark("WARN lines (binomial tests)");
 }
@@ -482,6 +483,7 @@ bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores
     int width = 1, ploidy = 2;                      // BCF's usual GT layout: int8, diploid
     if (p.use_ds) { width = 4; ploidy = 1; }        // FORMAT/DS: one float per sample
     bool seekable = true;                           // first try the index-driven pass (needs <file>.tbi / .csi)
+    bool dose32 = false;                            // a BGEN pass met a block that only 32-bit dosage rows hold
     for (int attempt = 0; attempt < 6; attempt++) {
         std::unique_ptr<VariantSource> vcf = open_variant_source(genotype_path, seekable);
         if (!vcf) return false;
@@ -490,7 +492,7 @@ bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores
         ScoreParams q = p;
         if (fixed == NPC_GT_BED && p.use_ds) throw InputError("--dosage: a PLINK fileset holds hard calls only, no FORMAT/DS");
         if (fixed != VariantSource::NO_FIXED_LAYOUT) {
-            width = fixed; ploidy = 2; seekable = false;
+            width = dose32 ? NPC_GT_DOSE32 : fixed; ploidy = 2; seekable = false;
             q.use_ds = false;                       // BGEN rows are dosages already: --dosage changes nothing
         }
         vcf->set_dosage_mode(q.use_ds);
@@ -501,6 +503,9 @@ bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores
             seekable = false;
         } catch (const LayoutOverflow &o) {         // rare: wider integers or higher ploidy -- rerun with that layout
             width = o.width; ploidy = o.ploidy;
+        } catch (const NeedsDose32 &e) {            // BGEN at another bit depth or with haploid samples: rerun with 32-bit rows
+            dose32 = true;
+            if (getenv("NIMPRESS_TIMING")) fprintf(stderr, "[nimpress timing] restart with 32-bit dosage rows: %s\n", e.what());
         } catch (const SlabOverflow &) {            // too many rows for one resident slab: one file at a time
             outs.assign(scores.size(), ScoreResult());
             for (size_t k = 0; k < scores.size(); k++)

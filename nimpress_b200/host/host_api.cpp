@@ -187,6 +187,8 @@ int nph_read_gt(const char *genotype_path, uint8_t *out, int64_t row_bytes, int6
         std::unique_ptr<VariantSource> vcf = open_variant_source(genotype_path);
         if (!vcf) return NPH_EOPEN_VCF;
         if (const char *e = getenv("NIMPRESS_READ_DS")) if (*e && *e != '0') vcf->set_dosage_mode(true);   // tests: FORMAT/DS instead of GT
+        int bgen_layout = NPC_GT_DOSE255;                                                                   // BGEN rows
+        if (const char *e = getenv("NIMPRESS_READ_DOSE32")) if (*e && *e != '0') bgen_layout = NPC_GT_DOSE32;
         VariantRecord rec;
         int64_t k = 0;
         *n_samples = vcf->n_samples();
@@ -194,8 +196,8 @@ int nph_read_gt(const char *genotype_path, uint8_t *out, int64_t row_bytes, int6
             if (k >= max_records) return NPH_ECAPACITY;
             if (rec.has_gt && vcf->fixed_layout() == NPC_GT_DOSE255) {
                 // BGEN: converted by the source's workers straight into the output row, as the driver has it done
-                if (npc_gt_row_bytes(vcf->n_samples(), 2, NPC_GT_DOSE255) > row_bytes) { vcf->wait_rows(); return NPH_ECAPACITY; }
-                vcf->load_gt_into(rec, out + k * row_bytes, NPC_GT_DOSE255, 2);
+                if (npc_gt_row_bytes(vcf->n_samples(), 2, bgen_layout) > row_bytes) { vcf->wait_rows(); return NPH_ECAPACITY; }
+                vcf->load_gt_into(rec, out + k * row_bytes, bgen_layout, 2);
                 *width = rec.gt_width; *ploidy = rec.ploidy;
             } else if (rec.has_gt) {
                 vcf->load_gt(rec);
@@ -277,10 +279,11 @@ static const char *USAGE =
     "                     Not with a PLINK fileset; with a BGEN file it changes nothing.\n"
     "PLINK 1 fileset (not a reference input): X.bed with X.bim and X.fam, recognised by its magic bytes.\n"
     "  REF = A2 (.bim column 6), ALT = A1 (column 5), sample names = .fam IID; FILTER is always \".\".\n"
-    "BGEN v1.2 file (not a reference input): layout 2, 8-bit probabilities, uncompressed or zlib, diploid\n"
-    "  biallelic variants, recognised by its magic bytes.  Scored as expected ALT dosages.  REF = allele 1,\n"
-    "  ALT = allele 2, CHROM compared literally; sample names = the embedded identifiers, else column 2\n"
-    "  (ID_2) of X.sample beside X.bgen; FILTER is always \".\".  No AF-mismatch warnings for its loci.\n"
+    "BGEN v1.2 file (not a reference input): layout 2, 1-16 bits per probability, uncompressed or zlib,\n"
+    "  haploid and diploid samples, biallelic variants, recognised by its magic bytes.  Scored as expected\n"
+    "  ALT dosages.  REF = allele 1, ALT = allele 2, CHROM compared literally; sample names = the embedded\n"
+    "  identifiers, else column 2 (ID_2) of X.sample beside X.bgen; FILTER is always \".\".  No AF-mismatch\n"
+    "  warnings for its loci.\n"
     "  --exact-order      Add every locus to the running sums in score-file order, bit for bit\n"
     "                     like the reference (default: sum tiles of four loci first; same\n"
     "                     products, scores equal to ~1e-15 relative) (not a reference option).\n";

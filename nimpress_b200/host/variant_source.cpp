@@ -954,12 +954,15 @@ private:
 };
 
 // ------------------------------------------------------------------------------------------
-// BGEN v1.2, layout 2, 8-bit probabilities (DESIGN.md 4.8) -- not a reference input
+// BGEN v1.2, layout 2, 1 to 16 bits per probability (DESIGN.md 4.8, 4.9) -- not a reference input
 // ------------------------------------------------------------------------------------------
 
-// One genotype block -> one row of fixed-point dosages (NPC_GT_DOSE255): per sample k = 255 x the expected ALT dosage as
-// a little-endian uint16, 0xFFFF for a missing sample.  Each thread that converts blocks has one of these: its own file
-// descriptor, inflate tables and buffers.
+// One genotype block -> one row of fixed-point dosages, in either layout:
+//   NPC_GT_DOSE255  8 bits, diploid: per sample k = 255 x the expected ALT dosage as a little-endian uint16, 0xFFFF for a
+//                   missing sample.  A well-formed block these rows cannot hold throws NeedsDose32.
+//   NPC_GT_DOSE32   1 to 16 bits, haploid and diploid samples: the row header (uint32 D = 2^B - 1, 12 zero bytes), then
+//                   per sample the uint32 word k | ploidy << 24, 0xFFFFFFFF for a missing sample (npc_dose32.cuh).
+// Each thread that converts blocks has one of these: its own file descriptor, inflate tables and buffers.
 class BgenBlockReader {
 public:
     BgenBlockReader(const std::string &path, int64_t n, bool compressed) : n_(n), compressed_(compressed) {
@@ -970,7 +973,8 @@ public:
     BgenBlockReader(const BgenBlockReader &) = delete;
     BgenBlockReader &operator=(const BgenBlockReader &) = delete;
     // off / C: file offset and length of the genotype block after its C field; what: the variant, for messages
-    void convert(int64_t off, uint32_t C, uint8_t *dst, const std::string &what) {
+    // layout: NPC_GT_DOSE255 or NPC_GT_DOSE32
+    void convert(int64_t off, uint32_t C, uint8_t *dst, const std::string &what, int layout) {
         in_.resize((size_t)C + 16);
         int64_t got = 0;
         while (got < (int64_t)C) {
@@ -1000,24 +1004,30 @@ public:
             }
             p = out_.data(); len = D;
         }
-        decode(p, len, dst, what);
+        if (layout == NPC_GT_DOSE32) decode32(p, len, dst, what);
+        else decode(p, len, dst, what);
     }
 private:
+    InputError bad(const std::string &what, const std::string &m) const { return InputError("BGEN: variant " + what + ": " + m); }
+    // NeedsDose32 when the block is well-formed; decode32 refuses it otherwise
+    NeedsDose32 needs32(const uint8_t *p, size_t len, const std::string &what, const std::string &m) const {
+        decode32(p, len, nullptr, what);
+        return NeedsDose32("BGEN: variant " + what + ": " + m + " (needs 32-bit dosage rows)");
+    }
     void decode(const uint8_t *p, size_t len, uint8_t *dst, const std::string &what) const {
-        auto bad = [&](const std::string &m) { return InputError("BGEN: variant " + what + ": " + m); };
-        if (len < 8) throw bad("genotype block too short");
+        if (len < 8) throw bad(what, "genotype block too short");
         uint32_t N; uint16_t K;
         memcpy(&N, p, 4); memcpy(&K, p + 4, 2);
         const int pmin = p[6], pmax = p[7];
-        if ((int64_t)N != n_) throw bad("genotype block holds " + std::to_string(N) + " samples, the header " + std::to_string(n_));
-        if (K != 2) throw bad(std::to_string(K) + " alleles (only biallelic variants are supported)");
-        if (pmin != 2 || pmax != 2) throw bad("ploidy " + std::to_string(pmin) + ".." + std::to_string(pmax) + " (only diploid samples are supported)");
-        if (len < 8 + (size_t)n_ + 2) throw bad("genotype block too short");
+        if ((int64_t)N != n_) throw bad(what, "genotype block holds " + std::to_string(N) + " samples, the header " + std::to_string(n_));
+        if (K != 2) throw bad(what, std::to_string(K) + " alleles (only biallelic variants are supported)");
+        if (pmin != 2 || pmax != 2) throw needs32(p, len, what, "ploidy " + std::to_string(pmin) + ".." + std::to_string(pmax));
+        if (len < 8 + (size_t)n_ + 2) throw bad(what, "genotype block too short");
         const uint8_t *ploidy = p + 8, *q = p + 8 + n_;
         const bool phased = q[0] != 0;
         const int B = q[1];
-        if (B != 8) throw bad(std::to_string(B) + " bits per probability (only 8 are supported)");
-        if (len < 8 + (size_t)n_ + 2 + 2 * (size_t)n_) throw bad("genotype block too short");
+        if (B != 8) throw needs32(p, len, what, std::to_string(B) + " bits per probability");
+        if (len < 8 + (size_t)n_ + 2 + 2 * (size_t)n_) throw bad(what, "genotype block too short");
         const uint8_t *pr = q + 2;
         for (int64_t i = 0; i < n_; i++) {
             const uint32_t a = pr[2 * i], b = pr[2 * i + 1];
@@ -1025,11 +1035,67 @@ private:
             if (ploidy[i] & 0x80) k = 0xFFFF;
             else if (phased) k = 510 - a - b;                             // (255 - h0) + (255 - h1)
             else {
-                if (a + b > 255) throw bad("sample " + std::to_string(i) + ": P(hom allele 1) + P(het) > 1");
+                if (a + b > 255) throw bad(what, "sample " + std::to_string(i) + ": P(hom allele 1) + P(het) > 1");
                 k = 510 - 2 * a - b;                                      // P(het) + 2 P(hom allele 2), in 1/255
             }
             const uint16_t v = (uint16_t)k;
             memcpy(dst + 2 * i, &v, 2);
+        }
+    }
+    // dst == nullptr: check the block only.  Each sample stores `ploidy` values of B bits (phased or not, K = 2), packed
+    // back to back least-significant bit first; a missing sample still occupies its values.
+    void decode32(const uint8_t *p, size_t len, uint8_t *dst, const std::string &what) const {
+        if (len < 8) throw bad(what, "genotype block too short");
+        uint32_t N; uint16_t K;
+        memcpy(&N, p, 4); memcpy(&K, p + 4, 2);
+        const int pmin = p[6], pmax = p[7];
+        if ((int64_t)N != n_) throw bad(what, "genotype block holds " + std::to_string(N) + " samples, the header " + std::to_string(n_));
+        if (K != 2) throw bad(what, std::to_string(K) + " alleles (only biallelic variants are supported)");
+        if (pmax > 2) throw bad(what, "ploidy " + std::to_string(pmin) + ".." + std::to_string(pmax) + " (only haploid and diploid samples are supported)");
+        if (len < 8 + (size_t)n_ + 2) throw bad(what, "genotype block too short");
+        const uint8_t *ploidy = p + 8, *q = p + 8 + n_;
+        const bool phased = q[0] != 0;
+        const int B = q[1];
+        if (B < 1 || B > 16) throw bad(what, std::to_string(B) + " bits per probability (1 to 16 are supported)");
+        uint64_t values = 0;
+        for (int64_t i = 0; i < n_; i++) {
+            const int pl = ploidy[i] & 0x3F;
+            if (pl < pmin || pl > pmax)
+                throw bad(what, "sample " + std::to_string(i) + ": ploidy " + std::to_string(pl) + " outside " + std::to_string(pmin) + ".." + std::to_string(pmax));
+            values += (uint64_t)pl;
+        }
+        if (len - (8 + (size_t)n_ + 2) < (values * (uint64_t)B + 7) / 8)
+            throw bad(what, "genotype block too short for " + std::to_string(n_) + " samples at " + std::to_string(B) + " bits");
+        const uint32_t D = (1u << B) - 1, mask = D;
+        const uint8_t *src = q + 2;
+        uint64_t acc = 0;
+        int have = 0;
+        auto next = [&]() -> uint32_t {                                   // the next B-bit value of the stream
+            while (have < B) { acc |= (uint64_t)*src++ << have; have += 8; }
+            const uint32_t v = (uint32_t)acc & mask;
+            acc >>= B; have -= B;
+            return v;
+        };
+        if (dst) {
+            memset(dst, 0, 16);
+            memcpy(dst, &D, 4);
+        }
+        for (int64_t i = 0; i < n_; i++) {
+            const int pl = ploidy[i] & 0x3F;
+            uint32_t w = 0xFFFFFFFFu;
+            if (pl == 1) {
+                const uint32_t a = next();
+                w = (D - a) | 1u << 24;                                   // P(allele 2), in 1/D
+            } else if (pl == 2) {
+                const uint32_t a = next(), b = next();
+                if (phased) w = (2 * D - a - b) | 2u << 24;               // (D - h0) + (D - h1)
+                else {
+                    if (a + b > D && !(ploidy[i] & 0x80)) throw bad(what, "sample " + std::to_string(i) + ": P(hom allele 1) + P(het) > 1");
+                    w = (2 * D - 2 * a - b) | 2u << 24;                   // P(het) + 2 P(hom allele 2), in 1/D
+                }
+            }
+            if (ploidy[i] & 0x80) w = 0xFFFFFFFFu;
+            if (dst) memcpy(dst + 16 + 4 * i, &w, 4);
         }
     }
     int fd_ = -1;
@@ -1042,8 +1108,9 @@ private:
 // The header and sample identifiers are read at open; next() walks the variant headers and skips each genotype block by
 // its length (there is no index: a .bgi is an SQLite file).  A block is read and converted only when a score row matched
 // its variant (load_gt / load_gt_into).  load_gt_into hands the block to a pool of NIMPRESS_THREADS workers and returns;
-// wait_rows() waits for every block posted so far.  Per variant: CHROM = chromosome (compared literally), POS, REF =
-// allele 1, ALT = allele 2 (and any further alleles), rlen = len(REF), FILTER ".".
+// wait_rows() waits for every block posted so far, and rethrows a worker's InputError (before a worker's NeedsDose32, so
+// that which of them is thrown does not depend on the workers' timing).  Per variant: CHROM = chromosome (compared
+// literally), POS, REF = allele 1, ALT = allele 2 (and any further alleles), rlen = len(REF), FILTER ".".
 class BgenSource : public VariantSource {
 public:
     ~BgenSource() override {
@@ -1118,27 +1185,29 @@ public:
     int fixed_layout() const override { return NPC_GT_DOSE255; }
     void load_gt(VariantRecord &rec) override {
         buf_.resize((size_t)std::max<int64_t>(2 * n_, 1));
-        inline_reader().convert(blk_off_, blk_len_, buf_.data(), what_);
-        fill(rec, buf_.data());
+        inline_reader().convert(blk_off_, blk_len_, buf_.data(), what_, NPC_GT_DOSE255);
+        fill(rec, buf_.data(), NPC_GT_DOSE255);
     }
     bool load_gt_into(VariantRecord &rec, uint8_t *dst, int want_width, int want_ploidy) override {
-        if (want_width != NPC_GT_DOSE255 || want_ploidy != 2) { load_gt(rec); return false; }
-        if (threads_ <= 1) inline_reader().convert(blk_off_, blk_len_, dst, what_);
+        if ((want_width != NPC_GT_DOSE255 && want_width != NPC_GT_DOSE32) || want_ploidy != 2) { load_gt(rec); return false; }
+        if (threads_ <= 1) inline_reader().convert(blk_off_, blk_len_, dst, what_, want_width);
         else {
             std::lock_guard<std::mutex> g(mu_);
             if (workers_.empty())
                 for (int t = 0; t < threads_; t++) workers_.emplace_back([this] { work(); });
-            jobs_.push_back(Job{ blk_off_, blk_len_, dst, what_ });
+            jobs_.push_back(Job{ blk_off_, blk_len_, dst, what_, want_width });
             pending_++;
             cv_.notify_one();
         }
-        fill(rec, dst);
+        fill(rec, dst, want_width);
         return true;
     }
     void wait_rows() override {
         std::unique_lock<std::mutex> lk(mu_);
         done_.wait(lk, [this] { return pending_ == 0; });
-        if (!err_.empty()) { std::string e; e.swap(err_); throw InputError(e); }
+        std::string e;
+        if (!err_.empty()) { e.swap(err_); need32_.clear(); throw InputError(e); }
+        if (!need32_.empty()) { e.swap(need32_); throw NeedsDose32(e); }
     }
 protected:
     bool next_raw(VariantRecord &rec) override {
@@ -1177,7 +1246,7 @@ protected:
     int contig_rank(const VariantRecord &rec) const override { return rec.contig_id; }
     int contig_rank(const std::string &) const override { return -1; }
 private:
-    struct Job { int64_t off; uint32_t len; uint8_t *dst; std::string what; };
+    struct Job { int64_t off; uint32_t len; uint8_t *dst; std::string what; int layout; };
     bool rd(void *dst, size_t n) {
         if (fread(dst, 1, n, fp_) != n) return false;
         pos_ += (int64_t)n;
@@ -1194,7 +1263,7 @@ private:
         if (!inline_) inline_ = std::make_unique<BgenBlockReader>(path_, n_, compressed_);
         return *inline_;
     }
-    void fill(VariantRecord &rec, const uint8_t *row) const { rec.has_gt = true; rec.gt = row; rec.gt_width = NPC_GT_DOSE255; rec.ploidy = 2; }
+    void fill(VariantRecord &rec, const uint8_t *row, int layout) const { rec.has_gt = true; rec.gt = row; rec.gt_width = layout; rec.ploidy = 2; }
     void work() {
         std::unique_ptr<BgenBlockReader> r;
         for (;;) {
@@ -1206,13 +1275,15 @@ private:
                 j = std::move(jobs_.front());
                 jobs_.pop_front();
             }
-            std::string e;
+            std::string e, e32;
             try {
                 if (!r) r = std::make_unique<BgenBlockReader>(path_, n_, compressed_);
-                r->convert(j.off, j.len, j.dst, j.what);
-            } catch (const InputError &x) { e = x.what(); }
+                r->convert(j.off, j.len, j.dst, j.what, j.layout);
+            } catch (const NeedsDose32 &x) { e32 = x.what(); }
+            catch (const InputError &x) { e = x.what(); }
             std::lock_guard<std::mutex> g(mu_);
             if (!e.empty() && err_.empty()) err_ = e;
+            if (!e32.empty() && need32_.empty()) need32_ = e32;
             if (--pending_ == 0) done_.notify_all();
         }
     }
@@ -1231,7 +1302,7 @@ private:
     std::deque<Job> jobs_;
     int64_t pending_ = 0;
     bool stop_ = false;
-    std::string err_;
+    std::string err_, need32_;
     std::vector<std::thread> workers_;
 };
 

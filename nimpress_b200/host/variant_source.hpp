@@ -103,7 +103,8 @@ public:
     virtual void set_dosage_mode(bool on) { dosage_ = on; }
     // The one device layout this source's rows come in, or NO_FIXED_LAYOUT for VCF / BCF (whose layout follows the records):
     // NPC_GT_BED for a PLINK 1 fileset (.bed rows as stored, ploidy 2, ceil(n/4) bytes), NPC_GT_DOSE255 for a BGEN file
-    // (one uint16 dosage numerator per sample, ploidy 2).
+    // (one uint16 dosage numerator per sample, ploidy 2).  A BGEN file also delivers NPC_GT_DOSE32 rows when load_gt_into
+    // asks for them, and throws NeedsDose32 where a matched block does not fit NPC_GT_DOSE255 rows.
     static constexpr int NO_FIXED_LAYOUT = -1;
     virtual int fixed_layout() const { return NO_FIXED_LAYOUT; }
     // Rows that load_gt_into handed to worker threads are complete once this returns; a worker's InputError is rethrown
@@ -128,6 +129,13 @@ private:
     size_t region_ = 0;
     bool filtering_ = false, positioned_ = false;
     int64_t seeks_ = 0;
+};
+
+// A matched BGEN genotype block that 2-byte dosage rows (NPC_GT_DOSE255) cannot hold and 32-bit rows (NPC_GT_DOSE32) can:
+// a bit depth other than 8, or samples that are not all diploid.  The driver restarts its pass with NPC_GT_DOSE32 rows;
+// to any other caller it is the InputError that names the variant.
+struct NeedsDose32 : InputError {
+    using InputError::InputError;
 };
 
 // nullptr: the file cannot be opened or is neither VCF, BCF, a PLINK 1 .bed nor a BGEN file (the reference: open() == false);

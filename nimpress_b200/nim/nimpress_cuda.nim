@@ -40,6 +40,7 @@ const
   npcClassMaxMis* = 4'i32 ## output only: nmissing/n > maxMissingRate     (:565-571)
   npcGtBed* = 0'i32       ## gtWidth of a context over PLINK 1 .bed rows (2 bits per sample, ploidy 2)
   npcGtDose255* = 255'i32 ## gtWidth of a context over BGEN fixed-point dosage rows (uint16 255 x dosage, ploidy 2)
+  npcGtDose32* = 32'i32   ## gtWidth of a context over BGEN 32-bit dosage rows (16-byte header with D, uint32 per sample, ploidy 2)
 
 {.push importc, cdecl, dynlib: npcLib.}
 proc npc_create*(ctx: ptr NpcCtx; device: cint; nSamples: int64; ploidy, gtWidth: int32;
@@ -76,7 +77,7 @@ proc npc_launch_count*(ctx: NpcCtx): int64
 proc npc_multi_contractions*(ctx: NpcCtx): int64
 proc npc_kernel_shape*(ctx: NpcCtx; shape: ptr array[8, int32]): cint
 proc npc_kernel_shape2*(ctx: NpcCtx; n_rows: int64; shape: ptr array[8, int32]): cint
-proc npc_gt_row_bytes*(n_samples: int64; ploidy, gt_width: int32): int64   ## bytes of a row (gt_width npcGtBed: 2-bit rows, npcGtDose255: 2 bytes per sample)
+proc npc_gt_row_bytes*(n_samples: int64; ploidy, gt_width: int32): int64   ## bytes of a row (gt_width npcGtBed: 2-bit rows, npcGtDose255: 2 bytes per sample, npcGtDose32: 16 + 4 per sample)
 proc npc_plan_shape*(n_samples: int64; gt_width, num_sms, max_smem: int32; n_rows: int64; exact: int32; plan: ptr array[16, int32]): cint
 proc npc_synth_fill_device*(ctx: NpcCtx; gtDev: pointer; rowStride, v0, nRows: int64; seed: uint64;
                             afThr16Dev, missThr24Dev: ptr uint32; altCodeDev: ptr int32): cint
