@@ -56,6 +56,24 @@
  * Accumulate: scores[s] += fl(fl(k'/D) * beta) (cm for a missing sample) in score-row order, the reference's chain, in
  * every mode.  With D = 255 and diploid samples a row scores bit for bit as the same NPC_GT_DOSE255 row; hard calls
  * (k' = 0, D, 2D) score bit for bit as the same genotypes in int8 GT rows in exact order, haploid samples included.
+ *
+ * Or, for a context created with gt_width = NPC_GT_PL (ploidy 2), FORMAT/PL rows as the host packs them from a biallelic
+ * VCF or BCF record's phred-scaled genotype likelihoods (DESIGN.md 4.10, npc_pl.cuh; NOT in the reference, parity
+ * unpinned): n little-endian uint32 words, one per sample.  With m the sample's smallest PL, j the index of its first
+ * occurrence and x_g = PL_g - m: bits 0-11 a and bits 12-23 b, the x of the two other genotypes in genotype order, each
+ * saturated at 4095 (b = 0 for a haploid sample); bits 24-25 j; bits 26-27 the ploidy (1: 2 PL values, 2: 3 values).
+ * The host writes 0xFFFFFFFF for a missing sample; any word with bit 31 set, a ploidy outside {1, 2} or j > ploidy is a
+ * missing sample.  All in fp64, round to nearest, no FMA contraction, with p = npc_row.eaf and q = fl(1 - p):
+ *   w_g = T[x_g], T[x] = fl(10^(-x/10)) correctly rounded (npc_pl_weight_table), 0 from x = 3237 on;
+ *   prior by c = effect-allele copies of g (ALT: c = g; REF: c = 2 - g diploid, 1 - g haploid): diploid pi(0) = fl(q*q),
+ *   pi(1) = fl(2*fl(p*q)), pi(2) = fl(p*p); haploid pi(0) = q, pi(1) = p; p NaN or outside [0, 1]: every sample missing;
+ *   u_g = fl(pi(c_g) * w_g); den = u_0 + u_1 (+ u_2) left to right; num = fl(u_1 + 2*u_2) (diploid, ALT), fl(2*u_0 + u_1)
+ *   (diploid, REF), u_1 (haploid, ALT), u_0 (haploid, REF); the sample is called iff den > 0, then d = fl(num / den).
+ * Tally, decision and accumulate as FORMAT/DS rows (npc_set_dosage_rows): nmiss an integer, neff = the fp64 sum of the
+ * called d in chunks of 8 samples left to right, a 32-way butterfly, blocks of 256 left to right, npc_locus.neff its IEEE
+ * bits; scores[s] += fl(d * beta) (cm for a missing sample) in score-row order, the reference's chain, in every mode.
+ * Decisive PLs (every other x >= 3237, 0 < eaf < 1, no underflow in the priors) give d in {0, 1, 2} exactly: such rows
+ * score bit for bit as the same genotypes in int8 GT rows in exact order, haploid samples included.
  */
 /*
  * Environment (diagnostics and tests; none is needed in normal use):
@@ -115,8 +133,17 @@ enum { NPC_KIND_GT = 0,      /* record found, FILTER passes: decode its genotype
  * above): ploidy must be 2.  Calls, effect alleles, exact order and the split calls as for NPC_GT_DOSE255. */
 #define NPC_GT_DOSE32 32
 
-/* Bytes of one genotype row of n samples in a layout (gt_width 1, 2, 4, NPC_GT_BED, NPC_GT_DOSE255 or NPC_GT_DOSE32). */
+/* gt_width of a context whose rows are FORMAT/PL rows (4 bytes per sample, see above): ploidy must be 2.  Calls, effect
+ * alleles, exact order and the split calls as for NPC_GT_DOSE255. */
+#define NPC_GT_PL 10
+
+/* Bytes of one genotype row of n samples in a layout (gt_width 1, 2, 4, NPC_GT_BED, NPC_GT_DOSE255, NPC_GT_DOSE32 or
+ * NPC_GT_PL). */
 int64_t npc_gt_row_bytes(int64_t n_samples, int32_t ploidy, int32_t gt_width);
+
+/* The weights of FORMAT/PL rows, no device needed: out[x] = T[x] = fl(10^(-x/10)) correctly rounded for x = 0 .. n - 1
+ * (0 from x = 3237 on), the table the PL kernels use. */
+int npc_pl_weight_table(double *out, int32_t n);
 
 typedef struct npc_ctx npc_ctx;
 
@@ -341,7 +368,8 @@ int npc_set_dosage_rows(npc_ctx *ctx, int32_t on);
  * shape[3] = samples per thread, shape[4] = rows per tile: 4 in the default mode, 1 in exact order),
  * 5 for NPC_GT_DOSE255 rows (k_count_dose255, k_decide_dose255, k_accum_dose255; then shape[1] = CTAs of the
  * accumulate pass, shape[2] = warps per CTA, shape[3] = 8 samples per thread), 6 for NPC_GT_DOSE32 rows (k_count_dose32,
- * k_decide_dose32, k_accum_dose32; shape[1..3] as for 5, with 4 samples per thread), 0 for the count/decide/accumulate sequence; then grid (tile kernel: sample slabs * 1000 + row
+ * k_decide_dose32, k_accum_dose32; shape[1..3] as for 5, with 4 samples per thread), 7 for NPC_GT_PL rows (k_count_pl,
+ * k_decide_pl, k_accum_pl; shape[1..3] as for 6), 0 for the count/decide/accumulate sequence; then grid (tile kernel: sample slabs * 1000 + row
  * groups), consumer warps, chunks per thread, rows
  * per tile, raw stages * 1000 + index-ring tiles, lag * 100 + tiles per decider pass * 10 + decider warps, dynamic
  * shared-memory bytes. */

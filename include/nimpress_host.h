@@ -24,6 +24,8 @@
  *   NIMPRESS_TIMING=1        phase wall times on stderr
  *   NIMPRESS_SLAB_ROWS=<n>   cap the device-resident genotype rows (tests: forces scoring in rounds)
  *   NIMPRESS_SPLIT=<k>       with one device: k contexts on it, combined by npc_reduce (tests of the multi-GPU path on one GPU)
+ *   NIMPRESS_READ_PL=1       nph_read_gt on a VCF / BCF: FORMAT/PL of every record as a packed PL row (NPC_GT_PL) instead
+ *                            of its GT
  *   NIMPRESS_READ_DOSE32=1   nph_read_gt on a BGEN file: every block as a 32-bit dosage row (NPC_GT_DOSE32) instead of a
  *                            2-byte one (NPC_GT_DOSE255, which refuses other bit depths and haploid samples)
  */
@@ -61,7 +63,9 @@ typedef struct {
     double  afmisp;
     int32_t use_ds;         /* 1: score FORMAT/DS (fp32 expected ALT dosage, biallelic effect alleles) instead of FORMAT/GT --
                                npc_set_dosage_rows; not in the reference (README.md:162-165 "Future") */
-    int32_t reserved;
+    int32_t use_pl;         /* 1: score FORMAT/PL (phred-scaled genotype likelihoods of biallelic VCF / BCF records) as posterior
+                               expected dosages at the score file's eaf (NPC_GT_PL rows, DESIGN.md 4.10) instead of FORMAT/GT;
+                               not with use_ds, a PLINK fileset or a BGEN file; not in the reference */
 } nph_params;
 
 typedef struct nph_result nph_result;

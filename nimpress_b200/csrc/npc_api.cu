@@ -18,6 +18,7 @@
 #include "npc_bed.cuh"
 #include "npc_dose255.cuh"
 #include "npc_dose32.cuh"
+#include "npc_pl.cuh"
 
 using namespace npc;
 
@@ -88,6 +89,8 @@ struct npc_ctx {
     // 32-bit fixed-point dosage rows from BGEN files at any bit depth (npc_dose32.cuh, gt_width = NPC_GT_DOSE32): a 16-byte
     // header holding the row's denominator, then uint32 per sample
     bool dose32 = false;
+    // FORMAT/PL rows (npc_pl.cuh, gt_width = NPC_GT_PL): a packed uint32 per sample; tallied as FORMAT/DS rows, into d_ds_part
+    bool pl = false;
     // cross-GPU combine (npc_reduce.cuh)
     cudaEvent_t ev_multi = nullptr;         // npc_score_resident_multi: orders its copy-stream work against the compute stream
     cudaEvent_t ev_reduce = nullptr;        // "this context's partial sums are final"
@@ -121,7 +124,15 @@ extern "C" int64_t npc_gt_row_bytes(int64_t n_samples, int32_t ploidy, int32_t g
     if (gt_width == NPC_GT_BED) return (n_samples + 3) / 4;
     if (gt_width == NPC_GT_DOSE255) return n_samples * 2;
     if (gt_width == NPC_GT_DOSE32) return D32_HEADER + n_samples * 4;
+    if (gt_width == NPC_GT_PL) return n_samples * 4;
     return n_samples * ploidy * gt_width;
+}
+
+extern "C" int npc_pl_weight_table(double *out, int32_t n) {
+    static const double tab[PL_TN] = { NPC_PL_TABLE_VALUES };
+    if (n < 0 || (n && !out)) return NPC_EINVAL;
+    for (int32_t x = 0; x < n; x++) out[x] = x < PL_TN ? tab[x] : 0.0;
+    return NPC_OK;
 }
 
 extern "C" int npc_warmup(int device) {
@@ -364,15 +375,15 @@ extern "C" int npc_create2(npc_ctx **out, int device, int64_t n_samples, int32_t
     *out = nullptr;
     if (n_samples < 0 || ploidy < 1 || ploidy > 64 ||
         (gt_width != 1 && gt_width != 2 && gt_width != 4 && gt_width != NPC_GT_BED && gt_width != NPC_GT_DOSE255 &&
-         gt_width != NPC_GT_DOSE32) ||
-        ((gt_width == NPC_GT_BED || gt_width == NPC_GT_DOSE255 || gt_width == NPC_GT_DOSE32) && ploidy != 2) ||
+         gt_width != NPC_GT_DOSE32 && gt_width != NPC_GT_PL) ||
+        ((gt_width == NPC_GT_BED || gt_width == NPC_GT_DOSE255 || gt_width == NPC_GT_DOSE32 || gt_width == NPC_GT_PL) && ploidy != 2) ||
         max_rows_per_block < 1 || n_slots < 0 || n_slots == 1 || staging_rows < 1 || staging_rows > max_rows_per_block) {
         g_create_error = "npc_create: invalid argument";
         return NPC_EINVAL;
     }
     npc_ctx *c = new npc_ctx();
     c->device = device; c->n = n_samples; c->ploidy = ploidy; c->width = gt_width; c->bed = gt_width == NPC_GT_BED;
-    c->dose255 = gt_width == NPC_GT_DOSE255; c->dose32 = gt_width == NPC_GT_DOSE32;
+    c->dose255 = gt_width == NPC_GT_DOSE255; c->dose32 = gt_width == NPC_GT_DOSE32; c->pl = gt_width == NPC_GT_PL;
     c->max_rows = max_rows_per_block; c->n_slots = n_slots; c->staging_rows = staging_rows;
     c->pol.imp_locus = NPC_LOCUS_PS; c->pol.imp_missing = NPC_MISSING_HOMREF; c->pol.imp_sample = NPC_SAMPLE_INT_PS;
     c->pol.mincs = 100; c->pol.maxmis = 0.05; c->pol.n_total = n_samples;      // defaults of main (:670-687)
@@ -443,13 +454,15 @@ static const npc_ctx::TileCfg &fast_config(const npc_ctx *c, int64_t n_rows) {
 // What a launch of n_rows rows runs (launch_block), and what npc_kernel_shape2 and npc_plan_shape report: 0 the generic
 // tally, decide, accumulate sequence, 1 the tile kernel in exact order, 2 in default order, 3 tally + decide, then the tile
 // kernel in decided mode over the wide slabs (only where no resident shape fits), 4 the sequence on PLINK .bed rows, 5 the
-// sequence on fixed-point dosage rows (BGEN), 6 the sequence on 32-bit fixed-point dosage rows (BGEN at any bit depth).
+// sequence on fixed-point dosage rows (BGEN), 6 the sequence on 32-bit fixed-point dosage rows (BGEN at any bit depth),
+// 7 the sequence on FORMAT/PL rows.
 // t: the tile kernel's shape in modes 1-3.
 static int launch_mode(const npc_ctx *c, bool exact, int64_t n_rows, const npc_ctx::TileCfg *&t) {
     t = nullptr;
     if (c->bed) return 4;
     if (c->dose255) return 5;
     if (c->dose32) return 6;
+    if (c->pl) return 7;
     t = exact ? &c->exact_cfg : &fast_config(c, n_rows);
     if (t->ok) return exact ? 1 : 2;
     t = exact ? &c->wide_exact : &c->wide;
@@ -468,6 +481,8 @@ extern "C" int npc_kernel_shape2(const npc_ctx *ctx, int64_t n_rows, int32_t sha
         shape[1] = (int32_t)((ctx->n + 8 * D255_THREADS - 1) / (8 * D255_THREADS)); shape[2] = D255_THREADS / 32; shape[3] = 8;
     } else if (shape[0] == 6) {
         shape[1] = (int32_t)((ctx->n + 4 * D32_THREADS - 1) / (4 * D32_THREADS)); shape[2] = D32_THREADS / 32; shape[3] = 4;
+    } else if (shape[0] == 7) {
+        shape[1] = (int32_t)((ctx->n + 4 * PL_THREADS - 1) / (4 * PL_THREADS)); shape[2] = PL_THREADS / 32; shape[3] = 4;
     } else if (shape[0]) {
         shape[1] = t->Gs * 1000 + t->Gr; shape[2] = t->nc; shape[3] = t->K;
         shape[4] = F5_R; shape[5] = t->Sr * 1000 + t->Sc; shape[6] = t->L * 100 + t->GD * 10 + t->A; shape[7] = (int32_t)t->smem;
@@ -537,7 +552,7 @@ static int check_block(npc_ctx *c, const void *gt, int64_t row_stride, int64_t n
 
 // .bed and dosage rows carry one ALT: a decoded row names REF (0) or that ALT (1).  Checked where the rows are on the host.
 static int check_bed_rows(npc_ctx *c, const npc_row *rows, int64_t n_rows, int on_device) {
-    if (!(c->bed || c->dose255 || c->dose32) || on_device) return NPC_OK;
+    if (!(c->bed || c->dose255 || c->dose32 || c->pl) || on_device) return NPC_OK;
     for (int64_t i = 0; i < n_rows; i++)
         if (rows[i].kind == NPC_KIND_GT && rows[i].gt_row >= 0 && rows[i].eaidx != 0 && rows[i].eaidx != 1)
             return fail(c, NPC_EINVAL, c->bed ? "PLINK .bed rows: the effect allele of a genotype row is REF (eaidx 0) or the one ALT (eaidx 1)"
@@ -561,15 +576,22 @@ static unsigned tally_grid_y(int64_t units, int64_t n_rows, int64_t min_units) {
     return (unsigned)std::min<int64_t>(std::max<int64_t>(std::min(std::max(want, s_min), s_max), 1), 65535);
 }
 
-// Tallies of n_rows rows into counts: two words a row; for dosage rows the missing count alone, the block sums of the
-// called dosages go to d_ds_part.
+// Tallies of n_rows rows into counts: two words a row; for FORMAT/DS and FORMAT/PL rows the missing count alone, the
+// block sums of the called dosages go to d_ds_part.
 static int launch_tally(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows,
                         ull *counts) {
-    NPC_CUDA(c, cudaMemsetAsync(counts, 0, n_rows * (c->ds ? 1 : 2) * sizeof(ull), c->stream));
+    NPC_CUDA(c, cudaMemsetAsync(counts, 0, n_rows * (c->ds || c->pl ? 1 : 2) * sizeof(ull), c->stream));
     if (n_rows == 0 || c->n == 0) return NPC_OK;
-    if (c->ds) {
-        const int64_t n_blocks = (c->n + DS_BLOCK - 1) / DS_BLOCK;
-        if (!c->d_ds_part) NPC_CUDA(c, cudaMalloc(&c->d_ds_part, (size_t)std::max<int64_t>(c->max_rows, 1) * (size_t)n_blocks * sizeof(double)));
+    const int64_t n_blocks = (c->n + DS_BLOCK - 1) / DS_BLOCK;
+    if ((c->ds || c->pl) && !c->d_ds_part)
+        NPC_CUDA(c, cudaMalloc(&c->d_ds_part, (size_t)std::max<int64_t>(c->max_rows, 1) * (size_t)n_blocks * sizeof(double)));
+    if (c->pl) {
+        // a CTA loads T once and takes every gridDim.y-th row: about 4096 CTAs in all
+        const unsigned gx = (unsigned)((n_blocks + 7) / 8);
+        const unsigned gy = (unsigned)std::min<int64_t>(n_rows, std::max<int64_t>(1, (4096 + gx - 1) / gx));
+        k_count_pl<<<dim3(gx, gy), 256, 0, c->stream>>>(gt, row_stride, d_rows, n_rows, c->n, n_blocks, c->d_ds_part, counts);
+        c->launches++;
+    } else if (c->ds) {
         for (int64_t r0 = 0; r0 < n_rows; r0 += 65535) {                                        // grid y: at most 65,535 rows
             const int64_t nr = std::min<int64_t>(65535, n_rows - r0);
             k_count_ds<<<dim3((unsigned)((n_blocks + 7) / 8), (unsigned)nr), 256, 0, c->stream>>>(gt, row_stride, d_rows + r0, c->n, n_blocks,
@@ -608,7 +630,10 @@ static int launch_decide(npc_ctx *c, const uint8_t *gt, int64_t row_stride, cons
     int rc = ensure_log(c, n_rows);
     if (rc) return rc;
     const unsigned grid = (unsigned)((n_rows + 127) / 128);
-    if (c->ds)
+    if (c->pl)
+        k_decide_pl<<<grid, 128, 0, c->stream>>>(d_rows, n_rows, c->d_ds_part, (c->n + DS_BLOCK - 1) / DS_BLOCK, counts, c->pol, c->n,
+                                                c->d_rowp, c->d_log + c->log_len, c->d_nloci);
+    else if (c->ds)
         k_decide_ds<<<grid, 128, 0, c->stream>>>(d_rows, n_rows, c->d_ds_part, (c->n + DS_BLOCK - 1) / DS_BLOCK, counts, c->pol, c->n,
                                                 c->d_rowp, c->d_log + c->log_len, c->d_nloci);
     else if (c->dose255)
@@ -652,6 +677,9 @@ static int launch_accum(npc_ctx *c, const uint8_t *gt, int64_t row_stride, int64
     } else if (c->dose32) {
         const unsigned grid = (unsigned)((c->n + 4 * D32_THREADS - 1) / (4 * D32_THREADS));
         k_accum_dose32<<<grid, D32_THREADS, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->d_sums);
+    } else if (c->pl) {
+        const unsigned grid = (unsigned)((c->n + 4 * PL_THREADS - 1) / (4 * PL_THREADS));
+        k_accum_pl<<<grid, PL_THREADS, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->d_sums);
     } else if (c->width == 1 && c->ploidy == 2) {
         const int64_t nchunks = (c->n + 7) / 8;
         k_accum_i8x2<64, 8><<<(unsigned)((nchunks + 255) / 256), 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows,
@@ -743,7 +771,7 @@ static int launch_block(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const
     switch (launch_mode(c, c->exact, n_rows, t)) {
     case 1: case 2: return launch_fused(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
     case 3: return launch_wide(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
-    default: {                                                                                  // 0, 4, 5, 6
+    default: {                                                                                  // 0, 4, 5, 6, 7
         int rc = launch_tally(c, gt, row_stride, d_rows, n_rows, c->d_counts);
         if (!rc) rc = launch_decide(c, gt, row_stride, d_rows, n_rows, c->d_counts);
         return rc ? rc : launch_accum(c, gt, row_stride, n_rows);
@@ -816,6 +844,7 @@ static int split_prologue(npc_ctx *c, const void *gt_dev, int64_t row_stride, in
     if (c->ds) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take hard-call (GT) rows only");
     if (c->bed) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not PLINK .bed rows");
     if (c->dose255 || c->dose32) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not BGEN dosage rows");
+    if (c->pl) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not FORMAT/PL rows");
     NPC_CUDA(c, cudaSetDevice(c->device));
     return upload_rows(c, rows, n_rows, rows_on_device, d_rows);
 }

@@ -16,6 +16,7 @@ KIND_GT, KIND_NOTCOV, KIND_ABSENT, KIND_FILTER, CLASS_MAXMIS = range(5)
 GT_BED = 0        # gt_width of a context over PLINK 1 .bed rows (2 bits per sample, ploidy 2): NPC_GT_BED
 GT_DOSE255 = 255  # gt_width of a context over fixed-point dosage rows of BGEN files (uint16 255 x dosage, ploidy 2): NPC_GT_DOSE255
 GT_DOSE32 = 32    # gt_width of a context over 32-bit fixed-point dosage rows of BGEN files at any bit depth (ploidy 2): NPC_GT_DOSE32
+GT_PL = 10        # gt_width of a context over FORMAT/PL rows (one packed uint32 per sample, ploidy 2): NPC_GT_PL
 
 
 def gt_row_bytes(n_samples, ploidy, gt_width):
@@ -96,6 +97,7 @@ def load_library():
         "npc_set_dosage_rows": (C.c_int, [vp, i32]),
         "npc_synth_fill_device": (C.c_int, [vp, vp, i64, i64, i64, C.c_uint64, vp, vp, vp]),
         "npc_gt_row_bytes": (i64, [i64, i32, i32]),
+        "npc_pl_weight_table": (C.c_int, [vp, i32]),
         "npc_version": (C.c_int, []),
         "npc_warmup": (C.c_int, [C.c_int]),
     }
@@ -129,6 +131,16 @@ def plan_shape(n_samples, gt_width=1, num_sms=148, max_smem=232448, n_rows=0, ex
     if rc != 0:
         raise NpcError(f"npc_plan_shape: error {rc}")
     return dict(zip(PLAN_KEYS, list(a)))
+
+
+def pl_weight_table(n=4096):
+    """npc_pl_weight_table: T[x] = fl(10^(-x/10)) correctly rounded for x = 0 .. n - 1 (0 from 3237 on), the weights of
+    FORMAT/PL rows -- host only, no device."""
+    out = np.zeros(n, np.float64)
+    rc = load_library().npc_pl_weight_table(out.ctypes.data, int(n))
+    if rc != 0:
+        raise NpcError(f"npc_pl_weight_table: error {rc}")
+    return out
 
 
 def reduce_contexts(engines, offset=None):

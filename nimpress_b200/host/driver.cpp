@@ -360,16 +360,20 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
                 memcpy(dst, first, (size_t)npc_gt_row_bytes(n, ploidy, gt_width));
             }
             else {
+                if (p.use_pl && rec.alts.size() != 1)
+                    throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/PL rows take biallelic records only (" +
+                                     std::to_string(rec.alts.size()) + " ALT alleles; split them with bcftools norm -m-)");
                 // BCF with the context's layout: the GT payload goes from the inflated blocks straight into the pinned row
                 const bool direct = vcf.load_gt_into(rec, dst, gt_width, ploidy);
                 if (!rec.has_gt || !rec.gt)
-                    throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + (p.use_ds ? " has no DS field" : " has no GT field"));
+                    throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) +
+                                     (p.use_pl ? " has no PL field" : p.use_ds ? " has no DS field" : " has no GT field"));
                 if (p.use_ds && (rec.ploidy != 1 || rec.gt_width != 4))
                     throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/DS with several values per sample is not supported");
                 if (!direct) {
                     if (rec.ploidy > ploidy || rec.gt_width > gt_width)
                         throw LayoutOverflow{ std::max(rec.gt_width, gt_width), std::max(rec.ploidy, ploidy) };
-                    if (rec.gt_width == gt_width && rec.ploidy == ploidy) memcpy(dst, rec.gt, (size_t)n * ploidy * gt_width);
+                    if (rec.gt_width == gt_width && rec.ploidy == ploidy) memcpy(dst, rec.gt, (size_t)npc_gt_row_bytes(n, ploidy, gt_width));
                     else convert_gt(rec, n, gt_width, ploidy, dst);
                 }
                 first = dst;
@@ -470,7 +474,7 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
         outs[k].loci.assign(scores[k]->entries.size(), npc_locus());
         for (size_t j = 0; j < order[k].size(); j++) outs[k].loci[order[k][j]] = logs[k][j];
         outs[k].warnings = make_warnings(*scores[k], *ps[k].M, outs[k].loci, n, p,
-                                         p.use_ds || gt_width == NPC_GT_DOSE255 || gt_width == NPC_GT_DOSE32);
+                                         p.use_ds || p.use_pl || gt_width == NPC_GT_DOSE255 || gt_width == NPC_GT_DOSE32);
     }
     timer.mark("WARN lines (binomial tests)");
 }
@@ -481,7 +485,9 @@ bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores
                                     const GenomeIntervals &cov, const ScoreParams &p, std::vector<ScoreResult> &outs) {
     for (int d : (p.devices.empty() ? std::vector<int>{ p.device } : p.devices)) start_warm(d);
     int width = 1, ploidy = 2;                      // BCF's usual GT layout: int8, diploid
+    if (p.use_ds && p.use_pl) throw InputError("--pl and --dosage: score either FORMAT/PL or FORMAT/DS");
     if (p.use_ds) { width = 4; ploidy = 1; }        // FORMAT/DS: one float per sample
+    if (p.use_pl) { width = NPC_GT_PL; ploidy = 2; }   // FORMAT/PL: one packed word per sample
     bool seekable = true;                           // first try the index-driven pass (needs <file>.tbi / .csi)
     bool dose32 = false;                            // a BGEN pass met a block that only 32-bit dosage rows hold
     for (int attempt = 0; attempt < 6; attempt++) {
@@ -491,11 +497,14 @@ bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores
         const int fixed = vcf->fixed_layout();
         ScoreParams q = p;
         if (fixed == NPC_GT_BED && p.use_ds) throw InputError("--dosage: a PLINK fileset holds hard calls only, no FORMAT/DS");
+        if (fixed == NPC_GT_BED && p.use_pl) throw InputError("--pl: a PLINK fileset holds hard calls only, no FORMAT/PL");
+        if (fixed == NPC_GT_DOSE255 && p.use_pl) throw InputError("--pl: a BGEN file holds genotype probabilities, no FORMAT/PL");
         if (fixed != VariantSource::NO_FIXED_LAYOUT) {
             width = dose32 ? NPC_GT_DOSE32 : fixed; ploidy = 2; seekable = false;
             q.use_ds = false;                       // BGEN rows are dosages already: --dosage changes nothing
         }
         vcf->set_dosage_mode(q.use_ds);
+        vcf->set_pl_mode(q.use_pl);
         try {
             run_pass(scores, *vcf, genotype_path, seekable, cov, q, width, ploidy, outs);
             return true;

@@ -28,6 +28,7 @@ struct ScoreParams {
     std::vector<int> devices;              // several GPUs: the score rows are split into contiguous ranges, one per device (empty: `device`)
     bool exact_order = false;              // npc_set_exact_order: bit-for-bit reference summation order
     bool use_ds = false;                   // score FORMAT/DS (fp32 expected ALT dosage) instead of FORMAT/GT -- not a reference option
+    bool use_pl = false;                   // score FORMAT/PL as posterior expected dosages (NPC_GT_PL rows) -- not a reference option
 };
 
 struct ScoreResult {

@@ -25,6 +25,7 @@ static ScoreParams to_params(const nph_params *p) {
     q.mincs = p->mincs; q.maxmis = p->maxmis; q.afmisp = p->afmisp;
     for (int d = 0; d < 32; d++) if (((uint32_t)p->device_mask >> d) & 1u) q.devices.push_back(d);
     q.use_ds = p->use_ds != 0;
+    q.use_pl = p->use_pl != 0;
     return q;
 }
 
@@ -187,6 +188,7 @@ int nph_read_gt(const char *genotype_path, uint8_t *out, int64_t row_bytes, int6
         std::unique_ptr<VariantSource> vcf = open_variant_source(genotype_path);
         if (!vcf) return NPH_EOPEN_VCF;
         if (const char *e = getenv("NIMPRESS_READ_DS")) if (*e && *e != '0') vcf->set_dosage_mode(true);   // tests: FORMAT/DS instead of GT
+        if (const char *e = getenv("NIMPRESS_READ_PL")) if (*e && *e != '0') vcf->set_pl_mode(true);       // tests: FORMAT/PL rows
         int bgen_layout = NPC_GT_DOSE255;                                                                   // BGEN rows
         if (const char *e = getenv("NIMPRESS_READ_DOSE32")) if (*e && *e != '0') bgen_layout = NPC_GT_DOSE32;
         VariantRecord rec;
@@ -277,6 +279,11 @@ static const char *USAGE =
     "  --dosage           Score FORMAT/DS (expected ALT-allele dosage, one float per sample) instead of\n"
     "                     FORMAT/GT (not a reference option: the reference lists it under Future).\n"
     "                     Not with a PLINK fileset; with a BGEN file it changes nothing.\n"
+    "  --pl               Score FORMAT/PL (phred-scaled genotype likelihoods) as the posterior expected\n"
+    "                     dosage under a Hardy-Weinberg prior at the score file's EAF, instead of\n"
+    "                     FORMAT/GT (not a reference option).  Biallelic records only (split others\n"
+    "                     with bcftools norm -m-); diploid and haploid samples.  Not with --dosage, a\n"
+    "                     PLINK fileset or a BGEN file.  No AF-mismatch warnings.\n"
     "PLINK 1 fileset (not a reference input): X.bed with X.bim and X.fam, recognised by its magic bytes.\n"
     "  REF = A2 (.bim column 6), ALT = A1 (column 5), sample names = .fam IID; FILTER is always \".\".\n"
     "BGEN v1.2 file (not a reference input): layout 2, 1-16 bits per probability, uncompressed or zlib,\n"
@@ -357,6 +364,7 @@ int nph_main(int argc, char **argv) {
             else if (a == "--ignorefilt") p.ignorefilt = 1;
             else if (a == "--exact-order") p.exact_order = 1;
             else if (a == "--dosage") p.use_ds = 1;
+            else if (a == "--pl") p.use_pl = 1;
             else if (a.size() > 1 && a[0] == '-') throw InputError("unknown option " + a);
             else if (npos < 2) pos[npos++] = a;
             else throw InputError("too many arguments");

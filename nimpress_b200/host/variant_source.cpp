@@ -375,6 +375,54 @@ static int64_t rlen_from_info(const char *info, size_t len, int64_t pos, int64_t
 }
 
 // ------------------------------------------------------------------------------------------
+// FORMAT/PL rows (DESIGN.md 4.10) -- not a reference input
+// ------------------------------------------------------------------------------------------
+
+// One sample's PL values -> its word of an NPC_GT_PL row: a | b << 12 | j << 24 | ploidy << 26 with m the smallest PL, j
+// the index of its first occurrence, a, b the other genotypes' PL - m in genotype order, saturated at 4095 (T is 0 from
+// 3237 on, so nothing is lost).  No value or any missing value: a missing sample.
+static uint32_t pl_word(const int64_t *v, int cnt, bool missing, const VariantRecord &rec, const std::string &sample) {
+    if (missing || cnt == 0) return 0xFFFFFFFFu;
+    auto bad = [&](const std::string &m) {
+        return InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/PL of sample " + sample + ": " + m);
+    };
+    if (cnt != 2 && cnt != 3)
+        throw bad(std::to_string(cnt) + " values (a biallelic record has 3 for a diploid sample, 2 for a haploid one)");
+    int j = 0;
+    for (int g = 0; g < cnt; g++) {
+        if (v[g] < 0) throw bad("negative value " + std::to_string(v[g]));
+        if (v[g] < v[j]) j = g;
+    }
+    uint32_t x[2] = { 0, 0 };
+    for (int g = 0, k = 0; g < cnt; g++)
+        if (g != j) x[k++] = (uint32_t)std::min<int64_t>(v[g] - v[j], 4095);
+    return x[0] | x[1] << 12 | (uint32_t)j << 24 | (uint32_t)(cnt - 1) << 26;
+}
+
+// A BCF PL field (per sample `len` integers of esz bytes, missing = MIN and vector_end = MIN + 1 of the width) -> n words
+static void pack_pl_typed(const uint8_t *q, size_t esz, uint32_t len, int64_t n, uint8_t *dst, const VariantRecord &rec,
+                          const std::vector<std::string> &samples) {
+    for (int64_t i = 0; i < n; i++) {
+        int64_t v[3];
+        int cnt = 0;
+        bool missing = false;
+        for (uint32_t k = 0; k < len; k++) {
+            const uint8_t *e = q + ((size_t)i * len + k) * esz;
+            int64_t x, miss, vend;
+            if (esz == 1) { x = (int8_t)*e; miss = INT8_MIN; vend = INT8_MIN + 1; }
+            else if (esz == 2) { int16_t t; memcpy(&t, e, 2); x = t; miss = INT16_MIN; vend = INT16_MIN + 1; }
+            else { int32_t t; memcpy(&t, e, 4); x = t; miss = INT32_MIN; vend = INT32_MIN + 1; }
+            if (x == vend) break;
+            if (x == miss) missing = true;
+            else if (cnt < 3) v[cnt] = x;
+            cnt++;
+        }
+        const uint32_t w = pl_word(v, cnt, missing, rec, samples[i]);
+        memcpy(dst + 4 * i, &w, 4);
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // VCF text
 // ------------------------------------------------------------------------------------------
 
@@ -434,7 +482,8 @@ public:
         for (const char *q = col[8], *qe = col[8] + len[8]; q <= qe; k++) {
             const char *t = (const char *)memchr(q, ':', qe - q);
             size_t l = (t ? t : qe) - q;
-            if (l == 2 && (dosage_ ? (q[0] == 'D' && q[1] == 'S') : (q[0] == 'G' && q[1] == 'T'))) gt_idx = k;
+            const char c0 = pl_ ? 'P' : dosage_ ? 'D' : 'G', c1 = pl_ ? 'L' : dosage_ ? 'S' : 'T';
+            if (l == 2 && q[0] == c0 && q[1] == c1) gt_idx = k;
             if (!t) break;
             q = t + 1;
         }
@@ -445,11 +494,25 @@ public:
         gt_p_ = p; gt_idx_ = gt_idx; gt_loaded_ = false;
         return true;
     }
+    bool load_gt_into(VariantRecord &rec, uint8_t *dst, int want_width, int want_ploidy) override {
+        if (!pl_ || want_width != NPC_GT_PL || want_ploidy != 2 || !rec.has_gt || gt_loaded_) {
+            load_gt(rec);
+            return false;
+        }
+        gt_loaded_ = true;
+        load_pl(rec, dst);
+        return true;
+    }
     void load_gt(VariantRecord &rec) override {
         if (!rec.has_gt || gt_loaded_) return;
         gt_loaded_ = true;
         const char *p = gt_p_, *end = line_.data() + line_.size();
         const int64_t n = n_samples();
+        if (pl_) {
+            gt_.resize((size_t)n * 4);
+            load_pl(rec, gt_.data());
+            return;
+        }
         if (dosage_) {                                   // DS sub-field of every sample -> BCF floats ("." = missing)
             gt_.resize((size_t)n * 4);
             int maxv = 1;
@@ -538,6 +601,55 @@ public:
         rec.ploidy = maxp; rec.gt = gt_.data();
     }
 private:
+    // PL sub-field of every sample -> packed words in dst ("." or an absent sub-field = a missing sample)
+    void load_pl(VariantRecord &rec, uint8_t *dst) {
+        const char *p = gt_p_, *end = line_.data() + line_.size();
+        const int64_t n = n_samples();
+        for (int64_t i = 0; i < n; i++) {
+            const char *s = p <= end ? p : end, *se = end;
+            if (p <= end) {
+                const char *t = (const char *)memchr(p, '\t', end - p);
+                se = t ? t : end;
+                p = t ? t + 1 : end + 1;
+            }
+            for (int f = 0; f < gt_idx_ && s < se; f++) {
+                const char *t = (const char *)memchr(s, ':', se - s);
+                s = t ? t + 1 : se;
+            }
+            const char *fe = (const char *)memchr(s, ':', se - s);
+            if (!fe) fe = se;
+            int64_t v[3];
+            int cnt = 0;
+            bool missing = false;
+            while (s < fe) {
+                const char *c = (const char *)memchr(s, ',', fe - s);
+                if (!c) c = fe;
+                if (c - s == 1 && *s == '.') missing = true;
+                else {
+                    const char *d = s;
+                    const bool neg = *d == '-';
+                    if (neg || *d == '+') d++;
+                    if (d == c || c - d > 10)
+                        throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/PL of sample " + samples_[i] +
+                                         ": value \"" + std::string(s, c - s) + "\" is not an integer");
+                    int64_t x = 0;
+                    for (; d < c; d++) {
+                        if (*d < '0' || *d > '9')
+                            throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/PL of sample " + samples_[i] +
+                                         ": value \"" + std::string(s, c - s) + "\" is not an integer");
+                        x = x * 10 + (*d - '0');
+                    }
+                    if (cnt < 3) v[cnt] = neg ? -x : x;
+                }
+                cnt++;
+                s = c + 1;
+                if (c == fe) break;
+            }
+            const uint32_t w = pl_word(v, cnt, missing, rec, samples_[i]);
+            memcpy(dst + 4 * i, &w, 4);
+        }
+        rec.ploidy = 2; rec.gt_width = NPC_GT_PL; rec.gt = dst;
+    }
     std::unique_ptr<InflateStream> in_;
     std::string line_, contig_;
     const char *gt_p_ = nullptr;
@@ -643,6 +755,7 @@ public:
             }
             q += bytes;
         }
+        pack_pl(rec, nullptr);
     }
     // The GT payload straight from the inflated blocks into dst (the pinned staging row) when its layout is the wanted
     // one: the only copy the genotypes make on the host.  The field headers in front of it are a few bytes each.
@@ -679,12 +792,13 @@ public:
                 if ((int64_t)n_sample_ != n_samples()) throw InputError("BCF: record sample count differs from header");
                 gt_done_ = true;
                 rec.has_gt = true; rec.gt_width = (int)esz; rec.ploidy = (int)len;
-                const bool direct = (int)esz == want_width && (int)len == want_ploidy;
+                const bool direct = !pl_ && (int)esz == want_width && (int)len == want_ploidy;
                 uint8_t *to = dst;
                 if (!direct) { indiv_.resize(bytes); to = indiv_.data(); }
                 if (!in_->read_exact(to, bytes)) throw InputError("BCF: truncated record");
                 rec.gt = to;
                 indiv_left_ = left - bytes;                                 // later fields: skipped when the next record is read
+                if (pl_) return pack_pl(rec, want_width == NPC_GT_PL && want_ploidy == 2 ? dst : nullptr);
                 return direct;
             }
             if (!in_->skip(bytes)) throw InputError("BCF: truncated record");
@@ -789,9 +903,12 @@ private:
         gt_key_ = it == seen.end() ? -1 : it->second;
         it = seen.find("DS");
         ds_key_ = it == seen.end() ? -1 : it->second;
+        it = seen.find("PL");
+        pl_key_ = it == seen.end() ? -1 : it->second;
     }
-    // the FORMAT field the caller reads: GT (typed ints) or, in dosage mode, DS (floats)
+    // the FORMAT field the caller reads: GT (typed ints), in dosage mode DS (floats), in PL mode PL (typed ints)
     bool wanted(int32_t key, int type) const {
+        if (pl_) return key == pl_key_ && (type == 1 || type == 2 || type == 3);
         return dosage_ ? (key == ds_key_ && type == 5) : (key == gt_key_ && (type == 1 || type == 2 || type == 3));
     }
     std::unique_ptr<InflateStream> in_;
@@ -818,8 +935,21 @@ private:
             if (wanted(key, type)) { rec.has_gt = true; rec.gt = q; rec.gt_width = (int)esz; rec.ploidy = (int)len; }
             q += bytes;
         }
+        pack_pl(rec, nullptr);
     }
-    int32_t gt_key_ = -1, ds_key_ = -1;
+    // PL mode: the typed integers rec.gt points at -> packed words in dst, or in pl_buf_ when dst is null; true when
+    // written to dst.  Nothing to do in the other modes or without a PL field.
+    bool pack_pl(VariantRecord &rec, uint8_t *dst) {
+        if (!pl_ || !rec.has_gt || !rec.gt) return false;
+        const int64_t n = n_samples();
+        if (!dst) { pl_buf_.resize((size_t)n * 4); }
+        uint8_t *to = dst ? dst : pl_buf_.data();
+        pack_pl_typed(rec.gt, (size_t)rec.gt_width, (uint32_t)rec.ploidy, n, to, rec, samples_);
+        rec.gt = to; rec.gt_width = NPC_GT_PL; rec.ploidy = 2;
+        return dst != nullptr;
+    }
+    std::vector<uint8_t> pl_buf_;
+    int32_t gt_key_ = -1, ds_key_ = -1, pl_key_ = -1;
     size_t indiv_left_ = 0;
     uint32_t n_fmt_ = 0, n_sample_ = 0;
     bool gt_done_ = true;

@@ -101,6 +101,10 @@ public:
     // FORMAT/DS instead of FORMAT/GT (not a reference feature: README.md:162-165 lists dosage input under "Future"):
     // load_gt / load_gt_into then deliver one BCF float per value, gt_width = 4, ploidy = values per sample.
     virtual void set_dosage_mode(bool on) { dosage_ = on; }
+    // FORMAT/PL instead of FORMAT/GT (not a reference feature, DESIGN.md 4.10): load_gt / load_gt_into then deliver one packed
+    // uint32 word per sample (npc_pl.cuh), gt_width = NPC_GT_PL, ploidy = 2.  A sample with a PL count other than 2 or 3
+    // (or none), or a negative PL, throws InputError naming the variant.
+    void set_pl_mode(bool on) { pl_ = on; }
     // The one device layout this source's rows come in, or NO_FIXED_LAYOUT for VCF / BCF (whose layout follows the records):
     // NPC_GT_BED for a PLINK 1 fileset (.bed rows as stored, ploidy 2, ceil(n/4) bytes), NPC_GT_DOSE255 for a BGEN file
     // (one uint16 dosage numerator per sample, ploidy 2).  A BGEN file also delivers NPC_GT_DOSE32 rows when load_gt_into
@@ -111,6 +115,7 @@ public:
     // here.  Call before the rows' bytes are read.
     virtual void wait_rows() {}
     bool dosage_mode() const { return dosage_; }
+    bool pl_mode() const { return pl_; }
     const std::vector<std::string> &samples() const { return samples_; }
     int64_t n_samples() const { return (int64_t)samples_.size(); }
 protected:
@@ -122,7 +127,7 @@ protected:
     virtual bool index_names_contigs() const { return true; }         // text VCF: the index must carry the contig names
     std::vector<std::string> samples_;
     std::unique_ptr<RegionIndex> index_;
-    bool dosage_ = false;
+    bool dosage_ = false, pl_ = false;
 private:
     struct Region { int ref; int64_t beg0, end0; };                   // 0-based half open
     std::vector<Region> regions_;

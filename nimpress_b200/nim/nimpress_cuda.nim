@@ -41,6 +41,7 @@ const
   npcGtBed* = 0'i32       ## gtWidth of a context over PLINK 1 .bed rows (2 bits per sample, ploidy 2)
   npcGtDose255* = 255'i32 ## gtWidth of a context over BGEN fixed-point dosage rows (uint16 255 x dosage, ploidy 2)
   npcGtDose32* = 32'i32   ## gtWidth of a context over BGEN 32-bit dosage rows (16-byte header with D, uint32 per sample, ploidy 2)
+  npcGtPl* = 10'i32       ## gtWidth of a context over FORMAT/PL rows (packed uint32 per sample, ploidy 2)
 
 {.push importc, cdecl, dynlib: npcLib.}
 proc npc_create*(ctx: ptr NpcCtx; device: cint; nSamples: int64; ploidy, gtWidth: int32;
@@ -77,7 +78,8 @@ proc npc_launch_count*(ctx: NpcCtx): int64
 proc npc_multi_contractions*(ctx: NpcCtx): int64
 proc npc_kernel_shape*(ctx: NpcCtx; shape: ptr array[8, int32]): cint
 proc npc_kernel_shape2*(ctx: NpcCtx; n_rows: int64; shape: ptr array[8, int32]): cint
-proc npc_gt_row_bytes*(n_samples: int64; ploidy, gt_width: int32): int64   ## bytes of a row (gt_width npcGtBed: 2-bit rows, npcGtDose255: 2 bytes per sample, npcGtDose32: 16 + 4 per sample)
+proc npc_gt_row_bytes*(n_samples: int64; ploidy, gt_width: int32): int64   ## bytes of a row (gt_width npcGtBed: 2-bit rows, npcGtDose255: 2 bytes per sample, npcGtDose32: 16 + 4 per sample, npcGtPl: 4 per sample)
+proc npc_pl_weight_table*(out_tab: ptr float64; n: int32): cint   ## T[x] = fl(10^(-x/10)) of FORMAT/PL rows, x = 0 .. n - 1; no device
 proc npc_plan_shape*(n_samples: int64; gt_width, num_sms, max_smem: int32; n_rows: int64; exact: int32; plan: ptr array[16, int32]): cint
 proc npc_synth_fill_device*(ctx: NpcCtx; gtDev: pointer; rowStride, v0, nRows: int64; seed: uint64;
                             afThr16Dev, missThr24Dev: ptr uint32; altCodeDev: ptr int32): cint
