@@ -193,6 +193,19 @@ int  npc_create(npc_ctx **out, int device, int64_t n_samples, int32_t ploidy, in
  * and large launches. */
 int  npc_create2(npc_ctx **out, int device, int64_t n_samples, int32_t ploidy, int32_t gt_width,
                  int64_t max_rows_per_block, int32_t n_slots, int64_t staging_rows);
+/* A context that scores n_keep of the n_row_samples samples its staged rows carry: keep[0..n_keep) ascending, distinct,
+ * < n_row_samples.  n_samples of the context is n_keep: sums, tallies, --maxmis, scores_out, launch shapes.  Staging slots
+ * (npc_stage_acquire) hold rows of n_row_samples samples; npc_score_block and npc_stage_upload compact them on the device.
+ * The *_device entry points, npc_resident_adopt and npc_score_resident_multi take compact rows (the context's layout).
+ * A compact row is byte for byte the row of a file holding only the kept samples, in the same order (DESIGN.md 4.11), so
+ * scoring through such a context gives exactly what a context of n_keep samples gives on that file.  NPC_EINVAL for
+ * a keep list that breaks these rules. */
+int npc_create_subset(npc_ctx **out, int device, int64_t n_row_samples, const int64_t *keep, int64_t n_keep, int32_t ploidy,
+                      int32_t gt_width, int64_t max_rows_per_block, int32_t n_slots, int64_t staging_rows);
+/* The compaction alone, for rows already in device memory (src rows of n_row_samples, dst rows of n_keep; both 16-byte
+ * aligned, strides multiples of 16 holding a whole row).  Asynchronous, on the context's stream (npc_set_stream).
+ * NPC_ESTATE for a context not created by npc_create_subset. */
+int npc_gather_rows_device(npc_ctx *ctx, const void *src, int64_t src_stride, int64_t n_rows, void *dst, int64_t dst_stride);
 void npc_destroy(npc_ctx *ctx);
 const char *npc_last_error(const npc_ctx *ctx);   /* ctx may be NULL: text of the last npc_create failure */
 

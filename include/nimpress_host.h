@@ -66,6 +66,14 @@ typedef struct {
     int32_t use_pl;         /* 1: score FORMAT/PL (phred-scaled genotype likelihoods of biallelic VCF / BCF records) as posterior
                                expected dosages at the score file's eaf (NPC_GT_PL rows, DESIGN.md 4.10) instead of FORMAT/GT;
                                not with use_ds, a PLINK fileset or a BGEN file; not in the reference */
+    const char *samples_path; /* NULL: score every sample.  Else a list of sample names, one per line (the whole line, a trailing
+                               \r stripped, blank lines skipped), matched against the names the results carry (VCF / BCF header,
+                               .fam IID, BGEN identifier or .sample ID_2): only the listed samples are scored, in the genotype
+                               file's order, exactly as a genotype file holding only them would be (cohort EAF, --maxmis, WARN
+                               lines; DESIGN.md 4.11).  An unknown or twice-listed name, a name the file holds twice, an empty
+                               subset or an unreadable list is NPH_EINPUT.  Not in the reference (plink --keep, bcftools -S) */
+    int32_t exclude_samples;  /* 1: score the samples the list does NOT name (plink --remove, bcftools -S ^FILE); names the file
+                               lacks are ignored */
 } nph_params;
 
 typedef struct nph_result nph_result;
@@ -93,7 +101,8 @@ const char *nph_result_warnings(const nph_result *r);    /* "WARN ...\n" lines, 
 void nph_result_free(nph_result *r);
 const char *nph_last_error(void);
 
-/* CPU only: per score row kind (NPC_KIND_*) and eaidx after coverage / lookup / FILTER. */
+/* CPU only: per score row kind (NPC_KIND_*) and eaidx after coverage / lookup / FILTER; *n_samples_out the samples a
+ * scoring call would score (the kept ones under samples_path). */
 int nph_plan(const char *score_path, const char *genotype_path, const char *bed_path, const nph_params *p,
              int32_t *kind_out, int32_t *eaidx_out, int64_t cap, int64_t *n_rows_out, int64_t *n_samples_out);
 /* The same through the reader the scoring calls use: when <genotypes>.tbi / .csi exists, the file is

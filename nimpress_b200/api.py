@@ -52,7 +52,7 @@ class _Params(C.Structure):
                 ("ignorefilt", C.c_int32), ("use_cov", C.c_int32), ("device", C.c_int32),
                 ("exact_order", C.c_int32), ("device_mask", C.c_int32),
                 ("mincs", C.c_int64), ("maxmis", C.c_double), ("afmisp", C.c_double),
-                ("use_ds", C.c_int32), ("use_pl", C.c_int32)]
+                ("use_ds", C.c_int32), ("use_pl", C.c_int32), ("samples_path", C.c_char_p), ("exclude_samples", C.c_int32)]
 
 
 _host = None
@@ -143,14 +143,16 @@ class Result:
 
 def run(score_path, genotype_path, bed_path=None, imp_locus=ImputeMethodLocus.ps, imp_missing=ImputeMethodMissing.homref,
         imp_sample=ImputeMethodSample.int_ps, maxmis=0.05, afmisp=0.001, mincs=100, ignorefilt=False, device=0,
-        exact_order=False, devices=None, dosage=False, pl=False):
+        exact_order=False, devices=None, dosage=False, pl=False, samples=None, exclude_samples=False):
     """nph_compute_polygenic_scores -> Result (scores, per-locus records, WARN text).  devices: list of CUDA
     device indices to split the score rows over (npc_reduce combines their partial sums).  dosage: score FORMAT/DS;
-    pl: score FORMAT/PL as posterior expected dosages at the score file's eaf (DESIGN.md 4.10)."""
+    pl: score FORMAT/PL as posterior expected dosages at the score file's eaf (DESIGN.md 4.10).  samples: path of a
+    list of sample names to score (one per line; DESIGN.md 4.11), exclude_samples: score the others instead."""
     L = load_host_library()
     mask = sum(1 << int(d) for d in set(devices)) if devices else 0
     p = _Params(int(imp_locus), int(imp_missing), int(imp_sample), int(ignorefilt), int(bed_path is not None), device,
-                int(bool(exact_order)), mask, int(mincs), float(maxmis), float(afmisp), int(bool(dosage)), int(bool(pl)))
+                int(bool(exact_order)), mask, int(mincs), float(maxmis), float(afmisp), int(bool(dosage)), int(bool(pl)),
+                os.fsencode(samples) if samples else None, int(bool(exclude_samples)))
     h = C.c_void_p()
     rc = L.nph_compute_polygenic_scores(os.fsencode(score_path), os.fsencode(genotype_path),
                                         os.fsencode(bed_path) if bed_path else None, C.byref(p), C.byref(h))
@@ -160,12 +162,13 @@ def run(score_path, genotype_path, bed_path=None, imp_locus=ImputeMethodLocus.ps
 
 def run_multi(score_paths, genotype_path, bed_path=None, imp_locus=ImputeMethodLocus.ps, imp_missing=ImputeMethodMissing.homref,
               imp_sample=ImputeMethodSample.int_ps, maxmis=0.05, afmisp=0.001, mincs=100, ignorefilt=False, device=0,
-              exact_order=False, pl=False):
+              exact_order=False, pl=False, samples=None, exclude_samples=False):
     """nph_compute_polygenic_scores_multi: several score files over one pass of the genotype file
     -> [Result], each equal to run() on that file alone."""
     L = load_host_library()
     p = _Params(int(imp_locus), int(imp_missing), int(imp_sample), int(ignorefilt), int(bed_path is not None), device,
-                int(bool(exact_order)), 0, int(mincs), float(maxmis), float(afmisp), 0, int(bool(pl)))
+                int(bool(exact_order)), 0, int(mincs), float(maxmis), float(afmisp), 0, int(bool(pl)),
+                os.fsencode(samples) if samples else None, int(bool(exclude_samples)))
     paths = (C.c_char_p * len(score_paths))(*[os.fsencode(s) for s in score_paths])
     hs = (C.c_void_p * len(score_paths))()
     rc = L.nph_compute_polygenic_scores_multi(paths, len(score_paths), os.fsencode(genotype_path),

@@ -19,6 +19,7 @@
 #include "npc_dose255.cuh"
 #include "npc_dose32.cuh"
 #include "npc_pl.cuh"
+#include "npc_subset.cuh"
 
 using namespace npc;
 
@@ -31,7 +32,15 @@ struct npc_ctx {
     int64_t max_rows = 0;
     int64_t staging_rows = 0;               // rows per pinned staging slot (<= max_rows)
     int32_t n_slots = 0;
-    int64_t row_stride = 0;                 // of the staging ring
+    int64_t row_stride = 0;                 // of the context's rows (the staging ring's too, unless a subset context)
+    int64_t stage_stride = 0;               // of the staging ring's rows: n_row samples
+    // subset context (npc_create_subset, npc_subset.cuh): staged rows carry n_row samples, the context scores the n of them
+    // that d_keep names; rows are compacted on the device after the H2D copy (into d_gt / the slab, from d_raw)
+    bool sub = false;
+    int64_t n_row = 0;
+    std::vector<int32_t> keep;              // the kept sample indices until create_impl uploads them
+    int32_t *d_keep = nullptr;              // n ascending sample indices, zero-padded to a multiple of SUB_PAD
+    std::vector<uint8_t *> d_raw;           // per staging slot: its full rows on the device
     cudaStream_t own_stream = nullptr, stream = nullptr, copy_stream = nullptr;
     std::vector<uint8_t *> h_gt, d_gt;
     std::vector<cudaEvent_t> ev_h2d, ev_done;
@@ -150,6 +159,8 @@ extern "C" void npc_destroy(npc_ctx *ctx) {
     cudaDeviceSynchronize();
     for (auto p : ctx->h_gt) if (p) cudaFreeHost(p);
     for (auto p : ctx->d_gt) if (p) cudaFree(p);
+    for (auto p : ctx->d_raw) if (p) cudaFree(p);
+    cudaFree(ctx->d_keep);
     for (auto e : ctx->ev_h2d) if (e) cudaEventDestroy(e);
     for (auto e : ctx->ev_done) if (e) cudaEventDestroy(e);
     cudaFree(ctx->d_sums); cudaFree(ctx->d_out); cudaFree(ctx->d_nloci); cudaFree(ctx->d_counts);
@@ -346,13 +357,21 @@ static int create_impl(npc_ctx *c) {
     NPC_CUDA(c, cudaMalloc(&c->d_log, c->log_cap * sizeof(npc_locus)));
     c->row_stride = ((npc_gt_row_bytes(c->n, c->ploidy, c->width) + 127) / 128) * 128;
     if (c->row_stride == 0) c->row_stride = 128;
-    c->h_gt.assign(c->n_slots, nullptr); c->d_gt.assign(c->n_slots, nullptr);
+    c->stage_stride = c->row_stride;
+    if (c->sub) {
+        c->stage_stride = std::max<int64_t>(128, ((npc_gt_row_bytes(c->n_row, c->ploidy, c->width) + 127) / 128) * 128);
+        c->keep.resize((size_t)((c->n + SUB_PAD - 1) / SUB_PAD * SUB_PAD), 0);
+        NPC_CUDA(c, cudaMalloc(&c->d_keep, c->keep.size() * sizeof(int32_t)));
+        NPC_CUDA(c, cudaMemcpy(c->d_keep, c->keep.data(), c->keep.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+        std::vector<int32_t>().swap(c->keep);
+    }
+    c->h_gt.assign(c->n_slots, nullptr); c->d_gt.assign(c->n_slots, nullptr); c->d_raw.assign(c->n_slots, nullptr);
     c->ev_h2d.assign(c->n_slots, nullptr); c->ev_done.assign(c->n_slots, nullptr);
     c->slot_state.assign(c->n_slots, 0);
     for (int s = 0; s < c->n_slots; s++) {
         // pinned host slots only: the device copy of a slot is allocated when npc_score_block first needs it
         // (the resident path uploads straight into the slab)
-        const size_t bytes = (size_t)c->row_stride * (size_t)std::max<int64_t>(c->staging_rows, 1);
+        const size_t bytes = (size_t)c->stage_stride * (size_t)std::max<int64_t>(c->staging_rows, 1);
         // (write-combined memory was measured no faster: the H2D copy runs at the PCIe rate either way)
         NPC_CUDA(c, cudaHostAlloc((void **)&c->h_gt[s], bytes, cudaHostAllocDefault));
         NPC_CUDA(c, cudaEventCreateWithFlags(&c->ev_h2d[s], cudaEventDisableTiming));
@@ -369,8 +388,9 @@ extern "C" int npc_create(npc_ctx **out, int device, int64_t n_samples, int32_t 
     return npc_create2(out, device, n_samples, ploidy, gt_width, max_rows_per_block, n_slots, max_rows_per_block);
 }
 
-extern "C" int npc_create2(npc_ctx **out, int device, int64_t n_samples, int32_t ploidy, int32_t gt_width,
-                           int64_t max_rows_per_block, int32_t n_slots, int64_t staging_rows) {
+// keep == nullptr: a context over n_samples samples (npc_create2); else over keep[0..n_samples) of rows of n_row samples
+static int create_ctx(npc_ctx **out, int device, int64_t n_row, const int64_t *keep, int64_t n_samples, int32_t ploidy,
+                      int32_t gt_width, int64_t max_rows_per_block, int32_t n_slots, int64_t staging_rows) {
     if (!out) return NPC_EINVAL;
     *out = nullptr;
     if (n_samples < 0 || ploidy < 1 || ploidy > 64 ||
@@ -382,6 +402,12 @@ extern "C" int npc_create2(npc_ctx **out, int device, int64_t n_samples, int32_t
         return NPC_EINVAL;
     }
     npc_ctx *c = new npc_ctx();
+    c->n_row = n_row;
+    if (keep) {
+        c->sub = true;
+        c->keep.resize((size_t)n_samples);
+        for (int64_t i = 0; i < n_samples; i++) c->keep[(size_t)i] = (int32_t)keep[i];
+    }
     c->device = device; c->n = n_samples; c->ploidy = ploidy; c->width = gt_width; c->bed = gt_width == NPC_GT_BED;
     c->dose255 = gt_width == NPC_GT_DOSE255; c->dose32 = gt_width == NPC_GT_DOSE32; c->pl = gt_width == NPC_GT_PL;
     c->max_rows = max_rows_per_block; c->n_slots = n_slots; c->staging_rows = staging_rows;
@@ -395,6 +421,26 @@ extern "C" int npc_create2(npc_ctx **out, int device, int64_t n_samples, int32_t
     }
     *out = c;
     return NPC_OK;
+}
+
+extern "C" int npc_create2(npc_ctx **out, int device, int64_t n_samples, int32_t ploidy, int32_t gt_width,
+                           int64_t max_rows_per_block, int32_t n_slots, int64_t staging_rows) {
+    return create_ctx(out, device, n_samples, nullptr, n_samples, ploidy, gt_width, max_rows_per_block, n_slots, staging_rows);
+}
+
+extern "C" int npc_create_subset(npc_ctx **out, int device, int64_t n_row_samples, const int64_t *keep, int64_t n_keep,
+                                 int32_t ploidy, int32_t gt_width, int64_t max_rows_per_block, int32_t n_slots,
+                                 int64_t staging_rows) {
+    if (!out) return NPC_EINVAL;
+    *out = nullptr;
+    // int32 indices on the device; ascending and distinct, so that a compact row keeps the file's sample order
+    bool ok = keep && n_keep >= 1 && n_row_samples >= n_keep && n_row_samples <= INT32_MAX;
+    for (int64_t i = 0; ok && i < n_keep; i++) ok = keep[i] >= 0 && keep[i] < n_row_samples && (i == 0 || keep[i] > keep[i - 1]);
+    if (!ok) {
+        g_create_error = "npc_create_subset: keep must hold 1 .. n_row_samples ascending, distinct indices below n_row_samples";
+        return NPC_EINVAL;
+    }
+    return create_ctx(out, device, n_row_samples, keep, n_keep, ploidy, gt_width, max_rows_per_block, n_slots, staging_rows);
 }
 
 extern "C" int npc_set_stream(npc_ctx *ctx, void *cuda_stream) {
@@ -779,6 +825,49 @@ static int launch_block(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const
     }
 }
 
+// ---- subset contexts: compaction ------------------------------------------------------------
+
+// n_rows full rows (n_row samples, src_stride apart) -> compact rows of the context's layout (dst_stride apart), on stream st
+static int launch_gather(npc_ctx *c, const uint8_t *src, int64_t src_stride, int64_t n_rows, uint8_t *dst, int64_t dst_stride,
+                         cudaStream_t st) {
+    if (n_rows == 0) return NPC_OK;
+    const int64_t E = c->bed ? 0 : c->dose255 ? 2 : (c->dose32 || c->pl) ? 4 : (int64_t)c->ploidy * c->width;
+    const int hdr = c->dose32 ? D32_HEADER : 0;
+    // threads per row: one per 16 output bytes (2- and 4-byte samples), 4 bytes (.bed) or unit; a grid-stride loop beyond
+    const int64_t per_row = c->bed ? (c->n + 15) / 16 : (E == 2 || E == 4) ? (c->n * E + 15) / 16 : c->n * (E % 4 ? E : E / 4);
+    const unsigned gx = (unsigned)std::max<int64_t>(1, std::min<int64_t>((per_row + SUB_THREADS - 1) / SUB_THREADS, 1024));
+    for (int64_t r0 = 0; r0 < n_rows; r0 += 65535) {                                            // grid y: at most 65,535 rows
+        const dim3 grid(gx, (unsigned)std::min<int64_t>(65535, n_rows - r0));
+        const uint8_t *s = src + r0 * src_stride;
+        uint8_t *d = dst + r0 * dst_stride;
+        if (c->bed) k_gather_bed<<<grid, SUB_THREADS, 0, st>>>(s, src_stride, d, dst_stride, c->d_keep, c->n);
+        else if (E == 2) k_gather_vec<uint16_t><<<grid, SUB_THREADS, 0, st>>>(s, src_stride, d, dst_stride, c->d_keep, c->n, hdr);
+        else if (E == 4) k_gather_vec<uint32_t><<<grid, SUB_THREADS, 0, st>>>(s, src_stride, d, dst_stride, c->d_keep, c->n, hdr);
+        else if (E % 4 == 0) k_gather_unit<uint32_t><<<grid, SUB_THREADS, 0, st>>>(s, src_stride, d, dst_stride, c->d_keep, c->n, (int)(E / 4));
+        else k_gather_unit<uint8_t><<<grid, SUB_THREADS, 0, st>>>(s, src_stride, d, dst_stride, c->d_keep, c->n, (int)E);
+        c->launches++;
+        NPC_CUDA(c, cudaGetLastError());
+    }
+    return NPC_OK;
+}
+
+extern "C" int npc_gather_rows_device(npc_ctx *ctx, const void *src, int64_t src_stride, int64_t n_rows, void *dst, int64_t dst_stride) {
+    if (!ctx) return NPC_EINVAL;
+    if (!ctx->sub) return fail(ctx, NPC_ESTATE, "npc_gather_rows_device: the context was not created with npc_create_subset");
+    if (n_rows < 0 || (n_rows && (!src || !dst)) || ((uintptr_t)src & 15) || ((uintptr_t)dst & 15) || (src_stride & 15) || (dst_stride & 15) ||
+        src_stride < npc_gt_row_bytes(ctx->n_row, ctx->ploidy, ctx->width) || dst_stride < npc_gt_row_bytes(ctx->n, ctx->ploidy, ctx->width))
+        return fail(ctx, NPC_EINVAL, "npc_gather_rows_device: rows must be 16-byte aligned, strides multiples of 16 holding a whole row");
+    NPC_CUDA(ctx, cudaSetDevice(ctx->device));
+    return launch_gather(ctx, (const uint8_t *)src, src_stride, n_rows, (uint8_t *)dst, dst_stride, ctx->stream);
+}
+
+// A subset context's H2D copy of a slot's n_gt_rows full rows, compacted into dst (dst_stride apart); on the copy stream
+static int upload_compact(npc_ctx *c, int32_t slot, int64_t n_gt_rows, uint8_t *dst, int64_t dst_stride) {
+    if (!c->d_raw[slot]) NPC_CUDA(c, cudaMalloc(&c->d_raw[slot], (size_t)c->stage_stride * (size_t)std::max<int64_t>(c->staging_rows, 1)));
+    NPC_CUDA(c, cudaMemcpyAsync(c->d_raw[slot], c->h_gt[slot], (size_t)n_gt_rows * c->stage_stride, cudaMemcpyHostToDevice, c->copy_stream));
+    return launch_gather(c, c->d_raw[slot], c->stage_stride, n_gt_rows, dst, dst_stride, c->copy_stream);
+}
+
 // ---- staged blocks -----------------------------------------------------------------------
 
 extern "C" int npc_stage_acquire(npc_ctx *ctx, int32_t *slot, void **gt_host, int64_t *row_stride) {
@@ -793,7 +882,7 @@ extern "C" int npc_stage_acquire(npc_ctx *ctx, int32_t *slot, void **gt_host, in
     }
     ctx->slot_state[s] = 1;
     ctx->next_slot = (s + 1) % ctx->n_slots;
-    *slot = s; *gt_host = ctx->h_gt[s]; *row_stride = ctx->row_stride;
+    *slot = s; *gt_host = ctx->h_gt[s]; *row_stride = ctx->stage_stride;
     return NPC_OK;
 }
 
@@ -807,7 +896,9 @@ extern "C" int npc_score_block(npc_ctx *ctx, int32_t slot, int64_t n_gt_rows, co
     int rc = check_block(ctx, ctx->d_gt[slot], ctx->row_stride, n_gt_rows, rows, n_rows);
     if (!rc) rc = check_bed_rows(ctx, rows, n_rows, 0);
     if (rc) return rc;
-    if (n_gt_rows)
+    if (n_gt_rows && ctx->sub) {
+        if ((rc = upload_compact(ctx, slot, n_gt_rows, ctx->d_gt[slot], ctx->row_stride))) return rc;
+    } else if (n_gt_rows)
         NPC_CUDA(ctx, cudaMemcpyAsync(ctx->d_gt[slot], ctx->h_gt[slot], (size_t)n_gt_rows * ctx->row_stride,
                                       cudaMemcpyHostToDevice, ctx->copy_stream));
     NPC_CUDA(ctx, cudaEventRecord(ctx->ev_h2d[slot], ctx->copy_stream));
@@ -907,7 +998,9 @@ extern "C" int npc_stage_upload(npc_ctx *ctx, int32_t slot, int64_t n_gt_rows, i
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     // a scoring launch may still be reading the slab rows we are about to overwrite
     NPC_CUDA(ctx, cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_slab, 0));
-    if (n_gt_rows)
+    if (n_gt_rows && ctx->sub) {
+        if (int rc = upload_compact(ctx, slot, n_gt_rows, ctx->d_slab + dst_row * ctx->row_stride, ctx->row_stride)) return rc;
+    } else if (n_gt_rows)
         NPC_CUDA(ctx, cudaMemcpyAsync(ctx->d_slab + dst_row * ctx->row_stride, ctx->h_gt[slot], (size_t)n_gt_rows * ctx->row_stride,
                                       cudaMemcpyHostToDevice, ctx->copy_stream));
     NPC_CUDA(ctx, cudaEventRecord(ctx->ev_h2d[slot], ctx->copy_stream));

@@ -61,6 +61,8 @@ def load_library():
     sig = {
         "npc_create": (C.c_int, [C.POINTER(vp), C.c_int, i64, i32, i32, i64, i32]),
         "npc_create2": (C.c_int, [C.POINTER(vp), C.c_int, i64, i32, i32, i64, i32, i64]),
+        "npc_create_subset": (C.c_int, [C.POINTER(vp), C.c_int, i64, vp, i64, i32, i32, i64, i32, i64]),
+        "npc_gather_rows_device": (C.c_int, [vp, vp, i64, i64, vp, i64]),
         "npc_destroy": (None, [vp]),
         "npc_last_error": (C.c_char_p, [vp]),
         "npc_set_stream": (C.c_int, [vp, vp]),
@@ -160,13 +162,22 @@ class Engine:
     """One scoring context on one GPU: the state of one computePolygenicScores call
     (src/nimpress.nim:592-649) -- per-sample fp64 sums, nloci and the per-locus log."""
 
-    def __init__(self, n_samples, ploidy=2, gt_width=1, max_rows_per_block=4096, n_slots=0, device=0, staging_rows=None):
+    def __init__(self, n_samples, ploidy=2, gt_width=1, max_rows_per_block=4096, n_slots=0, device=0, staging_rows=None,
+                 keep=None, n_row_samples=None):
+        """keep: indices of the samples to score among the n_row_samples that staged rows carry (npc_create_subset; the
+        context then holds len(keep) samples and n_samples is ignored)."""
         self.L = load_library()
-        self.n = int(n_samples)
         self.ploidy, self.gt_width, self.max_rows = int(ploidy), int(gt_width), int(max_rows_per_block)
         h = C.c_void_p()
         self.staging_rows = int(staging_rows) if staging_rows else self.max_rows
-        rc = self.L.npc_create2(C.byref(h), device, self.n, ploidy, gt_width, max_rows_per_block, n_slots, self.staging_rows)
+        if keep is None:
+            self.n = int(n_samples)
+            rc = self.L.npc_create2(C.byref(h), device, self.n, ploidy, gt_width, max_rows_per_block, n_slots, self.staging_rows)
+        else:
+            keep = np.ascontiguousarray(keep, dtype=np.int64)
+            self.n = len(keep)
+            rc = self.L.npc_create_subset(C.byref(h), device, int(n_row_samples), keep.ctypes.data, self.n, ploidy, gt_width,
+                                          max_rows_per_block, n_slots, self.staging_rows)
         if rc:
             raise NpcError(f"npc_create rc={rc}: {self.L.npc_last_error(None).decode()}")
         self.h = h
@@ -200,6 +211,10 @@ class Engine:
 
     def reset(self):
         self._ck(self.L.npc_reset(self.h))
+
+    def gather_rows_device(self, src, src_stride, n_rows, dst, dst_stride):
+        """npc_gather_rows_device: compact n_rows device rows of the staged width into dst (asynchronous)."""
+        self._ck(self.L.npc_gather_rows_device(self.h, _ptr(src), int(src_stride), int(n_rows), _ptr(dst), int(dst_stride)))
 
     # -- host blocks through the pinned ring
     def stage_acquire(self):

@@ -5,6 +5,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <fstream>
 #include <stdexcept>
 #include <future>
 #include <map>
@@ -100,6 +101,38 @@ void Matcher::finish() {
     for (auto &k : kind) if (k == PENDING) k = NPC_KIND_ABSENT;
 }
 
+std::vector<int64_t> sample_subset(const std::vector<std::string> &file_samples, const std::string &list_path, bool exclude) {
+    std::ifstream in(list_path, std::ios::binary);
+    if (!in) throw InputError("--samples: cannot read the sample list " + list_path);
+    std::vector<std::string> names;
+    for (std::string line; std::getline(in, line);) {
+        if (!line.empty() && line.back() == '\r') line.pop_back();
+        if (!line.empty()) names.push_back(line);
+    }
+    if (in.bad()) throw InputError("--samples: cannot read the sample list " + list_path);
+    std::unordered_map<std::string, int64_t> index;                  // name -> its index, -1 when the file has it twice
+    for (int64_t i = 0; i < (int64_t)file_samples.size(); i++) {
+        auto ins = index.emplace(file_samples[i], i);
+        if (!ins.second) ins.first->second = -1;
+    }
+    std::vector<uint8_t> listed(file_samples.size(), 0);
+    for (const std::string &nm : names) {
+        auto it = index.find(nm);
+        if (it == index.end()) {
+            if (exclude) continue;                                   // a withdrawal list may name samples of other files
+            throw InputError("--samples: sample " + nm + " is not in the genotype file");
+        }
+        if (it->second < 0) throw InputError("--samples: sample " + nm + " occurs more than once in the genotype file");
+        if (listed[it->second] && !exclude) throw InputError("--samples: sample " + nm + " is listed twice");
+        listed[it->second] = 1;
+    }
+    std::vector<int64_t> keep;
+    for (int64_t i = 0; i < (int64_t)file_samples.size(); i++) if (listed[i] != exclude) keep.push_back(i);
+    if (keep.empty()) throw InputError("--samples: no sample of the genotype file is left to score");
+    if ((int64_t)keep.size() == (int64_t)file_samples.size()) keep.clear();        // every sample: the plain path
+    return keep;
+}
+
 namespace {
 
 // NIMPRESS_TIMING=1: phase wall times on stderr
@@ -176,10 +209,18 @@ std::string make_warnings(const ScoreFile &score, const Matcher &M, const std::v
 // is uploaded once, and the resident slab is then scored for each file).  Throws LayoutOverflow
 // when a matched record needs a wider layout (the caller restarts the pass with it) and
 // SlabOverflow when several files are given and their rows do not fit device memory.
+// keep: the samples to score (sample_subset), empty for all.  The reader's rows carry the file's n_row samples; the devices
+// compact them to the n kept ones (npc_create_subset), which is all that the contexts, scores and WARN lines see.
 void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, const std::string &genotype_path, bool seekable,
-              const GenomeIntervals &cov, const ScoreParams &p, int gt_width, int ploidy, std::vector<ScoreResult> &outs) {
+              const GenomeIntervals &cov, const ScoreParams &p, int gt_width, int ploidy, const std::vector<int64_t> &keep,
+              std::vector<ScoreResult> &outs) {
     const int S = (int)scores.size();
-    const int64_t n = vcf.n_samples();
+    const int64_t n_row = vcf.n_samples(), n = keep.empty() ? n_row : (int64_t)keep.size();
+    std::vector<std::string> names = vcf.samples();
+    if (!keep.empty()) {
+        names.clear();
+        for (int64_t i : keep) names.push_back(vcf.samples()[(size_t)i]);
+    }
     struct PerScore {
         std::unique_ptr<Matcher> M;
         std::vector<int64_t> slab_row;              // per entry: row of its device's resident slab
@@ -194,7 +235,7 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
     {   // entries with the same (contig, pos, ref, ea) settle on the same record: count keys once
         std::unordered_map<std::string, int> keys;
         for (int k = 0; k < S; k++) {
-            outs[k].samples = vcf.samples();
+            outs[k].samples = names;
             ps[k].M.reset(new Matcher(*scores[k], cov, p));
             const int64_t nE = (int64_t)scores[k]->entries.size();
             ps[k].slab_row.assign(nE, -1); ps[k].done.assign(nE, 0);
@@ -234,7 +275,7 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
 
     // staging slots of ~8 MB: big enough for efficient H2D copies, small enough that pinning three of them per
     // device does not dominate a short run (pinning costs ~1 ms per MB); scoring launches are sized separately
-    const int64_t row_bytes = std::max<int64_t>(16, npc_gt_row_bytes(n, ploidy, gt_width));
+    const int64_t row_bytes = std::max<int64_t>(16, npc_gt_row_bytes(n_row, ploidy, gt_width));
     struct Dev {
         Ctx ctx;
         int32_t slot = -1; uint8_t *stage = nullptr; int64_t stride = 0, staged = 0, slab_base = 0, slab_cap = 0, block_rows = 1;
@@ -255,7 +296,9 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
             const int64_t want = std::max<int64_t>(dev_lookup[d], 1);
             v.block_rows = std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(4096, (8ll << 20) / row_bytes + 1), want));
             const int64_t launch_rows = std::max<int64_t>(v.block_rows, 32768);
-            v.ctx.ck(npc_create2(&v.ctx.h, dev_ids[d], n, ploidy, gt_width, launch_rows, 3, v.block_rows), "npc_create");
+            if (keep.empty()) v.ctx.ck(npc_create2(&v.ctx.h, dev_ids[d], n, ploidy, gt_width, launch_rows, 3, v.block_rows), "npc_create");
+            else v.ctx.ck(npc_create_subset(&v.ctx.h, dev_ids[d], n_row, keep.data(), n, ploidy, gt_width, launch_rows, 3, v.block_rows),
+                          "npc_create_subset");
             v.ctx.ck(npc_set_policy(v.ctx.h, &pol), "npc_set_policy");
             if (p.use_ds) v.ctx.ck(npc_set_dosage_rows(v.ctx.h, 1), "npc_set_dosage_rows");
             if (p.exact_order) v.ctx.ck(npc_set_exact_order(v.ctx.h, 1), "npc_set_exact_order");
@@ -357,7 +400,7 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
             uint8_t *dst = v.stage + v.staged * v.stride;
             if (first) {                                            // a record named by two ranges: same bytes
                 vcf.wait_rows();
-                memcpy(dst, first, (size_t)npc_gt_row_bytes(n, ploidy, gt_width));
+                memcpy(dst, first, (size_t)npc_gt_row_bytes(n_row, ploidy, gt_width));
             }
             else {
                 if (p.use_pl && rec.alts.size() != 1)
@@ -373,8 +416,8 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
                 if (!direct) {
                     if (rec.ploidy > ploidy || rec.gt_width > gt_width)
                         throw LayoutOverflow{ std::max(rec.gt_width, gt_width), std::max(rec.ploidy, ploidy) };
-                    if (rec.gt_width == gt_width && rec.ploidy == ploidy) memcpy(dst, rec.gt, (size_t)npc_gt_row_bytes(n, ploidy, gt_width));
-                    else convert_gt(rec, n, gt_width, ploidy, dst);
+                    if (rec.gt_width == gt_width && rec.ploidy == ploidy) memcpy(dst, rec.gt, (size_t)npc_gt_row_bytes(n_row, ploidy, gt_width));
+                    else convert_gt(rec, n_row, gt_width, ploidy, dst);
                 }
                 first = dst;
             }
@@ -493,6 +536,8 @@ bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores
     for (int attempt = 0; attempt < 6; attempt++) {
         std::unique_ptr<VariantSource> vcf = open_variant_source(genotype_path, seekable);
         if (!vcf) return false;
+        // before any context: a bad list fails without a device
+        const std::vector<int64_t> keep = p.samples_path.empty() ? std::vector<int64_t>() : sample_subset(vcf->samples(), p.samples_path, p.exclude_samples);
         // PLINK fileset, BGEN file: rows in a layout of their own, read by offset (no index pass)
         const int fixed = vcf->fixed_layout();
         ScoreParams q = p;
@@ -506,7 +551,7 @@ bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores
         vcf->set_dosage_mode(q.use_ds);
         vcf->set_pl_mode(q.use_pl);
         try {
-            run_pass(scores, *vcf, genotype_path, seekable, cov, q, width, ploidy, outs);
+            run_pass(scores, *vcf, genotype_path, seekable, cov, q, width, ploidy, keep, outs);
             return true;
         } catch (const NoIndex &) {
             seekable = false;

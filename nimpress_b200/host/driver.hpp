@@ -29,6 +29,8 @@ struct ScoreParams {
     bool exact_order = false;              // npc_set_exact_order: bit-for-bit reference summation order
     bool use_ds = false;                   // score FORMAT/DS (fp32 expected ALT dosage) instead of FORMAT/GT -- not a reference option
     bool use_pl = false;                   // score FORMAT/PL as posterior expected dosages (NPC_GT_PL rows) -- not a reference option
+    std::string samples_path;              // --samples: a list of sample names (empty: every sample) -- not a reference option
+    bool exclude_samples = false;          // --samples=^FILE: score every sample the list does not name
 };
 
 struct ScoreResult {
@@ -69,6 +71,13 @@ private:
     std::vector<int64_t> hits_;
     int64_t n_lookup_ = 0;
 };
+
+// --samples: the samples of `file_samples` (the genotype file's names, in its order) to score, as ascending indices; an
+// empty result means every sample (also when the list keeps them all).  The list file holds one name per line (the whole
+// line, a trailing \r stripped, blank lines skipped).  A keep list naming a sample the file lacks or naming one twice, a
+// listed name occurring more than once in the file, an empty subset or an unreadable list throw InputError; names of an
+// exclude list that the file lacks are ignored.
+std::vector<int64_t> sample_subset(const std::vector<std::string> &file_samples, const std::string &list_path, bool exclude);
 
 // Throws InputError where the reference raises; std::runtime_error on CUDA / library failure.
 // false: the genotype file cannot be opened (the reference: FATAL + quit(-1), :728-730).

@@ -26,7 +26,16 @@ static ScoreParams to_params(const nph_params *p) {
     for (int d = 0; d < 32; d++) if (((uint32_t)p->device_mask >> d) & 1u) q.devices.push_back(d);
     q.use_ds = p->use_ds != 0;
     q.use_pl = p->use_pl != 0;
+    if (p->samples_path) q.samples_path = p->samples_path;
+    q.exclude_samples = p->exclude_samples != 0;
     return q;
+}
+
+// samples a scoring call would score: the file's, or the kept ones under --samples
+static int64_t scored_samples(const VariantSource &vcf, const ScoreParams &q) {
+    if (q.samples_path.empty()) return vcf.n_samples();
+    const std::vector<int64_t> keep = sample_subset(vcf.samples(), q.samples_path, q.exclude_samples);
+    return keep.empty() ? vcf.n_samples() : (int64_t)keep.size();
 }
 
 // open(ScoreFile) + loadBedIntervals as main() sequences them (:728-740)
@@ -130,6 +139,7 @@ int nph_plan(const char *score_path, const char *genotype_path, const char *bed_
         ScoreParams q = to_params(p);
         std::unique_ptr<VariantSource> vcf = open_variant_source(genotype_path);
         if (!vcf) return NPH_EOPEN_VCF;
+        const int64_t n_scored = scored_samples(*vcf, q);
         ScoreFile sf; GenomeIntervals cov;
         int rc = load_inputs(score_path, bed_path, q, sf, cov, nullptr);
         if (rc) return rc;
@@ -140,7 +150,7 @@ int nph_plan(const char *score_path, const char *genotype_path, const char *bed_
         M.finish();
         for (size_t i = 0; i < sf.entries.size(); i++) { kind_out[i] = M.kind[i]; eaidx_out[i] = M.eaidx[i]; }
         *n_rows_out = (int64_t)sf.entries.size();
-        *n_samples_out = vcf->n_samples();
+        *n_samples_out = n_scored;
         return NPH_OK;
     } catch (const InputError &e) {
         g_err = e.what();
@@ -160,6 +170,7 @@ int nph_plan_indexed(const char *score_path, const char *genotype_path, const ch
         Matcher M(sf, cov, q);
         std::unique_ptr<VariantSource> vcf = open_variant_source(genotype_path, true);      // the driver's order: index first
         if (!vcf) return NPH_EOPEN_VCF;
+        const int64_t n_scored = scored_samples(*vcf, q);
         std::unordered_map<std::string, std::vector<std::pair<int64_t, int64_t>>> spans;
         M.add_spans(spans);
         if (!vcf->use_regions(spans, genotype_path)) {
@@ -172,7 +183,7 @@ int nph_plan_indexed(const char *score_path, const char *genotype_path, const ch
         M.finish();
         for (size_t i = 0; i < sf.entries.size(); i++) { kind_out[i] = M.kind[i]; eaidx_out[i] = M.eaidx[i]; }
         *n_rows_out = (int64_t)sf.entries.size();
-        *n_samples_out = vcf->n_samples();
+        *n_samples_out = n_scored;
         if (records_read_out) *records_read_out = nrec;
         if (index_seeks_out) *index_seeks_out = vcf->seeks();
         return NPH_OK;
@@ -293,7 +304,13 @@ static const char *USAGE =
     "  warnings for its loci.\n"
     "  --exact-order      Add every locus to the running sums in score-file order, bit for bit\n"
     "                     like the reference (default: sum tiles of four loci first; same\n"
-    "                     products, scores equal to ~1e-15 relative) (not a reference option).\n";
+    "                     products, scores equal to ~1e-15 relative) (not a reference option).\n"
+    "  --samples=<file>   Score only the samples named in <file>, one name per line (VCF/BCF header\n"
+    "                     name, .fam IID, BGEN identifier or .sample ID_2), in the genotype file's\n"
+    "                     order: exactly what a genotype file holding only them gives, cohort EAF,\n"
+    "                     --maxmis and WARN lines included (not a reference option).\n"
+    "  --samples=^<file>  Score every sample except those named in <file>; names the genotype file\n"
+    "                     lacks are ignored (not a reference option).\n";
 
 static int parse_enum(const std::string &v, std::initializer_list<const char *> names) {   // Nim parseEnum: style-insensitive beyond the first char is not reproduced
     int i = 0;
@@ -337,8 +354,8 @@ static void print_result(const nph_result *r) {
 }
 
 int nph_main(int argc, char **argv) {
-    nph_params p = { NPC_LOCUS_PS, NPC_MISSING_HOMREF, NPC_SAMPLE_INT_PS, 0, 0, 0, 0, 0, 100, 0.05, 0.001, 0, 0 };
-    std::string cov, pos[2];
+    nph_params p = { NPC_LOCUS_PS, NPC_MISSING_HOMREF, NPC_SAMPLE_INT_PS, 0, 0, 0, 0, 0, 100, 0.05, 0.001, 0, 0, nullptr, 0 };
+    std::string cov, samples_list, pos[2];
     int npos = 0;
     try {
         for (int i = 1; i < argc; i++) {
@@ -361,6 +378,12 @@ int nph_main(int argc, char **argv) {
             else if (is("--afmisp")) p.afmisp = parse_float_nim(val("--afmisp"), "--afmisp");
             else if (is("--devices")) p.device_mask = (int32_t)parse_device_list(val("--devices"));
             else if (is("--device")) p.device = (int)parse_int_nim(val("--device"), "--device");
+            else if (is("--samples")) {
+                samples_list = val("--samples");
+                p.exclude_samples = !samples_list.empty() && samples_list[0] == '^';
+                if (p.exclude_samples) samples_list.erase(0, 1);
+                if (samples_list.empty()) throw InputError("--samples requires a file name");
+            }
             else if (a == "--ignorefilt") p.ignorefilt = 1;
             else if (a == "--exact-order") p.exact_order = 1;
             else if (a == "--dosage") p.use_ds = 1;
@@ -370,6 +393,7 @@ int nph_main(int argc, char **argv) {
             else throw InputError("too many arguments");
         }
         if (npos != 2) throw InputError("expected <scoredef> <genotypes.vcf|.bcf|.bed>");
+        if (!samples_list.empty()) p.samples_path = samples_list.c_str();
     } catch (const InputError &e) {
         std::cerr << e.what() << "\n" << "Usage:\n  nimpress [options] <scoredef> <genotypes.vcf|.bcf|.bed>\n";
         return 1;
