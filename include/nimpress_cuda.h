@@ -206,6 +206,13 @@ int npc_create_subset(npc_ctx **out, int device, int64_t n_row_samples, const in
  * aligned, strides multiples of 16 holding a whole row).  Asynchronous, on the context's stream (npc_set_stream).
  * NPC_ESTATE for a context not created by npc_create_subset. */
 int npc_gather_rows_device(npc_ctx *ctx, const void *src, int64_t src_stride, int64_t n_rows, void *dst, int64_t dst_stride);
+/* Replaces the keep list of a context made by npc_create_subset, for rows uploaded after this call: keep[0..n_keep)
+ * ascending, distinct, below n_row_samples of the context; n_keep must equal the context's.  Rows staged or uploaded
+ * before the call (npc_stage_upload, npc_score_block, npc_gather_rows_device) are compacted with the list they were
+ * uploaded under: the call waits for those gathers, so flush a half-filled staging slot first.  Several genotype files
+ * whose rows carry different samples score through one context this way (DESIGN.md 4.12).  NPC_ESTATE for a context
+ * not made by npc_create_subset, NPC_EINVAL for a bad list. */
+int npc_set_keep(npc_ctx *ctx, const int64_t *keep, int64_t n_keep);
 void npc_destroy(npc_ctx *ctx);
 const char *npc_last_error(const npc_ctx *ctx);   /* ctx may be NULL: text of the last npc_create failure */
 

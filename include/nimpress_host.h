@@ -87,6 +87,14 @@ int nph_compute_polygenic_scores(const char *score_path, const char *genotype_pa
  * is one nimpress process per score file.  On failure nothing is returned in out. */
 int nph_compute_polygenic_scores_multi(const char *const *score_paths, int32_t n_scores, const char *genotype_path,
                                        const char *bed_path, const nph_params *p, nph_result **out);
+/* Several genotype files (e.g. one per chromosome or chunk), read in the order given: exactly what one run over their
+ * concatenation gives -- the records of file 1, then file 2, ..., with the common sample list (DESIGN.md 4.12).  out[k]
+ * is what score_paths[k] gets.  The files are VCF text / BCF (mixed freely), or all PLINK 1 filesets, or all BGEN; they
+ * carry the same samples in the same order, or keep the same sequence of samples under samples_path (applied to each
+ * file on its own).  Mixed kinds and differing samples are NPH_EINPUT naming the file; NPH_EOPEN_VCF names the first
+ * file that cannot be opened (nph_last_error).  All genotype files are opened before the score files. */
+int nph_compute_polygenic_scores_files(const char *const *score_paths, int32_t n_scores, const char *const *genotype_paths,
+                                       int32_t n_genotypes, const char *bed_path, const nph_params *p, nph_result **out);
 int64_t nph_result_n_samples(const nph_result *r);
 int64_t nph_result_n_loci(const nph_result *r);          /* score rows                      */
 int64_t nph_result_nloci_used(const nph_result *r);      /* loci in the sum (the divisor/2) */
@@ -113,6 +121,11 @@ int nph_plan(const char *score_path, const char *genotype_path, const char *bed_
 int nph_plan_indexed(const char *score_path, const char *genotype_path, const char *bed_path, const nph_params *p,
                      int32_t *kind_out, int32_t *eaidx_out, int64_t cap, int64_t *n_rows_out, int64_t *n_samples_out,
                      int64_t *records_read_out, int64_t *index_seeks_out);
+/* nph_plan_indexed over several genotype files, read as their concatenation (nph_compute_polygenic_scores_files): each
+ * file takes its index-driven pass or is streamed on its own; records_read and index_seeks are sums over the files. */
+int nph_plan_files(const char *score_path, const char *const *genotype_paths, int32_t n_genotypes, const char *bed_path,
+                   const nph_params *p, int32_t *kind_out, int32_t *eaidx_out, int64_t cap, int64_t *n_rows_out,
+                   int64_t *n_samples_out, int64_t *records_read_out, int64_t *index_seeks_out);
 
 /* CPU only: raw GT payload of every record of a VCF/BCF, for reader tests.  Record r occupies
  * out[r*row_bytes ..]; returns the record count, width and ploidy of the LAST record read. */
@@ -129,7 +142,8 @@ double nph_betai(double a, double b, double x);
 double nph_binom_test(int64_t x, int64_t n, double p);
 int nph_format_float(double v, char *buf, int32_t buflen);   /* Nim `$`(float), the output format */
 
-/* The command line of the reference: nimpress [options] <scoredef> <genotypes.vcf>; prints the
+/* The command line of the reference: nimpress [options] <scoredef> <genotypes.vcf> (and, beyond it, several score files
+ * and several genotype files: <scoredef>[,<scoredef>...] <genotypes> [<genotypes> ...]); prints the
  * reference's WARN lines and `sample<TAB>score` lines to stdout; returns the process exit code
  * (0, 1 on malformed input / bad option, 255 when a file cannot be opened). */
 int nph_main(int argc, char **argv);

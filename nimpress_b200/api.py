@@ -75,6 +75,8 @@ def load_host_library():
     sig = {
         "nph_compute_polygenic_scores": (C.c_int, [cp, cp, cp, C.POINTER(_Params), C.POINTER(vp)]),
         "nph_compute_polygenic_scores_multi": (C.c_int, [C.POINTER(cp), C.c_int32, cp, cp, C.POINTER(_Params), C.POINTER(vp)]),
+        "nph_compute_polygenic_scores_files": (C.c_int, [C.POINTER(cp), C.c_int32, C.POINTER(cp), C.c_int32, cp, C.POINTER(_Params),
+                                                         C.POINTER(vp)]),
         "nph_result_n_samples": (i64, [vp]), "nph_result_n_loci": (i64, [vp]), "nph_result_nloci_used": (i64, [vp]),
         "nph_result_rounds": (i64, [vp]), "nph_result_devices": (i64, [vp]), "nph_result_scores": (vp, [vp]), "nph_result_loci": (vp, [vp]),
         "nph_result_sample": (cp, [vp, i64]), "nph_result_warnings": (cp, [vp]), "nph_result_free": (None, [vp]),
@@ -82,6 +84,8 @@ def load_host_library():
         "nph_plan": (C.c_int, [cp, cp, cp, C.POINTER(_Params), vp, vp, i64, C.POINTER(i64), C.POINTER(i64)]),
         "nph_fast_inflate": (C.c_int, [vp, i64, vp, i64]),
         "nph_plan_indexed": (C.c_int, [cp, cp, cp, C.POINTER(_Params), vp, vp, i64, C.POINTER(i64), C.POINTER(i64), C.POINTER(i64), C.POINTER(i64)]),
+        "nph_plan_files": (C.c_int, [cp, C.POINTER(cp), C.c_int32, cp, C.POINTER(_Params), vp, vp, i64, C.POINTER(i64), C.POINTER(i64),
+                                     C.POINTER(i64), C.POINTER(i64)]),
         "nph_result_records_read": (i64, [vp]), "nph_result_index_seeks": (i64, [vp]),
         "nph_read_gt": (C.c_int, [cp, vp, i64, i64, C.POINTER(i64), C.POINTER(i64), C.POINTER(i32), C.POINTER(i32)]),
         "nph_dbinom": (f64, [i64, i64, f64]), "nph_pbinom": (f64, [i64, i64, f64]), "nph_betai": (f64, [f64, f64, f64]),
@@ -147,12 +151,15 @@ def run(score_path, genotype_path, bed_path=None, imp_locus=ImputeMethodLocus.ps
     """nph_compute_polygenic_scores -> Result (scores, per-locus records, WARN text).  devices: list of CUDA
     device indices to split the score rows over (npc_reduce combines their partial sums).  dosage: score FORMAT/DS;
     pl: score FORMAT/PL as posterior expected dosages at the score file's eaf (DESIGN.md 4.10).  samples: path of a
-    list of sample names to score (one per line; DESIGN.md 4.11), exclude_samples: score the others instead."""
+    list of sample names to score (one per line; DESIGN.md 4.11), exclude_samples: score the others instead.
+    genotype_path: one path, or a list of them (e.g. one file per chromosome) scored as their concatenation (DESIGN.md 4.12)."""
     L = load_host_library()
     mask = sum(1 << int(d) for d in set(devices)) if devices else 0
     p = _Params(int(imp_locus), int(imp_missing), int(imp_sample), int(ignorefilt), int(bed_path is not None), device,
                 int(bool(exact_order)), mask, int(mincs), float(maxmis), float(afmisp), int(bool(dosage)), int(bool(pl)),
                 os.fsencode(samples) if samples else None, int(bool(exclude_samples)))
+    if not isinstance(genotype_path, (str, bytes, os.PathLike)):
+        return _run_files([score_path], genotype_path, bed_path, p)[0]
     h = C.c_void_p()
     rc = L.nph_compute_polygenic_scores(os.fsencode(score_path), os.fsencode(genotype_path),
                                         os.fsencode(bed_path) if bed_path else None, C.byref(p), C.byref(h))
@@ -164,14 +171,29 @@ def run_multi(score_paths, genotype_path, bed_path=None, imp_locus=ImputeMethodL
               imp_sample=ImputeMethodSample.int_ps, maxmis=0.05, afmisp=0.001, mincs=100, ignorefilt=False, device=0,
               exact_order=False, pl=False, samples=None, exclude_samples=False):
     """nph_compute_polygenic_scores_multi: several score files over one pass of the genotype file
-    -> [Result], each equal to run() on that file alone."""
+    -> [Result], each equal to run() on that file alone.  genotype_path: one path or a list of them, as for run()."""
     L = load_host_library()
     p = _Params(int(imp_locus), int(imp_missing), int(imp_sample), int(ignorefilt), int(bed_path is not None), device,
                 int(bool(exact_order)), 0, int(mincs), float(maxmis), float(afmisp), 0, int(bool(pl)),
                 os.fsencode(samples) if samples else None, int(bool(exclude_samples)))
+    if not isinstance(genotype_path, (str, bytes, os.PathLike)):
+        return _run_files(score_paths, genotype_path, bed_path, p)
     paths = (C.c_char_p * len(score_paths))(*[os.fsencode(s) for s in score_paths])
     hs = (C.c_void_p * len(score_paths))()
     rc = L.nph_compute_polygenic_scores_multi(paths, len(score_paths), os.fsencode(genotype_path),
+                                              os.fsencode(bed_path) if bed_path else None, C.byref(p), hs)
+    _check(L, rc)
+    return [_take_result(L, C.c_void_p(h)) for h in hs]
+
+
+def _run_files(score_paths, genotype_paths, bed_path, p):
+    """nph_compute_polygenic_scores_files: the score files over the genotype files read as their concatenation."""
+    L = load_host_library()
+    genotype_paths = list(genotype_paths)
+    paths = (C.c_char_p * len(score_paths))(*[os.fsencode(s) for s in score_paths])
+    geno = (C.c_char_p * len(genotype_paths))(*[os.fsencode(g) for g in genotype_paths])
+    hs = (C.c_void_p * len(score_paths))()
+    rc = L.nph_compute_polygenic_scores_files(paths, len(score_paths), geno, len(genotype_paths),
                                               os.fsencode(bed_path) if bed_path else None, C.byref(p), hs)
     _check(L, rc)
     return [_take_result(L, C.c_void_p(h)) for h in hs]

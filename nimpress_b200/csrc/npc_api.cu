@@ -861,6 +861,23 @@ extern "C" int npc_gather_rows_device(npc_ctx *ctx, const void *src, int64_t src
     return launch_gather(ctx, (const uint8_t *)src, src_stride, n_rows, (uint8_t *)dst, dst_stride, ctx->stream);
 }
 
+extern "C" int npc_set_keep(npc_ctx *ctx, const int64_t *keep, int64_t n_keep) {
+    if (!ctx) return NPC_EINVAL;
+    if (!ctx->sub) return fail(ctx, NPC_ESTATE, "npc_set_keep: the context was not created with npc_create_subset");
+    bool ok = keep && n_keep == ctx->n;
+    for (int64_t i = 0; ok && i < n_keep; i++) ok = keep[i] >= 0 && keep[i] < ctx->n_row && (i == 0 || keep[i] > keep[i - 1]);
+    if (!ok) return fail(ctx, NPC_EINVAL, "npc_set_keep: keep must hold the context's n ascending, distinct indices below n_row_samples");
+    std::vector<int32_t> h((size_t)((ctx->n + SUB_PAD - 1) / SUB_PAD * SUB_PAD), 0);
+    for (int64_t i = 0; i < n_keep; i++) h[(size_t)i] = (int32_t)keep[i];
+    NPC_CUDA(ctx, cudaSetDevice(ctx->device));
+    // the gathers of rows uploaded so far (copy stream) and of npc_gather_rows_device (the context's stream) read d_keep:
+    // let them finish, then replace it with a blocking copy
+    NPC_CUDA(ctx, cudaStreamSynchronize(ctx->copy_stream));
+    NPC_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    NPC_CUDA(ctx, cudaMemcpy(ctx->d_keep, h.data(), h.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
+    return NPC_OK;
+}
+
 // A subset context's H2D copy of a slot's n_gt_rows full rows, compacted into dst (dst_stride apart); on the copy stream
 static int upload_compact(npc_ctx *c, int32_t slot, int64_t n_gt_rows, uint8_t *dst, int64_t dst_stride) {
     if (!c->d_raw[slot]) NPC_CUDA(c, cudaMalloc(&c->d_raw[slot], (size_t)c->stage_stride * (size_t)std::max<int64_t>(c->staging_rows, 1)));

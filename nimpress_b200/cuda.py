@@ -63,6 +63,7 @@ def load_library():
         "npc_create2": (C.c_int, [C.POINTER(vp), C.c_int, i64, i32, i32, i64, i32, i64]),
         "npc_create_subset": (C.c_int, [C.POINTER(vp), C.c_int, i64, vp, i64, i32, i32, i64, i32, i64]),
         "npc_gather_rows_device": (C.c_int, [vp, vp, i64, i64, vp, i64]),
+        "npc_set_keep": (C.c_int, [vp, vp, i64]),
         "npc_destroy": (None, [vp]),
         "npc_last_error": (C.c_char_p, [vp]),
         "npc_set_stream": (C.c_int, [vp, vp]),
@@ -215,6 +216,11 @@ class Engine:
     def gather_rows_device(self, src, src_stride, n_rows, dst, dst_stride):
         """npc_gather_rows_device: compact n_rows device rows of the staged width into dst (asynchronous)."""
         self._ck(self.L.npc_gather_rows_device(self.h, _ptr(src), int(src_stride), int(n_rows), _ptr(dst), int(dst_stride)))
+
+    def set_keep(self, keep):
+        """npc_set_keep: compact rows uploaded from now on with this keep list (same length, ascending)."""
+        keep = np.ascontiguousarray(keep, dtype=np.int64)
+        self._ck(self.L.npc_set_keep(self.h, keep.ctypes.data, len(keep)))
 
     # -- host blocks through the pinned ring
     def stage_acquire(self):

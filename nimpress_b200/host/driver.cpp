@@ -13,6 +13,7 @@
 #include <thread>
 #include <unordered_map>
 
+#include "region_index.hpp"
 #include "stats.hpp"
 
 namespace nph {
@@ -135,6 +136,108 @@ std::vector<int64_t> sample_subset(const std::vector<std::string> &file_samples,
 
 namespace {
 
+const char *kind_name(int fixed) {
+    return fixed == NPC_GT_BED ? "a PLINK 1 fileset" : fixed == NPC_GT_DOSE255 ? "BGEN" : "VCF/BCF";
+}
+
+// first position at which two name lists differ (the shorter one's length when one is a prefix of the other), -1 if equal
+int64_t first_difference(const std::vector<std::string> &a, const std::vector<std::string> &b) {
+    const size_t m = std::min(a.size(), b.size());
+    for (size_t i = 0; i < m; i++) if (a[i] != b[i]) return (int64_t)i;
+    return a.size() == b.size() ? -1 : (int64_t)m;
+}
+
+std::string name_at(const std::vector<std::string> &v, int64_t i) {
+    return i < (int64_t)v.size() ? v[(size_t)i] : "(none: " + std::to_string(v.size()) + " samples)";
+}
+
+}  // namespace
+
+bool GenotypeFiles::open(const ScoreParams &p, std::string *unopened) {
+    const size_t F = paths.size();
+    src.clear(); src.resize(F);
+    opened_seekable_.assign(F, 0);
+    n_row = 0;
+    keep.assign(F, std::vector<int64_t>());
+    std::vector<int64_t> n_file(F);
+    std::vector<std::string> kept0;                                            // the names file 0 scores
+    bool all = true;                                                           // every file scores all of its samples
+    for (size_t f = 0; f < F; f++) {
+        // Checked one at a time: a later file is opened (seekable, which starts no inflate threads), checked and closed
+        // again, so that hundreds of chunk files do not hold their buffers and descriptors at once; prepare() reopens it.
+        std::unique_ptr<VariantSource> v = open_variant_source(paths[f], f == 0 ? seekable[f] != 0 : true);
+        if (!v) { if (unopened) *unopened = paths[f]; return false; }
+        if (f == 0) kind = v->fixed_layout();
+        else if (v->fixed_layout() != kind)
+            throw InputError("genotype files " + paths[0] + " (" + kind_name(kind) + ") and " + paths[f] + " (" + kind_name(v->fixed_layout()) +
+                             ") are of different kinds: one run reads VCF/BCF files, PLINK 1 filesets or BGEN files");
+        n_file[f] = v->n_samples();
+        n_row = std::max(n_row, n_file[f]);
+        const std::vector<std::string> &s = v->samples();
+        if (!p.samples_path.empty()) {
+            try {
+                keep[f] = sample_subset(s, p.samples_path, p.exclude_samples);
+            } catch (const InputError &e) {
+                if (F == 1) throw;
+                throw InputError("genotype file " + paths[f] + ": " + e.what());
+            }
+        }
+        std::vector<std::string> kept;
+        if (keep[f].empty()) kept = s;
+        else { all = false; for (int64_t i : keep[f]) kept.push_back(s[(size_t)i]); }
+        if (f == 0) {
+            kept0 = std::move(kept);
+            opened_seekable_[0] = seekable[0];
+            src[0] = std::move(v);                                             // file 0 is read next: keep it open
+            continue;
+        }
+        const int64_t d = first_difference(kept0, kept);
+        if (d < 0) continue;
+        if (p.samples_path.empty())
+            throw InputError("genotype file " + paths[f] + ": sample " + std::to_string(d + 1) + " is " + name_at(kept, d) + ", in " + paths[0] +
+                             " it is " + name_at(kept0, d) + ": files scored together carry the same samples in the same order "
+                             "(--samples=FILE scores the samples it names from every file)");
+        throw InputError("--samples: genotype file " + paths[f] + " keeps " + name_at(kept, d) + " as sample " + std::to_string(d + 1) + ", " +
+                         paths[0] + " keeps " + name_at(kept0, d) + ": the kept samples must be the same, in the same order, in every file");
+    }
+    if (kind != VariantSource::NO_FIXED_LAYOUT) seekable.assign(F, 0);          // rows read by offset: no index pass
+    names = std::move(kept0);
+    if (all) keep.clear();
+    else for (size_t f = 0; f < F; f++)
+        if (keep[f].empty()) for (int64_t i = 0; i < n_file[f]; i++) keep[f].push_back(i);
+    return true;
+}
+
+void GenotypeFiles::set_modes(bool ds, bool pl) {
+    ds_ = ds; pl_ = pl;
+    for (auto &s : src) if (s) { s->set_dosage_mode(ds); s->set_pl_mode(pl); }
+}
+
+bool GenotypeFiles::reopen(size_t f, bool block_mode) {
+    src[f] = open_variant_source(paths[f], block_mode);
+    if (!src[f]) return false;
+    opened_seekable_[f] = block_mode;
+    src[f]->set_dosage_mode(ds_); src[f]->set_pl_mode(pl_);
+    return true;
+}
+
+bool GenotypeFiles::prepare(size_t f, const Spans &spans) {
+    if (!src[f]) {
+        // no .tbi / .csi beside the file: use_regions() would refuse, so open it to be streamed straight away
+        if (seekable[f] && !RegionIndex::present(paths[f])) seekable[f] = 0;
+        if (!reopen(f, seekable[f] != 0)) return false;
+    }
+    if (seekable[f]) {
+        if (src[f]->use_regions(spans, paths[f])) return true;
+        seekable[f] = 0;                                                       // streamed, with the inflate pool, from now on
+    } else if (!opened_seekable_[f] || kind != VariantSource::NO_FIXED_LAYOUT) {
+        return true;
+    }
+    return reopen(f, false);
+}
+
+namespace {
+
 // NIMPRESS_TIMING=1: phase wall times on stderr
 struct PhaseTimer {
     bool on = getenv("NIMPRESS_TIMING") != nullptr;
@@ -168,7 +271,7 @@ void wait_warm(int device) {
 
 struct LayoutOverflow { int width, ploidy; };      // a matched record does not fit the context's GT layout
 struct SlabOverflow {};                            // several score files, and their matched rows exceed device memory
-struct NoIndex {};                                 // the index-driven pass is not possible / not worthwhile: stream the file
+struct CannotOpen { std::string path; };           // a genotype file that opened before could not be reopened to be streamed
 
 // WARN lines of one score file, in the reference's order (:326, :527-530, :538-541, :554-557, :567-570, :575-579)
 // real_tally: dosage rows (FORMAT/DS, BGEN), whose effect-allele tally is not an integer allele count
@@ -209,18 +312,20 @@ std::string make_warnings(const ScoreFile &score, const Matcher &M, const std::v
 // is uploaded once, and the resident slab is then scored for each file).  Throws LayoutOverflow
 // when a matched record needs a wider layout (the caller restarts the pass with it) and
 // SlabOverflow when several files are given and their rows do not fit device memory.
-// keep: the samples to score (sample_subset), empty for all.  The reader's rows carry the file's n_row samples; the devices
-// compact them to the n kept ones (npc_create_subset), which is all that the contexts, scores and WARN lines see.
-void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, const std::string &genotype_path, bool seekable,
-              const GenomeIntervals &cov, const ScoreParams &p, int gt_width, int ploidy, const std::vector<int64_t> &keep,
-              std::vector<ScoreResult> &outs) {
+// The genotype files are read one after the other as one record stream (DESIGN.md 4.12).  files.keep: the samples each
+// file scores, empty for all.  The reader's rows carry a file's own samples, at the front of staging rows sized for the
+// widest file (n_row); the devices compact them to the n kept ones (npc_create_subset, npc_set_keep at each file), which
+// is all that the contexts, scores and WARN lines see.
+void run_pass(const std::vector<const ScoreFile *> &scores, GenotypeFiles &files, const GenomeIntervals &cov, const ScoreParams &p,
+              int gt_width, int ploidy, std::vector<ScoreResult> &outs) {
     const int S = (int)scores.size();
-    const int64_t n_row = vcf.n_samples(), n = keep.empty() ? n_row : (int64_t)keep.size();
-    std::vector<std::string> names = vcf.samples();
-    if (!keep.empty()) {
-        names.clear();
-        for (int64_t i : keep) names.push_back(vcf.samples()[(size_t)i]);
-    }
+    const int64_t n_row = files.n_row, n = (int64_t)files.names.size();
+    const std::vector<std::string> &names = files.names;
+    const bool subset = !files.keep.empty();
+    size_t cur = 0;                                   // the file being read
+    // the keep list of the file being read (or, after the stream, of the last one): a context opened lazily takes it; one
+    // opened after the stream receives no rows, so any file's list serves it
+    const int64_t *keep_now = subset ? files.keep[0].data() : nullptr;
     struct PerScore {
         std::unique_ptr<Matcher> M;
         std::vector<int64_t> slab_row;              // per entry: row of its device's resident slab
@@ -247,11 +352,11 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
         }
         if (S > 1) n_lookup = (int64_t)keys.size();
     }
-    if (seekable) {                                   // an index next to the file and few loci: read only where loci are
-        std::unordered_map<std::string, std::vector<std::pair<int64_t, int64_t>>> spans;
+    Spans spans;                                      // an index next to a file and few loci: read only where loci are
+    if (std::count(files.seekable.begin(), files.seekable.end(), 1))
         for (int k = 0; k < S; k++) ps[k].M->add_spans(spans);
-        if (!vcf.use_regions(spans, genotype_path)) throw NoIndex();
-    }
+    if (!files.prepare(0, spans)) throw CannotOpen{ files.paths[0] };
+    VariantSource *vcf = files.src[0].get();
     timer.mark("coverage + entry index");
 
     // Devices: one context per GPU.  With several, the score rows are partitioned into contiguous ranges in
@@ -286,8 +391,8 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
     // rows still being converted by the source's workers land in the devices' pinned slots: let them finish before the
     // slots go, whichever way this pass ends
     struct RowsGuard {
-        VariantSource &v;
-        ~RowsGuard() { try { v.wait_rows(); } catch (...) {} }
+        VariantSource *&v;
+        ~RowsGuard() { try { if (v) v->wait_rows(); } catch (...) {} }
     } rows_guard{ vcf };
     npc_policy pol = { p.imp_locus, p.imp_missing, p.imp_sample, 0, p.mincs, p.maxmis };
     auto open_dev = [&](int d) {
@@ -296,9 +401,9 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
             const int64_t want = std::max<int64_t>(dev_lookup[d], 1);
             v.block_rows = std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(4096, (8ll << 20) / row_bytes + 1), want));
             const int64_t launch_rows = std::max<int64_t>(v.block_rows, 32768);
-            if (keep.empty()) v.ctx.ck(npc_create2(&v.ctx.h, dev_ids[d], n, ploidy, gt_width, launch_rows, 3, v.block_rows), "npc_create");
-            else v.ctx.ck(npc_create_subset(&v.ctx.h, dev_ids[d], n_row, keep.data(), n, ploidy, gt_width, launch_rows, 3, v.block_rows),
-                          "npc_create_subset");
+            if (!subset) v.ctx.ck(npc_create2(&v.ctx.h, dev_ids[d], n, ploidy, gt_width, launch_rows, 3, v.block_rows), "npc_create");
+            else v.ctx.ck(npc_create_subset(&v.ctx.h, dev_ids[d], n_row, keep_now, n, ploidy, gt_width, launch_rows, 3,
+                                            v.block_rows), "npc_create_subset");
             v.ctx.ck(npc_set_policy(v.ctx.h, &pol), "npc_set_policy");
             if (p.use_ds) v.ctx.ck(npc_set_dosage_rows(v.ctx.h, 1), "npc_set_dosage_rows");
             if (p.exact_order) v.ctx.ck(npc_set_exact_order(v.ctx.h, 1), "npc_set_exact_order");
@@ -327,7 +432,7 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
 
     auto flush_stage = [&](Dev &v) {
         if (v.slot < 0) return;
-        vcf.wait_rows();
+        vcf->wait_rows();
         v.ctx.ck(npc_stage_upload(v.ctx.h, v.slot, v.staged, v.slab_base), "npc_stage_upload");
         v.slab_base += v.staged; v.staged = 0; v.slot = -1;
     };
@@ -363,82 +468,99 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
         rounds[d]++;
     };
 
-    // ---- one streaming pass over the genotype file (findVariant :353-364, eaidx :375-379) ---
+    // ---- one streaming pass over the genotype files (findVariant :353-364, eaidx :375-379) ---
     VariantRecord rec;
-    int64_t records_read = 0, records_matched = 0;
+    int64_t records_read = 0, records_matched = 0, seeks = 0;
     std::vector<int64_t> rec_row(D);                   // slab row this record got on each device, -1 = not uploaded there
-    while (vcf.next(rec)) {
-        records_read++;
-        bool any = false, need_gt = false;
-        uint32_t need_dev = 0;
-        for (int k = 0; k < S; k++) {
-            const std::vector<int64_t> &hits = ps[k].M->match(rec);
-            for (int64_t i : hits) {
-                any = true;
-                if (ps[k].M->kind[i] == NPC_KIND_GT) { need_gt = true; need_dev |= 1u << dev_of(k, i); }
-            }
-        }
-        if (!any) continue;
-        records_matched++;
-        if (!need_gt) continue;                                     // FILTER-failed: never decoded (:553-558)
-        const uint8_t *first = nullptr;
-        for (int d = 0; d < D; d++) {
-            rec_row[d] = -1;
-            if (!((need_dev >> d) & 1u)) continue;
-            ensure_open(d);
-            Dev &v = devs[d];
-            if (v.slab_base + v.staged >= v.slab_cap) {             // slab full: score its rows, start over
-                if (S > 1) throw SlabOverflow();
-                score_round(d, false);
-                v.slab_base = 0;
-            }
-            if (v.slot < 0) {
-                void *ptr;
-                v.ctx.ck(npc_stage_acquire(v.ctx.h, &v.slot, &ptr, &v.stride), "npc_stage_acquire");
-                v.stage = (uint8_t *)ptr; v.staged = 0;
-            }
-            uint8_t *dst = v.stage + v.staged * v.stride;
-            if (first) {                                            // a record named by two ranges: same bytes
-                vcf.wait_rows();
-                memcpy(dst, first, (size_t)npc_gt_row_bytes(n_row, ploidy, gt_width));
-            }
-            else {
-                if (p.use_pl && rec.alts.size() != 1)
-                    throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/PL rows take biallelic records only (" +
-                                     std::to_string(rec.alts.size()) + " ALT alleles; split them with bcftools norm -m-)");
-                // BCF with the context's layout: the GT payload goes from the inflated blocks straight into the pinned row
-                const bool direct = vcf.load_gt_into(rec, dst, gt_width, ploidy);
-                if (!rec.has_gt || !rec.gt)
-                    throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) +
-                                     (p.use_pl ? " has no PL field" : p.use_ds ? " has no DS field" : " has no GT field"));
-                if (p.use_ds && (rec.ploidy != 1 || rec.gt_width != 4))
-                    throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/DS with several values per sample is not supported");
-                if (!direct) {
-                    if (rec.ploidy > ploidy || rec.gt_width > gt_width)
-                        throw LayoutOverflow{ std::max(rec.gt_width, gt_width), std::max(rec.ploidy, ploidy) };
-                    if (rec.gt_width == gt_width && rec.ploidy == ploidy) memcpy(dst, rec.gt, (size_t)npc_gt_row_bytes(n_row, ploidy, gt_width));
-                    else convert_gt(rec, n_row, gt_width, ploidy, dst);
+    for (cur = 0; cur < files.src.size(); cur++) {
+        if (cur > 0) {
+            if (!files.prepare(cur, spans)) throw CannotOpen{ files.paths[cur] };
+            vcf = files.src[cur].get();
+            if (subset) {                                 // staged rows of the previous file are compacted with its list
+                keep_now = files.keep[cur].data();
+                for (int d = 0; d < D; d++) if (opened[d]) {
+                    flush_stage(devs[d]);
+                    devs[d].ctx.ck(npc_set_keep(devs[d].ctx.h, keep_now, n), "npc_set_keep");
                 }
-                first = dst;
             }
-            rec_row[d] = v.slab_base + v.staged;
-            v.staged++;
         }
-        for (int k = 0; k < S; k++) for (int64_t i : ps[k].M->match_last())
-            if (ps[k].M->kind[i] == NPC_KIND_GT) {
-                if (p.use_ds && ps[k].M->eaidx[i] > 1)
-                    throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/DS rows take the REF or the first ALT as effect allele");
-                ps[k].slab_row[i] = rec_row[dev_of(k, i)];
+        const size_t file_row_bytes = (size_t)npc_gt_row_bytes(vcf->n_samples(), ploidy, gt_width);   // the front of a staging row
+        while (vcf->next(rec)) {
+            records_read++;
+            bool any = false, need_gt = false;
+            uint32_t need_dev = 0;
+            for (int k = 0; k < S; k++) {
+                const std::vector<int64_t> &hits = ps[k].M->match(rec);
+                for (int64_t i : hits) {
+                    any = true;
+                    if (ps[k].M->kind[i] == NPC_KIND_GT) { need_gt = true; need_dev |= 1u << dev_of(k, i); }
+                }
             }
-        for (int d = 0; d < D; d++) if (devs[d].slot >= 0 && devs[d].staged == devs[d].block_rows) flush_stage(devs[d]);
+            if (!any) continue;
+            records_matched++;
+            if (!need_gt) continue;                                     // FILTER-failed: never decoded (:553-558)
+            const uint8_t *first = nullptr;
+            for (int d = 0; d < D; d++) {
+                rec_row[d] = -1;
+                if (!((need_dev >> d) & 1u)) continue;
+                ensure_open(d);
+                Dev &v = devs[d];
+                if (v.slab_base + v.staged >= v.slab_cap) {             // slab full: score its rows, start over
+                    if (S > 1) throw SlabOverflow();
+                    score_round(d, false);
+                    v.slab_base = 0;
+                }
+                if (v.slot < 0) {
+                    void *ptr;
+                    v.ctx.ck(npc_stage_acquire(v.ctx.h, &v.slot, &ptr, &v.stride), "npc_stage_acquire");
+                    v.stage = (uint8_t *)ptr; v.staged = 0;
+                }
+                uint8_t *dst = v.stage + v.staged * v.stride;
+                if (first) {                                            // a record named by two ranges: same bytes
+                    vcf->wait_rows();
+                    memcpy(dst, first, file_row_bytes);
+                }
+                else {
+                    if (p.use_pl && rec.alts.size() != 1)
+                        throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/PL rows take biallelic records only (" +
+                                         std::to_string(rec.alts.size()) + " ALT alleles; split them with bcftools norm -m-)");
+                    // BCF with the context's layout: the GT payload goes from the inflated blocks straight into the pinned row
+                    const bool direct = vcf->load_gt_into(rec, dst, gt_width, ploidy);
+                    if (!rec.has_gt || !rec.gt)
+                        throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) +
+                                         (p.use_pl ? " has no PL field" : p.use_ds ? " has no DS field" : " has no GT field"));
+                    if (p.use_ds && (rec.ploidy != 1 || rec.gt_width != 4))
+                        throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/DS with several values per sample is not supported");
+                    if (!direct) {
+                        if (rec.ploidy > ploidy || rec.gt_width > gt_width)
+                            throw LayoutOverflow{ std::max(rec.gt_width, gt_width), std::max(rec.ploidy, ploidy) };
+                        if (rec.gt_width == gt_width && rec.ploidy == ploidy) memcpy(dst, rec.gt, file_row_bytes);
+                        else convert_gt(rec, vcf->n_samples(), gt_width, ploidy, dst);
+                    }
+                    first = dst;
+                }
+                rec_row[d] = v.slab_base + v.staged;
+                v.staged++;
+            }
+            for (int k = 0; k < S; k++) for (int64_t i : ps[k].M->match_last())
+                if (ps[k].M->kind[i] == NPC_KIND_GT) {
+                    if (p.use_ds && ps[k].M->eaidx[i] > 1)
+                        throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/DS rows take the REF or the first ALT as effect allele");
+                    ps[k].slab_row[i] = rec_row[dev_of(k, i)];
+                }
+            for (int d = 0; d < D; d++) if (devs[d].slot >= 0 && devs[d].staged == devs[d].block_rows) flush_stage(devs[d]);
+        }
+        vcf->wait_rows();                                 // BGEN workers may still be writing this file's rows into pinned slots
+        seeks += vcf->seeks();
+        if (cur + 1 < files.src.size()) { files.src[cur].reset(); vcf = nullptr; }
     }
     for (int k = 0; k < S; k++) {
         ps[k].M->finish();
-        outs[k].records_read = records_read; outs[k].records_matched = records_matched; outs[k].index_seeks = vcf.seeks();
+        outs[k].records_read = records_read; outs[k].records_matched = records_matched; outs[k].index_seeks = seeks;
     }
     timer.mark("stream + match + upload");
     if (timer.on) fprintf(stderr, "[nimpress timing] records read %lld, matched %lld, index seeks %lld%s\n", (long long)records_read,
-                          (long long)records_matched, (long long)vcf.seeks(), vcf.seeks() ? " (.tbi / .csi used)" : "");
+                          (long long)records_matched, (long long)seeks, seeks ? " (.tbi / .csi used)" : "");
 
     // ---- score the slab(s), collect results ----------------------------------------------------
     std::vector<std::vector<npc_locus>> logs(S);
@@ -524,50 +646,57 @@ void run_pass(const std::vector<const ScoreFile *> &scores, VariantSource &vcf, 
 
 }  // namespace
 
-bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores, const std::string &genotype_path,
-                                    const GenomeIntervals &cov, const ScoreParams &p, std::vector<ScoreResult> &outs) {
+bool compute_polygenic_scores_files(const std::vector<const ScoreFile *> &scores, const std::vector<std::string> &genotype_paths,
+                                    const GenomeIntervals &cov, const ScoreParams &p, std::vector<ScoreResult> &outs, std::string *unopened) {
     for (int d : (p.devices.empty() ? std::vector<int>{ p.device } : p.devices)) start_warm(d);
     int width = 1, ploidy = 2;                      // BCF's usual GT layout: int8, diploid
     if (p.use_ds && p.use_pl) throw InputError("--pl and --dosage: score either FORMAT/PL or FORMAT/DS");
     if (p.use_ds) { width = 4; ploidy = 1; }        // FORMAT/DS: one float per sample
     if (p.use_pl) { width = NPC_GT_PL; ploidy = 2; }   // FORMAT/PL: one packed word per sample
-    bool seekable = true;                           // first try the index-driven pass (needs <file>.tbi / .csi)
+    GenotypeFiles files(genotype_paths);            // each file first tries the index-driven pass (needs <file>.tbi / .csi)
     bool dose32 = false;                            // a BGEN pass met a block that only 32-bit dosage rows hold
     for (int attempt = 0; attempt < 6; attempt++) {
-        std::unique_ptr<VariantSource> vcf = open_variant_source(genotype_path, seekable);
-        if (!vcf) return false;
-        // before any context: a bad list fails without a device
-        const std::vector<int64_t> keep = p.samples_path.empty() ? std::vector<int64_t>() : sample_subset(vcf->samples(), p.samples_path, p.exclude_samples);
-        // PLINK fileset, BGEN file: rows in a layout of their own, read by offset (no index pass)
-        const int fixed = vcf->fixed_layout();
+        // every file is (re)opened and its --samples list resolved before any context: a bad list fails without a device
+        if (!files.open(p, unopened)) return false;
+        // PLINK filesets, BGEN files: rows in a layout of their own, read by offset (no index pass)
+        const int fixed = files.kind;
         ScoreParams q = p;
         if (fixed == NPC_GT_BED && p.use_ds) throw InputError("--dosage: a PLINK fileset holds hard calls only, no FORMAT/DS");
         if (fixed == NPC_GT_BED && p.use_pl) throw InputError("--pl: a PLINK fileset holds hard calls only, no FORMAT/PL");
         if (fixed == NPC_GT_DOSE255 && p.use_pl) throw InputError("--pl: a BGEN file holds genotype probabilities, no FORMAT/PL");
         if (fixed != VariantSource::NO_FIXED_LAYOUT) {
-            width = dose32 ? NPC_GT_DOSE32 : fixed; ploidy = 2; seekable = false;
+            width = dose32 ? NPC_GT_DOSE32 : fixed; ploidy = 2;
             q.use_ds = false;                       // BGEN rows are dosages already: --dosage changes nothing
         }
-        vcf->set_dosage_mode(q.use_ds);
-        vcf->set_pl_mode(q.use_pl);
+        files.set_modes(q.use_ds, q.use_pl);
         try {
-            run_pass(scores, *vcf, genotype_path, seekable, cov, q, width, ploidy, keep, outs);
+            run_pass(scores, files, cov, q, width, ploidy, outs);
             return true;
-        } catch (const NoIndex &) {
-            seekable = false;
-        } catch (const LayoutOverflow &o) {         // rare: wider integers or higher ploidy -- rerun with that layout
+        } catch (const CannotOpen &e) {
+            if (unopened) *unopened = e.path;
+            return false;
+        } catch (const LayoutOverflow &o) {         // rare: wider integers or higher ploidy -- rerun every file with that layout
             width = o.width; ploidy = o.ploidy;
         } catch (const NeedsDose32 &e) {            // BGEN at another bit depth or with haploid samples: rerun with 32-bit rows
             dose32 = true;
             if (getenv("NIMPRESS_TIMING")) fprintf(stderr, "[nimpress timing] restart with 32-bit dosage rows: %s\n", e.what());
-        } catch (const SlabOverflow &) {            // too many rows for one resident slab: one file at a time
+        } catch (const SlabOverflow &) {            // too many rows for one resident slab: one score file at a time
+            files.src.clear();
             outs.assign(scores.size(), ScoreResult());
-            for (size_t k = 0; k < scores.size(); k++)
-                if (!compute_polygenic_scores(*scores[k], genotype_path, cov, p, outs[k])) return false;
+            for (size_t k = 0; k < scores.size(); k++) {
+                std::vector<ScoreResult> one;
+                if (!compute_polygenic_scores_files({ scores[k] }, genotype_paths, cov, p, one, unopened)) return false;
+                outs[k] = std::move(one[0]);
+            }
             return true;
         }
     }
     throw std::runtime_error("GT layout kept growing between passes");
+}
+
+bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores, const std::string &genotype_path,
+                                    const GenomeIntervals &cov, const ScoreParams &p, std::vector<ScoreResult> &outs) {
+    return compute_polygenic_scores_files(scores, { genotype_path }, cov, p, outs);
 }
 
 bool compute_polygenic_scores(const ScoreFile &score, const std::string &genotype_path, const GenomeIntervals &cov,

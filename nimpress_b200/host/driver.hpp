@@ -4,6 +4,7 @@
 // imputation / accumulation to libnimpress_cuda.
 #pragma once
 #include <cstdint>
+#include <memory>
 #include <string>
 #include <unordered_map>
 #include <vector>
@@ -79,6 +80,33 @@ private:
 // exclude list that the file lacks are ignored.
 std::vector<int64_t> sample_subset(const std::vector<std::string> &file_samples, const std::string &list_path, bool exclude);
 
+using Spans = std::unordered_map<std::string, std::vector<std::pair<int64_t, int64_t>>>;   // per contig, 1-based inclusive
+
+// The genotype files of one run, read one after the other as their concatenation (DESIGN.md 4.12).
+struct GenotypeFiles {
+    std::vector<std::string> paths;
+    std::vector<uint8_t> seekable;                     // per file: try its index-driven pass when it is read
+    std::vector<std::unique_ptr<VariantSource>> src;   // per file while open: file 0 from open(), the others from prepare()
+    int kind = VariantSource::NO_FIXED_LAYOUT;         // the files' common fixed_layout()
+    std::vector<std::vector<int64_t>> keep;            // per file: its scored samples, ascending; empty: every file scores all of its samples
+    std::vector<std::string> names;                    // the scored samples, in order
+    int64_t n_row = 0;                                 // samples of the widest file
+
+    explicit GenotypeFiles(const std::vector<std::string> &paths) : paths(paths), seekable(paths.size(), 1) {}
+    // Opens every file in turn, checks that they are of one kind (VCF text and BCF, or PLINK 1 filesets, or BGEN) and
+    // resolves --samples per file; the kept names must be the same sequence in every file.  Only file 0 stays open.  false,
+    // with *unopened = its path, at the first file that cannot be opened; InputError for mixed kinds or differing samples.
+    bool open(const ScoreParams &p, std::string *unopened);
+    void set_modes(bool ds, bool pl);                  // set_dosage_mode / set_pl_mode of every source, also of one reopened later
+    // Before file f is read: open it if it is closed, restrict it to these spans by its .tbi / .csi when seekable[f] and the
+    // index allows it, otherwise (re)open it to be streamed (false: it cannot be opened).
+    bool prepare(size_t f, const Spans &spans);
+private:
+    bool reopen(size_t f, bool block_mode);
+    bool ds_ = false, pl_ = false;
+    std::vector<uint8_t> opened_seekable_;             // per file: its source reads block by block (no inflate pool)
+};
+
 // Throws InputError where the reference raises; std::runtime_error on CUDA / library failure.
 // false: the genotype file cannot be opened (the reference: FATAL + quit(-1), :728-730).
 bool compute_polygenic_scores(const ScoreFile &score, const std::string &genotype_path, const GenomeIntervals &cov,
@@ -88,5 +116,11 @@ bool compute_polygenic_scores(const ScoreFile &score, const std::string &genotyp
 // compute_polygenic_scores gives for that file alone (the reference: one nimpress run per file).
 bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores, const std::string &genotype_path,
                                     const GenomeIntervals &cov, const ScoreParams &p, std::vector<ScoreResult> &outs);
+
+// The same over several genotype files, exactly as over their concatenation (DESIGN.md 4.12).  false: a genotype file
+// cannot be opened (*unopened, when given, names it).
+bool compute_polygenic_scores_files(const std::vector<const ScoreFile *> &scores, const std::vector<std::string> &genotype_paths,
+                                    const GenomeIntervals &cov, const ScoreParams &p, std::vector<ScoreResult> &outs,
+                                    std::string *unopened = nullptr);
 
 }  // namespace nph

@@ -52,44 +52,30 @@ static int load_inputs(const char *score_path, const char *bed_path, ScoreParams
 int nph_compute_polygenic_scores(const char *score_path, const char *genotype_path, const char *bed_path,
                                  const nph_params *p, nph_result **out) {
     if (!score_path || !genotype_path || !p || !out) return NPH_EINPUT;
-    *out = nullptr;
-    try {
-        ScoreParams q = to_params(p);
-        {   // main() opens the VCF first (:728): an unreadable VCF wins over an unreadable score file
-            std::unique_ptr<VariantSource> probe = open_variant_source(genotype_path);
-            if (!probe) { g_err = std::string("Could not open input VCF file ") + genotype_path; return NPH_EOPEN_VCF; }
-        }
-        ScoreFile sf; GenomeIntervals cov;
-        std::string fatal;
-        int rc = load_inputs(score_path, bed_path, q, sf, cov, &fatal);
-        if (rc) { g_err = std::string("Could not open polygenic score file ") + score_path; return rc; }
-        nph_result *res = new nph_result();
-        if (!compute_polygenic_scores(sf, genotype_path, cov, q, res->r)) {
-            delete res;
-            g_err = std::string("Could not open input VCF file ") + genotype_path;
-            return NPH_EOPEN_VCF;
-        }
-        res->r.warnings = fatal + res->r.warnings;
-        *out = res;
-        return NPH_OK;
-    } catch (const InputError &e) {
-        g_err = e.what();
-        return NPH_EINPUT;
-    } catch (const std::exception &e) {
-        g_err = e.what();
-        return NPH_EGPU;
-    }
+    return nph_compute_polygenic_scores_files(&score_path, 1, &genotype_path, 1, bed_path, p, out);
 }
 
 int nph_compute_polygenic_scores_multi(const char *const *score_paths, int32_t n_scores, const char *genotype_path,
                                        const char *bed_path, const nph_params *p, nph_result **out) {
-    if (!score_paths || n_scores < 1 || !genotype_path || !p || !out) return NPH_EINPUT;
+    if (!genotype_path) return NPH_EINPUT;
+    return nph_compute_polygenic_scores_files(score_paths, n_scores, &genotype_path, 1, bed_path, p, out);
+}
+
+int nph_compute_polygenic_scores_files(const char *const *score_paths, int32_t n_scores, const char *const *genotype_paths,
+                                       int32_t n_genotypes, const char *bed_path, const nph_params *p, nph_result **out) {
+    if (!score_paths || n_scores < 1 || !genotype_paths || n_genotypes < 1 || !p || !out) return NPH_EINPUT;
     for (int32_t k = 0; k < n_scores; k++) out[k] = nullptr;
     try {
         ScoreParams q = to_params(p);
-        {
-            std::unique_ptr<VariantSource> probe = open_variant_source(genotype_path);
-            if (!probe) { g_err = std::string("Could not open input VCF file ") + genotype_path; return NPH_EOPEN_VCF; }
+        std::vector<std::string> geno;
+        for (int32_t f = 0; f < n_genotypes; f++) {
+            if (!genotype_paths[f]) return NPH_EINPUT;
+            geno.push_back(genotype_paths[f]);
+        }
+        // main() opens the VCF first (:728): an unreadable genotype file wins over an unreadable score file
+        for (const std::string &g : geno) {
+            std::unique_ptr<VariantSource> probe = open_variant_source(g, true);
+            if (!probe) { g_err = "Could not open input VCF file " + g; return NPH_EOPEN_VCF; }
         }
         std::vector<ScoreFile> files((size_t)n_scores);
         std::vector<const ScoreFile *> ptrs;
@@ -99,10 +85,12 @@ int nph_compute_polygenic_scores_multi(const char *const *score_paths, int32_t n
             if (!files[k].load(score_paths[k])) { g_err = std::string("Could not open polygenic score file ") + score_paths[k]; return NPH_EOPEN_SCORE; }
             ptrs.push_back(&files[k]);
         }
+        // the reference logs FATAL but carries on (:739-740)
         if (q.use_cov && bed_path && !cov.load(bed_path)) fatal = std::string("FATAL Could not open coverage BED file ") + bed_path + "\n";
         std::vector<ScoreResult> rs;
-        if (!compute_polygenic_scores_multi(ptrs, genotype_path, cov, q, rs)) {
-            g_err = std::string("Could not open input VCF file ") + genotype_path;
+        std::string unopened = geno[0];
+        if (!compute_polygenic_scores_files(ptrs, geno, cov, q, rs, &unopened)) {
+            g_err = "Could not open input VCF file " + unopened;
             return NPH_EOPEN_VCF;
         }
         for (int32_t k = 0; k < n_scores; k++) {
@@ -161,31 +149,41 @@ int nph_plan(const char *score_path, const char *genotype_path, const char *bed_
 int nph_plan_indexed(const char *score_path, const char *genotype_path, const char *bed_path, const nph_params *p,
                      int32_t *kind_out, int32_t *eaidx_out, int64_t cap, int64_t *n_rows_out, int64_t *n_samples_out,
                      int64_t *records_read_out, int64_t *index_seeks_out) {
+    return nph_plan_files(score_path, &genotype_path, 1, bed_path, p, kind_out, eaidx_out, cap, n_rows_out, n_samples_out,
+                          records_read_out, index_seeks_out);
+}
+
+int nph_plan_files(const char *score_path, const char *const *genotype_paths, int32_t n_genotypes, const char *bed_path,
+                   const nph_params *p, int32_t *kind_out, int32_t *eaidx_out, int64_t cap, int64_t *n_rows_out,
+                   int64_t *n_samples_out, int64_t *records_read_out, int64_t *index_seeks_out) {
     try {
+        if (!genotype_paths || n_genotypes < 1) return NPH_EINPUT;
         ScoreParams q = to_params(p);
         ScoreFile sf; GenomeIntervals cov;
         int rc = load_inputs(score_path, bed_path, q, sf, cov, nullptr);
         if (rc) return rc;
         if ((int64_t)sf.entries.size() > cap) return NPH_ECAPACITY;
         Matcher M(sf, cov, q);
-        std::unique_ptr<VariantSource> vcf = open_variant_source(genotype_path, true);      // the driver's order: index first
-        if (!vcf) return NPH_EOPEN_VCF;
-        const int64_t n_scored = scored_samples(*vcf, q);
-        std::unordered_map<std::string, std::vector<std::pair<int64_t, int64_t>>> spans;
+        GenotypeFiles files(std::vector<std::string>(genotype_paths, genotype_paths + n_genotypes));
+        std::string unopened;
+        if (!files.open(q, &unopened)) { g_err = "Could not open input VCF file " + unopened; return NPH_EOPEN_VCF; }     // the driver's order: index first
+        Spans spans;
         M.add_spans(spans);
-        if (!vcf->use_regions(spans, genotype_path)) {
-            vcf = open_variant_source(genotype_path, false);
-            if (!vcf) return NPH_EOPEN_VCF;
-        }
         VariantRecord rec;
-        int64_t nrec = 0;
-        while (vcf->next(rec)) { nrec++; M.match(rec); }
+        int64_t nrec = 0, seeks = 0;
+        for (size_t f = 0; f < files.paths.size(); f++) {
+            if (!files.prepare(f, spans)) { g_err = "Could not open input VCF file " + files.paths[f]; return NPH_EOPEN_VCF; }
+            VariantSource &vcf = *files.src[f];
+            while (vcf.next(rec)) { nrec++; M.match(rec); }
+            seeks += vcf.seeks();
+            files.src[f].reset();
+        }
         M.finish();
         for (size_t i = 0; i < sf.entries.size(); i++) { kind_out[i] = M.kind[i]; eaidx_out[i] = M.eaidx[i]; }
         *n_rows_out = (int64_t)sf.entries.size();
-        *n_samples_out = n_scored;
+        *n_samples_out = (int64_t)files.names.size();
         if (records_read_out) *records_read_out = nrec;
-        if (index_seeks_out) *index_seeks_out = vcf->seeks();
+        if (index_seeks_out) *index_seeks_out = seeks;
         return NPH_OK;
     } catch (const InputError &e) {
         g_err = e.what();
@@ -257,6 +255,8 @@ static const char *USAGE =
     "  nimpress [options] <scoredef> <genotypes.vcf|.bcf|.bed>\n"
     "  nimpress [options] <scoredef1>,<scoredef2>,... <genotypes.vcf|.bcf|.bed>   (one pass, a \"#score\" line per file; not in the reference)\n"
     "  nimpress [options] <scoredef> <genotypes.bgen>\n"
+    "  nimpress [options] <scoredef>[,<scoredef>...] <genotypes> [<genotypes> ...]   (several genotype files, e.g. one per\n"
+    "                     chromosome: scored exactly as their concatenation; not in the reference)\n"
     "  nimpress (-h | --help)\n"
     "  nimpress --version\n\n"
     "Options:\n"
@@ -310,7 +310,11 @@ static const char *USAGE =
     "                     order: exactly what a genotype file holding only them gives, cohort EAF,\n"
     "                     --maxmis and WARN lines included (not a reference option).\n"
     "  --samples=^<file>  Score every sample except those named in <file>; names the genotype file\n"
-    "                     lacks are ignored (not a reference option).\n";
+    "                     lacks are ignored (not a reference option).\n"
+    "Several genotype files (not a reference input): VCF/BCF files (text and BCF may be mixed), PLINK 1 filesets\n"
+    "  or BGEN files, one kind per run, read in the order given; a site in two files is matched in the earlier one.\n"
+    "  Every file must carry the same samples in the same order, or, with --samples, keep the same samples in the\n"
+    "  same order.\n";
 
 static int parse_enum(const std::string &v, std::initializer_list<const char *> names) {   // Nim parseEnum: style-insensitive beyond the first char is not reproduced
     int i = 0;
@@ -355,8 +359,8 @@ static void print_result(const nph_result *r) {
 
 int nph_main(int argc, char **argv) {
     nph_params p = { NPC_LOCUS_PS, NPC_MISSING_HOMREF, NPC_SAMPLE_INT_PS, 0, 0, 0, 0, 0, 100, 0.05, 0.001, 0, 0, nullptr, 0 };
-    std::string cov, samples_list, pos[2];
-    int npos = 0;
+    std::string cov, samples_list;
+    std::vector<std::string> pos;                          // <scoredef>, then the genotype files
     try {
         for (int i = 1; i < argc; i++) {
             std::string a = argv[i];
@@ -389,15 +393,17 @@ int nph_main(int argc, char **argv) {
             else if (a == "--dosage") p.use_ds = 1;
             else if (a == "--pl") p.use_pl = 1;
             else if (a.size() > 1 && a[0] == '-') throw InputError("unknown option " + a);
-            else if (npos < 2) pos[npos++] = a;
-            else throw InputError("too many arguments");
+            else pos.push_back(a);
         }
-        if (npos != 2) throw InputError("expected <scoredef> <genotypes.vcf|.bcf|.bed>");
+        if (pos.size() < 2) throw InputError("expected <scoredef> <genotypes> [<genotypes> ...]");
         if (!samples_list.empty()) p.samples_path = samples_list.c_str();
     } catch (const InputError &e) {
-        std::cerr << e.what() << "\n" << "Usage:\n  nimpress [options] <scoredef> <genotypes.vcf|.bcf|.bed>\n";
+        std::cerr << e.what() << "\n" << "Usage:\n  nimpress [options] <scoredef>[,<scoredef>...] <genotypes> [<genotypes> ...]\n";
         return 1;
     }
+    std::vector<const char *> geno;                        // several genotype files: scored as their concatenation (DESIGN.md 4.12)
+    for (size_t f = 1; f < pos.size(); f++) geno.push_back(pos[f].c_str());
+    const char *bed = p.use_cov ? cov.c_str() : nullptr;
     // several score files, one pass (not a reference feature) -- unless the whole argument names a file, as it would for the reference
     if (pos[0].find(',') != std::string::npos && access(pos[0].c_str(), F_OK) != 0) {
         std::vector<std::string> paths;
@@ -405,9 +411,8 @@ int nph_main(int argc, char **argv) {
         std::vector<const char *> cp;
         for (auto &s : paths) cp.push_back(s.c_str());
         std::vector<nph_result *> rs(paths.size(), nullptr);
-        int rc = nph_compute_polygenic_scores_multi(cp.data(), (int32_t)cp.size(), pos[1].c_str(), p.use_cov ? cov.c_str() : nullptr, &p, rs.data());
-        if (rc == NPH_EOPEN_VCF) { std::cout << "FATAL Could not open input VCF file " << pos[1] << "\n"; return 255; }
-        if (rc == NPH_EOPEN_SCORE) { std::cout << "FATAL " << nph_last_error() << "\n"; return 255; }
+        int rc = nph_compute_polygenic_scores_files(cp.data(), (int32_t)cp.size(), geno.data(), (int32_t)geno.size(), bed, &p, rs.data());
+        if (rc == NPH_EOPEN_VCF || rc == NPH_EOPEN_SCORE) { std::cout << "FATAL " << nph_last_error() << "\n"; return 255; }
         if (rc) { std::cerr << "nimpress: " << nph_last_error() << "\n"; return 1; }
         for (size_t k = 0; k < rs.size(); k++) {           // per file: a "#score" line, then the reference's output for it
             std::cout << "#score\t" << paths[k] << "\n";
@@ -417,9 +422,10 @@ int nph_main(int argc, char **argv) {
         return 0;
     }
     nph_result *r = nullptr;
-    int rc = nph_compute_polygenic_scores(pos[0].c_str(), pos[1].c_str(), p.use_cov ? cov.c_str() : nullptr, &p, &r);
-    if (rc == NPH_EOPEN_VCF) { std::cout << "FATAL Could not open input VCF file " << pos[1] << "\n"; return 255; }          // :729-730
-    if (rc == NPH_EOPEN_SCORE) { std::cout << "FATAL Could not open polygenic score file " << pos[0] << "\n"; return 255; } // :733-734
+    const char *score = pos[0].c_str();
+    int rc = nph_compute_polygenic_scores_files(&score, 1, geno.data(), (int32_t)geno.size(), bed, &p, &r);
+    // "FATAL Could not open input VCF file <path>" (:729-730), "FATAL Could not open polygenic score file <path>" (:733-734)
+    if (rc == NPH_EOPEN_VCF || rc == NPH_EOPEN_SCORE) { std::cout << "FATAL " << nph_last_error() << "\n"; return 255; }
     if (rc) { std::cerr << "nimpress: " << nph_last_error() << "\n"; return 1; }
     print_result(r);
     nph_result_free(r);

@@ -22,6 +22,14 @@ struct Cur {
 };
 }  // namespace
 
+bool RegionIndex::present(const std::string &data_path) {
+    struct stat si, sd;
+    if (stat(data_path.c_str(), &sd) != 0) return false;
+    for (const char *ext : { ".tbi", ".csi" })
+        if (stat((data_path + ext).c_str(), &si) == 0 && si.st_mtime >= sd.st_mtime) return true;
+    return false;
+}
+
 std::unique_ptr<RegionIndex> RegionIndex::load(const std::string &data_path) {
     for (int k = 0; k < 2; k++) {
         const std::string path = data_path + (k == 0 ? ".tbi" : ".csi");

@@ -22,6 +22,8 @@ public:
     static constexpr uint64_t NONE = ~0ull;
     // <path>.tbi, then <path>.csi; nullptr when neither exists or parses
     static std::unique_ptr<RegionIndex> load(const std::string &data_path);
+    // whether load() can find an index for data_path at all: <data_path>.tbi or .csi, not older than the data file
+    static bool present(const std::string &data_path);
     // Virtual file offset (BGZF: block offset << 16 | offset in block) from which every record of
     // reference `ref` overlapping [beg0, end0) (0-based, half open) lies at or after; NONE: no such record.
     uint64_t query_start(int ref, int64_t beg0, int64_t end0) const;

@@ -91,6 +91,8 @@ proc npc_create_subset*(ctx: ptr NpcCtx; device: cint; nRowSamples: int64; keep:
                         maxRowsPerBlock: int64; nSlots: int32; stagingRows: int64): cint
   ## scores keep[0 ..< nKeep] (ascending) of the nRowSamples samples of the staged rows; compacts them on the device
 proc npc_gather_rows_device*(ctx: NpcCtx; src: pointer; srcStride, nRows: int64; dst: pointer; dstStride: int64): cint
+proc npc_set_keep*(ctx: NpcCtx; keep: ptr int64; nKeep: int64): cint
+  ## replaces the keep list of a subset context for rows uploaded after the call (several genotype files)
 proc npc_set_dosage_rows*(ctx: NpcCtx; on: int32): cint
 proc npc_trace*(ctx: NpcCtx; stamps: ptr array[8, uint64]): cint
 # several GPUs: one process (npc_reduce) or one process per GPU over NCCL (npc_comm_*)
