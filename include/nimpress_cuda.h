@@ -383,13 +383,13 @@ int npc_set_dosage_rows(npc_ctx *ctx, int32_t on);
 /* Which kernels npc_score_block* uses for this context: shape[0] = 2 for the fused tile kernel in
  * its default mode, 1 in exact-order mode (int8 / int16 diploid cohorts that fit one resident pass),
  * 3 for cohorts too wide for that (> ~1.2 M samples per GPU: tally + decide over all samples, then the
- * tile kernel in "decided" mode once per slab of the sample axis), 4 for NPC_GT_BED rows (k_count_bed,
+ * tile kernel in "decided" mode once per slab of the sample axis), 4 for NPC_GT_BED rows (k_count_chunks,
  * k_decide, k_accum_bed; then shape[1] = CTAs of the accumulate pass, shape[2] = warps per CTA,
  * shape[3] = samples per thread, shape[4] = rows per tile: 4 in the default mode, 1 in exact order),
- * 5 for NPC_GT_DOSE255 rows (k_count_dose255, k_decide_dose255, k_accum_dose255; then shape[1] = CTAs of the
- * accumulate pass, shape[2] = warps per CTA, shape[3] = 8 samples per thread), 6 for NPC_GT_DOSE32 rows (k_count_dose32,
- * k_decide_dose32, k_accum_dose32; shape[1..3] as for 5, with 4 samples per thread), 7 for NPC_GT_PL rows (k_count_pl,
- * k_decide_pl, k_accum_pl; shape[1..3] as for 6), 0 for the count/decide/accumulate sequence; then grid (tile kernel: sample slabs * 1000 + row
+ * 5 for NPC_GT_DOSE255 rows (k_count_chunks, k_decide, k_accum_dose255; then shape[1] = CTAs of the
+ * accumulate pass, shape[2] = warps per CTA, shape[3] = 8 samples per thread), 6 for NPC_GT_DOSE32 rows (k_count_chunks,
+ * k_decide, k_accum_dose32; shape[1..3] as for 5, with 4 samples per thread), 7 for NPC_GT_PL rows (k_count_pl,
+ * k_decide, k_accum_pl; shape[1..3] as for 6), 0 for the count/decide/accumulate sequence; then grid (tile kernel: sample slabs * 1000 + row
  * groups), consumer warps, chunks per thread, rows
  * per tile, raw stages * 1000 + index-ring tiles, lag * 100 + tiles per decider pass * 10 + decider warps, dynamic
  * shared-memory bytes. */

@@ -25,10 +25,54 @@ using namespace npc;
 
 static thread_local std::string g_create_error;
 
+// The layout of a context's genotype rows, set once from gt_width by npc_create*; npc_set_dosage_rows switches a ploidy-1,
+// width-4 context between GT and DS.
+enum class Layout { GT, DS, BED, DOSE255, DOSE32, PL };
+
+// What the launcher knows of each layout, indexed by Layout.
+struct LayoutInfo {
+    const char *name;                       // in error messages
+    int32_t sample_bits;                    // bits per sample of a row (0: ploidy x width bytes)
+    int32_t header;                         // bytes of a row before its first sample
+    bool diploid;                           // the context's ploidy must be 2
+    bool one_alt;                           // a decoded row names REF (eaidx 0) or the one ALT (eaidx 1)
+    bool real_tally;                        // tally: one count word a row (missing samples), the called dosages' block sums in d_ds_part
+    int32_t mode;                           // npc_kernel_shape mode (0: the GT path's choice, launch_mode)
+    int32_t threads, per_thread;            // accumulate pass of modes 4-7: threads per CTA, samples per thread
+    int32_t chunk;                          // k_count_chunks: samples per 16-byte chunk (0: another tally)
+};
+static constexpr LayoutInfo LAYOUTS[] = {
+    { "BCF GT rows", 0, 0, false, false, false, 0, 0, 0, 0 },
+    { "FORMAT/DS rows", 0, 0, false, false, true, 0, 0, 0, 0 },
+    { "PLINK .bed rows", 2, Bed::HEADER, true, true, false, 4, BED_THREADS, 8, Bed::PER16 },
+    { "BGEN dosage rows", 16, Dose255::HEADER, true, true, false, 5, D255_THREADS, 8, Dose255::PER16 },
+    { "BGEN dosage rows", 32, Dose32::HEADER, true, true, false, 6, D32_THREADS, 4, Dose32::PER16 },
+    { "FORMAT/PL rows", 32, 0, true, true, true, 7, PL_THREADS, 4, 0 },
+};
+static const LayoutInfo &info(Layout l) { return LAYOUTS[(int)l]; }
+
+// The layout of a gt_width; false for none.
+static bool layout_of(int32_t gt_width, Layout &l) {
+    switch (gt_width) {
+    case 1: case 2: case 4: l = Layout::GT; return true;
+    case NPC_GT_BED: l = Layout::BED; return true;
+    case NPC_GT_DOSE255: l = Layout::DOSE255; return true;
+    case NPC_GT_DOSE32: l = Layout::DOSE32; return true;
+    case NPC_GT_PL: l = Layout::PL; return true;
+    }
+    return false;
+}
+
+static int64_t row_bytes(Layout l, int64_t n_samples, int32_t ploidy, int32_t width) {
+    const LayoutInfo &L = info(l);
+    return L.sample_bits ? L.header + (n_samples * L.sample_bits + 7) / 8 : n_samples * ploidy * width;
+}
+
 struct npc_ctx {
     int device = 0;
     int64_t n = 0;
-    int32_t ploidy = 2, width = 1;
+    Layout layout = Layout::GT;
+    int32_t ploidy = 2, width = 1;          // width: bytes of a GT allele value (1, 2 or 4); 0 in the other layouts
     int64_t max_rows = 0;
     int64_t staging_rows = 0;               // rows per pinned staging slot (<= max_rows)
     int32_t n_slots = 0;
@@ -86,20 +130,9 @@ struct npc_ctx {
     size_t multi_scratch_bytes = 0;
     bool multi_attr_set = false;
     int64_t multi_contractions = 0;         // npc_score_resident_multi calls served by the tensor-core contraction
-    // FORMAT/DS rows (npc_dosage.cuh): fp32 dosages, one per sample
-    bool ds = false;
-    double *d_ds_part = nullptr;            // [max_rows][n_blocks] block sums of the tally pass
-    // PLINK 1 .bed rows (npc_bed.cuh, gt_width = NPC_GT_BED): 2 bits per sample
-    bool bed = false;
-    double *d_bed_tab = nullptr;            // per batch of BED_RB rows: the accumulate pass's value tables
+    double *d_ds_part = nullptr;            // FORMAT/DS and FORMAT/PL rows: [max_rows][n_blocks] block sums of the tally pass
+    double *d_bed_tab = nullptr;            // PLINK .bed rows, per batch of BED_RB rows: the accumulate pass's value tables
     int32_t *d_bed_off = nullptr;           // ... and the slab row of every row it loads
-    // fixed-point dosage rows from BGEN files (npc_dose255.cuh, gt_width = NPC_GT_DOSE255): uint16 per sample
-    bool dose255 = false;
-    // 32-bit fixed-point dosage rows from BGEN files at any bit depth (npc_dose32.cuh, gt_width = NPC_GT_DOSE32): a 16-byte
-    // header holding the row's denominator, then uint32 per sample
-    bool dose32 = false;
-    // FORMAT/PL rows (npc_pl.cuh, gt_width = NPC_GT_PL): a packed uint32 per sample; tallied as FORMAT/DS rows, into d_ds_part
-    bool pl = false;
     // cross-GPU combine (npc_reduce.cuh)
     cudaEvent_t ev_multi = nullptr;         // npc_score_resident_multi: orders its copy-stream work against the compute stream
     cudaEvent_t ev_reduce = nullptr;        // "this context's partial sums are final"
@@ -130,12 +163,12 @@ static int fail(npc_ctx *ctx, int code, const char *msg) {
 extern "C" int npc_version(void) { return 200; }
 
 extern "C" int64_t npc_gt_row_bytes(int64_t n_samples, int32_t ploidy, int32_t gt_width) {
-    if (gt_width == NPC_GT_BED) return (n_samples + 3) / 4;
-    if (gt_width == NPC_GT_DOSE255) return n_samples * 2;
-    if (gt_width == NPC_GT_DOSE32) return D32_HEADER + n_samples * 4;
-    if (gt_width == NPC_GT_PL) return n_samples * 4;
-    return n_samples * ploidy * gt_width;
+    Layout l = Layout::GT;
+    layout_of(gt_width, l);
+    return row_bytes(l, n_samples, ploidy, gt_width);
 }
+
+static int64_t ctx_row_bytes(const npc_ctx *c, int64_t n_samples) { return row_bytes(c->layout, n_samples, c->ploidy, c->width); }
 
 extern "C" int npc_pl_weight_table(double *out, int32_t n) {
     static const double tab[PL_TN] = { NPC_PL_TABLE_VALUES };
@@ -355,11 +388,11 @@ static int create_impl(npc_ctx *c) {
     NPC_CUDA(c, cudaMalloc(&c->d_rowp, r1 * sizeof(RowP)));
     c->log_cap = std::max<int64_t>(r1, 1024);
     NPC_CUDA(c, cudaMalloc(&c->d_log, c->log_cap * sizeof(npc_locus)));
-    c->row_stride = ((npc_gt_row_bytes(c->n, c->ploidy, c->width) + 127) / 128) * 128;
+    c->row_stride = ((ctx_row_bytes(c, c->n) + 127) / 128) * 128;
     if (c->row_stride == 0) c->row_stride = 128;
     c->stage_stride = c->row_stride;
     if (c->sub) {
-        c->stage_stride = std::max<int64_t>(128, ((npc_gt_row_bytes(c->n_row, c->ploidy, c->width) + 127) / 128) * 128);
+        c->stage_stride = std::max<int64_t>(128, ((ctx_row_bytes(c, c->n_row) + 127) / 128) * 128);
         c->keep.resize((size_t)((c->n + SUB_PAD - 1) / SUB_PAD * SUB_PAD), 0);
         NPC_CUDA(c, cudaMalloc(&c->d_keep, c->keep.size() * sizeof(int32_t)));
         NPC_CUDA(c, cudaMemcpy(c->d_keep, c->keep.data(), c->keep.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
@@ -393,10 +426,8 @@ static int create_ctx(npc_ctx **out, int device, int64_t n_row, const int64_t *k
                       int32_t gt_width, int64_t max_rows_per_block, int32_t n_slots, int64_t staging_rows) {
     if (!out) return NPC_EINVAL;
     *out = nullptr;
-    if (n_samples < 0 || ploidy < 1 || ploidy > 64 ||
-        (gt_width != 1 && gt_width != 2 && gt_width != 4 && gt_width != NPC_GT_BED && gt_width != NPC_GT_DOSE255 &&
-         gt_width != NPC_GT_DOSE32 && gt_width != NPC_GT_PL) ||
-        ((gt_width == NPC_GT_BED || gt_width == NPC_GT_DOSE255 || gt_width == NPC_GT_DOSE32 || gt_width == NPC_GT_PL) && ploidy != 2) ||
+    Layout layout = Layout::GT;
+    if (n_samples < 0 || ploidy < 1 || ploidy > 64 || !layout_of(gt_width, layout) || (info(layout).diploid && ploidy != 2) ||
         max_rows_per_block < 1 || n_slots < 0 || n_slots == 1 || staging_rows < 1 || staging_rows > max_rows_per_block) {
         g_create_error = "npc_create: invalid argument";
         return NPC_EINVAL;
@@ -408,8 +439,7 @@ static int create_ctx(npc_ctx **out, int device, int64_t n_row, const int64_t *k
         c->keep.resize((size_t)n_samples);
         for (int64_t i = 0; i < n_samples; i++) c->keep[(size_t)i] = (int32_t)keep[i];
     }
-    c->device = device; c->n = n_samples; c->ploidy = ploidy; c->width = gt_width; c->bed = gt_width == NPC_GT_BED;
-    c->dose255 = gt_width == NPC_GT_DOSE255; c->dose32 = gt_width == NPC_GT_DOSE32; c->pl = gt_width == NPC_GT_PL;
+    c->device = device; c->n = n_samples; c->ploidy = ploidy; c->layout = layout; c->width = layout == Layout::GT ? gt_width : 0;
     c->max_rows = max_rows_per_block; c->n_slots = n_slots; c->staging_rows = staging_rows;
     c->pol.imp_locus = NPC_LOCUS_PS; c->pol.imp_missing = NPC_MISSING_HOMREF; c->pol.imp_sample = NPC_SAMPLE_INT_PS;
     c->pol.mincs = 100; c->pol.maxmis = 0.05; c->pol.n_total = n_samples;      // defaults of main (:670-687)
@@ -505,10 +535,7 @@ static const npc_ctx::TileCfg &fast_config(const npc_ctx *c, int64_t n_rows) {
 // t: the tile kernel's shape in modes 1-3.
 static int launch_mode(const npc_ctx *c, bool exact, int64_t n_rows, const npc_ctx::TileCfg *&t) {
     t = nullptr;
-    if (c->bed) return 4;
-    if (c->dose255) return 5;
-    if (c->dose32) return 6;
-    if (c->pl) return 7;
+    if (const int mode = info(c->layout).mode) return mode;
     t = exact ? &c->exact_cfg : &fast_config(c, n_rows);
     if (t->ok) return exact ? 1 : 2;
     t = exact ? &c->wide_exact : &c->wide;
@@ -520,15 +547,11 @@ extern "C" int npc_kernel_shape2(const npc_ctx *ctx, int64_t n_rows, int32_t sha
     memset(shape, 0, 8 * sizeof(int32_t));
     const npc_ctx::TileCfg *t;
     shape[0] = launch_mode(ctx, ctx->exact, n_rows, t);
-    if (shape[0] == 4) {
-        shape[1] = (int32_t)((ctx->n + 8 * BED_THREADS - 1) / (8 * BED_THREADS)); shape[2] = BED_THREADS / 32;
-        shape[3] = 8; shape[4] = ctx->exact ? 1 : 4;
-    } else if (shape[0] == 5) {
-        shape[1] = (int32_t)((ctx->n + 8 * D255_THREADS - 1) / (8 * D255_THREADS)); shape[2] = D255_THREADS / 32; shape[3] = 8;
-    } else if (shape[0] == 6) {
-        shape[1] = (int32_t)((ctx->n + 4 * D32_THREADS - 1) / (4 * D32_THREADS)); shape[2] = D32_THREADS / 32; shape[3] = 4;
-    } else if (shape[0] == 7) {
-        shape[1] = (int32_t)((ctx->n + 4 * PL_THREADS - 1) / (4 * PL_THREADS)); shape[2] = PL_THREADS / 32; shape[3] = 4;
+    if (shape[0] >= 4) {
+        const LayoutInfo &L = info(ctx->layout);
+        const int64_t per_cta = (int64_t)L.threads * L.per_thread;
+        shape[1] = (int32_t)((ctx->n + per_cta - 1) / per_cta); shape[2] = L.threads / 32; shape[3] = L.per_thread;
+        if (ctx->layout == Layout::BED) shape[4] = ctx->exact ? 1 : 4;
     } else if (shape[0]) {
         shape[1] = t->Gs * 1000 + t->Gr; shape[2] = t->nc; shape[3] = t->K;
         shape[4] = F5_R; shape[5] = t->Sr * 1000 + t->Sc; shape[6] = t->L * 100 + t->GD * 10 + t->A; shape[7] = (int32_t)t->smem;
@@ -559,9 +582,10 @@ extern "C" int npc_plan_shape(int64_t n_samples, int32_t gt_width, int32_t num_s
 
 extern "C" int npc_set_dosage_rows(npc_ctx *ctx, int32_t on) {
     if (!ctx) return NPC_EINVAL;
-    if (on && (ctx->width != 4 || ctx->ploidy != 1 || ctx->bed))
+    const bool can = ctx->width == 4 && ctx->ploidy == 1;                   // a GT or DS context
+    if (on && !can)
         return fail(ctx, NPC_EINVAL, "npc_set_dosage_rows: create the context with ploidy 1 and gt_width 4 (one fp32 DS value per sample)");
-    ctx->ds = on != 0;
+    if (can) ctx->layout = on ? Layout::DS : Layout::GT;
     return NPC_OK;
 }
 
@@ -591,18 +615,18 @@ static int check_block(npc_ctx *c, const void *gt, int64_t row_stride, int64_t n
     if (n_rows < 0 || n_gt_rows < 0 || n_rows > c->max_rows || n_gt_rows > c->max_rows)
         return fail(c, NPC_EINVAL, "block larger than max_rows_per_block");
     if (n_rows && !rows) return fail(c, NPC_EINVAL, "rows is NULL");
-    if (n_gt_rows && (!gt || ((uintptr_t)gt & 15) || (row_stride & 15) || row_stride < npc_gt_row_bytes(c->n, c->ploidy, c->width)))
+    if (n_gt_rows && (!gt || ((uintptr_t)gt & 15) || (row_stride & 15) || row_stride < ctx_row_bytes(c, c->n)))
         return fail(c, NPC_EINVAL, "genotype slab must be 16-byte aligned with row_stride % 16 == 0 and >= the bytes of a row");
     return NPC_OK;
 }
 
-// .bed and dosage rows carry one ALT: a decoded row names REF (0) or that ALT (1).  Checked where the rows are on the host.
-static int check_bed_rows(npc_ctx *c, const npc_row *rows, int64_t n_rows, int on_device) {
-    if (!(c->bed || c->dose255 || c->dose32 || c->pl) || on_device) return NPC_OK;
+// .bed, BGEN and PL rows carry one ALT: a decoded row names REF (0) or that ALT (1).  Checked where the rows are on the host.
+static int check_one_alt(npc_ctx *c, const npc_row *rows, int64_t n_rows, int on_device) {
+    if (!info(c->layout).one_alt || on_device) return NPC_OK;
     for (int64_t i = 0; i < n_rows; i++)
         if (rows[i].kind == NPC_KIND_GT && rows[i].gt_row >= 0 && rows[i].eaidx != 0 && rows[i].eaidx != 1)
-            return fail(c, NPC_EINVAL, c->bed ? "PLINK .bed rows: the effect allele of a genotype row is REF (eaidx 0) or the one ALT (eaidx 1)"
-                                              : "dosage rows: the effect allele of a genotype row is REF (eaidx 0) or the one ALT (eaidx 1)");
+            return fail(c, NPC_EINVAL, (std::string(info(c->layout).name) +
+                                        ": the effect allele of a genotype row is REF (eaidx 0) or the one ALT (eaidx 1)").c_str());
     return NPC_OK;
 }
 
@@ -626,35 +650,16 @@ static unsigned tally_grid_y(int64_t units, int64_t n_rows, int64_t min_units) {
 // block sums of the called dosages go to d_ds_part.
 static int launch_tally(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows,
                         ull *counts) {
-    NPC_CUDA(c, cudaMemsetAsync(counts, 0, n_rows * (c->ds || c->pl ? 1 : 2) * sizeof(ull), c->stream));
+    const LayoutInfo &L = info(c->layout);
+    NPC_CUDA(c, cudaMemsetAsync(counts, 0, n_rows * (L.real_tally ? 1 : 2) * sizeof(ull), c->stream));
     if (n_rows == 0 || c->n == 0) return NPC_OK;
     const int64_t n_blocks = (c->n + DS_BLOCK - 1) / DS_BLOCK;
-    if ((c->ds || c->pl) && !c->d_ds_part)
+    if (L.real_tally && !c->d_ds_part)
         NPC_CUDA(c, cudaMalloc(&c->d_ds_part, (size_t)std::max<int64_t>(c->max_rows, 1) * (size_t)n_blocks * sizeof(double)));
-    if (c->pl) {
-        // a CTA loads T once and takes every gridDim.y-th row: about 4096 CTAs in all
-        const unsigned gx = (unsigned)((n_blocks + 7) / 8);
-        const unsigned gy = (unsigned)std::min<int64_t>(n_rows, std::max<int64_t>(1, (4096 + gx - 1) / gx));
-        k_count_pl<<<dim3(gx, gy), 256, 0, c->stream>>>(gt, row_stride, d_rows, n_rows, c->n, n_blocks, c->d_ds_part, counts);
-        c->launches++;
-    } else if (c->ds) {
-        for (int64_t r0 = 0; r0 < n_rows; r0 += 65535) {                                        // grid y: at most 65,535 rows
-            const int64_t nr = std::min<int64_t>(65535, n_rows - r0);
-            k_count_ds<<<dim3((unsigned)((n_blocks + 7) / 8), (unsigned)nr), 256, 0, c->stream>>>(gt, row_stride, d_rows + r0, c->n, n_blocks,
-                                                                                               c->d_ds_part + r0 * n_blocks, counts + r0);
-            c->launches++;
-        }
-    } else {
-        if (c->bed) {
-            const unsigned slabs = tally_grid_y((c->n + 63) / 64, n_rows, 1024);             // units: chunks of 64 samples
-            k_count_bed<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
-        } else if (c->dose255) {
-            const unsigned slabs = tally_grid_y((c->n + 7) / 8, n_rows, 1024);               // units: chunks of 8 samples
-            k_count_dose255<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
-        } else if (c->dose32) {
-            const unsigned slabs = tally_grid_y((c->n + 3) / 4, n_rows, 1024);               // units: chunks of 4 samples
-            k_count_dose32<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
-        } else if (c->width == 1 && c->ploidy == 2) {
+    void (*chunks)(const uint8_t *, int64_t, const npc_row *, int64_t, ull *) = nullptr;
+    switch (c->layout) {
+    case Layout::GT:
+        if (c->width == 1 && c->ploidy == 2) {
             const unsigned slabs = tally_grid_y((c->n + 7) / 8, n_rows, 1024);               // units: chunks of 8 samples
             k_count_i8x2<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
         } else {
@@ -663,6 +668,31 @@ static int launch_tally(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const
             else if (c->width == 2) k_count_generic<int16_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->ploidy, counts);
             else k_count_generic<int32_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, c->ploidy, counts);
         }
+        c->launches++;
+        break;
+    case Layout::DS:
+        for (int64_t r0 = 0; r0 < n_rows; r0 += 65535) {                                        // grid y: at most 65,535 rows
+            const int64_t nr = std::min<int64_t>(65535, n_rows - r0);
+            k_count_ds<<<dim3((unsigned)((n_blocks + 7) / 8), (unsigned)nr), 256, 0, c->stream>>>(gt, row_stride, d_rows + r0, c->n, n_blocks,
+                                                                                               c->d_ds_part + r0 * n_blocks, counts + r0);
+            c->launches++;
+        }
+        break;
+    case Layout::PL: {
+        // a CTA loads T once and takes every gridDim.y-th row: about 4096 CTAs in all
+        const unsigned gx = (unsigned)((n_blocks + 7) / 8);
+        const unsigned gy = (unsigned)std::min<int64_t>(n_rows, std::max<int64_t>(1, (4096 + gx - 1) / gx));
+        k_count_pl<<<dim3(gx, gy), 256, 0, c->stream>>>(gt, row_stride, d_rows, n_rows, c->n, n_blocks, c->d_ds_part, counts);
+        c->launches++;
+        break;
+    }
+    case Layout::BED: chunks = k_count_chunks<Bed>; break;
+    case Layout::DOSE255: chunks = k_count_chunks<Dose255>; break;
+    case Layout::DOSE32: chunks = k_count_chunks<Dose32>; break;
+    }
+    if (chunks) {
+        const unsigned slabs = tally_grid_y((c->n + L.chunk - 1) / L.chunk, n_rows, 1024);     // units: chunks
+        chunks<<<dim3((unsigned)n_rows, slabs), 256, 0, c->stream>>>(gt, row_stride, d_rows, c->n, counts);
         c->launches++;
     }
     NPC_CUDA(c, cudaGetLastError());
@@ -675,20 +705,17 @@ static int launch_decide(npc_ctx *c, const uint8_t *gt, int64_t row_stride, cons
     if (n_rows == 0) return NPC_OK;
     int rc = ensure_log(c, n_rows);
     if (rc) return rc;
-    const unsigned grid = (unsigned)((n_rows + 127) / 128);
-    if (c->pl)
-        k_decide_pl<<<grid, 128, 0, c->stream>>>(d_rows, n_rows, c->d_ds_part, (c->n + DS_BLOCK - 1) / DS_BLOCK, counts, c->pol, c->n,
-                                                c->d_rowp, c->d_log + c->log_len, c->d_nloci);
-    else if (c->ds)
-        k_decide_ds<<<grid, 128, 0, c->stream>>>(d_rows, n_rows, c->d_ds_part, (c->n + DS_BLOCK - 1) / DS_BLOCK, counts, c->pol, c->n,
-                                                c->d_rowp, c->d_log + c->log_len, c->d_nloci);
-    else if (c->dose255)
-        k_decide_dose255<<<grid, 128, 0, c->stream>>>(d_rows, n_rows, counts, c->pol, c->n, c->d_rowp, c->d_log + c->log_len, c->d_nloci);
-    else if (c->dose32)
-        k_decide_dose32<<<grid, 128, 0, c->stream>>>(gt, row_stride, d_rows, n_rows, counts, c->pol, c->n, c->d_rowp,
-                                                     c->d_log + c->log_len, c->d_nloci);
-    else
-        k_decide<<<grid, 128, 0, c->stream>>>(d_rows, n_rows, counts, c->pol, c->n, c->d_rowp, c->d_log + c->log_len, c->d_nloci);
+    auto decide = k_decide<CountTally>;
+    switch (c->layout) {
+    case Layout::GT: case Layout::BED: break;
+    case Layout::DS: decide = k_decide<DsTally>; break;
+    case Layout::DOSE255: decide = k_decide<Dose255::Tally>; break;
+    case Layout::DOSE32: decide = k_decide<Dose32::Tally>; break;
+    case Layout::PL: decide = k_decide<PlTally>; break;
+    }
+    const TallyIn in = { gt, row_stride, counts, c->d_ds_part, (c->n + DS_BLOCK - 1) / DS_BLOCK };
+    decide<<<(unsigned)((n_rows + 127) / 128), 128, 0, c->stream>>>(in, d_rows, n_rows, c->pol, c->n, c->d_rowp, c->d_log + c->log_len,
+                                                                  c->d_nloci);
     c->launches++;
     NPC_CUDA(c, cudaGetLastError());
     c->log_len += n_rows;
@@ -698,9 +725,25 @@ static int launch_decide(npc_ctx *c, const uint8_t *gt, int64_t row_stride, cons
 // The decided rows' contributions (d_rowp) added to the sums
 static int launch_accum(npc_ctx *c, const uint8_t *gt, int64_t row_stride, int64_t n_rows) {
     if (n_rows == 0 || c->n == 0) return NPC_OK;
-    if (c->ds) {
+    const LayoutInfo &L = info(c->layout);
+    const unsigned grid = L.threads ? (unsigned)((c->n + L.threads * L.per_thread - 1) / (L.threads * L.per_thread)) : 0;   // modes 4-7
+    switch (c->layout) {
+    case Layout::GT:
+        if (c->width == 1 && c->ploidy == 2) {
+            const int64_t nchunks = (c->n + 7) / 8;
+            k_accum_i8x2<64, 8><<<(unsigned)((nchunks + 255) / 256), 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows,
+                                                                                         c->n, c->d_sums);
+        } else {
+            const unsigned grid = (unsigned)((c->n + 255) / 256);
+            if (c->width == 1) k_accum_generic<int8_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
+            else if (c->width == 2) k_accum_generic<int16_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
+            else k_accum_generic<int32_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
+        }
+        break;
+    case Layout::DS:
         k_accum_ds<<<(unsigned)((c->n + 255) / 256), 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->d_sums);
-    } else if (c->bed) {
+        break;
+    case Layout::BED: {
         const int64_t n_batches = (n_rows + BED_RB - 1) / BED_RB, E = c->exact ? BED_RB * 4 : BED_RB * 8;
         if (!c->d_bed_tab) {
             const int64_t max_batches = (std::max<int64_t>(c->max_rows, 1) + BED_RB - 1) / BED_RB;
@@ -708,7 +751,6 @@ static int launch_accum(npc_ctx *c, const uint8_t *gt, int64_t row_stride, int64
             NPC_CUDA(c, cudaMalloc(&c->d_bed_off, (size_t)max_batches * BED_RB * sizeof(int32_t)));
         }
         const unsigned pgrid = (unsigned)((n_batches * E + 255) / 256);
-        const unsigned grid = (unsigned)((c->n + 8 * BED_THREADS - 1) / (8 * BED_THREADS));
         if (c->exact) {
             k_bed_prep<true><<<pgrid, 256, 0, c->stream>>>(c->d_rowp, n_rows, n_batches, c->d_bed_tab, c->d_bed_off);
             k_accum_bed<true><<<grid, BED_THREADS, 0, c->stream>>>(gt, row_stride, c->d_bed_tab, c->d_bed_off, n_rows, c->n, c->d_sums);
@@ -717,24 +759,17 @@ static int launch_accum(npc_ctx *c, const uint8_t *gt, int64_t row_stride, int64
             k_accum_bed<false><<<grid, BED_THREADS, 0, c->stream>>>(gt, row_stride, c->d_bed_tab, c->d_bed_off, n_rows, c->n, c->d_sums);
         }
         c->launches++;                                                                          // k_bed_prep
-    } else if (c->dose255) {
-        const unsigned grid = (unsigned)((c->n + 8 * D255_THREADS - 1) / (8 * D255_THREADS));
+        break;
+    }
+    case Layout::DOSE255:
         k_accum_dose255<<<grid, D255_THREADS, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->d_sums);
-    } else if (c->dose32) {
-        const unsigned grid = (unsigned)((c->n + 4 * D32_THREADS - 1) / (4 * D32_THREADS));
+        break;
+    case Layout::DOSE32:
         k_accum_dose32<<<grid, D32_THREADS, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->d_sums);
-    } else if (c->pl) {
-        const unsigned grid = (unsigned)((c->n + 4 * PL_THREADS - 1) / (4 * PL_THREADS));
+        break;
+    case Layout::PL:
         k_accum_pl<<<grid, PL_THREADS, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->d_sums);
-    } else if (c->width == 1 && c->ploidy == 2) {
-        const int64_t nchunks = (c->n + 7) / 8;
-        k_accum_i8x2<64, 8><<<(unsigned)((nchunks + 255) / 256), 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows,
-                                                                                     c->n, c->d_sums);
-    } else {
-        const unsigned grid = (unsigned)((c->n + 255) / 256);
-        if (c->width == 1) k_accum_generic<int8_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
-        else if (c->width == 2) k_accum_generic<int16_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
-        else k_accum_generic<int32_t><<<grid, 256, 0, c->stream>>>(gt, row_stride, c->d_rowp, n_rows, c->n, c->ploidy, c->d_sums);
+        break;
     }
     c->launches++;
     NPC_CUDA(c, cudaGetLastError());
@@ -831,16 +866,18 @@ static int launch_block(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const
 static int launch_gather(npc_ctx *c, const uint8_t *src, int64_t src_stride, int64_t n_rows, uint8_t *dst, int64_t dst_stride,
                          cudaStream_t st) {
     if (n_rows == 0) return NPC_OK;
-    const int64_t E = c->bed ? 0 : c->dose255 ? 2 : (c->dose32 || c->pl) ? 4 : (int64_t)c->ploidy * c->width;
-    const int hdr = c->dose32 ? D32_HEADER : 0;
+    const LayoutInfo &L = info(c->layout);
+    const bool bed = c->layout == Layout::BED;
+    const int64_t E = L.sample_bits ? L.sample_bits / 8 : (int64_t)c->ploidy * c->width;             // bytes per sample (.bed: 0)
+    const int hdr = L.header;
     // threads per row: one per 16 output bytes (2- and 4-byte samples), 4 bytes (.bed) or unit; a grid-stride loop beyond
-    const int64_t per_row = c->bed ? (c->n + 15) / 16 : (E == 2 || E == 4) ? (c->n * E + 15) / 16 : c->n * (E % 4 ? E : E / 4);
+    const int64_t per_row = bed ? (c->n + 15) / 16 : (E == 2 || E == 4) ? (c->n * E + 15) / 16 : c->n * (E % 4 ? E : E / 4);
     const unsigned gx = (unsigned)std::max<int64_t>(1, std::min<int64_t>((per_row + SUB_THREADS - 1) / SUB_THREADS, 1024));
     for (int64_t r0 = 0; r0 < n_rows; r0 += 65535) {                                            // grid y: at most 65,535 rows
         const dim3 grid(gx, (unsigned)std::min<int64_t>(65535, n_rows - r0));
         const uint8_t *s = src + r0 * src_stride;
         uint8_t *d = dst + r0 * dst_stride;
-        if (c->bed) k_gather_bed<<<grid, SUB_THREADS, 0, st>>>(s, src_stride, d, dst_stride, c->d_keep, c->n);
+        if (bed) k_gather_bed<<<grid, SUB_THREADS, 0, st>>>(s, src_stride, d, dst_stride, c->d_keep, c->n);
         else if (E == 2) k_gather_vec<uint16_t><<<grid, SUB_THREADS, 0, st>>>(s, src_stride, d, dst_stride, c->d_keep, c->n, hdr);
         else if (E == 4) k_gather_vec<uint32_t><<<grid, SUB_THREADS, 0, st>>>(s, src_stride, d, dst_stride, c->d_keep, c->n, hdr);
         else if (E % 4 == 0) k_gather_unit<uint32_t><<<grid, SUB_THREADS, 0, st>>>(s, src_stride, d, dst_stride, c->d_keep, c->n, (int)(E / 4));
@@ -855,7 +892,7 @@ extern "C" int npc_gather_rows_device(npc_ctx *ctx, const void *src, int64_t src
     if (!ctx) return NPC_EINVAL;
     if (!ctx->sub) return fail(ctx, NPC_ESTATE, "npc_gather_rows_device: the context was not created with npc_create_subset");
     if (n_rows < 0 || (n_rows && (!src || !dst)) || ((uintptr_t)src & 15) || ((uintptr_t)dst & 15) || (src_stride & 15) || (dst_stride & 15) ||
-        src_stride < npc_gt_row_bytes(ctx->n_row, ctx->ploidy, ctx->width) || dst_stride < npc_gt_row_bytes(ctx->n, ctx->ploidy, ctx->width))
+        src_stride < ctx_row_bytes(ctx, ctx->n_row) || dst_stride < ctx_row_bytes(ctx, ctx->n))
         return fail(ctx, NPC_EINVAL, "npc_gather_rows_device: rows must be 16-byte aligned, strides multiples of 16 holding a whole row");
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     return launch_gather(ctx, (const uint8_t *)src, src_stride, n_rows, (uint8_t *)dst, dst_stride, ctx->stream);
@@ -911,7 +948,7 @@ extern "C" int npc_score_block(npc_ctx *ctx, int32_t slot, int64_t n_gt_rows, co
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     if (!ctx->d_gt[slot]) NPC_CUDA(ctx, cudaMalloc(&ctx->d_gt[slot], (size_t)ctx->row_stride * (size_t)std::max<int64_t>(ctx->staging_rows, 1)));
     int rc = check_block(ctx, ctx->d_gt[slot], ctx->row_stride, n_gt_rows, rows, n_rows);
-    if (!rc) rc = check_bed_rows(ctx, rows, n_rows, 0);
+    if (!rc) rc = check_one_alt(ctx, rows, n_rows, 0);
     if (rc) return rc;
     if (n_gt_rows && ctx->sub) {
         if ((rc = upload_compact(ctx, slot, n_gt_rows, ctx->d_gt[slot], ctx->row_stride))) return rc;
@@ -935,7 +972,7 @@ extern "C" int npc_score_block(npc_ctx *ctx, int32_t slot, int64_t n_gt_rows, co
 extern "C" int npc_score_block_device(npc_ctx *ctx, const void *gt_dev, int64_t row_stride, int64_t n_gt_rows,
                                       const npc_row *rows, int64_t n_rows, int32_t rows_on_device) {
     int rc = check_block(ctx, gt_dev, row_stride, n_gt_rows, rows, n_rows);
-    if (!rc) rc = check_bed_rows(ctx, rows, n_rows, rows_on_device);
+    if (!rc) rc = check_one_alt(ctx, rows, n_rows, rows_on_device);
     if (rc) return rc;
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     const npc_row *d_rows;
@@ -949,10 +986,8 @@ static int split_prologue(npc_ctx *c, const void *gt_dev, int64_t row_stride, in
     int rc = check_block(c, gt_dev, row_stride, n_gt_rows, rows, n_rows);
     if (rc) return rc;
     if (!counts_dev) return fail(c, NPC_EINVAL, "counts_dev is NULL");
-    if (c->ds) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take hard-call (GT) rows only");
-    if (c->bed) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not PLINK .bed rows");
-    if (c->dose255 || c->dose32) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not BGEN dosage rows");
-    if (c->pl) return fail(c, NPC_EUNSUPPORTED, "the split count / accumulate calls take BCF GT rows, not FORMAT/PL rows");
+    if (c->layout != Layout::GT)
+        return fail(c, NPC_EUNSUPPORTED, (std::string("the split count / accumulate calls take BCF GT rows, not ") + info(c->layout).name).c_str());
     NPC_CUDA(c, cudaSetDevice(c->device));
     return upload_rows(c, rows, n_rows, rows_on_device, d_rows);
 }
@@ -996,7 +1031,7 @@ extern "C" int npc_resident_reserve(npc_ctx *ctx, int64_t capacity_rows, int64_t
 
 extern "C" int npc_resident_adopt(npc_ctx *ctx, const void *gt_dev, int64_t row_stride, int64_t n_gt_rows) {
     if (!ctx || n_gt_rows < 0 || (n_gt_rows && !gt_dev)) return NPC_EINVAL;
-    if (((uintptr_t)gt_dev & 15) || (row_stride & 15) || row_stride < npc_gt_row_bytes(ctx->n, ctx->ploidy, ctx->width))
+    if (((uintptr_t)gt_dev & 15) || (row_stride & 15) || row_stride < ctx_row_bytes(ctx, ctx->n))
         return fail(ctx, NPC_EINVAL, "npc_resident_adopt: slab must be 16-byte aligned, row_stride a multiple of 16 holding a whole row");
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     NPC_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1032,7 +1067,7 @@ extern "C" int npc_score_resident(npc_ctx *ctx, const npc_row *rows, int64_t n_r
     for (int64_t i = 0; i < n_rows; i++)
         if (rows[i].kind == NPC_KIND_GT && rows[i].gt_row >= ctx->slab_rows)
             return fail(ctx, NPC_EINVAL, "npc_score_resident: gt_row outside the resident slab");
-    if (int rc = check_bed_rows(ctx, rows, n_rows, 0)) return rc;
+    if (int rc = check_one_alt(ctx, rows, n_rows, 0)) return rc;
     // every upload issued so far must have landed
     for (int s = 0; s < ctx->n_slots; s++) NPC_CUDA(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_h2d[s], 0));
     for (int64_t r0 = 0; r0 < n_rows; r0 += ctx->max_rows) {
@@ -1230,8 +1265,9 @@ static int multi_contract(npc_ctx *c, int32_t S, const npc_row *const *rows, con
         c->launches++;
     }
     for (int k = 0; k < S; k++) if (n_rows[k]) {
-        k_decide<<<(unsigned)((n_rows[k] + 127) / 128), 128, 0, st>>>(d_all + row0[k], n_rows[k], d_counts + 2 * row0[k], c->pol, c->n,
-                                                                     d_rowp + row0[k], d_log + row0[k], d_nloci + k);
+        const TallyIn in = { nullptr, 0, d_counts + 2 * row0[k], nullptr, 0 };
+        k_decide<CountTally><<<(unsigned)((n_rows[k] + 127) / 128), 128, 0, st>>>(in, d_all + row0[k], n_rows[k], c->pol, c->n,
+                                                                                 d_rowp + row0[k], d_log + row0[k], d_nloci + k);
         c->launches++;
     }
     k_multi_scale<<<S, 256, 0, st>>>(d_rowp, d_row0, d_scale);

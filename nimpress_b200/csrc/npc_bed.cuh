@@ -7,8 +7,8 @@
 //               sample n-1 are padding (PLINK writes 00) and are never counted or stored.
 //   code        00 hom A1, 01 missing, 10 het, 11 hom A2; A2 = REF (eaidx 0), A1 = the one ALT (eaidx 1):
 //               dosage for eaidx 1 = 2 / NaN / 1 / 0, for eaidx 0 = 0 / NaN / 1 / 2.
-//   k_count_bed (nmiss, neff) per score row from masks and popc over 32-bit words (16 samples), as exact integers.
-//   k_decide    unchanged (npc_kernels.cuh).
+//   Bed::Count  (nmiss, neff) per score row from masks and popc over 32-bit words (16 samples), as exact integers,
+//               in k_count_chunks; k_decide as for GT rows (npc_kernels.cuh).
 //   k_accum_bed the 2-bit code indexes the row's value table {contribution of code 0, 1, 2, 3}: no decode.
 //               A CONST row's table holds its constant in every entry, a dropped row's holds +0.0.
 //     EXACT     acc = acc + T_r[c_r], row by row: the reference's chain (:639-640), bit for bit.
@@ -38,49 +38,27 @@ __device__ __forceinline__ double bed_value(const RowP &rp, int c) {
     return (c == 0) == (rp.eaidx == 1) ? rp.c2 : rp.c0;          // 00 = two A1 (ALT) alleles, 11 = two A2 (REF)
 }
 
-// tallyAlleles (:32-47) on 2-bit rows.  One 16-byte load = 64 samples; four in flight per thread.
-__global__ void __launch_bounds__(256)
-k_count_bed(const uint8_t *__restrict__ gt, int64_t row_stride, const npc_row *__restrict__ rows, int64_t n,
-            ull *__restrict__ counts) {
-    const int r = blockIdx.x;
-    const npc_row row = rows[r];
-    if (row.kind != NPC_KIND_GT || row.gt_row < 0) return;
-    __shared__ ull s_m, s_e;
-    if (threadIdx.x == 0) { s_m = 0; s_e = 0; }
-    __syncthreads();
-    const uint4 *base = reinterpret_cast<const uint4 *>(gt + (int64_t)row.gt_row * row_stride);
-    const int64_t nchunks = (n + 63) >> 6;
-    const bool alt = row.eaidx == 1;
-    uint32_t nm = 0, ne = 0;                      // per thread: < 2^32 for any cohort below 2^25 samples per thread
-    constexpr int U = 4;
-    for (int64_t c0 = (int64_t)blockIdx.y * blockDim.x * U + threadIdx.x; c0 < nchunks; c0 += (int64_t)gridDim.y * blockDim.x * U) {
-        uint4 wv[U];
-#pragma unroll
-        for (int u = 0; u < U; u++) {
-            const int64_t c = c0 + (int64_t)u * blockDim.x;
-            wv[u] = c < nchunks ? ldg_stream(base + c) : make_uint4(0, 0, 0, 0);
-        }
-#pragma unroll
-        for (int u = 0; u < U; u++) {
-            const int64_t c = c0 + (int64_t)u * blockDim.x;
-            if (c >= nchunks) break;
-            const uint32_t ww[4] = { wv[u].x, wv[u].y, wv[u].z, wv[u].w };
+// The layout type of k_count_chunks (npc_kernels.cuh): tallyAlleles (:32-47) on 2-bit rows.  One 16-byte chunk = 64
+// samples, 32-bit words of 16.  Per thread: < 2^32 for any cohort below 2^25 samples per thread.
+struct Bed {
+    static constexpr int PER16 = 64, HEADER = 0;  // samples per 16-byte chunk, bytes before the first
+    struct Count {
+        bool alt;
+        __device__ Count(const uint8_t *, const npc_row &row) : alt(row.eaidx == 1) {}
+        __device__ void operator()(const uint4 &w, int64_t left, uint32_t &nm, uint32_t &ne) const {
+            const uint32_t ww[4] = { w.x, w.y, w.z, w.w };
 #pragma unroll
             for (int k = 0; k < 4; k++) {
-                const int64_t left = n - (c * 64 + k * 16);               // samples of this word still in the row
-                const uint32_t m = left >= 16 ? 0x55555555u : left <= 0 ? 0u : 0x55555555u & ((1u << (2 * left)) - 1u);
+                const int64_t l = left - k * 16;                                  // samples of this word still in the row
+                const uint32_t m = l >= 16 ? 0x55555555u : l <= 0 ? 0u : 0x55555555u & ((1u << (2 * l)) - 1u);
                 const uint32_t lo = ww[k] & m, hi = (ww[k] >> 1) & m;
-                nm += __popc(lo & ~hi);                                   // 01
+                nm += __popc(lo & ~hi);                                           // 01
                 // effect alleles: ALT = A1 counts 2 for 00 and 1 for 10; REF = A2 counts 1 for 10 and 2 for 11
                 ne += alt ? __popc(m & ~lo & ~hi) + __popc(m & ~lo) : __popc(hi) + __popc(lo & hi);
             }
         }
-    }
-    const ull m64 = __reduce_add_sync(0xffffffffu, nm), e64 = __reduce_add_sync(0xffffffffu, ne);
-    if ((threadIdx.x & 31) == 0) { atomicAdd(&s_m, m64); atomicAdd(&s_e, e64); }
-    __syncthreads();
-    if (threadIdx.x == 0) { atomicAdd(&counts[2 * r], s_m); atomicAdd(&counts[2 * r + 1], s_e); }
-}
+    };
+};
 
 // Per batch of BED_RB rows, what the accumulate pass reads: the value tables (EXACT: [row][code], 4 per row; default:
 // [tile][half][pair index], 32 per tile) and the slab row of every row it loads (-1: constant or dropped row, or past

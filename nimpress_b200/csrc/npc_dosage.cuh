@@ -70,27 +70,15 @@ k_count_ds(const uint8_t *__restrict__ gt, int64_t row_stride, const npc_row *__
     }
 }
 
-// decide for dosage rows: block sums left to right -> neff, then the common decision
-__global__ void __launch_bounds__(128)
-k_decide_ds(const npc_row *__restrict__ rows, int64_t n_rows, const double *__restrict__ part, int64_t n_blocks,
-            const ull *__restrict__ miss, Policy p, int64_t n_local, RowP *__restrict__ rowp, npc_locus *__restrict__ log,
-            ull *__restrict__ nloci) {
-    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    int used = 0;
-    if (r < n_rows) {
-        const npc_row row = rows[r];
-        double neff = 0.0;
+// The tally of k_decide for dosage rows: block sums left to right -> neff; the record holds its IEEE-754 bits.
+struct DsTally : RowTally {
+    __device__ DsTally(const TallyIn &in, const npc_row &row, int64_t r) {
+        neff = 0.0;
         if (row.kind == NPC_KIND_GT && row.gt_row >= 0)
-            for (int64_t b = 0; b < n_blocks; b++) neff = __dadd_rn(neff, part[r * n_blocks + b]);
-        RowP out; npc_locus rec;
-        decide_row_real(p, row, miss[r], neff, __double_as_longlong(neff), n_local, out, rec);
-        rowp[r] = out;
-        log[r] = rec;
-        used = rec.used;
+            for (int64_t b = 0; b < in.n_blocks; b++) neff = __dadd_rn(neff, in.part[r * in.n_blocks + b]);
+        nmiss = in.counts[r]; neff_rec = __double_as_longlong(neff);
     }
-    used = __reduce_add_sync(0xffffffffu, used);
-    if ((threadIdx.x & 31) == 0 && used) atomicAdd(nloci, (ull)used);
-}
+};
 
 // scores[s] += contribution(row, s), rows in order: the reference's chain
 __global__ void __launch_bounds__(256)

@@ -29,34 +29,18 @@ constexpr int D255_THREADS = 128;                 // accumulate pass: threads pe
 constexpr int D255_RB = 8;                        // rows per batch
 constexpr uint32_t D255_MAX = 510;                // 255 x the largest dosage; anything above is a missing sample
 
-// tallyAlleles (:32-47) on dosage rows: one 16-byte load = 8 samples, four in flight per thread.
-__global__ void __launch_bounds__(256)
-k_count_dose255(const uint8_t *__restrict__ gt, int64_t row_stride, const npc_row *__restrict__ rows, int64_t n,
-                ull *__restrict__ counts) {
-    const int r = blockIdx.x;
-    const npc_row row = rows[r];
-    if (row.kind != NPC_KIND_GT || row.gt_row < 0) return;
-    __shared__ ull s_m, s_e;
-    if (threadIdx.x == 0) { s_m = 0; s_e = 0; }
-    __syncthreads();
-    const uint4 *base = reinterpret_cast<const uint4 *>(gt + (int64_t)row.gt_row * row_stride);
-    const int64_t nchunks = (n + 7) >> 3;
-    const uint32_t flip = row.eaidx == 0 ? D255_MAX : 0u;            // k' = |k - flip|
-    uint32_t nm = 0, ne = 0;         // per thread: tally_grid_y gives a thread at most 64 chunks, 512 samples x 510
-    constexpr int U = 4;
-    for (int64_t c0 = (int64_t)blockIdx.y * blockDim.x * U + threadIdx.x; c0 < nchunks; c0 += (int64_t)gridDim.y * blockDim.x * U) {
-        uint4 wv[U];
-#pragma unroll
-        for (int u = 0; u < U; u++) {
-            const int64_t c = c0 + (int64_t)u * blockDim.x;
-            wv[u] = c < nchunks ? ldg_stream(base + c) : make_uint4(0, 0, 0, 0);
-        }
-#pragma unroll
-        for (int u = 0; u < U; u++) {
-            const int64_t c = c0 + (int64_t)u * blockDim.x;
-            if (c >= nchunks) break;
-            const int valid = (int)min((int64_t)8, n - c * 8);
-            const uint32_t ww[4] = { wv[u].x, wv[u].y, wv[u].z, wv[u].w };
+// The layout type of k_count_chunks and k_decide (npc_kernels.cuh).
+struct Dose255 {
+    static constexpr int PER16 = 8, HEADER = 0;   // samples per 16-byte word, bytes before the first
+
+    // tallyAlleles (:32-47): k' = |k - flip| summed over the called samples of a chunk.  Per thread: tally_grid_y gives a
+    // thread at most 64 chunks, 512 samples x 510.
+    struct Count {
+        uint32_t flip;
+        __device__ Count(const uint8_t *, const npc_row &row) : flip(row.eaidx == 0 ? D255_MAX : 0u) {}
+        __device__ void operator()(const uint4 &w, int64_t left, uint32_t &nm, uint32_t &ne) const {
+            const int valid = (int)min((int64_t)8, left);
+            const uint32_t ww[4] = { w.x, w.y, w.z, w.w };
 #pragma unroll
             for (int k = 0; k < 8; k++) {
                 if (k >= valid) break;
@@ -65,30 +49,16 @@ k_count_dose255(const uint8_t *__restrict__ gt, int64_t row_stride, const npc_ro
                 else ne += (uint32_t)abs((int)v - (int)flip);
             }
         }
-    }
-    const ull m64 = __reduce_add_sync(0xffffffffu, nm), e64 = __reduce_add_sync(0xffffffffu, ne);
-    if ((threadIdx.x & 31) == 0) { atomicAdd(&s_m, m64); atomicAdd(&s_e, e64); }
-    __syncthreads();
-    if (threadIdx.x == 0) { atomicAdd(&counts[2 * r], s_m); atomicAdd(&counts[2 * r + 1], s_e); }
-}
+    };
 
-// The common decision on the integer tallies: neff = fl(neff_num / 255), the record reports neff_num.
-__global__ void __launch_bounds__(128)
-k_decide_dose255(const npc_row *__restrict__ rows, int64_t n_rows, const ull *__restrict__ counts, Policy p,
-                 int64_t n_local, RowP *__restrict__ rowp, npc_locus *__restrict__ log, ull *__restrict__ nloci) {
-    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    int used = 0;
-    if (r < n_rows) {
-        RowP out; npc_locus rec;
-        const ull num = counts[2 * r + 1];
-        decide_row_real(p, rows[r], counts[2 * r], __ddiv_rn((double)num, 255.0), (long long)num, n_local, out, rec);
-        rowp[r] = out;
-        log[r] = rec;
-        used = rec.used;
-    }
-    used = __reduce_add_sync(0xffffffffu, used);
-    if ((threadIdx.x & 31) == 0 && used) atomicAdd(nloci, (ull)used);
-}
+    // The common decision on the integer tallies: neff = fl(neff_num / 255), the record reports neff_num.
+    struct Tally : RowTally {
+        __device__ Tally(const TallyIn &in, const npc_row &, int64_t r) {
+            const ull num = in.counts[2 * r + 1];
+            nmiss = in.counts[2 * r]; neff = __ddiv_rn((double)num, 255.0); neff_rec = (long long)num;
+        }
+    };
+};
 
 // Staged per row: mode word (0 dropped, 1 constant, 2 decode with k' = k, 3 decode with k' = 510 - k), beta (c0 for a
 // constant row) and cm; the slab row of every row whose loads go out (-1: not read).

@@ -34,11 +34,10 @@ namespace npc {
 
 constexpr int D32_THREADS = 128;                  // accumulate pass: threads per CTA (4 samples each)
 constexpr int D32_RB = 8;                         // rows per batch
-constexpr int D32_HEADER = 16;                    // bytes before the first sample word
 
 // The row's D, from its header.
-__device__ __forceinline__ uint32_t d32_den(const uint8_t *__restrict__ gt, int64_t row_stride, int32_t gt_row) {
-    return __ldg(reinterpret_cast<const uint32_t *>(gt + (int64_t)gt_row * row_stride));
+__device__ __forceinline__ uint32_t d32_den(const uint8_t *__restrict__ row) {
+    return __ldg(reinterpret_cast<const uint32_t *>(row));
 }
 
 // One sample word -> k' (eaidx 0: p*D - k); false for a missing sample.
@@ -56,36 +55,19 @@ __device__ __forceinline__ double d32_quot(uint32_t kk, double D, double r) {
     return __fma_rn(e, r, q0);
 }
 
-// tallyAlleles (:32-47) on dosage rows: one 16-byte load = 4 samples, four in flight per thread.
-__global__ void __launch_bounds__(256)
-k_count_dose32(const uint8_t *__restrict__ gt, int64_t row_stride, const npc_row *__restrict__ rows, int64_t n,
-               ull *__restrict__ counts) {
-    const int r = blockIdx.x;
-    const npc_row row = rows[r];
-    if (row.kind != NPC_KIND_GT || row.gt_row < 0) return;
-    __shared__ ull s_m, s_e;
-    if (threadIdx.x == 0) { s_m = 0; s_e = 0; }
-    __syncthreads();
-    const uint32_t D = d32_den(gt, row_stride, row.gt_row);
-    const uint4 *base = reinterpret_cast<const uint4 *>(gt + (int64_t)row.gt_row * row_stride + D32_HEADER);
-    const int64_t nchunks = (n + 3) >> 2;
-    const bool ref = row.eaidx == 0;
-    // per thread: tally_grid_y gives a thread at most 64 chunks, 256 samples x 2 x 65,535 < 2^25
-    uint32_t nm = 0, ne = 0;
-    constexpr int U = 4;
-    for (int64_t c0 = (int64_t)blockIdx.y * blockDim.x * U + threadIdx.x; c0 < nchunks; c0 += (int64_t)gridDim.y * blockDim.x * U) {
-        uint4 wv[U];
-#pragma unroll
-        for (int u = 0; u < U; u++) {
-            const int64_t c = c0 + (int64_t)u * blockDim.x;
-            wv[u] = c < nchunks ? ldg_stream(base + c) : make_uint4(0, 0, 0, 0);
-        }
-#pragma unroll
-        for (int u = 0; u < U; u++) {
-            const int64_t c = c0 + (int64_t)u * blockDim.x;
-            if (c >= nchunks) break;
-            const int valid = (int)min((int64_t)4, n - c * 4);
-            const uint32_t ww[4] = { wv[u].x, wv[u].y, wv[u].z, wv[u].w };
+// The layout type of k_count_chunks and k_decide (npc_kernels.cuh).
+struct Dose32 {
+    static constexpr int PER16 = 4, HEADER = 16;  // samples per 16-byte word, bytes before the first sample word
+
+    // tallyAlleles (:32-47) with D and the flip from the row.  Per thread: tally_grid_y gives a thread at most 64 chunks,
+    // 256 samples x 2 x 65,535 < 2^25; a warp's sum of ne can pass 2^32, which k_count_chunks' 64-bit reduction holds.
+    struct Count {
+        uint32_t D;
+        bool ref;
+        __device__ Count(const uint8_t *row, const npc_row &r) : D(d32_den(row)), ref(r.eaidx == 0) {}
+        __device__ void operator()(const uint4 &w, int64_t left, uint32_t &nm, uint32_t &ne) const {
+            const int valid = (int)min((int64_t)4, left);
+            const uint32_t ww[4] = { w.x, w.y, w.z, w.w };
 #pragma unroll
             for (int k = 0; k < 4; k++) {
                 if (k >= valid) break;
@@ -94,40 +76,20 @@ k_count_dose32(const uint8_t *__restrict__ gt, int64_t row_stride, const npc_row
                 else nm++;
             }
         }
-    }
-    // a warp's sum of ne can pass 2^32: reduce in 64 bits
-    ull m64 = nm, e64 = ne;
-    for (int o = 16; o; o >>= 1) {
-        m64 += __shfl_xor_sync(0xffffffffu, m64, o);
-        e64 += __shfl_xor_sync(0xffffffffu, e64, o);
-    }
-    if ((threadIdx.x & 31) == 0) { atomicAdd(&s_m, m64); atomicAdd(&s_e, e64); }
-    __syncthreads();
-    if (threadIdx.x == 0) { atomicAdd(&counts[2 * r], s_m); atomicAdd(&counts[2 * r + 1], s_e); }
-}
+    };
 
-// The common decision on the integer tallies: neff = fl(neff_num / D), the record reports neff_num.  RowP::pad carries
-// the row's D to the accumulate pass.
-__global__ void __launch_bounds__(128)
-k_decide_dose32(const uint8_t *__restrict__ gt, int64_t row_stride, const npc_row *__restrict__ rows, int64_t n_rows,
-                const ull *__restrict__ counts, Policy p, int64_t n_local, RowP *__restrict__ rowp,
-                npc_locus *__restrict__ log, ull *__restrict__ nloci) {
-    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    int used = 0;
-    if (r < n_rows) {
-        const npc_row row = rows[r];
-        const uint32_t D = row.kind == NPC_KIND_GT && row.gt_row >= 0 ? d32_den(gt, row_stride, row.gt_row) : 1u;
-        RowP out; npc_locus rec;
-        const ull num = counts[2 * r + 1];
-        decide_row_real(p, row, counts[2 * r], __ddiv_rn((double)num, (double)D), (long long)num, n_local, out, rec);
-        out.pad = (int32_t)D;
-        rowp[r] = out;
-        log[r] = rec;
-        used = rec.used;
-    }
-    used = __reduce_add_sync(0xffffffffu, used);
-    if ((threadIdx.x & 31) == 0 && used) atomicAdd(nloci, (ull)used);
-}
+    // The common decision on the integer tallies: neff = fl(neff_num / D), the record reports neff_num.  RowP::pad carries
+    // the row's D to the accumulate pass.
+    struct Tally : RowTally {
+        uint32_t D;
+        __device__ Tally(const TallyIn &in, const npc_row &row, int64_t r) {
+            D = row.kind == NPC_KIND_GT && row.gt_row >= 0 ? d32_den(in.gt + (int64_t)row.gt_row * in.row_stride) : 1u;
+            const ull num = in.counts[2 * r + 1];
+            nmiss = in.counts[2 * r]; neff = __ddiv_rn((double)num, (double)D); neff_rec = (long long)num;
+        }
+        __device__ void extra(const npc_row &, RowP &out) const { out.pad = (int32_t)D; }
+    };
+};
 
 // Staged per row: mode word (0 dropped, 1 constant, 2 decode with k' = k, 3 decode with k' = p*D - k), beta (c0 for a
 // constant row), cm and D; the slab row of every row whose loads go out (-1: not read).
@@ -160,7 +122,7 @@ k_accum_dose32(const uint8_t *__restrict__ gt, int64_t row_stride, const RowP *_
     double acc[4];
 #pragma unroll
     for (int k = 0; k < 4; k++) acc[k] = k < valid ? sums[t * 4 + k] : 0.0;
-    const uint4 *col = reinterpret_cast<const uint4 *>(gt + D32_HEADER) + (active ? t : 0);
+    const uint4 *col = reinterpret_cast<const uint4 *>(gt + Dose32::HEADER) + (active ? t : 0);
     const int64_t stride16 = row_stride >> 4;
     if (threadIdx.x < D32_RB) {
         uint32_t D;

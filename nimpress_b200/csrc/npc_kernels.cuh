@@ -217,6 +217,49 @@ k_count_i8x2(const uint8_t *__restrict__ gt, int64_t row_stride, const npc_row *
     if (threadIdx.x == 0) { atomicAdd(&counts[2 * r], (ull)s_m); atomicAdd(&counts[2 * r + 1], (ull)s_e); }
 }
 
+// Rows read as 16-byte chunks of L::PER16 samples after L::HEADER bytes (.bed and fixed-point dosage rows): one CTA per row
+// and slab of the sample axis, four chunks in flight per thread.  L::Count, made once per row, adds one chunk to the
+// thread's (nmiss, neff) words; a warp sums them in 64 bits, then shared and global 64-bit atomics (order-free).
+template <class L>
+__global__ void __launch_bounds__(256)
+k_count_chunks(const uint8_t *__restrict__ gt, int64_t row_stride, const npc_row *__restrict__ rows, int64_t n,
+               ull *__restrict__ counts) {
+    const int r = blockIdx.x;
+    const npc_row row = rows[r];
+    if (row.kind != NPC_KIND_GT || row.gt_row < 0) return;
+    __shared__ ull s_m, s_e;
+    if (threadIdx.x == 0) { s_m = 0; s_e = 0; }
+    __syncthreads();
+    const uint8_t *p = gt + (int64_t)row.gt_row * row_stride;
+    const typename L::Count count(p, row);
+    const uint4 *base = reinterpret_cast<const uint4 *>(p + L::HEADER);
+    const int64_t nchunks = (n + L::PER16 - 1) / L::PER16;
+    uint32_t nm = 0, ne = 0;
+    constexpr int U = 4;
+    for (int64_t c0 = (int64_t)blockIdx.y * blockDim.x * U + threadIdx.x; c0 < nchunks; c0 += (int64_t)gridDim.y * blockDim.x * U) {
+        uint4 wv[U];
+#pragma unroll
+        for (int u = 0; u < U; u++) {
+            const int64_t c = c0 + (int64_t)u * blockDim.x;
+            wv[u] = c < nchunks ? ldg_stream(base + c) : make_uint4(0, 0, 0, 0);
+        }
+#pragma unroll
+        for (int u = 0; u < U; u++) {
+            const int64_t c = c0 + (int64_t)u * blockDim.x;
+            if (c >= nchunks) break;
+            count(wv[u], n - c * L::PER16, nm, ne);
+        }
+    }
+    ull m64 = nm, e64 = ne;
+    for (int o = 16; o; o >>= 1) {
+        m64 += __shfl_xor_sync(0xffffffffu, m64, o);
+        e64 += __shfl_xor_sync(0xffffffffu, e64, o);
+    }
+    if ((threadIdx.x & 31) == 0) { atomicAdd(&s_m, m64); atomicAdd(&s_e, e64); }
+    __syncthreads();
+    if (threadIdx.x == 0) { atomicAdd(&counts[2 * r], s_m); atomicAdd(&counts[2 * r + 1], s_e); }
+}
+
 // ------------------------------------------------------------------------------------------
 // decide: one thread per score row.  Everything the reference decides in fp64 is decided here
 // with the same IEEE operations on the same integers.
@@ -287,14 +330,44 @@ __device__ __forceinline__ void decide_row(const Policy &p, const npc_row &row, 
     decide_row_real(p, row, nmiss_u, (double)neff_u, (long long)neff_u, n_local, out, rec);
 }
 
+// What the tally pass left for k_decide: integer layouts two words a row in counts, real-valued ones (FORMAT/DS, FORMAT/PL)
+// the missing count in counts and n_blocks block sums a row in part; gt, row_stride: the slab, for rows with a header.
+struct TallyIn {
+    const uint8_t *gt;
+    int64_t row_stride;
+    const ull *counts;
+    const double *part;
+    int64_t n_blocks;
+};
+
+// A row's tally as decide_row_real takes it.  Each layout's tally type derives from it, fills it from (TallyIn, row, r) in
+// its constructor and may hide extra(), which sets a RowP field the layout's accumulate pass needs beyond the decision.
+struct RowTally {
+    ull nmiss;
+    double neff;
+    long long neff_rec;
+    __device__ void extra(const npc_row &, RowP &) const {}
+};
+
+// GT and .bed rows: counts[2r] = nmiss, counts[2r+1] = neff.
+struct CountTally : RowTally {
+    __device__ CountTally(const TallyIn &in, const npc_row &, int64_t r) {
+        nmiss = in.counts[2 * r]; neff = (double)in.counts[2 * r + 1]; neff_rec = (long long)in.counts[2 * r + 1];
+    }
+};
+
+template <class T>
 __global__ void __launch_bounds__(128)
-k_decide(const npc_row *__restrict__ rows, int64_t n_rows, const ull *__restrict__ counts, Policy p,
-         int64_t n_local, RowP *__restrict__ rowp, npc_locus *__restrict__ log, ull *__restrict__ nloci) {
+k_decide(TallyIn in, const npc_row *__restrict__ rows, int64_t n_rows, Policy p, int64_t n_local, RowP *__restrict__ rowp,
+         npc_locus *__restrict__ log, ull *__restrict__ nloci) {
     const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     int used = 0;
     if (r < n_rows) {
+        const npc_row row = rows[r];
+        const T t(in, row, r);
         RowP out; npc_locus rec;
-        decide_row(p, rows[r], counts[2 * r], counts[2 * r + 1], n_local, out, rec);
+        decide_row_real(p, row, t.nmiss, t.neff, t.neff_rec, n_local, out, rec);
+        t.extra(row, out);
         rowp[r] = out;
         log[r] = rec;
         used = rec.used;

@@ -22,7 +22,7 @@
 //                allele ALT), fl(2 u_0 + u_1) (diploid, REF), u_1 (haploid, ALT), u_0 (haploid, REF).  Called iff
 //                den > 0; d = fl(num / den)
 //   tally        as FORMAT/DS rows (npc_dosage.cuh): nmiss an integer, neff = the fp64 sum of the called d in chunks of
-//                8 samples, a 32-way butterfly, blocks of 256 left to right; k_decide_pl = k_decide_ds + the row's eaf
+//                8 samples, a 32-way butterfly, blocks of 256 left to right; PlTally = DsTally + the row's eaf
 //   accumulate   scores[s] = fl(scores[s] + fl(d beta)) (cm for a missing sample, c0 for a constant row), rows in
 //                score-row order: the reference's chain in every mode.
 //
@@ -120,28 +120,14 @@ k_count_pl(const uint8_t *__restrict__ gt, int64_t row_stride, const npc_row *__
     }
 }
 
-// k_decide_ds, and a decoded row carries its eaf in RowP::c0 (unused by this format) to the accumulate pass
-__global__ void __launch_bounds__(128)
-k_decide_pl(const npc_row *__restrict__ rows, int64_t n_rows, const double *__restrict__ part, int64_t n_blocks,
-            const ull *__restrict__ miss, Policy p, int64_t n_local, RowP *__restrict__ rowp, npc_locus *__restrict__ log,
-            ull *__restrict__ nloci) {
-    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    int used = 0;
-    if (r < n_rows) {
-        const npc_row row = rows[r];
-        double neff = 0.0;
-        if (row.kind == NPC_KIND_GT && row.gt_row >= 0)
-            for (int64_t b = 0; b < n_blocks; b++) neff = __dadd_rn(neff, part[r * n_blocks + b]);
-        RowP out; npc_locus rec;
-        decide_row_real(p, row, miss[r], neff, __double_as_longlong(neff), n_local, out, rec);
+// The tally of k_decide for FORMAT/DS rows, and a decoded row carries its eaf in RowP::c0 (unused by this format) to the
+// accumulate pass.
+struct PlTally : DsTally {
+    __device__ PlTally(const TallyIn &in, const npc_row &row, int64_t r) : DsTally(in, row, r) {}
+    __device__ void extra(const npc_row &row, RowP &out) const {
         if (out.mode == MODE_DECODE) out.c0 = row.eaf;
-        rowp[r] = out;
-        log[r] = rec;
-        used = rec.used;
     }
-    used = __reduce_add_sync(0xffffffffu, used);
-    if ((threadIdx.x & 31) == 0 && used) atomicAdd(nloci, (ull)used);
-}
+};
 
 // Staged per row: mode (0 dropped, 1 constant, 2 decode with effect allele ALT, 3 decode with REF), beta (the constant
 // of a constant row; cm for a decoded row whose eaf makes every sample missing), cm and the priors.
