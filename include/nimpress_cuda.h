@@ -296,11 +296,14 @@ int npc_score_resident(npc_ctx *ctx, const npc_row *rows, int64_t n_rows);
  * formed as one dense contraction on the tensor cores (npc_multi.cuh): the genotypes are read
  * once for the tallies and once per 18 definitions (16 when some imputed contribution is NaN)
  * instead of once per definition.  Per-locus
- * records and nloci are bit-equal to the one-by-one path; scores agree with it within 1e-9
- * relative (exact integer arithmetic on coefficients rounded to 2^-53 of the definition's
- * largest; measured ~1e-15).  Inputs it does not represent (effect-allele index > 62, a
- * definition naming one slab row with one allele more than four times, infinite coefficients)
- * take the one-by-one path.  npc_multi_contractions counts the calls the contraction served. */
+ * records and nloci are bit-equal to the one-by-one path.  Scores come from exact integer
+ * arithmetic on coefficients rounded to a fixed-point grid: per sample they are within
+ * 2^-52 * (the definition's largest |coefficient|) per unit of plane value (dosage 0/1/2, 1 for
+ * a missing call) per row, plus fp64 rounding, of the exact sum -- an absolute bound, not a
+ * relative one (DESIGN 4.5).  Inputs it does not represent (effect-allele index > 62, a
+ * definition naming one slab row with one allele more than four times, a coefficient that is
+ * infinite or above 1.79e308, more than 2^22 distinct (row, allele) entries) take the one-by-one
+ * path.  npc_multi_contractions counts the calls the contraction served. */
 int npc_score_resident_multi(npc_ctx *ctx, int32_t n_scores, const npc_row *const *rows, const int64_t *n_rows,
                              const double *offsets, double *const *scores_out, int64_t *nloci_out,
                              npc_locus *const *loci_out);

@@ -15,11 +15,15 @@
 // integer and split into seven balanced base-256 digits; tcgen05.mma.kind::i8 multiplies the digit
 // rows (operand A, int8) with the d / m planes (operand B, int8 values 0,1,2) into int32
 // accumulators in tensor memory; the epilogue recombines the seven digit sums as two int64 and
-// converts once.  The only approximation is the fixed-point rounding of the coefficients: at most
-// 2^-53 of the largest |coefficient| of that score per term (the reference's own fp64 chain rounds
-// every add at 2^-53 of the running sum).  Stated tolerance: scores within 1e-9 relative of the
-// reference (tests measure ~1e-15).  Per-locus records and nloci come from the same k_decide as
-// every other path: bit-equal.
+// converts once.  The only approximation is the fixed-point rounding of the coefficients: with
+// F = 52 - ex (max|c| = m * 2^ex, 0.5 <= m < 1) a coefficient is off by at most half a quantum,
+// 2^(ex-53) <= 2^-52 * max|c| of its score, reached when max|c| is a power of two.  Stated tolerance,
+// absolute: per sample, 2^-52 * max|c| times the sum of the plane values (dosage 0/1/2, 1 for a
+// missing call) over the score's rows, plus fp64 rounding of the constant sum, the conversion, the
+// k-split adds and the normalisation.  The errors add up over rows, so no relative bound holds: a
+// score whose coefficients span many binades loses its smallest ones (tests/test_multi_exact_gpu.py
+// checks this bound against the exact sum).  Per-locus records and nloci come from the same k_decide
+// as every other path: bit-equal.
 //
 // When some imputed contribution is NaN (--imp-sample=fail / int_fail, eaf = NaN) an eighth row per
 // score counts, per sample, the missing calls at those entries: count > 0 -> score NaN, as the
@@ -407,7 +411,8 @@ __global__ void __launch_bounds__(256) k_multi_scale(const RowP *__restrict__ ro
         const RowP rp = rowp[r];
         if (rp.mode == MODE_CONST) cs = __dadd_rn(cs, rp.c0);
         else if (rp.mode == MODE_DECODE) {
-            if (!(fabs(rp.c1) <= 1.79e308) || rp.c0 != 0.0) cs = __dadd_rn(cs, __longlong_as_double(0x7FF8000000000000ll));   // beta NaN / inf: every sample NaN
+            if (rp.c1 != rp.c1) cs = __dadd_rn(cs, __longlong_as_double(0x7FF8000000000000ll));   // beta NaN: every sample NaN, as in the reference
+            else if (!(fabs(rp.c1) <= 1.79e308)) flags |= 1;             // beta +-inf or near DBL_MAX: +-inf, NaN only at dosage 0 -> one by one
             else {
                 mx = fmax(mx, fabs(rp.c1));
                 if (rp.cm == rp.cm) { if (fabs(rp.cm) > 1.79e308) flags |= 1; else mx = fmax(mx, fabs(rp.cm)); }
@@ -438,7 +443,7 @@ __global__ void k_multi_coef(const RowP *__restrict__ rowp, const int32_t *__res
     const RowP rp = rowp[r];
     const int32_t e = ent[r];
     if (rp.mode != MODE_DECODE || e < 0) return;
-    if (!(fabs(rp.c1) <= 1.79e308) || rp.c0 != 0.0) return;             // counted as a NaN constant by k_multi_scale
+    if (rp.c1 != rp.c1) return;                                        // beta NaN: counted as a NaN constant by k_multi_scale
     const int k = score_of[r] - k0;                                    // score within this launch
     const int F = fexp[k];
     atomicAdd((ull *)&coef[((int64_t)k * 2 + 0) * E + e], (ull)__double2ll_rn(scalbn(rp.c1, F)));
