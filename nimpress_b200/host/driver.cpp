@@ -12,6 +12,7 @@
 #include <mutex>
 #include <thread>
 #include <unordered_map>
+#include <unordered_set>
 
 #include "region_index.hpp"
 #include "stats.hpp"
@@ -63,7 +64,7 @@ Matcher::Matcher(const ScoreFile &score, const GenomeIntervals &cov, const Score
         ci.by_pos.emplace_back(E_[i].pos, i);
         ci.max_reflen = std::max<int64_t>(ci.max_reflen, (int64_t)E_[i].refseq.size());
     }
-    for (auto &kv : index_) { std::sort(kv.second.by_pos.begin(), kv.second.by_pos.end()); n_lookup_ += (int64_t)kv.second.by_pos.size(); }
+    for (auto &kv : index_) std::sort(kv.second.by_pos.begin(), kv.second.by_pos.end());
 }
 
 const std::vector<int64_t> &Matcher::match(const VariantRecord &rec) {
@@ -273,8 +274,30 @@ struct LayoutOverflow { int width, ploidy; };      // a matched record does not 
 struct SlabOverflow {};                            // several score files, and their matched rows exceed device memory
 struct CannotOpen { std::string path; };           // a genotype file that opened before could not be reopened to be streamed
 
+// The row format of one pass: what the staging rows and the contexts hold
+struct RowLayout {
+    int width = 1, ploidy = 2;                     // BCF's usual GT layout: int8, diploid
+    bool ds = false, pl = false;                   // FORMAT/DS rows (one float per sample), FORMAT/PL rows (one packed word per sample)
+    // dosage rows (FORMAT/DS, FORMAT/PL, BGEN): the effect-allele tally is not an integer allele count
+    bool real_tally() const { return ds || pl || width == NPC_GT_DOSE255 || width == NPC_GT_DOSE32; }
+};
+
+// The layout a pass over genotype files of this kind (GenotypeFiles::kind) starts with; dose32: a BGEN pass met a block
+// that only 32-bit dosage rows hold.  InputError when the files cannot give the rows p asks for.
+RowLayout row_layout(int kind, const ScoreParams &p, bool dose32) {
+    if (p.use_ds && p.use_pl) throw InputError("--pl and --dosage: score either FORMAT/PL or FORMAT/DS");
+    if (kind == NPC_GT_BED && p.use_ds) throw InputError("--dosage: a PLINK fileset holds hard calls only, no FORMAT/DS");
+    if (kind == NPC_GT_BED && p.use_pl) throw InputError("--pl: a PLINK fileset holds hard calls only, no FORMAT/PL");
+    if (kind == NPC_GT_DOSE255 && p.use_pl) throw InputError("--pl: a BGEN file holds genotype probabilities, no FORMAT/PL");
+    RowLayout L;
+    if (kind != VariantSource::NO_FIXED_LAYOUT) L.width = dose32 ? NPC_GT_DOSE32 : kind;   // BGEN rows are dosages already: --dosage changes nothing
+    else if (p.use_ds) { L.width = 4; L.ploidy = 1; L.ds = true; }
+    else if (p.use_pl) { L.width = NPC_GT_PL; L.pl = true; }
+    return L;
+}
+
 // WARN lines of one score file, in the reference's order (:326, :527-530, :538-541, :554-557, :567-570, :575-579)
-// real_tally: dosage rows (FORMAT/DS, BGEN), whose effect-allele tally is not an integer allele count
+// real_tally: RowLayout::real_tally() of the pass
 std::string make_warnings(const ScoreFile &score, const Matcher &M, const std::vector<npc_locus> &loci, int64_t n, const ScoreParams &p,
                           bool real_tally) {
     std::string w;
@@ -307,7 +330,291 @@ std::string make_warnings(const ScoreFile &score, const Matcher &M, const std::v
     return w;
 }
 
-// One pass over the genotype file with a fixed GT layout, for one score file or several at once
+// One score file's side of a pass
+struct ScoreState {
+    const ScoreFile &score;
+    Matcher M;
+    int D;                                         // devices of the pass
+    std::vector<int64_t> slab_row;                 // per entry: row of its device's resident slab
+    std::vector<uint8_t> done;                     // per entry: taken by a round
+    ScoreState(const ScoreFile &s, const GenomeIntervals &cov, const ScoreParams &p, int D)
+        : score(s), M(s, cov, p), D(D), slab_row(s.entries.size(), -1), done(s.entries.size(), 0) {}
+    // entry i belongs to device i * D / (entries): contiguous ranges of EVERY file in its own order
+    int dev_of(int64_t i) const {
+        return D == 1 ? 0 : (int)std::min<int64_t>(D - 1, i * D / std::max<int64_t>((int64_t)score.entries.size(), 1));
+    }
+};
+
+// Rows of each device's ranges that need a record (an upper bound when score files share records).  One device and
+// several score files: entries with the same (contig, pos, ref, ea) settle on the same record, so a key counts once.
+std::vector<int64_t> lookup_counts(const std::vector<ScoreState> &ps, int D) {
+    const bool dedup = D == 1 && ps.size() > 1;
+    std::vector<int64_t> c(D, 0);
+    std::unordered_set<std::string> keys;
+    for (const ScoreState &s : ps)
+        for (int64_t i = 0; i < (int64_t)s.score.entries.size(); i++) if (s.M.kind[i] == Matcher::PENDING) {
+            const ScoreEntry &e = s.score.entries[i];
+            c[s.dev_of(i)]++;
+            if (dedup) keys.insert(e.contig + "\t" + std::to_string(e.pos) + "\t" + e.refseq + "\t" + e.easeq);
+        }
+    if (dedup) c[0] = (int64_t)keys.size();
+    return c;
+}
+
+// The rows of score file s that a round takes on device d, in score-file order: a final round takes every row not taken
+// yet, an earlier one the rows whose genotypes sit in the slab.  Their entry indices are appended to submitted.
+void collect_rows(ScoreState &s, int d, bool final_round, std::vector<npc_row> &rows, std::vector<int64_t> &submitted) {
+    const std::vector<ScoreEntry> &E = s.score.entries;
+    rows.clear();
+    for (int64_t i = 0; i < (int64_t)E.size(); i++) {
+        if (s.done[i] || s.dev_of(i) != d) continue;
+        const int32_t kind = s.M.kind[i];
+        if (!final_round && !(kind == NPC_KIND_GT && s.slab_row[i] >= 0)) continue;
+        npc_row r;
+        r.gt_row = kind == NPC_KIND_GT ? (int32_t)s.slab_row[i] : -1;
+        r.eaidx = s.M.eaidx[i]; r.beta = E[i].beta; r.eaf = E[i].eaf;
+        r.ref_is_ea = E[i].ref_is_ea() ? 1 : 0; r.kind = kind;
+        rows.push_back(r);
+        submitted.push_back(i);
+        s.done[i] = 1;
+    }
+}
+
+// What the contexts of a pass are created with, and the file being read
+struct Pass {
+    const ScoreParams &p;
+    const RowLayout &lay;
+    int64_t n, n_row, row_bytes;                   // scored samples, samples of the widest file, bytes of a staging row
+    VariantSource *src;                            // the file being read (after the stream: the last one)
+    // its keep list, nullptr when every file scores all of its samples: a context opened lazily takes it; one opened after
+    // the stream receives no rows, so any file's list serves it
+    const int64_t *keep;
+    double waited_ms = 0.0;                        // spent opening contexts
+};
+
+// Devices: one context per GPU.  With several, the score rows are partitioned into contiguous ranges in
+// score-file order (a contig / region partition for a sorted score file): context d scores range d over all
+// samples, a matched record is uploaded to the device(s) whose ranges name it, and the partial sums are
+// combined in range order by npc_reduce.  Several score files at once: every file is cut into D ranges of its own,
+// device d scores range d of every file in one npc_score_resident_multi call (raw partial sums), and the host adds
+// the partials of each file in device order and normalises once.
+struct Device {
+    Pass *pass = nullptr;
+    int d = 0, id = 0;                             // index in the pass, CUDA device
+    int64_t lookup = 0;                            // rows of its ranges that need a record
+    Ctx ctx;
+    bool opened = false;
+    int32_t slot = -1; uint8_t *stage = nullptr; int64_t stride = 0, staged = 0, slab_base = 0, slab_cap = 0, block_rows = 1, rounds = 0;
+    int64_t taken = -1;                            // slab row of the last row take_row() handed out
+    std::vector<npc_row> rows; std::vector<int64_t> submitted;   // one score file: this device's rows, entry index of each
+
+    // A context is opened when its first row arrives (or at the end, for its constant rows): contexts come up one after
+    // the other inside the driver (~1 s each), and a sorted file reaches the later ranges later -- the first device's
+    // rows stream while the others' contexts are still being created.
+    void open() {
+        if (opened) return;
+        const auto t0 = std::chrono::steady_clock::now();
+        wait_warm(id);
+        const Pass &P = *pass;
+        // staging slots of ~8 MB: big enough for efficient H2D copies, small enough that pinning three of them per
+        // device does not dominate a short run (pinning costs ~1 ms per MB); scoring launches are sized separately
+        const int64_t want = std::max<int64_t>(lookup, 1);
+        block_rows = std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(4096, (8ll << 20) / P.row_bytes + 1), want));
+        const int64_t launch_rows = std::max<int64_t>(block_rows, 32768);
+        if (!P.keep) ctx.ck(npc_create2(&ctx.h, id, P.n, P.lay.ploidy, P.lay.width, launch_rows, 3, block_rows), "npc_create");
+        else ctx.ck(npc_create_subset(&ctx.h, id, P.n_row, P.keep, P.n, P.lay.ploidy, P.lay.width, launch_rows, 3, block_rows),
+                    "npc_create_subset");
+        const npc_policy pol = { P.p.imp_locus, P.p.imp_missing, P.p.imp_sample, 0, P.p.mincs, P.p.maxmis };
+        ctx.ck(npc_set_policy(ctx.h, &pol), "npc_set_policy");
+        if (P.lay.ds) ctx.ck(npc_set_dosage_rows(ctx.h, 1), "npc_set_dosage_rows");
+        if (P.p.exact_order) ctx.ck(npc_set_exact_order(ctx.h, 1), "npc_set_exact_order");
+        ctx.ck(npc_reset(ctx.h), "npc_reset");
+        int64_t slab_want = want;
+        if (const char *e = getenv("NIMPRESS_SLAB_ROWS")) if (*e) slab_want = std::max<int64_t>(1, std::min<int64_t>(slab_want, atoll(e)));   // tests: force rounds
+        ctx.ck(npc_resident_reserve(ctx.h, slab_want, &slab_cap), "npc_resident_reserve");
+        pass->waited_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
+        opened = true;
+    }
+    // The next staging row (its slab row in `taken`).  A full slab is scored (one score file, ps[0]; several throw
+    // SlabOverflow) and refilled from row 0; a slot is acquired when none is held.
+    uint8_t *take_row(std::vector<ScoreState> &ps) {
+        open();
+        if (slab_base + staged >= slab_cap) {
+            if (ps.size() > 1) throw SlabOverflow();
+            score_round(ps[0], false);
+            slab_base = 0;
+        }
+        if (slot < 0) {
+            void *ptr;
+            ctx.ck(npc_stage_acquire(ctx.h, &slot, &ptr, &stride), "npc_stage_acquire");
+            stage = (uint8_t *)ptr; staged = 0;
+        }
+        taken = slab_base + staged;
+        return stage + staged++ * stride;
+    }
+    void flush() {                                 // uploads the held slot once the reader's workers have filled its rows
+        if (slot < 0) return;
+        pass->src->wait_rows();
+        ctx.ck(npc_stage_upload(ctx.h, slot, staged, slab_base), "npc_stage_upload");
+        slab_base += staged; staged = 0; slot = -1;
+    }
+    // A round scores rows over the resident slab in score-file order.  The normal case is ONE final round per device
+    // holding every row of its range: exactly the reference's loop order (:634-641).  Only when the matched genotype rows
+    // exceed device memory are there earlier rounds; those take the rows whose genotypes sit in the slab, and the
+    // summation order then differs from the reference's by a reordering of terms (scores agree to ~1 ulp of the partial
+    // sums, not bit for bit).  One score file only.
+    void score_round(ScoreState &s, bool final_round) {
+        flush();
+        collect_rows(s, d, final_round, rows, submitted);
+        if (!rows.empty()) ctx.ck(npc_score_resident(ctx.h, rows.data(), (int64_t)rows.size()), "npc_score_resident");
+        rounds++;
+    }
+};
+
+std::string record_at(const VariantRecord &rec) { return "record " + *rec.contig + ":" + std::to_string(rec.pos); }
+
+// Fills one staging row from the record src just returned (row_bytes: a row of the file's own samples).  InputError for
+// a record these rows cannot take, LayoutOverflow when it needs a wider GT layout.
+void load_row(VariantRecord &rec, VariantSource &src, const RowLayout &lay, size_t row_bytes, uint8_t *dst) {
+    if (lay.pl && rec.alts.size() != 1)
+        throw InputError(record_at(rec) + ": FORMAT/PL rows take biallelic records only (" + std::to_string(rec.alts.size()) +
+                         " ALT alleles; split them with bcftools norm -m-)");
+    // BCF with the context's layout: the GT payload goes from the inflated blocks straight into the pinned row
+    const bool direct = src.load_gt_into(rec, dst, lay.width, lay.ploidy);
+    if (!rec.has_gt || !rec.gt)
+        throw InputError(record_at(rec) + (lay.pl ? " has no PL field" : lay.ds ? " has no DS field" : " has no GT field"));
+    if (lay.ds && (rec.ploidy != 1 || rec.gt_width != 4))
+        throw InputError(record_at(rec) + ": FORMAT/DS with several values per sample is not supported");
+    if (direct) return;
+    if (rec.ploidy > lay.ploidy || rec.gt_width > lay.width)
+        throw LayoutOverflow{ std::max(rec.gt_width, lay.width), std::max(rec.ploidy, lay.ploidy) };
+    if (rec.gt_width == lay.width && rec.ploidy == lay.ploidy) memcpy(dst, rec.gt, row_bytes);
+    else convert_gt(rec, src.n_samples(), lay.width, lay.ploidy, dst);
+}
+
+// One streaming pass over the genotype files, one after the other (findVariant :353-364, eaidx :375-379): a record whose
+// genotypes a score file needs is staged once on every device whose ranges name it.  Sets the record counters of outs.
+void stream_files(GenotypeFiles &files, const Spans &spans, Pass &P, std::vector<ScoreState> &ps, std::vector<Device> &devs,
+                  std::vector<ScoreResult> &outs) {
+    VariantRecord rec;
+    int64_t records_read = 0, records_matched = 0, seeks = 0;
+    for (size_t cur = 0; cur < files.src.size(); cur++) {
+        if (cur > 0) {
+            if (!files.prepare(cur, spans)) throw CannotOpen{ files.paths[cur] };
+            P.src = files.src[cur].get();
+            if (P.keep) {                             // staged rows of the previous file are compacted with its list
+                P.keep = files.keep[cur].data();
+                for (Device &v : devs) if (v.opened) {
+                    v.flush();
+                    v.ctx.ck(npc_set_keep(v.ctx.h, P.keep, P.n), "npc_set_keep");
+                }
+            }
+        }
+        VariantSource &src = *P.src;
+        const size_t file_row_bytes = (size_t)npc_gt_row_bytes(src.n_samples(), P.lay.ploidy, P.lay.width);   // the front of a staging row
+        while (src.next(rec)) {
+            records_read++;
+            bool any = false;
+            uint32_t need_dev = 0;                    // devices that take the record's genotypes
+            for (ScoreState &s : ps)
+                for (int64_t i : s.M.match(rec)) {
+                    any = true;
+                    if (s.M.kind[i] == NPC_KIND_GT) need_dev |= 1u << s.dev_of(i);
+                }
+            if (!any) continue;
+            records_matched++;
+            if (!need_dev) continue;                  // FILTER-failed: never decoded (:553-558)
+            const uint8_t *first = nullptr;
+            for (size_t d = 0; d < devs.size(); d++) {
+                if (!((need_dev >> d) & 1u)) continue;
+                uint8_t *dst = devs[d].take_row(ps);
+                if (first) {                          // a record named by two ranges: same bytes
+                    src.wait_rows();
+                    memcpy(dst, first, file_row_bytes);
+                } else {
+                    load_row(rec, src, P.lay, file_row_bytes, dst);
+                    first = dst;
+                }
+            }
+            for (ScoreState &s : ps)
+                for (int64_t i : s.M.match_last()) if (s.M.kind[i] == NPC_KIND_GT) {
+                    if (P.lay.ds && s.M.eaidx[i] > 1)
+                        throw InputError(record_at(rec) + ": FORMAT/DS rows take the REF or the first ALT as effect allele");
+                    s.slab_row[i] = devs[s.dev_of(i)].taken;
+                }
+            for (Device &v : devs) if (v.slot >= 0 && v.staged == v.block_rows) v.flush();
+        }
+        src.wait_rows();                              // BGEN workers may still be writing this file's rows into pinned slots
+        seeks += src.seeks();
+        if (cur + 1 < files.src.size()) { files.src[cur].reset(); P.src = nullptr; }
+    }
+    for (size_t k = 0; k < ps.size(); k++) {
+        ps[k].M.finish();
+        outs[k].records_read = records_read; outs[k].records_matched = records_matched; outs[k].index_seeks = seeks;
+    }
+}
+
+// One score file: every device scores the rest of its range in a final round.  One device's npc_finish gives the scores;
+// with several, npc_reduce combines their partial sums in range order and npc_partial gives each one's locus records.
+void score_single(ScoreState &s, std::vector<Device> &devs, int64_t n, ScoreResult &out) {
+    const int D = (int)devs.size();
+    std::vector<npc_ctx *> hs;
+    for (Device &v : devs) {
+        v.score_round(s, true);
+        out.rounds = std::max(out.rounds, v.rounds);
+        hs.push_back(v.ctx.h);
+    }
+    out.scores.assign(n, 0.0);
+    out.devices = D;
+    if (D > 1) devs[0].ctx.ck(npc_reduce(hs.data(), D, &s.score.offset, out.scores.data(), &out.nloci), "npc_reduce");
+    std::vector<double> scratch(D > 1 ? (size_t)std::max<int64_t>(n, 1) : 0);
+    for (Device &v : devs) {
+        std::vector<npc_locus> log(v.submitted.size());
+        int64_t nlog = 0, nl = 0;
+        if (D == 1)
+            v.ctx.ck(npc_finish(v.ctx.h, s.score.offset, out.scores.data(), &out.nloci, log.data(), (int64_t)log.size(), &nlog), "npc_finish");
+        else v.ctx.ck(npc_partial(v.ctx.h, scratch.data(), &nl, log.data(), (int64_t)log.size(), &nlog), "npc_partial");
+        if (nlog != (int64_t)v.submitted.size()) throw std::runtime_error("locus log length mismatch");
+        for (size_t j = 0; j < log.size(); j++) out.loci[v.submitted[j]] = log[j];
+    }
+}
+
+// Several score files: device d scores range d of every file in one npc_score_resident_multi call.  One device gives the
+// normalised scores straight away; several give raw partial sums, device 0's into the scores and the others' added to
+// them in device order (= score-file order of the ranges), normalised once.
+void score_multi(std::vector<ScoreState> &ps, std::vector<Device> &devs, int64_t n, std::vector<ScoreResult> &outs) {
+    const int S = (int)ps.size(), D = (int)devs.size();
+    std::vector<std::vector<double>> part(S);
+    for (int k = 0; k < S; k++) { outs[k].scores.assign(n, 0.0); outs[k].rounds = 1; outs[k].devices = D; if (D > 1) part[k].assign((size_t)n, 0.0); }
+    for (Device &v : devs) {
+        v.flush();
+        std::vector<std::vector<npc_row>> rows(S);
+        std::vector<std::vector<int64_t>> entries(S);
+        std::vector<std::vector<npc_locus>> log(S);
+        std::vector<const npc_row *> row_ptr(S);
+        std::vector<int64_t> n_rows(S), nloci(S);
+        std::vector<double> offsets(S);
+        std::vector<double *> sc(S);
+        std::vector<npc_locus *> log_ptr(S);
+        for (int k = 0; k < S; k++) {
+            collect_rows(ps[k], v.d, true, rows[k], entries[k]);
+            row_ptr[k] = rows[k].data(); n_rows[k] = (int64_t)rows[k].size(); offsets[k] = ps[k].score.offset;
+            sc[k] = v.d == 0 ? outs[k].scores.data() : part[k].data();
+            log[k].resize(rows[k].size()); log_ptr[k] = log[k].data();
+        }
+        // one device: normalised scores; several: raw partial sums (offsets = NULL)
+        v.ctx.ck(npc_score_resident_multi(v.ctx.h, S, row_ptr.data(), n_rows.data(), D == 1 ? offsets.data() : nullptr, sc.data(),
+                                          nloci.data(), log_ptr.data()), "npc_score_resident_multi");
+        for (int k = 0; k < S; k++) {
+            outs[k].nloci += nloci[k];
+            for (size_t j = 0; j < log[k].size(); j++) outs[k].loci[entries[k][j]] = log[k][j];
+            if (v.d > 0) for (int64_t i = 0; i < n; i++) outs[k].scores[i] += part[k][i];
+        }
+    }
+    if (D > 1) for (int k = 0; k < S; k++) npc_normalise(outs[k].scores.data(), n, outs[k].nloci, ps[k].score.offset);
+}
+
+// One pass over the genotype files with a fixed row layout, for one score file or several at once
 // (BASELINE config 4: every score file sees the same record stream, a record any of them matches
 // is uploaded once, and the resident slab is then scored for each file).  Throws LayoutOverflow
 // when a matched record needs a wider layout (the caller restarts the pass with it) and
@@ -317,330 +624,55 @@ std::string make_warnings(const ScoreFile &score, const Matcher &M, const std::v
 // widest file (n_row); the devices compact them to the n kept ones (npc_create_subset, npc_set_keep at each file), which
 // is all that the contexts, scores and WARN lines see.
 void run_pass(const std::vector<const ScoreFile *> &scores, GenotypeFiles &files, const GenomeIntervals &cov, const ScoreParams &p,
-              int gt_width, int ploidy, std::vector<ScoreResult> &outs) {
+              const RowLayout &lay, std::vector<ScoreResult> &outs) {
     const int S = (int)scores.size();
-    const int64_t n_row = files.n_row, n = (int64_t)files.names.size();
-    const std::vector<std::string> &names = files.names;
-    const bool subset = !files.keep.empty();
-    size_t cur = 0;                                   // the file being read
-    // the keep list of the file being read (or, after the stream, of the last one): a context opened lazily takes it; one
-    // opened after the stream receives no rows, so any file's list serves it
-    const int64_t *keep_now = subset ? files.keep[0].data() : nullptr;
-    struct PerScore {
-        std::unique_ptr<Matcher> M;
-        std::vector<int64_t> slab_row;              // per entry: row of its device's resident slab
-        std::vector<uint8_t> done;
-        std::vector<npc_row> rows;
-    };
-    std::vector<PerScore> ps(S);
-    outs.assign(S, ScoreResult());
-
+    const int64_t n = (int64_t)files.names.size();
     PhaseTimer timer;
-    int64_t n_lookup = 0;
-    {   // entries with the same (contig, pos, ref, ea) settle on the same record: count keys once
-        std::unordered_map<std::string, int> keys;
-        for (int k = 0; k < S; k++) {
-            outs[k].samples = names;
-            ps[k].M.reset(new Matcher(*scores[k], cov, p));
-            const int64_t nE = (int64_t)scores[k]->entries.size();
-            ps[k].slab_row.assign(nE, -1); ps[k].done.assign(nE, 0);
-            if (S == 1) { n_lookup = ps[k].M->n_lookup(); break; }
-            for (int64_t i = 0; i < nE; i++) if (ps[k].M->kind[i] == Matcher::PENDING) {
-                const ScoreEntry &e = scores[k]->entries[i];
-                keys.emplace(e.contig + "\t" + std::to_string(e.pos) + "\t" + e.refseq + "\t" + e.easeq, 0);
-            }
-        }
-        if (S > 1) n_lookup = (int64_t)keys.size();
-    }
-    Spans spans;                                      // an index next to a file and few loci: read only where loci are
-    if (std::count(files.seekable.begin(), files.seekable.end(), 1))
-        for (int k = 0; k < S; k++) ps[k].M->add_spans(spans);
-    if (!files.prepare(0, spans)) throw CannotOpen{ files.paths[0] };
-    VariantSource *vcf = files.src[0].get();
-    timer.mark("coverage + entry index");
-
-    // Devices: one context per GPU.  With several, the score rows are partitioned into contiguous ranges in
-    // score-file order (a contig / region partition for a sorted score file): context d scores range d over all
-    // samples, a matched record is uploaded to the device(s) whose ranges name it, and the partial sums are
-    // combined in range order by npc_reduce.  Several score files at once: every file is cut into D ranges of its own,
-    // device d scores range d of every file in one npc_score_resident_multi call (raw partial sums), and the host adds
-    // the partials of each file in device order and normalises once.
     std::vector<int> dev_ids = p.devices.empty() ? std::vector<int>{ p.device } : p.devices;
     if (const char *e = getenv("NIMPRESS_SPLIT")) if (*e && dev_ids.size() == 1 && atoi(e) > 1)      // tests: several contexts on one GPU
         dev_ids.assign((size_t)std::min(atoi(e), 16), dev_ids[0]);
     const int D = (int)dev_ids.size();
-    // entry i of score file k belongs to device i * D / (entries of k): contiguous ranges of EVERY file in its own order
-    auto dev_of = [&](int k, int64_t i) -> int {
-        return D == 1 ? 0 : (int)std::min<int64_t>(D - 1, i * D / std::max<int64_t>((int64_t)scores[k]->entries.size(), 1));
-    };
-    std::vector<int64_t> dev_lookup(D, 0);            // rows of each device's ranges that need a record (an upper bound when files share records)
-    if (D == 1) dev_lookup[0] = n_lookup;
-    else for (int k = 0; k < S; k++)
-        for (int64_t i = 0; i < (int64_t)scores[k]->entries.size(); i++) if (ps[k].M->kind[i] == Matcher::PENDING) dev_lookup[dev_of(k, i)]++;
+    outs.assign(S, ScoreResult());
+    std::vector<ScoreState> ps;
+    ps.reserve(S);
+    for (int k = 0; k < S; k++) {
+        outs[k].samples = files.names;
+        outs[k].loci.assign(scores[k]->entries.size(), npc_locus());
+        ps.emplace_back(*scores[k], cov, p, D);
+    }
+    const std::vector<int64_t> lookup = lookup_counts(ps, D);
+    Spans spans;                                      // an index next to a file and few loci: read only where loci are
+    if (std::count(files.seekable.begin(), files.seekable.end(), 1)) for (const ScoreState &s : ps) s.M.add_spans(spans);
+    if (!files.prepare(0, spans)) throw CannotOpen{ files.paths[0] };
+    timer.mark("coverage + entry index");
 
-    // staging slots of ~8 MB: big enough for efficient H2D copies, small enough that pinning three of them per
-    // device does not dominate a short run (pinning costs ~1 ms per MB); scoring launches are sized separately
-    const int64_t row_bytes = std::max<int64_t>(16, npc_gt_row_bytes(n_row, ploidy, gt_width));
-    struct Dev {
-        Ctx ctx;
-        int32_t slot = -1; uint8_t *stage = nullptr; int64_t stride = 0, staged = 0, slab_base = 0, slab_cap = 0, block_rows = 1;
-        std::vector<npc_row> rows; std::vector<int64_t> submitted;   // S == 1: this device's rows, entry index of each
-        std::string err;
-    };
-    std::vector<Dev> devs(D);
+    Pass P{ p, lay, n, files.n_row, std::max<int64_t>(16, npc_gt_row_bytes(files.n_row, lay.ploidy, lay.width)), files.src[0].get(),
+            files.keep.empty() ? nullptr : files.keep[0].data() };
+    std::vector<Device> devs(D);
+    for (int d = 0; d < D; d++) {
+        devs[d].pass = &P; devs[d].d = d; devs[d].id = dev_ids[d]; devs[d].lookup = lookup[d];
+    }
     // rows still being converted by the source's workers land in the devices' pinned slots: let them finish before the
     // slots go, whichever way this pass ends
     struct RowsGuard {
         VariantSource *&v;
         ~RowsGuard() { try { if (v) v->wait_rows(); } catch (...) {} }
-    } rows_guard{ vcf };
-    npc_policy pol = { p.imp_locus, p.imp_missing, p.imp_sample, 0, p.mincs, p.maxmis };
-    auto open_dev = [&](int d) {
-        Dev &v = devs[d];
-        try {
-            const int64_t want = std::max<int64_t>(dev_lookup[d], 1);
-            v.block_rows = std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(4096, (8ll << 20) / row_bytes + 1), want));
-            const int64_t launch_rows = std::max<int64_t>(v.block_rows, 32768);
-            if (!subset) v.ctx.ck(npc_create2(&v.ctx.h, dev_ids[d], n, ploidy, gt_width, launch_rows, 3, v.block_rows), "npc_create");
-            else v.ctx.ck(npc_create_subset(&v.ctx.h, dev_ids[d], n_row, keep_now, n, ploidy, gt_width, launch_rows, 3,
-                                            v.block_rows), "npc_create_subset");
-            v.ctx.ck(npc_set_policy(v.ctx.h, &pol), "npc_set_policy");
-            if (p.use_ds) v.ctx.ck(npc_set_dosage_rows(v.ctx.h, 1), "npc_set_dosage_rows");
-            if (p.exact_order) v.ctx.ck(npc_set_exact_order(v.ctx.h, 1), "npc_set_exact_order");
-            v.ctx.ck(npc_reset(v.ctx.h), "npc_reset");
-            int64_t slab_want = want;
-            if (const char *e = getenv("NIMPRESS_SLAB_ROWS")) if (*e) slab_want = std::max<int64_t>(1, std::min<int64_t>(slab_want, atoll(e)));   // tests: force rounds
-            v.ctx.ck(npc_resident_reserve(v.ctx.h, slab_want, &v.slab_cap), "npc_resident_reserve");
-        } catch (const std::exception &e) { v.err = e.what(); }
-    };
-    // A device is opened when its first row arrives (or at the end, for its constant rows): contexts come up one after
-    // the other inside the driver (~1 s each), and a sorted file reaches the later ranges later -- the first device's
-    // rows stream while the others' contexts are still being created.
-    std::vector<uint8_t> opened(D, 0);
-    double waited_ms = 0.0;
-    auto ensure_open = [&](int d) {
-        if (opened[d]) return;
-        const auto t0 = std::chrono::steady_clock::now();
-        wait_warm(dev_ids[d]);
-        open_dev(d);
-        waited_ms += std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t0).count();
-        if (!devs[d].err.empty()) throw std::runtime_error(devs[d].err);
-        opened[d] = 1;
-    };
-    ensure_open(0);
+    } rows_guard{ P.src };
+    devs[0].open();
     timer.mark("first GPU context + buffers");
 
-    auto flush_stage = [&](Dev &v) {
-        if (v.slot < 0) return;
-        vcf->wait_rows();
-        v.ctx.ck(npc_stage_upload(v.ctx.h, v.slot, v.staged, v.slab_base), "npc_stage_upload");
-        v.slab_base += v.staged; v.staged = 0; v.slot = -1;
-    };
-    // the rows of score k that a round takes on device d, in score-file order
-    auto collect_rows = [&](int k, int d, bool final_round, std::vector<npc_row> &rows, std::vector<int64_t> &submitted) {
-        PerScore &q = ps[k];
-        const std::vector<ScoreEntry> &E = scores[k]->entries;
-        rows.clear();
-        for (int64_t i = 0; i < (int64_t)E.size(); i++) {
-            if (q.done[i] || dev_of(k, i) != d) continue;
-            const int32_t kind = q.M->kind[i];
-            if (!final_round && !(kind == NPC_KIND_GT && q.slab_row[i] >= 0)) continue;
-            npc_row r;
-            r.gt_row = kind == NPC_KIND_GT ? (int32_t)q.slab_row[i] : -1;
-            r.eaidx = q.M->eaidx[i]; r.beta = E[i].beta; r.eaf = E[i].eaf;
-            r.ref_is_ea = E[i].ref_is_ea() ? 1 : 0; r.kind = kind;
-            rows.push_back(r);
-            submitted.push_back(i);
-            q.done[i] = 1;
-        }
-    };
-    // A round scores rows over a device's resident slab in score-file order.  The normal case is ONE
-    // final round per device holding every row of its range: exactly the reference's loop order
-    // (:634-641).  Only when the matched genotype rows exceed device memory are there earlier rounds;
-    // those take the rows whose genotypes sit in the slab, and the summation order then differs from
-    // the reference's by a reordering of terms (scores agree to ~1 ulp of the partial sums, not bit for bit).
-    std::vector<int64_t> rounds(D, 0);
-    auto score_round = [&](int d, bool final_round) {     // one score file only
-        Dev &v = devs[d];
-        flush_stage(v);
-        collect_rows(0, d, final_round, v.rows, v.submitted);
-        if (!v.rows.empty()) v.ctx.ck(npc_score_resident(v.ctx.h, v.rows.data(), (int64_t)v.rows.size()), "npc_score_resident");
-        rounds[d]++;
-    };
-
-    // ---- one streaming pass over the genotype files (findVariant :353-364, eaidx :375-379) ---
-    VariantRecord rec;
-    int64_t records_read = 0, records_matched = 0, seeks = 0;
-    std::vector<int64_t> rec_row(D);                   // slab row this record got on each device, -1 = not uploaded there
-    for (cur = 0; cur < files.src.size(); cur++) {
-        if (cur > 0) {
-            if (!files.prepare(cur, spans)) throw CannotOpen{ files.paths[cur] };
-            vcf = files.src[cur].get();
-            if (subset) {                                 // staged rows of the previous file are compacted with its list
-                keep_now = files.keep[cur].data();
-                for (int d = 0; d < D; d++) if (opened[d]) {
-                    flush_stage(devs[d]);
-                    devs[d].ctx.ck(npc_set_keep(devs[d].ctx.h, keep_now, n), "npc_set_keep");
-                }
-            }
-        }
-        const size_t file_row_bytes = (size_t)npc_gt_row_bytes(vcf->n_samples(), ploidy, gt_width);   // the front of a staging row
-        while (vcf->next(rec)) {
-            records_read++;
-            bool any = false, need_gt = false;
-            uint32_t need_dev = 0;
-            for (int k = 0; k < S; k++) {
-                const std::vector<int64_t> &hits = ps[k].M->match(rec);
-                for (int64_t i : hits) {
-                    any = true;
-                    if (ps[k].M->kind[i] == NPC_KIND_GT) { need_gt = true; need_dev |= 1u << dev_of(k, i); }
-                }
-            }
-            if (!any) continue;
-            records_matched++;
-            if (!need_gt) continue;                                     // FILTER-failed: never decoded (:553-558)
-            const uint8_t *first = nullptr;
-            for (int d = 0; d < D; d++) {
-                rec_row[d] = -1;
-                if (!((need_dev >> d) & 1u)) continue;
-                ensure_open(d);
-                Dev &v = devs[d];
-                if (v.slab_base + v.staged >= v.slab_cap) {             // slab full: score its rows, start over
-                    if (S > 1) throw SlabOverflow();
-                    score_round(d, false);
-                    v.slab_base = 0;
-                }
-                if (v.slot < 0) {
-                    void *ptr;
-                    v.ctx.ck(npc_stage_acquire(v.ctx.h, &v.slot, &ptr, &v.stride), "npc_stage_acquire");
-                    v.stage = (uint8_t *)ptr; v.staged = 0;
-                }
-                uint8_t *dst = v.stage + v.staged * v.stride;
-                if (first) {                                            // a record named by two ranges: same bytes
-                    vcf->wait_rows();
-                    memcpy(dst, first, file_row_bytes);
-                }
-                else {
-                    if (p.use_pl && rec.alts.size() != 1)
-                        throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/PL rows take biallelic records only (" +
-                                         std::to_string(rec.alts.size()) + " ALT alleles; split them with bcftools norm -m-)");
-                    // BCF with the context's layout: the GT payload goes from the inflated blocks straight into the pinned row
-                    const bool direct = vcf->load_gt_into(rec, dst, gt_width, ploidy);
-                    if (!rec.has_gt || !rec.gt)
-                        throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) +
-                                         (p.use_pl ? " has no PL field" : p.use_ds ? " has no DS field" : " has no GT field"));
-                    if (p.use_ds && (rec.ploidy != 1 || rec.gt_width != 4))
-                        throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/DS with several values per sample is not supported");
-                    if (!direct) {
-                        if (rec.ploidy > ploidy || rec.gt_width > gt_width)
-                            throw LayoutOverflow{ std::max(rec.gt_width, gt_width), std::max(rec.ploidy, ploidy) };
-                        if (rec.gt_width == gt_width && rec.ploidy == ploidy) memcpy(dst, rec.gt, file_row_bytes);
-                        else convert_gt(rec, vcf->n_samples(), gt_width, ploidy, dst);
-                    }
-                    first = dst;
-                }
-                rec_row[d] = v.slab_base + v.staged;
-                v.staged++;
-            }
-            for (int k = 0; k < S; k++) for (int64_t i : ps[k].M->match_last())
-                if (ps[k].M->kind[i] == NPC_KIND_GT) {
-                    if (p.use_ds && ps[k].M->eaidx[i] > 1)
-                        throw InputError("record " + *rec.contig + ":" + std::to_string(rec.pos) + ": FORMAT/DS rows take the REF or the first ALT as effect allele");
-                    ps[k].slab_row[i] = rec_row[dev_of(k, i)];
-                }
-            for (int d = 0; d < D; d++) if (devs[d].slot >= 0 && devs[d].staged == devs[d].block_rows) flush_stage(devs[d]);
-        }
-        vcf->wait_rows();                                 // BGEN workers may still be writing this file's rows into pinned slots
-        seeks += vcf->seeks();
-        if (cur + 1 < files.src.size()) { files.src[cur].reset(); vcf = nullptr; }
-    }
-    for (int k = 0; k < S; k++) {
-        ps[k].M->finish();
-        outs[k].records_read = records_read; outs[k].records_matched = records_matched; outs[k].index_seeks = seeks;
-    }
+    stream_files(files, spans, P, ps, devs, outs);
     timer.mark("stream + match + upload");
-    if (timer.on) fprintf(stderr, "[nimpress timing] records read %lld, matched %lld, index seeks %lld%s\n", (long long)records_read,
-                          (long long)records_matched, (long long)seeks, seeks ? " (.tbi / .csi used)" : "");
+    const ScoreResult &o = outs[0];
+    if (timer.on) fprintf(stderr, "[nimpress timing] records read %lld, matched %lld, index seeks %lld%s\n", (long long)o.records_read,
+                          (long long)o.records_matched, (long long)o.index_seeks, o.index_seeks ? " (.tbi / .csi used)" : "");
 
-    // ---- score the slab(s), collect results ----------------------------------------------------
-    std::vector<std::vector<npc_locus>> logs(S);
-    std::vector<std::vector<int64_t>> order(S);          // entry index of every log record
-    for (int d = 0; d < D; d++) ensure_open(d);
-    if (timer.on && D > 1) fprintf(stderr, "[nimpress timing] waited for GPU contexts + buffers, all devices %8.1f ms\n", waited_ms);
-    if (S == 1) {
-        for (int d = 0; d < D; d++) score_round(d, true);
-        outs[0].scores.assign(n, 0.0);
-        outs[0].rounds = *std::max_element(rounds.begin(), rounds.end());
-        outs[0].devices = D;
-        if (D == 1) {
-            Dev &v = devs[0];
-            logs[0].resize(v.submitted.size());
-            int64_t nlog = 0;
-            v.ctx.ck(npc_finish(v.ctx.h, scores[0]->offset, outs[0].scores.data(), &outs[0].nloci, logs[0].data(), (int64_t)logs[0].size(), &nlog), "npc_finish");
-            if (nlog != (int64_t)v.submitted.size()) throw std::runtime_error("locus log length mismatch");
-            order[0] = v.submitted;
-        } else {
-            std::vector<npc_ctx *> hs(D);
-            for (int d = 0; d < D; d++) hs[d] = devs[d].ctx.h;
-            const double off = scores[0]->offset;
-            devs[0].ctx.ck(npc_reduce(hs.data(), D, &off, outs[0].scores.data(), &outs[0].nloci), "npc_reduce");
-            std::vector<double> scratch((size_t)std::max<int64_t>(n, 1));
-            for (int d = 0; d < D; d++) {
-                Dev &v = devs[d];
-                std::vector<npc_locus> lg(v.submitted.size());
-                int64_t nlog = 0, nl = 0;
-                v.ctx.ck(npc_partial(v.ctx.h, scratch.data(), &nl, lg.data(), (int64_t)lg.size(), &nlog), "npc_partial");
-                if (nlog != (int64_t)v.submitted.size()) throw std::runtime_error("locus log length mismatch");
-                logs[0].insert(logs[0].end(), lg.begin(), lg.end());
-                order[0].insert(order[0].end(), v.submitted.begin(), v.submitted.end());
-            }
-        }
-    } else {
-        std::vector<int64_t> nloci_tot(S, 0);
-        std::vector<std::vector<double>> part(S);
-        for (int k = 0; k < S; k++) { outs[k].scores.assign(n, 0.0); outs[k].rounds = 1; outs[k].devices = D; if (D > 1) part[k].assign((size_t)n, 0.0); }
-        for (int d = 0; d < D; d++) {
-            Dev &v = devs[d];
-            flush_stage(v);
-            std::vector<std::vector<npc_row>> drows(S);
-            std::vector<std::vector<npc_locus>> dlog(S);
-            std::vector<const npc_row *> rows(S);
-            std::vector<int64_t> n_rows(S), nloci(S);
-            std::vector<double> offsets(S);
-            std::vector<double *> sc(S);
-            std::vector<npc_locus *> lg(S);
-            for (int k = 0; k < S; k++) {
-                collect_rows(k, d, true, drows[k], order[k]);
-                rows[k] = drows[k].data(); n_rows[k] = (int64_t)drows[k].size(); offsets[k] = scores[k]->offset;
-                sc[k] = D == 1 ? outs[k].scores.data() : part[k].data();
-                dlog[k].resize(drows[k].size()); lg[k] = dlog[k].data();
-            }
-            // one device: normalised scores straight away; several: raw partial sums (offsets = NULL), combined below
-            v.ctx.ck(npc_score_resident_multi(v.ctx.h, S, rows.data(), n_rows.data(), D == 1 ? offsets.data() : nullptr, sc.data(), nloci.data(), lg.data()),
-                     "npc_score_resident_multi");
-            for (int k = 0; k < S; k++) {
-                nloci_tot[k] += nloci[k];
-                logs[k].insert(logs[k].end(), dlog[k].begin(), dlog[k].end());
-                if (D > 1) {
-                    double *tot = outs[k].scores.data();
-                    const double *pk = part[k].data();
-                    if (d == 0) memcpy(tot, pk, (size_t)n * sizeof(double));
-                    else for (int64_t i = 0; i < n; i++) tot[i] += pk[i];            // device order = score-file order of the ranges
-                }
-            }
-        }
-        for (int k = 0; k < S; k++) {
-            outs[k].nloci = nloci_tot[k];
-            if (D > 1) npc_normalise(outs[k].scores.data(), n, nloci_tot[k], scores[k]->offset);
-        }
-    }
+    for (Device &v : devs) v.open();
+    if (timer.on && D > 1) fprintf(stderr, "[nimpress timing] waited for GPU contexts + buffers, all devices %8.1f ms\n", P.waited_ms);
+    if (S == 1) score_single(ps[0], devs, n, outs[0]);
+    else score_multi(ps, devs, n, outs);
     timer.mark("score + finish (GPU)");
-    for (int k = 0; k < S; k++) {
-        outs[k].loci.assign(scores[k]->entries.size(), npc_locus());
-        for (size_t j = 0; j < order[k].size(); j++) outs[k].loci[order[k][j]] = logs[k][j];
-        outs[k].warnings = make_warnings(*scores[k], *ps[k].M, outs[k].loci, n, p,
-                                         p.use_ds || p.use_pl || gt_width == NPC_GT_DOSE255 || gt_width == NPC_GT_DOSE32);
-    }
+    for (int k = 0; k < S; k++) outs[k].warnings = make_warnings(*scores[k], ps[k].M, outs[k].loci, n, p, lay.real_tally());
     timer.mark("WARN lines (binomial tests)");
 }
 
@@ -649,34 +681,24 @@ void run_pass(const std::vector<const ScoreFile *> &scores, GenotypeFiles &files
 bool compute_polygenic_scores_files(const std::vector<const ScoreFile *> &scores, const std::vector<std::string> &genotype_paths,
                                     const GenomeIntervals &cov, const ScoreParams &p, std::vector<ScoreResult> &outs, std::string *unopened) {
     for (int d : (p.devices.empty() ? std::vector<int>{ p.device } : p.devices)) start_warm(d);
-    int width = 1, ploidy = 2;                      // BCF's usual GT layout: int8, diploid
-    if (p.use_ds && p.use_pl) throw InputError("--pl and --dosage: score either FORMAT/PL or FORMAT/DS");
-    if (p.use_ds) { width = 4; ploidy = 1; }        // FORMAT/DS: one float per sample
-    if (p.use_pl) { width = NPC_GT_PL; ploidy = 2; }   // FORMAT/PL: one packed word per sample
+    RowLayout lay = row_layout(VariantSource::NO_FIXED_LAYOUT, p, false);   // --pl with --dosage fails before any file is opened
     GenotypeFiles files(genotype_paths);            // each file first tries the index-driven pass (needs <file>.tbi / .csi)
     bool dose32 = false;                            // a BGEN pass met a block that only 32-bit dosage rows hold
     for (int attempt = 0; attempt < 6; attempt++) {
         // every file is (re)opened and its --samples list resolved before any context: a bad list fails without a device
         if (!files.open(p, unopened)) return false;
-        // PLINK filesets, BGEN files: rows in a layout of their own, read by offset (no index pass)
-        const int fixed = files.kind;
-        ScoreParams q = p;
-        if (fixed == NPC_GT_BED && p.use_ds) throw InputError("--dosage: a PLINK fileset holds hard calls only, no FORMAT/DS");
-        if (fixed == NPC_GT_BED && p.use_pl) throw InputError("--pl: a PLINK fileset holds hard calls only, no FORMAT/PL");
-        if (fixed == NPC_GT_DOSE255 && p.use_pl) throw InputError("--pl: a BGEN file holds genotype probabilities, no FORMAT/PL");
-        if (fixed != VariantSource::NO_FIXED_LAYOUT) {
-            width = dose32 ? NPC_GT_DOSE32 : fixed; ploidy = 2;
-            q.use_ds = false;                       // BGEN rows are dosages already: --dosage changes nothing
-        }
-        files.set_modes(q.use_ds, q.use_pl);
+        // PLINK filesets, BGEN files: rows in a layout of their own, read by offset (no index pass); VCF/BCF rows keep
+        // the layout the last LayoutOverflow grew them to
+        if (files.kind != VariantSource::NO_FIXED_LAYOUT) lay = row_layout(files.kind, p, dose32);
+        files.set_modes(lay.ds, lay.pl);
         try {
-            run_pass(scores, files, cov, q, width, ploidy, outs);
+            run_pass(scores, files, cov, p, lay, outs);
             return true;
         } catch (const CannotOpen &e) {
             if (unopened) *unopened = e.path;
             return false;
         } catch (const LayoutOverflow &o) {         // rare: wider integers or higher ploidy -- rerun every file with that layout
-            width = o.width; ploidy = o.ploidy;
+            lay.width = o.width; lay.ploidy = o.ploidy;
         } catch (const NeedsDose32 &e) {            // BGEN at another bit depth or with haploid samples: rerun with 32-bit rows
             dose32 = true;
             if (getenv("NIMPRESS_TIMING")) fprintf(stderr, "[nimpress timing] restart with 32-bit dosage rows: %s\n", e.what());
@@ -692,19 +714,6 @@ bool compute_polygenic_scores_files(const std::vector<const ScoreFile *> &scores
         }
     }
     throw std::runtime_error("GT layout kept growing between passes");
-}
-
-bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores, const std::string &genotype_path,
-                                    const GenomeIntervals &cov, const ScoreParams &p, std::vector<ScoreResult> &outs) {
-    return compute_polygenic_scores_files(scores, { genotype_path }, cov, p, outs);
-}
-
-bool compute_polygenic_scores(const ScoreFile &score, const std::string &genotype_path, const GenomeIntervals &cov,
-                              const ScoreParams &p, ScoreResult &out) {
-    std::vector<ScoreResult> outs;
-    if (!compute_polygenic_scores_multi({ &score }, genotype_path, cov, p, outs)) return false;
-    out = std::move(outs[0]);
-    return true;
 }
 
 }  // namespace nph

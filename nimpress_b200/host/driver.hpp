@@ -56,7 +56,6 @@ public:
     const std::vector<int64_t> &match_last() const { return hits_; }   // what the last match() returned
     void finish();                                  // everything still pending is ABSENT (:536)
     bool has_contig(const std::string &c) const { return index_.count(c) != 0; }
-    int64_t n_lookup() const { return n_lookup_; }
     // 1-based inclusive [pos, stop] of every entry that needs a record lookup, per contig (for the index-driven reader)
     void add_spans(std::unordered_map<std::string, std::vector<std::pair<int64_t, int64_t>>> &spans) const;
 
@@ -70,7 +69,6 @@ private:
     bool ignorefilt_;
     std::unordered_map<std::string, ContigIndex> index_;
     std::vector<int64_t> hits_;
-    int64_t n_lookup_ = 0;
 };
 
 // --samples: the samples of `file_samples` (the genotype file's names, in its order) to score, as ascending indices; an
@@ -107,18 +105,10 @@ private:
     std::vector<uint8_t> opened_seekable_;             // per file: its source reads block by block (no inflate pool)
 };
 
-// Throws InputError where the reference raises; std::runtime_error on CUDA / library failure.
-// false: the genotype file cannot be opened (the reference: FATAL + quit(-1), :728-730).
-bool compute_polygenic_scores(const ScoreFile &score, const std::string &genotype_path, const GenomeIntervals &cov,
-                              const ScoreParams &p, ScoreResult &out);
-
-// Several score files over ONE pass of the genotype file (BASELINE config 4).  Each result is what
-// compute_polygenic_scores gives for that file alone (the reference: one nimpress run per file).
-bool compute_polygenic_scores_multi(const std::vector<const ScoreFile *> &scores, const std::string &genotype_path,
-                                    const GenomeIntervals &cov, const ScoreParams &p, std::vector<ScoreResult> &outs);
-
-// The same over several genotype files, exactly as over their concatenation (DESIGN.md 4.12).  false: a genotype file
-// cannot be opened (*unopened, when given, names it).
+// computePolygenicScores for one score file or several over ONE pass of the genotype files (BASELINE config 4), read
+// exactly as their concatenation (DESIGN.md 4.12).  Each result is what that score file alone gives (the reference: one
+// nimpress run per file).  Throws InputError where the reference raises; std::runtime_error on CUDA / library failure.
+// false: a genotype file cannot be opened (the reference: FATAL + quit(-1), :728-730; *unopened, when given, names it).
 bool compute_polygenic_scores_files(const std::vector<const ScoreFile *> &scores, const std::vector<std::string> &genotype_paths,
                                     const GenomeIntervals &cov, const ScoreParams &p, std::vector<ScoreResult> &outs,
                                     std::string *unopened = nullptr);
