@@ -227,9 +227,20 @@ int npc_set_policy(npc_ctx *ctx, const npc_policy *p);
  * (defaults to n_samples). */
 int npc_set_cohort_size(npc_ctx *ctx, int64_t n_total);
 
-/* Zero the per-sample sums, nloci and the locus log: start of a computePolygenicScores call
- * (src/nimpress.nim:626-632). */
+/* Zero the per-sample sums, nloci and the locus log (and the observed counts, npc_set_observed): start of a
+ * computePolygenicScores call (src/nimpress.nim:626-632). */
 int npc_reset(npc_ctx *ctx);
+
+/* Not in the reference (DESIGN 4.13).  on != 0: from now on every scoring launch (npc_score_block, npc_score_block_device,
+ * npc_score_resident, npc_accumulate_block_device) also adds, per sample, the number of its score rows whose record has
+ * class OK (klass 0) and at which the sample has a called genotype -- one with no nmiss count in the layout's tally --
+ * into a per-context vector of int64 counts: one more kernel on the context's stream per launch.  Rows of the other
+ * classes never count (their dosage is the locus constant).  Loci, not alleles: PLINK's ALLELE_CT is twice this for
+ * diploid calls.  npc_reset zeroes the vector; on = 0 stops adding to it.  Off (the default) launches nothing more. */
+int npc_set_observed(npc_ctx *ctx, int32_t on);
+/* Waits for the submitted work, then copies the context's n_samples counts out.  Variant-sharded contexts: add them
+ * (integers: any order).  NPC_ESTATE when npc_set_observed was never turned on. */
+int npc_observed(npc_ctx *ctx, int64_t *out);
 
 /* ---- streaming blocks from host memory (pinned, double-buffered) ---------------------- */
 
@@ -289,7 +300,7 @@ int npc_score_resident(npc_ctx *ctx, const npc_row *rows, int64_t n_rows);
  * npc_finish(offsets[k], scores_out[k], &nloci_out[k], loci_out[k], n_rows[k]) gives:
  * scores_out[k][n_samples] normalised, loci_out[k][n_rows[k]] in row order (loci_out or
  * loci_out[k] may be NULL).  Synchronous; the context's own running sums and locus log are
- * overwritten.  offsets == NULL: scores_out[k] receives the raw partial sums instead (what
+ * overwritten, and its observed counts (npc_set_observed) are left zero.  offsets == NULL: scores_out[k] receives the raw partial sums instead (what
  * npc_partial gives) -- for variant-sharded cohorts, where the caller adds the shards' partials
  * per definition in shard order and applies npc_normalise once.
  *   With three or more definitions on an int8 diploid slab (and exact order off) the sums are
@@ -307,6 +318,14 @@ int npc_score_resident(npc_ctx *ctx, const npc_row *rows, int64_t n_rows);
 int npc_score_resident_multi(npc_ctx *ctx, int32_t n_scores, const npc_row *const *rows, const int64_t *n_rows,
                              const double *offsets, double *const *scores_out, int64_t *nloci_out,
                              npc_locus *const *loci_out);
+/* npc_score_resident_multi, and per definition the count of scored loci that used each sample's own genotype
+ * (npc_set_observed, DESIGN 4.13): observed_out[k][n_samples], or nothing when observed_out or observed_out[k] is NULL.
+ * The counts come from the definitions' records, one pass over the slab per group of up to 8 definitions, whichever
+ * path (contraction or one by one) scored them: the same integers either way.  The context's own observed vector
+ * (npc_set_observed) is not added to; like its running sums, it is reset: both multi calls leave it zero, on either path. */
+int npc_score_resident_multi_observed(npc_ctx *ctx, int32_t n_scores, const npc_row *const *rows, const int64_t *n_rows,
+                                      const double *offsets, double *const *scores_out, int64_t *nloci_out,
+                                      npc_locus *const *loci_out, int64_t *const *observed_out);
 
 /* ---- results ---------------------------------------------------------------------------- */
 

@@ -74,6 +74,9 @@ typedef struct {
                                subset or an unreadable list is NPH_EINPUT.  Not in the reference (plink --keep, bcftools -S) */
     int32_t exclude_samples;  /* 1: score the samples the list does NOT name (plink --remove, bcftools -S ^FILE); names the file
                                lacks are ignored */
+    int32_t observed;       /* 1: also count, per sample, the score rows of class OK at which the sample has a called genotype
+                               (nph_result_observed; DESIGN.md 4.13); scores and records are the same either way.  Not in the
+                               reference (PLINK's CNT, PRSice's CNT, pgsc_calc's DENOM) */
 } nph_params;
 
 typedef struct nph_result nph_result;
@@ -103,6 +106,9 @@ int64_t nph_result_devices(const nph_result *r);         /* GPUs that scored thi
 int64_t nph_result_records_read(const nph_result *r);    /* records the reader handed to the matcher         */
 int64_t nph_result_index_seeks(const nph_result *r);     /* > 0: the file's .tbi / .csi index was used        */
 const double *nph_result_scores(const nph_result *r);
+/* Per sample: score rows of class OK (klass 0) at which the sample has a called genotype, i.e. nloci minus the loci imputed
+ * for it (DESIGN.md 4.13).  NULL exactly when nph_params.observed was not set (never NULL when it was, even for no samples). */
+const int64_t *nph_result_observed(const nph_result *r);
 const npc_locus *nph_result_loci(const nph_result *r);   /* score-file order */
 const char *nph_result_sample(const nph_result *r, int64_t i);
 const char *nph_result_warnings(const nph_result *r);    /* "WARN ...\n" lines, reference order */

@@ -52,7 +52,8 @@ class _Params(C.Structure):
                 ("ignorefilt", C.c_int32), ("use_cov", C.c_int32), ("device", C.c_int32),
                 ("exact_order", C.c_int32), ("device_mask", C.c_int32),
                 ("mincs", C.c_int64), ("maxmis", C.c_double), ("afmisp", C.c_double),
-                ("use_ds", C.c_int32), ("use_pl", C.c_int32), ("samples_path", C.c_char_p), ("exclude_samples", C.c_int32)]
+                ("use_ds", C.c_int32), ("use_pl", C.c_int32), ("samples_path", C.c_char_p), ("exclude_samples", C.c_int32),
+                ("observed", C.c_int32)]
 
 
 _host = None
@@ -79,7 +80,7 @@ def load_host_library():
                                                          C.POINTER(vp)]),
         "nph_result_n_samples": (i64, [vp]), "nph_result_n_loci": (i64, [vp]), "nph_result_nloci_used": (i64, [vp]),
         "nph_result_rounds": (i64, [vp]), "nph_result_devices": (i64, [vp]), "nph_result_scores": (vp, [vp]), "nph_result_loci": (vp, [vp]),
-        "nph_result_sample": (cp, [vp, i64]), "nph_result_warnings": (cp, [vp]), "nph_result_free": (None, [vp]),
+        "nph_result_sample": (cp, [vp, i64]), "nph_result_observed": (vp, [vp]), "nph_result_warnings": (cp, [vp]), "nph_result_free": (None, [vp]),
         "nph_last_error": (cp, []),
         "nph_plan": (C.c_int, [cp, cp, cp, C.POINTER(_Params), vp, vp, i64, C.POINTER(i64), C.POINTER(i64)]),
         "nph_fast_inflate": (C.c_int, [vp, i64, vp, i64]),
@@ -140,24 +141,26 @@ def loadBedIntervals(ivals, path):
 
 
 class Result:
-    def __init__(self, scores, loci, nloci, samples, warnings, rounds, records_read=0, index_seeks=0):
+    def __init__(self, scores, loci, nloci, samples, warnings, rounds, records_read=0, index_seeks=0, observed=None):
         self.scores, self.loci, self.nloci, self.samples, self.warnings, self.rounds = scores, loci, nloci, samples, warnings, rounds
         self.records_read, self.index_seeks = records_read, index_seeks     # index_seeks > 0: the .tbi / .csi index was used
+        self.observed = observed            # int64 per sample with observed=True (DESIGN.md 4.13), else None
 
 
 def run(score_path, genotype_path, bed_path=None, imp_locus=ImputeMethodLocus.ps, imp_missing=ImputeMethodMissing.homref,
         imp_sample=ImputeMethodSample.int_ps, maxmis=0.05, afmisp=0.001, mincs=100, ignorefilt=False, device=0,
-        exact_order=False, devices=None, dosage=False, pl=False, samples=None, exclude_samples=False):
+        exact_order=False, devices=None, dosage=False, pl=False, samples=None, exclude_samples=False, observed=False):
     """nph_compute_polygenic_scores -> Result (scores, per-locus records, WARN text).  devices: list of CUDA
     device indices to split the score rows over (npc_reduce combines their partial sums).  dosage: score FORMAT/DS;
     pl: score FORMAT/PL as posterior expected dosages at the score file's eaf (DESIGN.md 4.10).  samples: path of a
     list of sample names to score (one per line; DESIGN.md 4.11), exclude_samples: score the others instead.
-    genotype_path: one path, or a list of them (e.g. one file per chromosome) scored as their concatenation (DESIGN.md 4.12)."""
+    genotype_path: one path, or a list of them (e.g. one file per chromosome) scored as their concatenation (DESIGN.md 4.12).
+    observed: also fill Result.observed, per sample the OK loci at which it has a called genotype (DESIGN.md 4.13)."""
     L = load_host_library()
     mask = sum(1 << int(d) for d in set(devices)) if devices else 0
     p = _Params(int(imp_locus), int(imp_missing), int(imp_sample), int(ignorefilt), int(bed_path is not None), device,
                 int(bool(exact_order)), mask, int(mincs), float(maxmis), float(afmisp), int(bool(dosage)), int(bool(pl)),
-                os.fsencode(samples) if samples else None, int(bool(exclude_samples)))
+                os.fsencode(samples) if samples else None, int(bool(exclude_samples)), int(bool(observed)))
     if not isinstance(genotype_path, (str, bytes, os.PathLike)):
         return _run_files([score_path], genotype_path, bed_path, p)[0]
     h = C.c_void_p()
@@ -169,13 +172,13 @@ def run(score_path, genotype_path, bed_path=None, imp_locus=ImputeMethodLocus.ps
 
 def run_multi(score_paths, genotype_path, bed_path=None, imp_locus=ImputeMethodLocus.ps, imp_missing=ImputeMethodMissing.homref,
               imp_sample=ImputeMethodSample.int_ps, maxmis=0.05, afmisp=0.001, mincs=100, ignorefilt=False, device=0,
-              exact_order=False, pl=False, samples=None, exclude_samples=False):
+              exact_order=False, pl=False, samples=None, exclude_samples=False, observed=False):
     """nph_compute_polygenic_scores_multi: several score files over one pass of the genotype file
     -> [Result], each equal to run() on that file alone.  genotype_path: one path or a list of them, as for run()."""
     L = load_host_library()
     p = _Params(int(imp_locus), int(imp_missing), int(imp_sample), int(ignorefilt), int(bed_path is not None), device,
                 int(bool(exact_order)), 0, int(mincs), float(maxmis), float(afmisp), 0, int(bool(pl)),
-                os.fsencode(samples) if samples else None, int(bool(exclude_samples)))
+                os.fsencode(samples) if samples else None, int(bool(exclude_samples)), int(bool(observed)))
     if not isinstance(genotype_path, (str, bytes, os.PathLike)):
         return _run_files(score_paths, genotype_path, bed_path, p)
     paths = (C.c_char_p * len(score_paths))(*[os.fsencode(s) for s in score_paths])
@@ -215,8 +218,11 @@ def _take_result(L, h):
         loci = np.frombuffer(C.string_at(L.nph_result_loci(h), nl * LOCUS_DTYPE.itemsize), dtype=LOCUS_DTYPE).copy() if nl \
             else np.zeros(0, LOCUS_DTYPE)
         samples = [L.nph_result_sample(h, i).decode() for i in range(n)]
+        op = L.nph_result_observed(h)
+        observed = np.ctypeslib.as_array(C.cast(op, C.POINTER(C.c_int64)), (n,)).copy() if op and n else \
+            (np.zeros(0, np.int64) if op is not None else None)
         r = Result(scores, loci, L.nph_result_nloci_used(h), samples, L.nph_result_warnings(h).decode(),
-                   L.nph_result_rounds(h), L.nph_result_records_read(h), L.nph_result_index_seeks(h))
+                   L.nph_result_rounds(h), L.nph_result_records_read(h), L.nph_result_index_seeks(h), observed)
         r.devices = L.nph_result_devices(h)
         return r
     finally:

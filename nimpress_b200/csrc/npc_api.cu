@@ -2,6 +2,7 @@
 // double-buffered staging ring, stream/event plumbing and kernel launches.  No CPU fallback:
 // every entry point either runs the CUDA kernels or fails.
 #include <algorithm>
+#include <array>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -20,6 +21,7 @@
 #include "npc_dose32.cuh"
 #include "npc_pl.cuh"
 #include "npc_subset.cuh"
+#include "npc_observed.cuh"
 
 using namespace npc;
 
@@ -142,6 +144,11 @@ struct npc_ctx {
     void *comm = nullptr;                   // ncclComm_t of npc_comm_init
     int comm_rank = 0, comm_world = 1;
     double *d_gather = nullptr;             // [world][n] all-gathered partial sums
+    // per-sample observed counts (npc_observed.cuh): while `observed`, every scoring launch adds its OK rows' counts to d_obs
+    bool observed = false;
+    ull *d_obs = nullptr;
+    uint8_t *d_obs_scratch = nullptr;       // npc_score_resident_multi_observed: a group's entries, weights and counts
+    size_t obs_scratch_bytes = 0;
 };
 
 static npc::NcclApi g_nccl;
@@ -202,6 +209,7 @@ extern "C" void npc_destroy(npc_ctx *ctx) {
     if (ctx->ev_reduce) cudaEventDestroy(ctx->ev_reduce);
     if (ctx->ev_multi) cudaEventDestroy(ctx->ev_multi);
     cudaFree(ctx->d_nloci_total); cudaFree(ctx->d_bridge); cudaFree(ctx->d_gather); cudaFree(ctx->d_ds_part); cudaFree(ctx->d_bed_tab); cudaFree(ctx->d_bed_off);
+    cudaFree(ctx->d_obs); cudaFree(ctx->d_obs_scratch);
     if (ctx->comm && g_nccl.lib) g_nccl.CommDestroy(ctx->comm);
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
@@ -500,6 +508,7 @@ extern "C" int npc_reset(npc_ctx *ctx) {
     NPC_CUDA(ctx, cudaSetDevice(ctx->device));
     NPC_CUDA(ctx, cudaMemsetAsync(ctx->d_sums, 0, std::max<int64_t>(ctx->n, 1) * sizeof(double), ctx->stream));
     NPC_CUDA(ctx, cudaMemsetAsync(ctx->d_nloci, 0, sizeof(ull), ctx->stream));
+    if (ctx->d_obs) NPC_CUDA(ctx, cudaMemsetAsync(ctx->d_obs, 0, std::max<int64_t>(ctx->n, 1) * sizeof(ull), ctx->stream));
     ctx->log_len = 0;
     return NPC_OK;
 }
@@ -776,6 +785,48 @@ static int launch_accum(npc_ctx *c, const uint8_t *gt, int64_t row_stride, int64
     return NPC_OK;
 }
 
+// The observed pass (npc_observed.cuh) over n_ent entries: out[g * n + s] += called(entry, s) x weight.  w == nullptr: a
+// group of one weighted by the records in log; else OBS_G definitions, w[g * n_ent + e].
+template <class L>
+static int observed_launch(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *ent, const npc_locus *log,
+                           const uint32_t *w, int64_t n_ent, ull *out) {
+    const unsigned gx = (unsigned)((c->n + (int64_t)L::P * OBS_THREADS - 1) / ((int64_t)L::P * OBS_THREADS));
+    // the entries split over gridDim.y until ~16 CTAs an SM, at least 64 entries each
+    const int64_t sms = c->num_sms > 0 ? c->num_sms : 148;
+    const int64_t gy = std::max<int64_t>(1, std::min<int64_t>({ (sms * 16 + gx - 1) / gx, (n_ent + 63) / 64, 65535 }));
+    const int64_t per_y = (n_ent + gy - 1) / gy;
+    auto k = w ? k_observed<L, OBS_G> : k_observed<L, 1>;
+    k<<<dim3(gx, (unsigned)((n_ent + per_y - 1) / per_y)), OBS_THREADS, 0, c->stream>>>(gt, row_stride, c->ploidy, ent, log, w, n_ent, per_y,
+                                                                                     c->n, out);
+    c->launches++;
+    NPC_CUDA(c, cudaGetLastError());
+    return NPC_OK;
+}
+
+static int launch_observed(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *ent, const npc_locus *log,
+                           const uint32_t *w, int64_t n_ent, ull *out) {
+    if (n_ent == 0 || c->n == 0) return NPC_OK;
+    switch (c->layout) {
+    case Layout::GT:
+        if (c->width == 1 && c->ploidy == 2) return observed_launch<ObsI8x2>(c, gt, row_stride, ent, log, w, n_ent, out);
+        if (c->width == 1) return observed_launch<ObsGT<int8_t>>(c, gt, row_stride, ent, log, w, n_ent, out);
+        if (c->width == 2) return observed_launch<ObsGT<int16_t>>(c, gt, row_stride, ent, log, w, n_ent, out);
+        return observed_launch<ObsGT<int32_t>>(c, gt, row_stride, ent, log, w, n_ent, out);
+    case Layout::DS: return observed_launch<ObsDs>(c, gt, row_stride, ent, log, w, n_ent, out);
+    case Layout::BED: return observed_launch<ObsBed>(c, gt, row_stride, ent, log, w, n_ent, out);
+    case Layout::DOSE255: return observed_launch<ObsDose255>(c, gt, row_stride, ent, log, w, n_ent, out);
+    case Layout::DOSE32: return observed_launch<ObsDose32>(c, gt, row_stride, ent, log, w, n_ent, out);
+    case Layout::PL: return observed_launch<ObsPl>(c, gt, row_stride, ent, log, w, n_ent, out);
+    }
+    return NPC_OK;
+}
+
+// After a launch's scoring sequence: its n_rows rows and their records (the last n_rows of the log) into d_obs
+static int observe_launch(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows) {
+    if (!c->observed || n_rows == 0) return NPC_OK;
+    return launch_observed(c, gt, row_stride, d_rows, c->d_log + c->log_len - n_rows, nullptr, n_rows, c->d_obs);
+}
+
 // The tile kernel's parameters for shape t over every sample and one row group; each mode then sets its own fields
 static FusedParams fused_params(const npc_ctx *c, const npc_ctx::TileCfg &t, const uint8_t *gt, int64_t row_stride,
                                 const npc_row *d_rows, int64_t n_rows) {
@@ -849,15 +900,16 @@ static int launch_wide(npc_ctx *c, const npc_ctx::TileCfg &t, bool exact, const 
 
 static int launch_block(npc_ctx *c, const uint8_t *gt, int64_t row_stride, const npc_row *d_rows, int64_t n_rows) {
     const npc_ctx::TileCfg *t;
+    int rc;
     switch (launch_mode(c, c->exact, n_rows, t)) {
-    case 1: case 2: return launch_fused(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
-    case 3: return launch_wide(c, *t, c->exact, gt, row_stride, d_rows, n_rows);
-    default: {                                                                                  // 0, 4, 5, 6, 7
-        int rc = launch_tally(c, gt, row_stride, d_rows, n_rows, c->d_counts);
+    case 1: case 2: rc = launch_fused(c, *t, c->exact, gt, row_stride, d_rows, n_rows); break;
+    case 3: rc = launch_wide(c, *t, c->exact, gt, row_stride, d_rows, n_rows); break;
+    default:                                                                                    // 0, 4, 5, 6, 7
+        rc = launch_tally(c, gt, row_stride, d_rows, n_rows, c->d_counts);
         if (!rc) rc = launch_decide(c, gt, row_stride, d_rows, n_rows, c->d_counts);
-        return rc ? rc : launch_accum(c, gt, row_stride, n_rows);
+        if (!rc) rc = launch_accum(c, gt, row_stride, n_rows);
     }
-    }
+    return rc ? rc : observe_launch(c, gt, row_stride, d_rows, n_rows);
 }
 
 // ---- subset contexts: compaction ------------------------------------------------------------
@@ -1006,7 +1058,8 @@ extern "C" int npc_accumulate_block_device(npc_ctx *ctx, const void *gt_dev, int
     const npc_row *d_rows;
     int rc = split_prologue(ctx, gt_dev, row_stride, n_gt_rows, rows, n_rows, rows_on_device, counts_dev, &d_rows);
     if (!rc) rc = launch_decide(ctx, (const uint8_t *)gt_dev, row_stride, d_rows, n_rows, (const ull *)counts_dev);
-    return rc ? rc : launch_accum(ctx, (const uint8_t *)gt_dev, row_stride, n_rows);
+    if (!rc) rc = launch_accum(ctx, (const uint8_t *)gt_dev, row_stride, n_rows);
+    return rc ? rc : observe_launch(ctx, (const uint8_t *)gt_dev, row_stride, d_rows, n_rows);
 }
 
 // ---- resident slab ---------------------------------------------------------------------------
@@ -1347,12 +1400,8 @@ static int multi_contract(npc_ctx *c, int32_t S, const npc_row *const *rows, con
     return 0;
 }
 
-extern "C" int npc_score_resident_multi(npc_ctx *ctx, int32_t n_scores, const npc_row *const *rows, const int64_t *n_rows,
-                                        const double *offsets, double *const *scores_out, int64_t *nloci_out,
-                                        npc_locus *const *loci_out) {
-    if (!ctx || n_scores < 0 || (n_scores && (!rows || !n_rows || !scores_out))) return NPC_EINVAL;
-    for (int32_t k = 0; k < n_scores; k++) if (n_rows[k] < 0 || (n_rows[k] && !rows[k]) || !scores_out[k]) return NPC_EINVAL;
-    NPC_CUDA(ctx, cudaSetDevice(ctx->device));
+static int score_multi(npc_ctx *ctx, int32_t n_scores, const npc_row *const *rows, const int64_t *n_rows, const double *offsets,
+                       double *const *scores_out, int64_t *nloci_out, npc_locus *const *loci_out) {
     // the contraction pays one tally pass + one pass per 16 definitions; below three definitions the fused kernel is as cheap
     const char *env = getenv("NPC_MULTI");
     const int min_scores = env && *env ? (atoi(env) ? 1 : 1 << 30) : 3;
@@ -1361,6 +1410,132 @@ extern "C" int npc_score_resident_multi(npc_ctx *ctx, int32_t n_scores, const np
         if (rc <= 0) { if (rc == 0) ctx->multi_contractions++; return rc; }
     }
     return multi_one_by_one(ctx, n_scores, rows, n_rows, offsets, scores_out, nloci_out, loci_out);
+}
+
+// Observed counts of the definitions with observed_out[k] != NULL from their records (loci[k]), OBS_G definitions per pass
+// over the slab.  An entry is a slab row (FORMAT/PL: a slab row, effect allele and eaf, which decide whether a sample is
+// called); its weight for a definition is the number of the definition's OK rows that name it.
+static int multi_observed(npc_ctx *c, int32_t S, const npc_row *const *rows, const int64_t *n_rows, npc_locus *const *loci,
+                          int64_t *const *observed_out) {
+    std::vector<int32_t> defs;
+    for (int32_t k = 0; k < S; k++) if (observed_out[k]) defs.push_back(k);
+    const bool pl = c->layout == Layout::PL;
+    const int64_t n1 = std::max<int64_t>(c->n, 1);
+    for (size_t k0 = 0; k0 < defs.size(); k0 += OBS_G) {
+        const size_t ng = std::min<size_t>(OBS_G, defs.size() - k0);
+        std::vector<npc_row> ent;
+        std::vector<std::array<uint32_t, OBS_G>> wt;
+        std::vector<int32_t> by_row((size_t)c->slab_rows, -1);
+        std::unordered_map<std::string, int32_t> by_key;                // FORMAT/PL entries
+        for (size_t g = 0; g < ng; g++) {
+            const int32_t k = defs[k0 + g];
+            for (int64_t i = 0; i < n_rows[k]; i++) {
+                const npc_row &r = rows[k][i];
+                const npc_locus &rec = loci[k][i];
+                if (rec.klass != 0 || !rec.used || r.kind != NPC_KIND_GT || r.gt_row < 0) continue;
+                int32_t *slot = &by_row[(size_t)r.gt_row];
+                if (pl) {
+                    std::string key((const char *)&r.gt_row, 4);
+                    key.append((const char *)&r.eaidx, 4).append((const char *)&r.eaf, 8);
+                    slot = &by_key.emplace(key, -1).first->second;
+                }
+                if (*slot < 0) {
+                    *slot = (int32_t)ent.size();
+                    ent.push_back(r);
+                    wt.push_back({});
+                }
+                wt[(size_t)*slot][g]++;
+            }
+        }
+        const int64_t E = (int64_t)ent.size();
+        std::vector<uint32_t> w((size_t)(OBS_G * E));
+        for (int64_t e = 0; e < E; e++) for (int g = 0; g < OBS_G; g++) w[(size_t)(g * E + e)] = wt[(size_t)e][g];
+        const size_t o_out = 0, o_ent = OBS_G * n1 * sizeof(ull), o_w = o_ent + ((E * sizeof(npc_row) + 255) & ~(size_t)255);
+        const size_t need = o_w + std::max<size_t>(w.size() * sizeof(uint32_t), 16);
+        if (need > c->obs_scratch_bytes) {
+            NPC_CUDA(c, cudaStreamSynchronize(c->stream));
+            cudaFree(c->d_obs_scratch); c->d_obs_scratch = nullptr; c->obs_scratch_bytes = 0;
+            NPC_CUDA(c, cudaMalloc(&c->d_obs_scratch, need));
+            c->obs_scratch_bytes = need;
+        }
+        ull *d_out = (ull *)(c->d_obs_scratch + o_out);
+        npc_row *d_ent = (npc_row *)(c->d_obs_scratch + o_ent);
+        uint32_t *d_w = (uint32_t *)(c->d_obs_scratch + o_w);
+        NPC_CUDA(c, cudaMemsetAsync(d_out, 0, OBS_G * n1 * sizeof(ull), c->stream));
+        if (E) {
+            NPC_CUDA(c, cudaMemcpyAsync(d_ent, ent.data(), E * sizeof(npc_row), cudaMemcpyHostToDevice, c->stream));
+            NPC_CUDA(c, cudaMemcpyAsync(d_w, w.data(), w.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+            if (int rc = launch_observed(c, c->d_slab, c->slab_stride, d_ent, nullptr, d_w, E, d_out)) return rc;
+        }
+        for (size_t g = 0; g < ng; g++)
+            if (c->n) NPC_CUDA(c, cudaMemcpyAsync(observed_out[defs[k0 + g]], d_out + g * n1, c->n * sizeof(ull), cudaMemcpyDeviceToHost, c->stream));
+        NPC_CUDA(c, cudaStreamSynchronize(c->stream));                      // the host tables above go out of scope
+    }
+    NPC_CUDA(c, cudaEventRecord(c->ev_slab, c->stream));
+    return NPC_OK;
+}
+
+// The context's own observed counts after a multi call: zero whichever path scored (the one-by-one path resets the
+// context per definition, the contraction does not touch it)
+static int zero_observed(npc_ctx *c) {
+    if (c->d_obs) NPC_CUDA(c, cudaMemsetAsync(c->d_obs, 0, std::max<int64_t>(c->n, 1) * sizeof(ull), c->stream));
+    return NPC_OK;
+}
+
+extern "C" int npc_score_resident_multi_observed(npc_ctx *ctx, int32_t n_scores, const npc_row *const *rows, const int64_t *n_rows,
+                                                 const double *offsets, double *const *scores_out, int64_t *nloci_out,
+                                                 npc_locus *const *loci_out, int64_t *const *observed_out) {
+    if (!ctx || n_scores < 0 || (n_scores && (!rows || !n_rows || !scores_out))) return NPC_EINVAL;
+    for (int32_t k = 0; k < n_scores; k++) if (n_rows[k] < 0 || (n_rows[k] && !rows[k]) || !scores_out[k]) return NPC_EINVAL;
+    NPC_CUDA(ctx, cudaSetDevice(ctx->device));
+    bool want = false;
+    for (int32_t k = 0; observed_out && k < n_scores; k++) want = want || observed_out[k];
+    // the counts come from one pass per group below, whichever path scored: the per-launch pass stays off meanwhile
+    const bool hook = ctx->observed;
+    ctx->observed = false;
+    if (!want) {
+        const int rc = score_multi(ctx, n_scores, rows, n_rows, offsets, scores_out, nloci_out, loci_out);
+        ctx->observed = hook;
+        return rc ? rc : zero_observed(ctx);
+    }
+    if (!ctx->ev_slab) NPC_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_slab, cudaEventDisableTiming));
+    std::vector<std::vector<npc_locus>> own((size_t)n_scores);                // records of definitions the caller does not take
+    std::vector<npc_locus *> loci((size_t)n_scores);
+    for (int32_t k = 0; k < n_scores; k++) {
+        if (loci_out && loci_out[k]) loci[k] = loci_out[k];
+        else { own[k].resize((size_t)n_rows[k]); loci[k] = own[k].data(); }
+    }
+    int rc = score_multi(ctx, n_scores, rows, n_rows, offsets, scores_out, nloci_out, loci.data());
+    ctx->observed = hook;
+    if (!rc) rc = multi_observed(ctx, n_scores, rows, n_rows, loci.data(), observed_out);
+    return rc ? rc : zero_observed(ctx);
+}
+
+extern "C" int npc_score_resident_multi(npc_ctx *ctx, int32_t n_scores, const npc_row *const *rows, const int64_t *n_rows,
+                                        const double *offsets, double *const *scores_out, int64_t *nloci_out,
+                                        npc_locus *const *loci_out) {
+    return npc_score_resident_multi_observed(ctx, n_scores, rows, n_rows, offsets, scores_out, nloci_out, loci_out, nullptr);
+}
+
+extern "C" int npc_set_observed(npc_ctx *ctx, int32_t on) {
+    if (!ctx) return NPC_EINVAL;
+    if (on && !ctx->d_obs) {
+        NPC_CUDA(ctx, cudaSetDevice(ctx->device));
+        const size_t bytes = (size_t)std::max<int64_t>(ctx->n, 1) * sizeof(ull);
+        NPC_CUDA(ctx, cudaMalloc(&ctx->d_obs, bytes));
+        NPC_CUDA(ctx, cudaMemsetAsync(ctx->d_obs, 0, bytes, ctx->stream));
+    }
+    ctx->observed = on != 0;
+    return NPC_OK;
+}
+
+extern "C" int npc_observed(npc_ctx *ctx, int64_t *out) {
+    if (!ctx || !out) return NPC_EINVAL;
+    if (!ctx->d_obs) return fail(ctx, NPC_ESTATE, "npc_observed: npc_set_observed was never turned on for this context");
+    NPC_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (ctx->n) NPC_CUDA(ctx, cudaMemcpyAsync(out, ctx->d_obs, ctx->n * sizeof(ull), cudaMemcpyDeviceToHost, ctx->stream));
+    NPC_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return NPC_OK;
 }
 
 extern "C" int npc_partial(npc_ctx *ctx, double *sums_out, int64_t *nloci_out, npc_locus *loci_out, int64_t loci_cap,

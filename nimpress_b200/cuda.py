@@ -81,6 +81,9 @@ def load_library():
         "npc_score_resident": (C.c_int, [vp, vp, i64]),
         "npc_multi_contractions": (C.c_int64, [vp]),
         "npc_score_resident_multi": (C.c_int, [vp, i32, vp, vp, vp, vp, vp, vp]),
+        "npc_score_resident_multi_observed": (C.c_int, [vp, i32, vp, vp, vp, vp, vp, vp, vp]),
+        "npc_set_observed": (C.c_int, [vp, i32]),
+        "npc_observed": (C.c_int, [vp, vp]),
         "npc_finish": (C.c_int, [vp, f64, vp, pi64, vp, i64, pi64]),
         "npc_partial": (C.c_int, [vp, vp, pi64, vp, i64, pi64]),
         "npc_partial_device_ptr": (C.c_int, [vp, C.POINTER(vp), C.POINTER(vp)]),
@@ -259,9 +262,11 @@ class Engine:
         rows = np.ascontiguousarray(rows, dtype=ROW_DTYPE)
         self._ck(self.L.npc_score_resident(self.h, rows.ctypes.data, len(rows)))
 
-    def score_resident_multi(self, rows_list, offsets, scores=None, loci=None):
+    def score_resident_multi(self, rows_list, offsets, scores=None, loci=None, observed=False):
         """npc_score_resident_multi -> [(scores, nloci, loci)] per score definition.  scores / loci:
-        optional preallocated output arrays (e.g. views of pinned memory), one per definition."""
+        optional preallocated output arrays (e.g. views of pinned memory), one per definition.
+        observed=True: npc_score_resident_multi_observed, [(scores, nloci, loci, observed)] with each definition's
+        per-sample observed counts (int64; DESIGN.md 4.13)."""
         S = len(rows_list)
         rows_list = [np.ascontiguousarray(r, dtype=ROW_DTYPE) for r in rows_list]
         rp = (C.c_void_p * S)(*[r.ctypes.data for r in rows_list])
@@ -272,8 +277,24 @@ class Engine:
         sp = (C.c_void_p * S)(*[a.ctypes.data for a in scores])
         lp = (C.c_void_p * S)(*[a.ctypes.data for a in loci])
         nloci = np.zeros(S, dtype=np.int64)
+        if observed:
+            obs = [np.zeros(self.n, dtype=np.int64) for _ in range(S)]
+            op = (C.c_void_p * S)(*[a.ctypes.data for a in obs])
+            self._ck(self.L.npc_score_resident_multi_observed(self.h, S, rp, nr.ctypes.data, off.ctypes.data if off is not None else None,
+                                                              sp, nloci.ctypes.data, lp, op))
+            return [(scores[k], int(nloci[k]), loci[k], obs[k]) for k in range(S)]
         self._ck(self.L.npc_score_resident_multi(self.h, S, rp, nr.ctypes.data, off.ctypes.data if off is not None else None, sp, nloci.ctypes.data, lp))
         return [(scores[k], int(nloci[k]), loci[k]) for k in range(S)]
+
+    def set_observed(self, on=True):
+        """npc_set_observed: every later scoring launch adds its per-sample observed counts (DESIGN.md 4.13)."""
+        self._ck(self.L.npc_set_observed(self.h, int(bool(on))))
+
+    def observed(self):
+        """npc_observed: the context's per-sample counts of OK score rows with a called genotype (int64)."""
+        out = np.zeros(self.n, dtype=np.int64)
+        self._ck(self.L.npc_observed(self.h, out.ctypes.data))
+        return out
 
     @property
     def multi_contractions(self):

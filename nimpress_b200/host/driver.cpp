@@ -428,6 +428,7 @@ struct Device {
         ctx.ck(npc_set_policy(ctx.h, &pol), "npc_set_policy");
         if (P.lay.ds) ctx.ck(npc_set_dosage_rows(ctx.h, 1), "npc_set_dosage_rows");
         if (P.p.exact_order) ctx.ck(npc_set_exact_order(ctx.h, 1), "npc_set_exact_order");
+        if (P.p.observed) ctx.ck(npc_set_observed(ctx.h, 1), "npc_set_observed");      // rounds add up in the context
         ctx.ck(npc_reset(ctx.h), "npc_reset");
         int64_t slab_want = want;
         if (const char *e = getenv("NIMPRESS_SLAB_ROWS")) if (*e) slab_want = std::max<int64_t>(1, std::min<int64_t>(slab_want, atoll(e)));   // tests: force rounds
@@ -577,6 +578,15 @@ void score_single(ScoreState &s, std::vector<Device> &devs, int64_t n, ScoreResu
         if (nlog != (int64_t)v.submitted.size()) throw std::runtime_error("locus log length mismatch");
         for (size_t j = 0; j < log.size(); j++) out.loci[v.submitted[j]] = log[j];
     }
+    if (!devs[0].pass->p.observed) return;
+    // integer counts: the devices' vectors add up in any order
+    out.has_observed = true;
+    out.observed.assign((size_t)n, 0);
+    std::vector<int64_t> obs((size_t)n);
+    for (Device &v : devs) {
+        v.ctx.ck(npc_observed(v.ctx.h, obs.data()), "npc_observed");
+        for (int64_t i = 0; i < n; i++) out.observed[(size_t)i] += obs[(size_t)i];
+    }
 }
 
 // Several score files: device d scores range d of every file in one npc_score_resident_multi call.  One device gives the
@@ -584,8 +594,14 @@ void score_single(ScoreState &s, std::vector<Device> &devs, int64_t n, ScoreResu
 // them in device order (= score-file order of the ranges), normalised once.
 void score_multi(std::vector<ScoreState> &ps, std::vector<Device> &devs, int64_t n, std::vector<ScoreResult> &outs) {
     const int S = (int)ps.size(), D = (int)devs.size();
+    const bool observed = devs[0].pass->p.observed;
     std::vector<std::vector<double>> part(S);
-    for (int k = 0; k < S; k++) { outs[k].scores.assign(n, 0.0); outs[k].rounds = 1; outs[k].devices = D; if (D > 1) part[k].assign((size_t)n, 0.0); }
+    std::vector<std::vector<int64_t>> obs(S);
+    for (int k = 0; k < S; k++) {
+        outs[k].scores.assign(n, 0.0); outs[k].rounds = 1; outs[k].devices = D;
+        if (D > 1) part[k].assign((size_t)n, 0.0);
+        if (observed) { outs[k].has_observed = true; outs[k].observed.assign((size_t)n, 0); obs[k].assign((size_t)n, 0); }
+    }
     for (Device &v : devs) {
         v.flush();
         std::vector<std::vector<npc_row>> rows(S);
@@ -596,17 +612,21 @@ void score_multi(std::vector<ScoreState> &ps, std::vector<Device> &devs, int64_t
         std::vector<double> offsets(S);
         std::vector<double *> sc(S);
         std::vector<npc_locus *> log_ptr(S);
+        std::vector<int64_t *> obs_ptr(S);
         for (int k = 0; k < S; k++) {
+            obs_ptr[k] = observed ? obs[k].data() : nullptr;
             collect_rows(ps[k], v.d, true, rows[k], entries[k]);
             row_ptr[k] = rows[k].data(); n_rows[k] = (int64_t)rows[k].size(); offsets[k] = ps[k].score.offset;
             sc[k] = v.d == 0 ? outs[k].scores.data() : part[k].data();
             log[k].resize(rows[k].size()); log_ptr[k] = log[k].data();
         }
         // one device: normalised scores; several: raw partial sums (offsets = NULL)
-        v.ctx.ck(npc_score_resident_multi(v.ctx.h, S, row_ptr.data(), n_rows.data(), D == 1 ? offsets.data() : nullptr, sc.data(),
-                                          nloci.data(), log_ptr.data()), "npc_score_resident_multi");
+        v.ctx.ck(npc_score_resident_multi_observed(v.ctx.h, S, row_ptr.data(), n_rows.data(), D == 1 ? offsets.data() : nullptr, sc.data(),
+                                                   nloci.data(), log_ptr.data(), observed ? obs_ptr.data() : nullptr),
+                 "npc_score_resident_multi");
         for (int k = 0; k < S; k++) {
             outs[k].nloci += nloci[k];
+            if (observed) for (int64_t i = 0; i < n; i++) outs[k].observed[(size_t)i] += obs[k][(size_t)i];
             for (size_t j = 0; j < log[k].size(); j++) outs[k].loci[entries[k][j]] = log[k][j];
             if (v.d > 0) for (int64_t i = 0; i < n; i++) outs[k].scores[i] += part[k][i];
         }

@@ -32,11 +32,14 @@ struct ScoreParams {
     bool use_pl = false;                   // score FORMAT/PL as posterior expected dosages (NPC_GT_PL rows) -- not a reference option
     std::string samples_path;              // --samples: a list of sample names (empty: every sample) -- not a reference option
     bool exclude_samples = false;          // --samples=^FILE: score every sample the list does not name
+    bool observed = false;                 // --observed: per-sample counts of OK loci with a called genotype -- not a reference option
 };
 
 struct ScoreResult {
     std::vector<std::string> samples;
     std::vector<double> scores;            // per sample, after /(2*nloci) and +offset
+    bool has_observed = false;             // ScoreParams::observed was set
+    std::vector<int64_t> observed;         // per sample: OK score rows at which it has a called genotype (DESIGN.md 4.13)
     std::vector<npc_locus> loci;           // per score row, score-file order
     int64_t nloci = 0;
     std::string warnings;                  // the "WARN ..." lines the reference logs, in its order

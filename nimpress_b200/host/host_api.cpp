@@ -28,6 +28,7 @@ static ScoreParams to_params(const nph_params *p) {
     q.use_pl = p->use_pl != 0;
     if (p->samples_path) q.samples_path = p->samples_path;
     q.exclude_samples = p->exclude_samples != 0;
+    q.observed = p->observed != 0;
     return q;
 }
 
@@ -116,6 +117,11 @@ int64_t nph_result_devices(const nph_result *r) { return r->r.devices; }
 int64_t nph_result_records_read(const nph_result *r) { return r->r.records_read; }
 int64_t nph_result_index_seeks(const nph_result *r) { return r->r.index_seeks; }
 const double *nph_result_scores(const nph_result *r) { return r->r.scores.data(); }
+const int64_t *nph_result_observed(const nph_result *r) {
+    static const int64_t none = 0;                          // option on, no samples: still not NULL
+    if (!r->r.has_observed) return nullptr;
+    return r->r.observed.empty() ? &none : r->r.observed.data();
+}
 const npc_locus *nph_result_loci(const nph_result *r) { return r->r.loci.data(); }
 const char *nph_result_sample(const nph_result *r, int64_t i) { return r->r.samples[(size_t)i].c_str(); }
 const char *nph_result_warnings(const nph_result *r) { return r->r.warnings.c_str(); }
@@ -311,6 +317,10 @@ static const char *USAGE =
     "                     --maxmis and WARN lines included (not a reference option).\n"
     "  --samples=^<file>  Score every sample except those named in <file>; names the genotype file\n"
     "                     lacks are ignored (not a reference option).\n"
+    "  --observed         Print a third column: per sample, the number of loci in the score whose\n"
+    "                     genotype was read from that sample's own call (locus scored, call not\n"
+    "                     missing); nloci minus it were imputed for the sample.  Loci, not alleles\n"
+    "                     (PLINK's ALLELE_CT is twice this for diploid calls) (not a reference option).\n"
     "Several genotype files (not a reference input): VCF/BCF files (text and BCF may be mixed), PLINK 1 filesets\n"
     "  or BGEN files, one kind per run, read in the order given; a site in two files is matched in the earlier one.\n"
     "  Every file must carry the same samples in the same order, or, with --samples, keep the same samples in the\n"
@@ -340,7 +350,8 @@ static uint32_t parse_device_list(const std::string &v) {
     return mask;
 }
 
-// WARN lines, then one `name<TAB>$score` line per sample (:752-753), formatted into one buffer
+// WARN lines, then one `name<TAB>$score` line per sample (:752-753), formatted into one buffer; with --observed a third
+// column, the sample's observed count
 static void print_result(const nph_result *r) {
     std::string out = r->r.warnings;
     const std::vector<double> &s = r->r.scores;
@@ -352,13 +363,14 @@ static void print_result(const nph_result *r) {
         out += r->r.samples[i];
         out += '\t';
         out.append(buf, (size_t)format_float_nim_to(s[i], buf));
+        if (r->r.has_observed) { out += '\t'; out += std::to_string(r->r.observed[i]); }
         out += '\n';
     }
     std::cout.write(out.data(), (std::streamsize)out.size());
 }
 
 int nph_main(int argc, char **argv) {
-    nph_params p = { NPC_LOCUS_PS, NPC_MISSING_HOMREF, NPC_SAMPLE_INT_PS, 0, 0, 0, 0, 0, 100, 0.05, 0.001, 0, 0, nullptr, 0 };
+    nph_params p = { NPC_LOCUS_PS, NPC_MISSING_HOMREF, NPC_SAMPLE_INT_PS, 0, 0, 0, 0, 0, 100, 0.05, 0.001, 0, 0, nullptr, 0, 0 };
     std::string cov, samples_list;
     std::vector<std::string> pos;                          // <scoredef>, then the genotype files
     try {
@@ -392,6 +404,7 @@ int nph_main(int argc, char **argv) {
             else if (a == "--exact-order") p.exact_order = 1;
             else if (a == "--dosage") p.use_ds = 1;
             else if (a == "--pl") p.use_pl = 1;
+            else if (a == "--observed") p.observed = 1;
             else if (a.size() > 1 && a[0] == '-') throw InputError("unknown option " + a);
             else pos.push_back(a);
         }

@@ -68,6 +68,11 @@ proc npc_score_resident*(ctx: NpcCtx; rows: ptr NpcRow; nRows: int64): cint
 proc npc_score_resident_multi*(ctx: NpcCtx; nScores: int32; rows: ptr ptr NpcRow; nRows: ptr int64;
                                offsets: ptr float64; scoresOut: ptr ptr float64; nlociOut: ptr int64;
                                lociOut: ptr ptr NpcLocus): cint
+proc npc_score_resident_multi_observed*(ctx: NpcCtx; nScores: int32; rows: ptr ptr NpcRow; nRows: ptr int64;
+                                        offsets: ptr float64; scoresOut: ptr ptr float64; nlociOut: ptr int64;
+                                        lociOut: ptr ptr NpcLocus; observedOut: ptr ptr int64): cint
+proc npc_set_observed*(ctx: NpcCtx; on: int32): cint   ## per-sample counts of OK loci with a called genotype (DESIGN.md 4.13)
+proc npc_observed*(ctx: NpcCtx; observedOut: ptr int64): cint
 proc npc_finish*(ctx: NpcCtx; offset: float64; scoresOut: ptr float64; nlociOut: ptr int64;
                  lociOut: ptr NpcLocus; lociCap: int64; nLociOut: ptr int64): cint
 proc npc_partial*(ctx: NpcCtx; sumsOut: ptr float64; nlociOut: ptr int64; lociOut: ptr NpcLocus;
